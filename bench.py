@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (default: every config below)
     python bench.py --impl reference --gpus N --steps K ...  # CPU reference arm (rank 0 only)
     python bench.py --config 2|3|4 ...                       # one config only
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as .npy
 
 Headline (BASELINE configs[2]): audio-seconds generated per second at B = 64 x 510 tokens per GPU.  A "step" is one
 pass of the whole forward over one batch of 64 synthetic utterances (kokorox_b200.synth.synth_batch: 510 ids ~
@@ -25,11 +26,14 @@ asks (NCCL, one rank per GPU) and is used only for the barrier around the timed 
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -37,15 +41,50 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree as it found it (it may be read-only)
 
-from kokorox_b200.synth import (ensure_second_weights, ensure_weights, synth_batch, synth_case,  # noqa: E402
-                                synth_requests_cfg4, synth_voice_table)
+from kokorox_b200.synth import (ensure_weights, synth_batch, synth_case, synth_requests_cfg4,  # noqa: E402
+                                synth_voice_table)
 
 # SURVEY.md 8d work model: MACs per token (attention term scaled by N/512) and per frame
 MAC_TOKEN_FIXED = 88.86e6 - 9.44e6
 MAC_TOKEN_ATTN = 9.44e6
 MAC_FRAME = 658.55e6
 REF_SUBSET = (0, 1)      # utterances of the batch the reference arm runs every step (fixed, stated)
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this many bytes in all
+DUMP_SEED = 0            # fixed sample of a waveform too large to dump whole
+
+_checkpoint_dir = None
+
+
+def checkpoint(seed: int = 1234) -> str:
+    """The random-init checkpoint of `seed` (kokorox_b200.synth), generated on first use.  None ships with the project
+    and the tree may be read-only, so it goes to a temporary directory of this process, removed at exit.  A file named
+    by $KKX_WEIGHTS stands in for the seed-1234 one."""
+    global _checkpoint_dir
+    if seed == 1234 and "KKX_WEIGHTS" in os.environ:
+        return ensure_weights()
+    if _checkpoint_dir is None:
+        _checkpoint_dir = tempfile.mkdtemp(prefix="kkx_bench_")
+        atexit.register(shutil.rmtree, _checkpoint_dir, True)
+    return ensure_weights(os.path.join(_checkpoint_dir, f"kokoro_random_{seed}.kkxw"), seed=seed)
+
+
+def dump_arrays(audio: np.ndarray, sample_offsets: np.ndarray, durations: np.ndarray) -> dict:
+    """What --dump-outputs writes for one staged step: the flat waveform of the batch, where each utterance starts in
+    it, and the integer frame durations of every token.  A waveform too large for what DUMP_BYTES leaves after the
+    other arrays is replaced by a seeded, sorted sample of its positions (`audio_index`), the same for the same
+    length, so that two builds can be compared array for array."""
+    out = {"sample_offsets": sample_offsets.astype(np.float64), "durations": durations.astype(np.float64)}
+    room = DUMP_BYTES - 4096 - sum(a.nbytes for a in out.values())     # 4 KB for the .npy headers
+    audio = np.asarray(audio, dtype=np.float32)
+    if audio.nbytes > room:
+        n = room // (4 + 8)                               # f32 sample + f64 index per kept position
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(audio.size, n, replace=False))
+        out["audio_index"] = idx.astype(np.float64)
+        audio = audio[idx]
+    out["audio"] = audio
+    return out
 
 
 def load_peaks():
@@ -109,7 +148,7 @@ def make_cpu_reference(threads: int):
         return (lambda t, s: ref.infer(t, s, 1.0)), "ort", f"ONNX Runtime CPU EP on {os.path.basename(why)}"
     from kokorox_b200.weightfile import read_weights
     from oracle.kokoro_ref import KokoroOracle
-    o = KokoroOracle(read_weights(ensure_weights()), threads=threads)
+    o = KokoroOracle(read_weights(checkpoint()), threads=threads)
     k = [0]
 
     def run(t, s):
@@ -206,7 +245,7 @@ def run_cfg3(local_rank: int, conc="1,4,16,64", requests=8, tokens=128):
         return {"error": "kkx_loadgen not built"}
     sampler = ClockSampler(local_rank).start()
     t0 = time.perf_counter()
-    r = subprocess.run([exe, ensure_weights(), "--device", str(local_rank), "--tokens", str(tokens), "--requests",
+    r = subprocess.run([exe, checkpoint(), "--device", str(local_rank), "--tokens", str(tokens), "--requests",
                         str(requests), "--conc", conc, "--modes", "serial,coalesce,async"],
                        capture_output=True, text=True, timeout=900)
     wall = time.perf_counter() - t0
@@ -233,7 +272,7 @@ def run_cfg4(rank, local_rank, world, barrier, passes=1, n_req=4096):
     table = synth_voice_table(54)
     vt = {f"v{v:02d}": table[v] for v in range(54)}
     sessions = {}
-    for lang, wp in (("en", ensure_weights()), ("zh", ensure_second_weights())):
+    for lang, wp in (("en", checkpoint()), ("zh", checkpoint(4321))):
         m = B200Koko.new(wp, device=local_rank)
         m.load_voices(vt)
         sessions[lang] = m
@@ -323,7 +362,12 @@ def main():
                     help="1 = tensor-core configuration (the library default), 0 = fp32 SIMT everywhere")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-out", default=None, help="write the per-kernel timing table of one step here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step of the headline path computed to DIR/<name>.npy "
+                         "(waveform, utterance offsets, token durations; at most 64 MB, a seeded sample of the waveform)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config in ("3", "4")):
+        ap.error("--dump-outputs writes the headline path's results: it needs --impl ours and --config all or 2")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -353,12 +397,10 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    # the synthetic checkpoints are written once (rank 0), not raced for by every rank
-    if rank == 0:
-        ensure_weights()
-        if args.config in ("all", "4"):
-            ensure_second_weights()
-    barrier()
+    # every process generates the synthetic checkpoints it reads, in its own temporary directory, before any timing
+    checkpoint()
+    if args.config in ("all", "4"):
+        checkpoint(4321)
 
     if args.config == "3":
         if rank == 0:
@@ -385,7 +427,7 @@ def main():
             dist.destroy_process_group()
         return
 
-    m = B200Koko.new(ensure_weights(), device=local_rank)
+    m = B200Koko.new(checkpoint(), device=local_rank)
     default_precision = m.get_stat("precision")          # what an unconfigured session runs (ADVICE r1: stated)
     m.set_option("precision", args.precision)
     # weak scaling: every rank runs the SAME 64 utterances (per-GPU work fixed; rank-dependent seeds made the ranks'
@@ -415,6 +457,10 @@ def main():
     frames = m.get_stat("last_frames")
     groups = m.get_stat("frame_groups")
     audio_s_step = totals[-1] / 24000.0
+    if args.dump_outputs and rank == 0:          # every rank runs the same batch
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump_arrays(*m.fetch_staged(totals[-1])).items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     # one profiled step (not part of the timed region) for the roofline of the dominant kernel
     m.profile_enable(True)

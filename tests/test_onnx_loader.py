@@ -10,8 +10,6 @@ node names carrying the torch scope path.  CPU tests convert through the host-on
 compare the recovered state dict bit for bit; the GPU test loads the .onnx through kkx_create and requires audio
 bit-identical to the KKXW load.
 """
-import os
-
 import numpy as np
 import pytest
 
@@ -266,7 +264,7 @@ def test_q4_matmulnbits_export(built, ref, tmp_path):
     check(built, tmp_path, blob, expect, "q4")
 
 
-def test_bias_fallback_and_unresolved_report(built, ref, tmp_path):
+def test_bias_fallback_and_unresolved_report(built, ref, tmp_path, weights_path):
     # exporters that do not name nodes by scope ("MatMul_12"): modules are recovered from the bias a Conv consumes or
     # the Add behind a MatMul adds; bias-less convs (conv1x1) and LSTMs cannot be, and the error must list them
     blob, _ = build_export(ref, "fp32", no_node_names=True)
@@ -284,15 +282,14 @@ def test_bias_fallback_and_unresolved_report(built, ref, tmp_path):
     with pytest.raises(built.KkxError):
         built.convert_model_file(str(junk), str(tmp_path / "junk.kkxw"))
     # a corrupt KKXW header (offset wraps) is an error, not a crash (ADVICE r1)
-    good = open(os.path.join(os.path.dirname(__file__), "..", "weights", "kokoro_random_1234.kkxw"), "rb").read(4096) \
-        if os.path.exists(os.path.join(os.path.dirname(__file__), "..", "weights", "kokoro_random_1234.kkxw")) else None
-    if good:
-        bad = bytearray(good)
-        p = 16 + 2 + int.from_bytes(good[16:18], "little") + 8 + 4 * int.from_bytes(good[16 + 2 + int.from_bytes(good[16:18], "little") + 4:][:4], "little")
-        bad[p:p + 8] = (2 ** 64 - 64).to_bytes(8, "little")
-        (tmp_path / "bad.kkxw").write_bytes(bytes(bad))
-        with pytest.raises(built.KkxError):
-            built.convert_model_file(str(tmp_path / "bad.kkxw"), str(tmp_path / "bad2.kkxw"))
+    with open(weights_path, "rb") as f:
+        good = f.read(4096)
+    bad = bytearray(good)
+    p = 16 + 2 + int.from_bytes(good[16:18], "little") + 8 + 4 * int.from_bytes(good[16 + 2 + int.from_bytes(good[16:18], "little") + 4:][:4], "little")
+    bad[p:p + 8] = (2 ** 64 - 64).to_bytes(8, "little")
+    (tmp_path / "bad.kkxw").write_bytes(bytes(bad))
+    with pytest.raises(built.KkxError):
+        built.convert_model_file(str(tmp_path / "bad.kkxw"), str(tmp_path / "bad2.kkxw"))
 
 
 @pytest.mark.gpu

@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from tests.conftest import REF_EXAMPLE_IDS, REF_TOKENIZE_IDS, make_noise, synth_case
+from tests.test_parity_gpu import avg_spectrum_db_diff
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -72,9 +73,17 @@ def test_oracle_reproduces_golden(oracle, name):
     assert r["audio"].shape == g["audio"].shape == (600 * int(g["pred_dur"].sum()),)
     np.testing.assert_allclose(r["stages"]["dur_float"], g["stage.dur_float"], rtol=0, atol=2e-5)
     np.testing.assert_allclose(r["stages"]["F0"], g["stage.F0"], rtol=0, atol=2e-3)
-    # same torch build, same kernels -> near bit-identical; allow libm / thread-count jitter
-    err = np.abs(r["audio"] - g["audio"]).max()
-    assert err < 2e-3, err
+    np.testing.assert_allclose(r["stages"]["N"], g["stage.N"], rtol=0, atol=1e-4)
+    # torch's CPU reductions follow the thread count: with 16 threads instead of the 8 the vectors were made with, F0
+    # moves by 5e-4 and N by 1e-5, and since the harmonic source integrates F0 into a phase of 1e4..1e5 rad the
+    # free-running waveform moves by up to 0.08 (test_parity_gpu.py).  So it is compared phase-insensitively (measured
+    # 0.07 dB), and the waveform is held sample for sample with the pinned F0 / N curves teacher-forced (2e-7).
+    assert avg_spectrum_db_diff(g["audio"], r["audio"]) < 0.5
+    t = oracle.forward(g["tokens"], g["style"], float(g["speed"]), noise=noise, stages=True,
+                       inject={"pred_dur": g["pred_dur"], "F0": g["stage.F0"], "N": g["stage.N"]})
+    np.testing.assert_allclose(t["stages"]["har_source"], g["stage.har_source"], rtol=0, atol=1e-5)
+    err = np.abs(t["audio"] - g["audio"]).max()
+    assert err < 1e-4, err
 
 
 def test_oracle_structure_properties(oracle):
