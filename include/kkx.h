@@ -78,8 +78,9 @@ KKX_API const char* kkx_last_error(const kkx_ctx* ctx);
  *              2 <= n_tokens <= 512, ids in 0..177 (tts/vocab.rs:5-20)   -- "input_ids"
  *   style256   [256] f32 (koko.rs:1255-1306 mix_styles row)             -- "style"
  *   speed      in [0.1, 10] (durations are 50/speed frames per token at most) -- "speed"
- *   out_audio  receives a library-owned pinned host buffer of *out_samples f32 (24 kHz mono,
- *              = 600 * sum(pred_dur)); valid until kkx_release(ctx, ptr) -- outputs[0]
+ *   out_audio  receives a library-owned pinned host buffer of *out_samples f32 mono at the session's "out_rate"
+ *              (default 24 kHz: 600 * sum(pred_dur) samples; at rate r: ceil(600 * sum(pred_dur) * U / D), see
+ *              "out_rate"); valid until kkx_release(ctx, ptr) -- outputs[0]
  *   out_pred_dur  nullable; [n_tokens] predicted integer frame durations (not observable
  *              through the reference graph; exposed for parity tests).
  * Thread-safe.  By default concurrent callers run one after another, like the reference's
@@ -139,12 +140,26 @@ KKX_API int kkx_infer_batch_voices(kkx_ctx* ctx, int32_t batch, const int64_t* t
 
 /* kkx_infer_batch_pcm16: like kkx_infer_batch, but the waveform comes back as 16-bit PCM,
  *   pcm = trunc(clamp(s, -1, 1) * 32767) -- the f32 -> i16 conversion of the reference's WebSocket server
- *   (kokorox-websocket/src/lib.rs:699-703) fused into the iSTFT kernel; half the device->host bytes.
+ *   (kokorox-websocket/src/lib.rs:699-703) fused into the iSTFT kernel; half the device->host bytes.  At an
+ *   "out_rate" other than 24000 the same conversion is applied to the resampled value, inside the resampling kernel.
  *   Release the buffer with kkx_release_pcm16. */
 KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                           const float* styles, const float* speeds, int16_t** out_pcm,
                           int64_t* out_sample_offsets, int32_t* out_pred_dur);
 KKX_API void kkx_release_pcm16(kkx_ctx* ctx, int16_t* pcm);
+
+/* kkx_infer_batch_g711: like kkx_infer_batch_pcm16, but every sample comes back as one ITU-T G.711 byte, for
+ *   telephony (SIP / PSTN, PCMU / PCMA media streams): law 0 = mu-law (PCMU), 1 = A-law (PCMA); any other value is
+ *   KKX_ERR_ARG.  The code of a sample is the G.711 encoding of the same 16-bit value p that kkx_infer_batch_pcm16
+ *   returns -- mu-law of the 14-bit p >> 2 (bias 33, clip 8159), A-law of the 13-bit p >> 3 -- i.e. the Sun reference
+ *   g711.c, equal to Python's audioop.lin2ulaw / lin2alaw(..., 2).  Works at every "out_rate" (8000 is the G.711 rate;
+ *   at 24000 the codes are those of the model's own waveform).  Offsets count codes (= samples).  One pass (no
+ *   "max_tokens" split); release the buffer with kkx_release_g711.  No WAV container: telephony transports carry
+ *   raw codes. */
+KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                                 const float* styles, const float* speeds, int32_t law /* 0 = mu-law, 1 = A-law */,
+                                 uint8_t** out_codes, int64_t* out_sample_offsets, int32_t* out_pred_dur);
+KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes);
 
 /* ---- output containers (host-side byte work after the pcm16 / f32 result; no GPU involved, no ctx needed).
  * kkx_wav_header_pcm16: the 44-byte RIFF/WAVE header of the WebSocket server's `encode_audio`
@@ -162,7 +177,7 @@ KKX_API int64_t kkx_encode_wav16_base64(const int16_t* pcm, int64_t n_samples, i
 /* ---- device-resident variant (bench.py `value`: inputs already in HBM, output stays in HBM).
  * Stages the batch on the device once; kkx_run_staged() then runs the whole forward with no
  * host<->device payload traffic (only the per-item frame counts cross, 4 bytes per item).
- * Returns total samples in *out_total_samples and kernel launches in *out_launches
+ * Returns total samples (at "out_rate") in *out_total_samples and kernel launches in *out_launches
  * (either may be NULL). */
 KKX_API int kkx_stage_batch(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                     const float* styles, const float* speeds);
@@ -199,10 +214,24 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *   tensor-core configuration; fp32-grade, not the same bits as libm) and "fuse_noise_stats" (the generator's 22 -> 128
  *   noise conv in fp32 together with the statistics of its output instead of bf16 operands on the tensor cores);
  *   "stream_bf16" (default 0) keeps the res-block residual stream in bf16.
+ *   "out_rate"    sample rate of every waveform the session returns (default 24000, the model's rate; nothing is
+ *                 resampled then).  Accepted: r in 8000..48000 with U = r/g, D = 24000/g (g = gcd(r, 24000)) and
+ *                 max(U, D) <= 320 -- 8000, 11025, 12000, 16000, 22050, 24000, 32000, 44100, 48000; anything else is
+ *                 KKX_ERR_ARG naming the reduced ratio, and the session keeps its rate.  Applies to every waveform entry
+ *                 point (kkx_infer, _batch, _batch_voices, _batch_pcm16, _batch_g711, kkx_wait and coalesced / async
+ *                 batches, kkx_run_staged / kkx_fetch_staged) for runs that start after the call; every sample count
+ *                 and offset is then in output-rate samples.  One rate per session (sessions of one file share the
+ *                 device weights, so a server holds one session per rate).  Each utterance is resampled on its own,
+ *                 with zeros outside it, exactly as scipy.signal.resample_poly(x, U, D) with its defaults:
+ *                   H = 10 max(U, D),  h = U * firwin(2H + 1, 1 / max(U, D), window = ("kaiser", 5.0))
+ *                   y[m] = sum over k ascending, 0 <= k < n, 0 <= mD - kU + H <= 2H, of x[k] * h[mD - kU + H],
+ *                   0 <= m < ceil(n U / D)   (n = 600 T input samples)
+ *                 accumulated in fp32 (taps designed in double, stored as fp32), one output per thread on the GPU, so
+ *                 results stay bit-identical to the item's own B = 1 call.  16-bit PCM and G.711 are converted from y.
  * kkx_get_stat keys: "launches", "last_frames", "gpu_us", "precision", "coalesced_batches",
  * "coalesced_requests", "coalesced_largest", "async_batches", "async_requests", "frame_groups",
  * "group_first:<g>" (first item of frame group g of the last run), "weights_sessions" (sessions sharing this
- * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays". */
+ * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate". */
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value);
 KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "last_frames", "gpu_us" ... */
 

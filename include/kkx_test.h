@@ -115,6 +115,16 @@ KKX_API int kkx_test_arb_conv_stream(int device, const float* x, int B, const in
                                      const float* shift, const float* alpha, const float* w, const float* bias, int ks,
                                      int dil, const float* res, float oscale, int accumulate, int want_bf16, float* out,
                                      float* sums);
+/* Output resampling (kernels_signal.cu resample_kernel).
+ * kkx_test_resample_taps: host only -- the fp32 filter the library designs for out_rate (U * firwin(2H + 1,
+ *   1 / max(U, D), ("kaiser", 5.0)), H = 10 max(U, D)); copies at most `capacity` taps to dst (nullable) and returns
+ *   the tap count, or < 0 for a rate "out_rate" rejects; at 24000 the filter is the identity (one tap 1.0).
+ * kkx_test_resample: B items packed back to back in x (item b has lens[b] >= 1 samples, any length) -> out (packed, item
+ *   b has ceil(lens[b] U / D) samples); pcm (nullable) the 16-bit twin, codes (nullable) the G.711 twin of law 0 / 1
+ *   (law -1 = none).  At 24000 the kernel runs its pass-through mode (U = D = 1, no filter). */
+KKX_API int64_t kkx_test_resample_taps(int32_t out_rate, float* dst, int64_t capacity);
+KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64_t* lens, int32_t out_rate, int32_t law,
+                              float* out, int16_t* pcm, uint8_t* codes);
 KKX_API const char* kkx_test_last_error(void);
 
 #ifdef __cplusplus

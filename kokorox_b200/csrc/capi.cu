@@ -11,6 +11,7 @@
 #include <deque>
 #include <mutex>
 #include <map>
+#include <numeric>
 #include <set>
 #include <sstream>
 #include <atomic>
@@ -364,7 +365,7 @@ static void serve_coalesced(kkx_ctx* ctx, const std::vector<kkx_ctx::Waiter*>& b
     for (int i = 0; i < B; i++) {
       kkx_ctx::Waiter& w = *batch[i];
       w.audio = host + soff[i];
-      w.samples = soff[i + 1] - soff[i];   // >= 600: every token lasts at least one frame, so view addresses are distinct
+      w.samples = soff[i + 1] - soff[i];   // >= 200: every token lasts at least one frame, so view addresses are distinct
       if (w.pred_dur) memcpy(w.pred_dur, &dur[offs[i]], (size_t)w.n * sizeof(int32_t));
       w.rc = KKX_OK;
       ctx->views[w.audio] = sb;
@@ -486,6 +487,34 @@ KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* to
 }
 
 KKX_API void kkx_release_pcm16(kkx_ctx* ctx, int16_t* pcm) { kkx_release(ctx, reinterpret_cast<float*>(pcm)); }
+
+KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                                 const float* styles, const float* speeds, int32_t law, uint8_t** out_codes,
+                                 int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+  int rc = check_ctx(ctx);
+  if (rc) return rc;
+  if (out_codes) *out_codes = nullptr;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(ctx, [&] {
+    if (!out_codes) throw ArgError("out_codes is null");
+    if (law != 0 && law != 1) throw ArgError("law must be 0 (mu-law) or 1 (A-law), got " + std::to_string(law));
+    Model& m = *ctx->model;
+    m.stage(batch, tokens, tok_offsets, styles, speeds);
+    m.set_g711(law);
+    try { m.run(); } catch (...) { m.set_g711(-1); throw; }
+    m.set_g711(-1);
+    const long long n = m.total_samples();
+    size_t cap = 0;
+    float* host = take_pinned(ctx, (size_t)(n + 3) / 4, &cap);   // n one-byte codes = n/4 floats of the same pool
+    try {
+      m.fetch_g711(reinterpret_cast<unsigned char*>(host), n, out_sample_offsets, out_pred_dur);
+    } catch (...) { cudaFreeHost(host); throw; }
+    hand_out(ctx, host, cap);
+    *out_codes = reinterpret_cast<uint8_t*>(host);
+  });
+}
+
+KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes) { kkx_release(ctx, reinterpret_cast<float*>(codes)); }
 
 // ---- output containers: host-side byte work (little-endian host assumed, as everywhere in this library)
 static void put_u16(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }
@@ -758,6 +787,16 @@ KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
     } else if (k == "async_batch") {
       if (value < 1 || value > kMaxCoalesce) throw ArgError("async_batch must be in 1..512");
       ctx->async_batch.store((int)value);
+    } else if (k == "out_rate") {
+      int U = 0, D = 0;
+      if (value < 8000 || value > 48000 || !resample_ratio((int)value, &U, &D)) {
+        const long long g = value > 0 ? std::gcd<long long>(value, 24000) : 1;
+        throw ArgError("out_rate " + std::to_string(value) + " Hz is not supported: out_rate / 24000 reduces to U/D = " +
+                       std::to_string(value / g) + "/" + std::to_string(24000 / g) +
+                       "; accepted are 8000..48000 Hz with max(U, D) <= 320 (8000, 11025, 12000, 16000, 22050, 24000, "
+                       "32000, 44100, 48000)");
+      }
+      o.out_rate = (int)value;
     }
     else throw ArgError("unknown option: " + k);
   });
@@ -771,6 +810,7 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   if (k == "last_frames") return ctx->model->last_frames;
   if (k == "gpu_us") return (int64_t)ctx->model->last_gpu_us;
   if (k == "precision") return ctx->model->opt.precision;
+  if (k == "out_rate") return ctx->model->opt.out_rate;
   if (k == "coalesced_batches") return ctx->coalesced_batches;
   if (k == "coalesced_requests") return ctx->coalesced_requests;
   if (k == "coalesced_largest") return ctx->coalesced_largest;

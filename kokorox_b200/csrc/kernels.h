@@ -270,6 +270,21 @@ void launch_stft(const float* x, const long long* s_off, float* har, int ldh, co
 void launch_istft(const float* cp, int ldc, const int* h_off, const int* h_len, float* audio, short* pcm /*nullable*/,
                   const long long* s_off, int fast, int B, int max_len, cudaStream_t st);
 
+// Output sample-rate conversion 24 kHz -> out_rate (scipy.signal.resample_poly with its defaults), per utterance.
+//   resample_ratio: U / D = out_rate / 24000 reduced; false unless 8000 <= out_rate <= 48000 and max(U, D) <= 320.
+//   resample_design: the 2H + 1 fp32 taps U * firwin(2H + 1, 1 / max(U, D), ("kaiser", 5.0)), H = 10 max(U, D),
+//                    designed in double on the host; returns the tap count, or -1 for a rejected rate.  24000 is the
+//                    identity: one tap 1.0, H = 0 (firwin has no filter with cutoff 1; resample_poly copies its input).
+//   launch_resample: item b reads x[in_off[b] .. + in_len[b]) and writes ceil(in_len[b] U / D) samples at out_off[b]
+//                    as f32 and optionally as 16-bit PCM (trunc(clamp(y, -1, 1) * 32767)) and / or G.711 codes of that
+//                    PCM value (law 0 = mu-law, 1 = A-law); U = D = 1 with H = 0 is a pass-through (no taps).
+//                    max_out = largest per-item output length.  Profile name "resample".
+bool resample_ratio(int out_rate, int* U, int* D);
+int resample_design(int out_rate, std::vector<float>* taps, int* U, int* D, int* H);
+void launch_resample(const float* x, const long long* in_off, const long long* in_len, const long long* out_off,
+                     const float* taps, int U, int D, int H, float* out, short* pcm /*nullable*/,
+                     unsigned char* codes /*nullable*/, int law, int B, long long max_out, cudaStream_t st);
+
 // mix_styles (koko.rs:1255-1306) on a device-resident voice table [V][511][256]
 void launch_mix_styles(const float* table, const int* mix_off, const int* voice_ids, const float* portions,
                        const int* rows, float* styles, int B, cudaStream_t st);

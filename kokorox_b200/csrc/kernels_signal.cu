@@ -1,8 +1,12 @@
 // kernels_signal.cu -- HBM-bound kernels: instance-norm statistics, duration head + exact
-// integer length regulation (K4/K5), harmonic source (K9), STFT (K10), iSTFT head (K11).
+// integer length regulation (K4/K5), harmonic source (K9), STFT (K10), iSTFT head (K11), output resampling.
 #include "kernels.h"
 #include <cuda_bf16.h>
 #include <math.h>
+#include <algorithm>
+#include <cmath>
+#include <numeric>
+#include <vector>
 
 namespace kkx {
 
@@ -688,6 +692,11 @@ __host__ __device__ constexpr float tw_cos(int m) {   // cos(2 pi m / 20), m tak
   return c[m % 20];
 }
 __host__ __device__ constexpr float tw_sin(int m) { return tw_cos(m + 15); }   // sin(x) = cos(x - pi/2)
+// 16-bit PCM of an output sample: trunc(clamp(s, -1, 1) * 32767), the f32 -> i16 conversion of the reference's WebSocket
+// server (kokorox-websocket/src/lib.rs:699-703; Rust `as i16` truncates toward zero, NaN -> 0)
+__device__ __forceinline__ short pcm16_of(float s) {
+  return (short)__float2int_rz(fminf(fmaxf(s, -1.0f), 1.0f) * 32767.0f);
+}
 
 template <bool FAST>
 __global__ void __launch_bounds__(128) istft_kernel(const float* __restrict__ cp, int ldc,
@@ -797,16 +806,13 @@ __global__ void __launch_bounds__(128) istft_kernel(const float* __restrict__ cp
     }
   }
   if (pcm) {
-    // optional 16-bit PCM: trunc(clamp(s, -1, 1) * 32767), the f32 -> i16 conversion of the reference's WebSocket
-    // server (kokorox-websocket/src/lib.rs:699-703; Rust `as i16` truncates toward zero, NaN -> 0)
-    short* pd = pcm + s_off[b] + n0;
-    auto to_i16 = [](float x) { return (short)__float2int_rz(fminf(fmaxf(x, -1.0f), 1.0f) * 32767.0f); };
+    short* pd = pcm + s_off[b] + n0;   // optional 16-bit PCM (pcm16_of)
     for (int v = t; v * 4 < count; v += 128) {
       if (v * 4 + 4 <= count) {
-        *reinterpret_cast<short4*>(pd + v * 4) = make_short4(to_i16(s_out[v * 4]), to_i16(s_out[v * 4 + 1]),
-                                                             to_i16(s_out[v * 4 + 2]), to_i16(s_out[v * 4 + 3]));
+        *reinterpret_cast<short4*>(pd + v * 4) = make_short4(pcm16_of(s_out[v * 4]), pcm16_of(s_out[v * 4 + 1]),
+                                                             pcm16_of(s_out[v * 4 + 2]), pcm16_of(s_out[v * 4 + 3]));
       } else {
-        for (int e = 0; v * 4 + e < count; e++) pd[v * 4 + e] = to_i16(s_out[v * 4 + e]);
+        for (int e = 0; v * 4 + e < count; e++) pd[v * 4 + e] = pcm16_of(s_out[v * 4 + e]);
       }
     }
   }
@@ -821,6 +827,181 @@ void launch_istft(const float* cp, int ldc, const int* h_off, const int* h_len, 
   if (fast) istft_kernel<true><<<g, 128, 0, st>>>(cp, ldc, h_off, h_len, audio, s_off, pcm);
   else istft_kernel<false><<<g, 128, 0, st>>>(cp, ldc, h_off, h_len, audio, s_off, pcm);
   post_launch("istft", st);
+}
+
+// ------------------------------------------------------------------------------------------
+// Output sample-rate conversion: 24 kHz -> out_rate by the polyphase FIR of scipy.signal.resample_poly (its defaults:
+// Kaiser beta 5, half length 10 * max(U, D)), each utterance on its own with zeros outside it.
+bool resample_ratio(int out_rate, int* U, int* D) {
+  if (out_rate < 8000 || out_rate > 48000) return false;
+  const int g = std::gcd(out_rate, 24000);
+  *U = out_rate / g;
+  *D = 24000 / g;
+  return std::max(*U, *D) <= 320;
+}
+
+static double bessel_i0(double x) {   // power series of the modified Bessel function I0 (x <= 5 here: ~25 terms)
+  double sum = 1.0, term = 1.0;
+  const double q = 0.25 * x * x;
+  for (int k = 1; k < 200; k++) {
+    term *= q / ((double)k * k);
+    sum += term;
+    if (term < 1e-17 * sum) break;
+  }
+  return sum;
+}
+
+int resample_design(int out_rate, std::vector<float>* taps, int* U, int* D, int* H) {
+  int u = 0, d = 0;
+  if (!resample_ratio(out_rate, &u, &d)) return -1;
+  if (u == 1 && d == 1) {   // 24 kHz: the identity (resample_poly returns its input), the pass-through mode's H = 0
+    if (taps) taps->assign(1, 1.0f);
+    if (U) *U = 1;
+    if (D) *D = 1;
+    if (H) *H = 0;
+    return 1;
+  }
+  const int half = 10 * std::max(u, d), n = 2 * half + 1;
+  // U * firwin(2H + 1, 1 / max(U, D), window = ("kaiser", 5.0)), in double: windowed sinc, normalised to unit DC gain
+  const double fc = 1.0 / std::max(u, d), beta = 5.0, i0b = bessel_i0(beta);
+  std::vector<double> h(n);
+  double sum = 0.0;
+  for (int i = 0; i < n; i++) {
+    const double m = i - half, a = fc * m;
+    const double sinc = m == 0 ? 1.0 : std::sin(M_PI * a) / (M_PI * a);
+    const double r = m / half;
+    h[i] = fc * sinc * bessel_i0(beta * std::sqrt(std::max(0.0, 1.0 - r * r))) / i0b;
+    sum += h[i];
+  }
+  if (taps) {
+    taps->resize(n);
+    for (int i = 0; i < n; i++) (*taps)[i] = (float)(u * (h[i] / sum));
+  }
+  if (U) *U = u;
+  if (D) *D = d;
+  if (H) *H = half;
+  return n;
+}
+
+// ITU-T G.711 of a 16-bit sample, Sun reference g711.c (what audioop.lin2ulaw / lin2alaw(..., 2) return):
+// mu-law from the 14-bit value p >> 2 (bias 33, clip 8159), A-law from the 13-bit value p >> 3.
+__device__ __forceinline__ unsigned char g711_ulaw(int p) {
+  int v = p >> 2;
+  const int mask = v < 0 ? 0x7F : 0xFF;
+  v = min(abs(v), 8159) + 33;                       // 34 .. 8192: segment = position of the top bit above bit 5
+  const int seg = max(0, 31 - __clz(v) - 5);        // first seg with v <= 0x3F << seg (v <= 8192 -> seg <= 7)
+  if (seg >= 8) return (unsigned char)(0x7F ^ mask);
+  return (unsigned char)(((seg << 4) | ((v >> (seg + 1)) & 0xF)) ^ mask);
+}
+__device__ __forceinline__ unsigned char g711_alaw(int p) {
+  int v = p >> 3;
+  const int mask = v >= 0 ? 0xD5 : 0x55;
+  if (v < 0) v = -v - 1;                            // 0 .. 4095
+  const int seg = max(0, 31 - __clz(v | 1) - 4);    // first seg with v <= 0x1F << seg
+  const int q = (seg < 2 ? v >> 1 : v >> seg) & 0xF;
+  return (unsigned char)(((seg << 4) | q) ^ mask);
+}
+
+// y_b[m] = sum over k ascending (0 <= k < n_b, 0 <= m D - k U + H <= 2H) of x_b[k] * taps[m D - k U + H], fp32 FMA.
+// Grid (output tiles of kRsTile = 2048 samples, items), 256 threads, 8 outputs per thread.  The CTA stages the
+// input span its tile reads (zero outside the item) and all 2H + 1 taps in shared memory with coalesced loads.  Each
+// output sample is a function of its item alone, so results do not depend on the batch around it.  Output offsets
+// need not be multiples of 4 (at 11025 / 22050 / 44100 Hz they are not): every store is a scalar, coalesced across
+// the warp.  PASS: U = D = 1 without a filter (the G.711 codes of the 24 kHz waveform itself).
+constexpr int kRsThreads = 256, kRsPer = 8, kRsTile = kRsThreads * kRsPer;
+__host__ __device__ inline long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+template <bool PASS>
+__global__ void __launch_bounds__(kRsThreads) resample_kernel(const float* __restrict__ x, const long long* __restrict__ in_off,
+                                                              const long long* __restrict__ in_len,
+                                                              const long long* __restrict__ out_off,
+                                                              const float* __restrict__ taps, int U, int D, int H,
+                                                              float* __restrict__ out, short* __restrict__ pcm,
+                                                              unsigned char* __restrict__ codes, int law) {
+  extern __shared__ float rs_smem[];
+  const int b = blockIdx.y, t = threadIdx.x;
+  const long long n = in_len[b];
+  const long long n_out = (n * U + D - 1) / D;
+  const long long m0 = (long long)blockIdx.x * kRsTile;
+  if (m0 >= n_out) return;
+  const float* xb = x + in_off[b];
+  const long long ob = out_off[b];
+  float y[kRsPer];
+  if (PASS) {
+#pragma unroll
+    for (int i = 0; i < kRsPer; i++) {
+      const long long m = m0 + t + i * kRsThreads;
+      y[i] = m < n_out ? xb[m] : 0.f;
+    }
+  } else {
+    const int ntap = 2 * H + 1;
+    float* s_h = rs_smem;
+    float* s_x = rs_smem + ((ntap + 3) & ~3);
+    const long long m1 = min(m0 + kRsTile, n_out) - 1;
+    const long long k0 = floor_div(m0 * D - H + U - 1, U);   // ceil((m0 D - H) / U): first input any output reads
+    const long long k1 = floor_div(m1 * D + H, U);
+    const int span = (int)(k1 - k0 + 1);
+    for (int i = t; i < ntap; i += kRsThreads) s_h[i] = __ldg(taps + i);
+    for (int i = t; i < span; i += kRsThreads) {
+      const long long k = k0 + i;
+      s_x[i] = (k >= 0 && k < n) ? __ldg(xb + k) : 0.f;
+    }
+    __syncthreads();
+    // tile-relative 32-bit index math: a = m D - k0 U lies in (H - U, H + (kRsTile - 1) D]; k counts from k0
+    const int a0 = (int)(m0 * D - k0 * U);
+    const int kfirst = (int)max(-k0, 0LL);                       // input index >= 0
+    const int klast = (int)(min(n - 1, k1) - k0);                // input index < n
+#pragma unroll
+    for (int i = 0; i < kRsPer; i++) {
+      const int r = t + i * kRsThreads;
+      float acc = 0.f;
+      if (m0 + r < n_out) {
+        const int a = a0 + r * D;
+        int k = a > H ? (int)((unsigned)(a - H + U - 1) / (unsigned)U) : 0;   // ceil((a - H) / U): first tap <= 2H
+        k = max(k, kfirst);
+        // tap of input k is j = a - k U + H; the filter ends where j < 0
+        for (int j = a - k * U + H; k <= klast && j >= 0; k++, j -= U) acc = fmaf(s_x[k], s_h[j], acc);
+      }
+      y[i] = acc;
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < kRsPer; i++) {
+    const long long m = m0 + t + i * kRsThreads;
+    if (m >= n_out) break;
+    out[ob + m] = y[i];
+    if (pcm || codes) {
+      const short p = pcm16_of(y[i]);
+      if (pcm) pcm[ob + m] = p;
+      if (codes) codes[ob + m] = law ? g711_alaw(p) : g711_ulaw(p);
+    }
+  }
+}
+
+size_t resample_smem_bytes(int U, int D, int H) {
+  if (U == 1 && D == 1 && H == 0) return 0;
+  const long long span = ((long long)(kRsTile - 1) * D + 2 * H) / U + 2;
+  return (size_t)(((2 * H + 1 + 3) & ~3) + span) * sizeof(float);
+}
+
+void launch_resample(const float* x, const long long* in_off, const long long* in_len, const long long* out_off,
+                     const float* taps, int U, int D, int H, float* out, short* pcm, unsigned char* codes, int law,
+                     int B, long long max_out, cudaStream_t st) {
+  if (g_dry_run) return;
+  const bool pass = U == 1 && D == 1 && H == 0;
+  if (!pass && !taps) throw ArgError("launch_resample: filter taps missing");
+  if (max_out <= 0) return;
+  const long long tiles = (max_out + kRsTile - 1) / kRsTile;
+  if (tiles > 0x7FFFFFFFLL || B > 65535) throw ArgError("launch_resample: grid too large");
+  // at most 42.6 KB (11 025 Hz: 6404 taps + a 4501-sample span), inside the default 48 KB of dynamic shared memory
+  const size_t smem = resample_smem_bytes(U, D, H);
+  if (smem > 48 * 1024) throw ArgError("launch_resample: filter too long for one CTA");
+  dim3 g((unsigned)tiles, B);
+  if (pass)
+    resample_kernel<true><<<g, kRsThreads, 0, st>>>(x, in_off, in_len, out_off, nullptr, 1, 1, 0, out, pcm, codes, law);
+  else
+    resample_kernel<false><<<g, kRsThreads, smem, st>>>(x, in_off, in_len, out_off, taps, U, D, H, out, pcm, codes, law);
+  post_launch("resample", st);
 }
 
 // ------------------------------------------------------------------------------------------

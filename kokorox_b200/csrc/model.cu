@@ -172,6 +172,8 @@ Model::~Model() {
   clear_graphs();
   if (d_audio_) cudaFree(d_audio_);
   if (d_pcm_) cudaFree(d_pcm_);
+  if (d_g711_) cudaFree(d_g711_);
+  if (d_taps_) cudaFree(d_taps_);
   if (d_voices_) cudaFree(d_voices_);
   if (d_noise_) cudaFree(d_noise_);
   if (h_pred_dur_) cudaFreeHost(h_pred_dur_);
@@ -774,6 +776,36 @@ void Model::fetch_pcm16(short* dst, long long capacity, int64_t* sample_offsets,
   }
 }
 
+void Model::fetch_g711(unsigned char* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur) {
+  if (!ran_) throw StateError("no completed run to fetch from");
+  if (!d_g711_ || !g711_valid_) throw ArgError("the last run did not produce G.711 codes");
+  fetch(nullptr, 0, sample_offsets, pred_dur);
+  if (dst) {
+    if (capacity < total_samples_) throw ArgError("code buffer too small");
+    KKX_CUDA(cudaMemcpyAsync(dst, d_g711_, total_samples_, cudaMemcpyDeviceToHost, stream_));
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+  }
+}
+
+// The resampling pass of this run: off at 24 kHz unless G.711 codes are wanted (then a pass-through, U = D = 1).  The
+// taps live on the device per Model and are rebuilt only when the rate changes.
+void Model::prepare_resample() {
+  resample_ = opt.out_rate != 24000 || want_law_ >= 0;
+  rs_U_ = 1; rs_D_ = 1; rs_H_ = 0;
+  if (opt.out_rate == 24000) return;
+  std::vector<float> taps;
+  if (resample_design(opt.out_rate, &taps, &rs_U_, &rs_D_, &rs_H_) < 0)
+    throw ArgError("out_rate " + std::to_string(opt.out_rate) + " is not supported");
+  if (taps_rate_ != opt.out_rate) {
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+    if (d_taps_) cudaFree(d_taps_);
+    d_taps_ = nullptr; taps_rate_ = 0;
+    KKX_CUDA(cudaMalloc(&d_taps_, taps.size() * sizeof(float)));
+    KKX_CUDA(cudaMemcpy(d_taps_, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice));
+    taps_rate_ = opt.out_rate;
+  }
+}
+
 void Model::fetch(float* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur) {
   if (!ran_ || B_ <= 0 || (int)sample_off_.size() != B_ + 1) throw StateError("no completed run to fetch from");
   KKX_CUDA(cudaSetDevice(device_));
@@ -797,6 +829,7 @@ void Model::run() {
   KKX_CUDA(cudaSetDevice(device_));
   ran_ = false;
   use_lane(0);
+  prepare_resample();
   g_launch_stats = &stats;
   stats.launches = 0;
   stats.conv_flops = 0;
@@ -824,12 +857,16 @@ void Model::run() {
     throw;
   }
 
-  // frame-phase groups under the frame budget
+  // frame-phase groups under the frame budget; sample counts at the output rate: item b has ceil(600 T_b U / D)
   sample_off_.assign(B_ + 1, 0);
-  long long tot = 0;
-  for (int b = 0; b < B_; b++) { sample_off_[b] = tot * 600; tot += r.T[b]; }
-  sample_off_[B_] = tot * 600;
-  total_samples_ = tot * 600;
+  long long tot = 0, ns = 0;
+  for (int b = 0; b < B_; b++) {
+    sample_off_[b] = ns;
+    tot += r.T[b];
+    ns += (600LL * r.T[b] * rs_U_ + rs_D_ - 1) / rs_D_;
+  }
+  sample_off_[B_] = ns;
+  total_samples_ = ns;
   last_frames = tot;
   if ((size_t)total_samples_ > audio_cap_) {
     KKX_CUDA(cudaStreamSynchronize(stream_));
@@ -847,7 +884,16 @@ void Model::run() {
     KKX_CUDA(cudaMalloc(&d_pcm_, cap * sizeof(short)));
     pcm_cap_ = cap;
   }
+  if (want_law_ >= 0 && (size_t)total_samples_ > g711_cap_) {
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+    if (d_g711_) cudaFree(d_g711_);
+    d_g711_ = nullptr; g711_cap_ = 0;
+    const size_t cap = (size_t)total_samples_ + (size_t)total_samples_ / 4;
+    KKX_CUDA(cudaMalloc(&d_g711_, cap));
+    g711_cap_ = cap;
+  }
   pcm_valid_ = want_pcm_;
+  g711_valid_ = want_law_ >= 0;
   sink_filled_ = false;
   float* sink = (host_sink && !debug_) ? host_sink(total_samples_) : nullptr;
   // (both streams are idle here: the previous run synchronised them, and d_audio_ was sized above)

@@ -168,6 +168,8 @@ struct Options {
   // LSTM gate non-linearities on the SFU (ex2 / rcp approximations, |error| ~ 1e-7) in the tensor-core configuration;
   // precision = 0 always uses libm's expf / tanhf and IEEE division
   int lstm_fast_gates = 1;
+  // sample rate of every waveform a run returns (kkx.h "out_rate"); 24000 = the model's own rate, no resampling
+  int out_rate = 24000;
 };
 
 // Device-resident weights of one checkpoint on one GPU: every layout the kernels read (fp32 SIMT, bf16 / split-TF32
@@ -196,7 +198,8 @@ class WeightSet {
 
 // Hard limits that keep every row / sample index inside int32 and the frame arena inside one GPU (ADVICE r1):
 constexpr float kMinSpeed = 0.1f, kMaxSpeed = 10.f;   // dur per token <= 50 / speed <= 500 frames
-constexpr int kMaxItemFrames = 65536;                  // one utterance: <= 27 min of audio (120*T+1 rows fit int32)
+constexpr int kMaxItemFrames = 65536;                  // one utterance: <= 27 min of audio (120*T+1 rows fit int32;
+                                                       // at out_rate 48000: 1 200 samples per frame, 7.9e7 per utterance)
 
 class Model {
  public:
@@ -214,6 +217,9 @@ class Model {
                     const int32_t* voice_ids, const float* portions, const int32_t* style_rows, const float* speeds);
   void set_pcm16(bool on) { want_pcm_ = on; }
   void fetch_pcm16(short* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
+  // G.711 codes of the 16-bit PCM value (law 0 = mu-law, 1 = A-law, -1 = none) written by the resampling pass
+  void set_g711(int law) { want_law_ = law; }
+  void fetch_g711(unsigned char* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
   // Optional host sink for the waveform: called once the total sample count is known (after the token phase);
   // returns a pinned buffer of >= n floats.  Each frame group's audio is then copied to it on a second stream as
   // soon as the group's iSTFT is done, overlapping the device->host copy with the next group's kernels.
@@ -345,6 +351,11 @@ class Model {
   // outputs
   float* d_audio_ = nullptr; size_t audio_cap_ = 0;
   short* d_pcm_ = nullptr; size_t pcm_cap_ = 0; bool want_pcm_ = false, pcm_valid_ = false;   // optional 16-bit PCM twin of d_audio_
+  unsigned char* d_g711_ = nullptr; size_t g711_cap_ = 0; int want_law_ = -1; bool g711_valid_ = false;  // optional G.711 twin
+  // output resampling of the current run (opt.out_rate): U / D, half length H; d_taps_ holds the filter of taps_rate_
+  bool resample_ = false; int rs_U_ = 1, rs_D_ = 1, rs_H_ = 0;
+  float* d_taps_ = nullptr; int taps_rate_ = 0;
+  void prepare_resample();
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
   std::vector<long long> sample_off_;
   int* h_pred_dur_ = nullptr; size_t h_pred_dur_cap_ = 0;                  // pinned: per-row integer durations of the last run

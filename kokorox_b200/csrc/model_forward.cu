@@ -603,6 +603,21 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
   upload(d_ph_off, ph_off.data(), B * sizeof(int));
   upload(d_s_loc, s_loc.data(), B * sizeof(long long));
   upload(d_s_glob, s_glob.data(), B * sizeof(long long));
+  // output resampling: the iSTFT writes the group's 24 kHz audio here (group-local offsets s_loc), the resampling
+  // pass reads it and writes d_audio_ at the output-rate offsets s_glob
+  float* wav24 = nullptr;
+  long long* d_s_len = nullptr;
+  long long max_out = 0;
+  if (resample_) {
+    std::vector<long long> s_len(B);
+    for (int b = 0; b < B; b++) {
+      s_len[b] = 600LL * T[b];
+      max_out = std::max(max_out, (s_len[b] * rs_U_ + rs_D_ - 1) / rs_D_);
+    }
+    wav24 = A.alloc<float>((size_t)(s_loc[B - 1] + s_len[B - 1]));
+    d_s_len = A.alloc<long long>(B);
+    upload(d_s_len, s_len.data(), B * sizeof(long long));
+  }
 
   // ---- length regulation (K4/K5)
   int* idx = A.alloc<int>(FR.rows);
@@ -897,7 +912,13 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
     launch_conv_f32(c, st);
   }
   capture("conv_post", cp, 24, 0, 22, G120, b0);
-  launch_istft(cp, 24, G120.d_off, G120.d_len, d_audio_, want_pcm_ ? d_pcm_ : nullptr, d_s_glob, opt.precision == 1, B, G120.max_len, st);
+  if (!resample_) {
+    launch_istft(cp, 24, G120.d_off, G120.d_len, d_audio_, want_pcm_ ? d_pcm_ : nullptr, d_s_glob, opt.precision == 1, B, G120.max_len, st);
+    return;
+  }
+  launch_istft(cp, 24, G120.d_off, G120.d_len, wav24, nullptr, d_s_loc, opt.precision == 1, B, G120.max_len, st);
+  launch_resample(wav24, d_s_loc, d_s_len, d_s_glob, d_taps_, rs_U_, rs_D_, rs_H_, d_audio_, want_pcm_ ? d_pcm_ : nullptr,
+                  want_law_ >= 0 ? d_g711_ : nullptr, want_law_ > 0 ? 1 : 0, B, max_out, st);
 }
 
 }  // namespace kkx

@@ -56,6 +56,42 @@ KKX_API int64_t kkx_test_tensor_specs(char* buf, int64_t capacity) {
   return (int64_t)s.size();
 }
 
+KKX_API int64_t kkx_test_resample_taps(int32_t out_rate, float* dst, int64_t capacity) {
+  std::vector<float> taps;
+  const int n = resample_design(out_rate, &taps, nullptr, nullptr, nullptr);
+  if (n < 0) return KKX_ERR_ARG;
+  if (dst && capacity > 0) memcpy(dst, taps.data(), (size_t)std::min<int64_t>(capacity, n) * sizeof(float));
+  return n;
+}
+
+KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64_t* lens, int32_t out_rate, int32_t law,
+                              float* out, int16_t* pcm, uint8_t* codes) {
+  return run(device, [&] {
+    if (!x || !lens || !out || B < 1 || law < -1 || law > 1) throw ArgError("kkx_test_resample: bad argument");
+    std::vector<float> taps;
+    int U = 1, D = 1, H = 0;
+    if (out_rate != 24000 && resample_design(out_rate, &taps, &U, &D, &H) < 0) throw ArgError("rejected out_rate");
+    std::vector<long long> in_off(B), in_len(B), out_off(B);
+    long long ni = 0, no = 0, max_out = 0;
+    for (int b = 0; b < B; b++) {
+      if (lens[b] < 1) throw ArgError("kkx_test_resample: every item needs >= 1 sample");
+      const long long m = (lens[b] * U + D - 1) / D;
+      in_off[b] = ni; in_len[b] = lens[b]; out_off[b] = no;
+      ni += lens[b]; no += m; max_out = std::max(max_out, m);
+    }
+    DevBuf dx(x, (size_t)ni * 4), dt(taps.data(), taps.size() * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8);
+    DevBuf doo(out_off.data(), B * 8), dout(nullptr, (size_t)no * 4), dpcm(nullptr, pcm ? (size_t)no * 2 : 0);
+    DevBuf dcode(nullptr, codes && law >= 0 ? (size_t)no : 0);
+    launch_resample(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), doo.as<long long>(),
+                    taps.empty() ? nullptr : dt.as<float>(), U, D, H, dout.as<float>(), pcm ? dpcm.as<short>() : nullptr,
+                    codes && law >= 0 ? dcode.as<unsigned char>() : nullptr, law > 0 ? 1 : 0, B, max_out, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(out, dout.p, (size_t)no * 4, cudaMemcpyDeviceToHost));
+    if (pcm) KKX_CUDA(cudaMemcpy(pcm, dpcm.p, (size_t)no * 2, cudaMemcpyDeviceToHost));
+    if (codes && law >= 0) KKX_CUDA(cudaMemcpy(codes, dcode.p, (size_t)no, cudaMemcpyDeviceToHost));
+  });
+}
+
 KKX_API int kkx_test_conv(int device, const float* in, int rows_in, int ldi, int Ci, const float* w,
                           const float* bias, int Co, int ks, int dil, int pad, int stride,
                           const float* pscale, const float* pshift, int pact, float pslope,

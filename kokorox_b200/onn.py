@@ -67,6 +67,10 @@ def load_library(path: Optional[str] = None):
         lib.kkx_infer_batch_pcm16.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), P(P(i16)), P(i64), P(i32)]
         lib.kkx_release_pcm16.argtypes = [vp, P(i16)]
         lib.kkx_release_pcm16.restype = None
+        u8 = C.c_uint8
+        lib.kkx_infer_batch_g711.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), i32, P(P(u8)), P(i64), P(i32)]
+        lib.kkx_release_g711.argtypes = [vp, P(u8)]
+        lib.kkx_release_g711.restype = None
         lib.kkx_wav_header_pcm16.argtypes = [P(C.c_uint8), i64, i32]
         lib.kkx_wav_header_f32_stream.argtypes = [P(C.c_uint8), i32, i32]
         lib.kkx_encode_wav16_base64.argtypes = [P(i16), i64, i32, C.c_char_p, i64]
@@ -93,6 +97,9 @@ def load_library(path: Optional[str] = None):
                                               C.c_int, C.c_int, C.c_int, P(f32), f32, P(f32)]
         lib.kkx_test_arb_conv_stream.argtypes = [C.c_int, P(f32), C.c_int, P(i32), C.c_int, P(f32), P(f32), P(f32), P(f32),
                                                  P(f32), C.c_int, C.c_int, P(f32), f32, C.c_int, C.c_int, P(f32), P(f32)]
+        lib.kkx_test_resample_taps.argtypes = [i32, P(f32), i64]
+        lib.kkx_test_resample_taps.restype = i64
+        lib.kkx_test_resample.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(i16), P(u8)]
         lib.kkx_test_attention_batch.argtypes = [C.c_int, P(f32), C.c_int, P(i32), P(i32), C.c_int, C.c_int, P(f32)]
         lib.kkx_debug_stage.argtypes = [vp, C.c_char_p, i32, P(f32), i64, P(i64), P(i64)]
         lib.kkx_debug_stage.restype = i64
@@ -466,6 +473,42 @@ class B200Koko:
         weakref.finalize(base, B200Koko._release_buffer, self, C.cast(pcm, C.c_void_p).value)
         outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
         del base
+        return outs
+
+    def infer_batch_g711(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float], law: str = "ulaw",
+                         return_durations: bool = False):
+        """Like infer_batch_pcm16, but every sample comes back as one G.711 byte (``law`` "ulaw" = PCMU or "alaw" =
+        PCMA) of that 16-bit value, at the session's ``out_rate`` (set it to 8000 for telephony).  Returns a list of
+        uint8 arrays, views into a library-owned buffer released like the pcm16 ones."""
+        self._require()
+        laws = {"ulaw": 0, "alaw": 1}
+        if law not in laws:
+            raise KkxError(-1, f"law must be 'ulaw' or 'alaw', got {law!r}")
+        B = len(tokens)
+        if B == 0:
+            raise KkxError(-1, "empty batch")
+        lens = [len(t) for t in tokens]
+        offs = np.zeros(B + 1, dtype=np.int32)
+        offs[1:] = np.cumsum(lens)
+        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
+        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, 256))
+        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        codes = C.POINTER(C.c_uint8)()
+        soff = np.zeros(B + 1, dtype=np.int64)
+        dur = np.zeros(int(offs[-1]), dtype=np.int32)
+        self._check(self._lib.kkx_infer_batch_g711(
+            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
+            _fp(st), _fp(sp), laws[law], C.byref(codes), soff.ctypes.data_as(C.POINTER(C.c_int64)),
+            dur.ctypes.data_as(C.POINTER(C.c_int32))))
+        total = int(soff[-1])
+        base = np.ctypeslib.as_array(codes, shape=(max(total, 1),))
+        with self._count_lock:
+            self._outstanding += 1
+        weakref.finalize(base, B200Koko._release_buffer, self, C.cast(codes, C.c_void_p).value)
+        outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
+        del base
+        if return_durations:
+            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
 
     # -- device-resident path (bench `value`) ---------------------------------------------

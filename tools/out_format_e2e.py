@@ -1,0 +1,99 @@
+"""End-to-end cost of the output formats: the benchmark's B = 64 x 510 batch through the public calls with host
+buffers (warm-up, then a timed loop; every call ends in a device synchronise and the result in pinned host memory),
+comparing
+
+  * infer_batch        at 24 kHz, f32      (the benchmark's e2e leg)
+  * infer_batch_pcm16  at 16 kHz, int16    ("out_rate" 16000)
+  * infer_batch_g711   at  8 kHz, mu-law   ("out_rate" 8000)
+
+One session switches "out_rate" before each format's warm-up (a server would hold one session per rate; those share the
+device weights), and the formats alternate over --rounds rounds so that drift on a shared host hits all of them alike.
+
+    python tools/out_format_e2e.py [--batch 64] [--tokens 510] [--steps 10] [--warmup 3] [--rounds 2] [--out FILE]
+Prints one JSON object: per format the wall time per step (every round), audio seconds per step, audio-s/s and the
+device-to-host bytes per step (waveform payload + the per-token durations the call also returns).
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+from kokorox_b200.synth import ensure_weights, synth_batch  # noqa: E402
+
+FORMATS = (   # name, out_rate, bytes per sample, per-token durations fetched by the binding
+    ("f32_24k", 24000, 4, True),
+    ("pcm16_16k", 16000, 2, False),
+    ("g711_ulaw_8k", 8000, 1, True),
+)
+
+
+def gpu_info():
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()
+        return q[0] if q else "unknown"
+    except (OSError, subprocess.SubprocessError):
+        return "unknown"
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--batch", type=int, default=64)
+    ap.add_argument("--tokens", type=int, default=510)
+    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--rounds", type=int, default=2)
+    ap.add_argument("--out", default="")
+    a = ap.parse_args()
+    from kokorox_b200.onn import B200Koko, init_ort
+    init_ort()
+    wp = ensure_weights()
+    toks, styles, speeds = synth_batch(a.batch, a.tokens, 0)
+    sum_n = sum(len(t) for t in toks)
+    m = B200Koko.new(wp)
+
+    def call(name):
+        if name.startswith("f32"):
+            return m.infer_batch(toks, styles, speeds)
+        if name.startswith("pcm16"):
+            return m.infer_batch_pcm16(toks, styles, speeds)
+        return m.infer_batch_g711(toks, styles, speeds, law="ulaw")
+
+    res = {name: {"out_rate": rate, "wall_ms_per_step": []} for name, rate, _, _ in FORMATS}
+    for _ in range(a.rounds):
+        for name, rate, bps, with_dur in FORMATS:
+            m.set_option("out_rate", rate)
+            outs = None
+            for _ in range(a.warmup):      # the previous result stays alive during the next call, as in bench.py
+                outs = call(name)
+            t0 = time.perf_counter()
+            for _ in range(a.steps):
+                outs = call(name)
+            wall = (time.perf_counter() - t0) / a.steps
+            n = sum(len(o) for o in outs)
+            del outs
+            r = res[name]
+            r["wall_ms_per_step"].append(round(wall * 1e3, 3))
+            r["samples_per_step"] = n
+            r["audio_s_per_step"] = n / rate
+            r["d2h_bytes_per_step"] = n * bps + (sum_n * 4 if with_dur else 0)
+    for name, _, _, _ in FORMATS:
+        r = res[name]
+        best = min(r["wall_ms_per_step"])
+        r["audio_s_per_s_best"] = round(r["audio_s_per_step"] / (best / 1e3), 1)
+    out = {"gpu": gpu_info(), "batch": a.batch, "tokens": a.tokens, "steps": a.steps, "warmup": a.warmup,
+           "rounds": a.rounds, "formats": res}
+    print(json.dumps(out, indent=1))
+    if a.out:
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        with open(a.out, "w") as f:
+            json.dump(out, f, indent=1)
+    m.close()
+
+
+if __name__ == "__main__":
+    main()
