@@ -161,6 +161,38 @@ KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tok
                                  uint8_t** out_codes, int64_t* out_sample_offsets, int32_t* out_pred_dur);
 KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes);
 
+/* kkx_infer_batch_flac: like kkx_infer_batch_pcm16, but item b comes back as one complete FLAC file (RFC 9639,
+ *   streamable subset): bytes [out_byte_offsets[b], out_byte_offsets[b+1]) of *out_bytes.  Decoding it yields exactly
+ *   the int16 samples kkx_infer_batch_pcm16 returns for that item, at the session's "out_rate".
+ *   out_sample_offsets (nullable) as in kkx_infer_batch_pcm16.  One pass (no "max_tokens" split).  Encoded on the
+ *   device; the bytes are a function of the item's samples alone (same bytes in any batch).  For n samples p[0..n)
+ *   at rate r:
+ *   head     "fLaC", metadata block header (last 1, type 0 STREAMINFO, length 34), STREAMINFO: min = max block size
+ *            4096, min / max frame size = this stream's smallest / largest frame in bytes, rate r, 1 channel,
+ *            16 bits, n total samples, MD5 all zero ("not computed").
+ *   frames   frame i holds p[4096 i, min(n, 4096 (i + 1))) (bs samples); no prediction crosses a frame.  Header:
+ *            FF F8, block-size code (4096: 1100; a short last block: its table code 192 / 576 / 1152 / 2304 /
+ *            256 / 512 / 1024 / 2048, else 0110 + 8-bit bs - 1 if bs <= 256, else 0111 + 16-bit bs - 1),
+ *            sample-rate code (8000 0100, 16000 0101, 22050 0110, 24000 0111, 32000 1000, 44100 1001,
+ *            48000 1010, 12000 1100 + byte 12, 11025 1101 + 16-bit 11025), byte 08 (mono, 16 bits), frame number
+ *            i in FLAC's UTF-8 coding, CRC-8 (poly 0x07, init 0).  Footer: zero bits to a byte boundary, CRC-16
+ *            of the frame (poly 0x8005, init 0, big-endian).
+ *   subframe one per frame, wasted-bits flag 0:
+ *            CONSTANT (00, 16-bit value) if all bs samples are equal (bs = 1 included); else the cheapest FIXED
+ *            (10 | o << 1): order o in 0..4 (o < bs), warm-up = first o samples (16 bits each), Rice method 0,
+ *            partition order q in 0..8 (bs % 2^q == 0, (bs >> q) > o; the first partition holds (bs >> q) - o
+ *            residuals), per partition the k in 0..14 minimising sum (u >> k) + n_part (k + 1), residual
+ *            e folded to u = e >= 0 ? 2e : -2e - 1 and coded as (u >> k) zeros, a one, the low k bits.  Cost
+ *            8 + 16 o + 6 + sum over partitions (4 + sum (u >> k) + n_part (k + 1)) bits; ties go to the smaller
+ *            o, then q, then k.  VERBATIM (02, bs x 16 bits) only if strictly cheaper (8 + 16 bs bits), so no
+ *            frame is larger than verbatim.  No Rice escapes, no LPC.
+ *   Release the buffer with kkx_release_flac.  KKX_ERR_ARG for a null out_bytes or out_byte_offsets. */
+KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                                 const float* styles, const float* speeds, uint8_t** out_bytes,
+                                 int64_t* out_byte_offsets /* [batch + 1], required */,
+                                 int64_t* out_sample_offsets /* [batch + 1], nullable */, int32_t* out_pred_dur);
+KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes);
+
 /* ---- output containers (host-side byte work after the pcm16 / f32 result; no GPU involved, no ctx needed).
  * kkx_wav_header_pcm16: the 44-byte RIFF/WAVE header of the WebSocket server's `encode_audio`
  *   (kokorox-websocket/src/lib.rs:707-731): PCM format 1, mono, 16 bit, sizes filled in from n_samples.

@@ -125,6 +125,11 @@ KKX_API int kkx_test_arb_conv_stream(int device, const float* x, int B, const in
 KKX_API int64_t kkx_test_resample_taps(int32_t out_rate, float* dst, int64_t capacity);
 KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64_t* lens, int32_t out_rate, int32_t law,
                               float* out, int16_t* pcm, uint8_t* codes);
+/* FLAC encoder (kernels_flac.cu) on caller-supplied PCM: B items packed back to back (item b has lens[b] >= 1
+ * samples), rate = any accepted "out_rate".  Writes the B FLAC files back to back into dst (nullable: size query)
+ * and their offsets into byte_offsets [B + 1]; returns the total byte count or < 0. */
+KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
+                              uint8_t* dst, int64_t capacity, int64_t* byte_offsets);
 KKX_API const char* kkx_test_last_error(void);
 
 #ifdef __cplusplus

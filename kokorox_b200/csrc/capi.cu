@@ -516,6 +516,35 @@ KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tok
 
 KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes) { kkx_release(ctx, reinterpret_cast<float*>(codes)); }
 
+KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                                 const float* styles, const float* speeds, uint8_t** out_bytes,
+                                 int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+  int rc = check_ctx(ctx);
+  if (rc) return rc;
+  if (out_bytes) *out_bytes = nullptr;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(ctx, [&] {
+    if (!out_bytes) throw ArgError("out_bytes is null");
+    if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
+    Model& m = *ctx->model;
+    m.stage(batch, tokens, tok_offsets, styles, speeds);
+    m.set_pcm16(true);
+    try { m.run(); } catch (...) { m.set_pcm16(false); throw; }
+    m.set_pcm16(false);
+    m.encode_flac();
+    const long long n = m.flac_bytes();
+    size_t cap = 0;
+    float* host = take_pinned(ctx, (size_t)(n + 3) / 4, &cap);   // n bytes = n/4 floats of the same pool
+    try {
+      m.fetch_flac(reinterpret_cast<unsigned char*>(host), n, out_byte_offsets, out_sample_offsets, out_pred_dur);
+    } catch (...) { cudaFreeHost(host); throw; }
+    hand_out(ctx, host, cap);
+    *out_bytes = reinterpret_cast<uint8_t*>(host);
+  });
+}
+
+KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes) { kkx_release(ctx, reinterpret_cast<float*>(bytes)); }
+
 // ---- output containers: host-side byte work (little-endian host assumed, as everywhere in this library)
 static void put_u16(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }
 static void put_u32(uint8_t* p, uint32_t v) { put_u16(p, v & 0xFFFF); put_u16(p + 2, v >> 16); }

@@ -285,6 +285,19 @@ void launch_resample(const float* x, const long long* in_off, const long long* i
                      const float* taps, int U, int D, int H, float* out, short* pcm /*nullable*/,
                      unsigned char* codes /*nullable*/, int law, int B, long long max_out, cudaStream_t st);
 
+// Lossless FLAC of 16-bit mono PCM (kernels_flac.cu; the bitstream rules are in kkx.h, kkx_infer_batch_flac).
+//   Item b is pcm[soff[b] .. soff[b + 1]) (>= 1 sample) and has flac_frames(n_b) frames of 4096 samples; foff[b + 1]
+//   is the prefix sum of those counts (F = foff[B] frames).  launch_flac writes item b's stream to
+//   out[item_off[b] .. item_off[b + 1]) (item_off [B + 1], device); out must hold flac_bound(B, F, samples) bytes and
+//   work flac_work_bytes(F).  rate: one of the nine "out_rate" values.  Three launches, profile names
+//   "flac_analyze", "flac_scan", "flac_pack".
+long long flac_frames(long long n);
+long long flac_bound(long long n_items, long long n_frames, long long n_samples);
+size_t flac_work_bytes(long long n_frames);
+bool flac_rate_ok(int rate);
+void launch_flac(const short* pcm, const long long* soff, const int* foff, int B, int F, int rate, void* work,
+                 unsigned char* out, long long* item_off, cudaStream_t st);
+
 // mix_styles (koko.rs:1255-1306) on a device-resident voice table [V][511][256]
 void launch_mix_styles(const float* table, const int* mix_off, const int* voice_ids, const float* portions,
                        const int* rows, float* styles, int B, cudaStream_t st);

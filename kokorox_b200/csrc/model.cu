@@ -173,6 +173,8 @@ Model::~Model() {
   if (d_audio_) cudaFree(d_audio_);
   if (d_pcm_) cudaFree(d_pcm_);
   if (d_g711_) cudaFree(d_g711_);
+  if (d_flac_) cudaFree(d_flac_);
+  if (d_flac_meta_) cudaFree(d_flac_meta_);
   if (d_taps_) cudaFree(d_taps_);
   if (d_voices_) cudaFree(d_voices_);
   if (d_noise_) cudaFree(d_noise_);
@@ -787,6 +789,87 @@ void Model::fetch_g711(unsigned char* dst, long long capacity, int64_t* sample_o
   }
 }
 
+void Model::encode_flac() {
+  if (!ran_) throw StateError("no completed run to encode");
+  if (!d_pcm_ || !pcm_valid_) throw ArgError("the last run did not produce 16-bit PCM");
+  KKX_CUDA(cudaSetDevice(device_));
+  flac_valid_ = false;
+  // frames per item (4096 samples each) and the device tables: sample offsets, frame prefix, item byte offsets
+  std::vector<int> foff(B_ + 1, 0);
+  for (int b = 0; b < B_; b++) {
+    const long long nf = flac_frames(sample_off_[b + 1] - sample_off_[b]);
+    if (foff[b] + nf > 0x7FFFFFFFLL) throw ArgError("batch too long for one FLAC encode");
+    foff[b + 1] = foff[b] + (int)nf;
+  }
+  const int F = foff[B_];
+  const size_t bound = (size_t)flac_bound(B_, F, total_samples_);
+  const size_t t_soff = 0, t_foff = t_soff + (((size_t)(B_ + 1) * 8 + 255) & ~size_t(255));
+  const size_t t_ioff = t_foff + (((size_t)(B_ + 1) * 4 + 255) & ~size_t(255));
+  const size_t t_work = t_ioff + (((size_t)(B_ + 1) * 8 + 255) & ~size_t(255));
+  const size_t meta = t_work + flac_work_bytes(F);
+  if (bound > flac_cap_) {
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+    if (d_flac_) cudaFree(d_flac_);
+    d_flac_ = nullptr; flac_cap_ = 0;
+    const size_t cap = bound + bound / 4;
+    KKX_CUDA(cudaMalloc(&d_flac_, cap));
+    flac_cap_ = cap;
+  }
+  if (meta > flac_meta_cap_) {
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+    if (d_flac_meta_) cudaFree(d_flac_meta_);
+    d_flac_meta_ = nullptr; flac_meta_cap_ = 0;
+    const size_t cap = meta + meta / 4;
+    KKX_CUDA(cudaMalloc(&d_flac_meta_, cap));
+    flac_meta_cap_ = cap;
+  }
+  long long* d_soff = reinterpret_cast<long long*>(d_flac_meta_ + t_soff);
+  int* d_foff = reinterpret_cast<int*>(d_flac_meta_ + t_foff);
+  long long* d_ioff = reinterpret_cast<long long*>(d_flac_meta_ + t_ioff);
+  KKX_CUDA(cudaMemcpyAsync(d_soff, sample_off_.data(), (size_t)(B_ + 1) * 8, cudaMemcpyHostToDevice, stream_));
+  KKX_CUDA(cudaMemcpyAsync(d_foff, foff.data(), (size_t)(B_ + 1) * 4, cudaMemcpyHostToDevice, stream_));
+  // the encoder's launches count in "launches" and appear in kkx_profile_json beside the run's kernels
+  g_launch_stats = &stats;
+  const size_t e0 = stats.n_events;
+  if (stats.profile) {   // a new start event; the name keeps names[i] = launch between events[i] and [i + 1]
+    cudaEventRecord(stats.next_event(), stream_);
+    stats.names.push_back("(host)");
+  }
+  try {
+    launch_flac(d_pcm_, d_soff, d_foff, B_, F, opt.out_rate, d_flac_meta_ + t_work, d_flac_, d_ioff, stream_);
+    flac_off_.assign(B_ + 1, 0);
+    KKX_CUDA(cudaMemcpyAsync(flac_off_.data(), d_ioff, (size_t)(B_ + 1) * 8, cudaMemcpyDeviceToHost, stream_));
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+  } catch (...) {
+    cudaStreamSynchronize(stream_);
+    g_launch_stats = nullptr;
+    throw;
+  }
+  if (stats.profile)
+    for (size_t i = e0; i + 1 < stats.n_events && i < stats.names.size(); i++) {
+      float dt = 0.f;
+      cudaEventElapsedTime(&dt, stats.events[i], stats.events[i + 1]);
+      auto& e = prof_[stats.names[i]];
+      e.first += 1; e.second += dt * 1e3;
+    }
+  g_launch_stats = nullptr;
+  flac_valid_ = true;
+}
+
+void Model::fetch_flac(unsigned char* dst, long long capacity, int64_t* byte_offsets, int64_t* sample_offsets,
+                       int32_t* pred_dur) {
+  if (!ran_) throw StateError("no completed run to fetch from");
+  if (!flac_valid_) throw ArgError("the last run was not FLAC-encoded");
+  fetch(nullptr, 0, sample_offsets, pred_dur);
+  if (byte_offsets)
+    for (int b = 0; b <= B_; b++) byte_offsets[b] = flac_off_[b];
+  if (dst) {
+    if (capacity < flac_off_[B_]) throw ArgError("FLAC buffer too small");
+    KKX_CUDA(cudaMemcpyAsync(dst, d_flac_, (size_t)flac_off_[B_], cudaMemcpyDeviceToHost, stream_));
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+  }
+}
+
 // The resampling pass of this run: off at 24 kHz unless G.711 codes are wanted (then a pass-through, U = D = 1).  The
 // taps live on the device per Model and are rebuilt only when the rate changes.
 void Model::prepare_resample() {
@@ -828,6 +911,7 @@ void Model::run() {
   if (!staged_ || B_ <= 0) throw StateError("no batch staged");
   KKX_CUDA(cudaSetDevice(device_));
   ran_ = false;
+  flac_valid_ = false;
   use_lane(0);
   prepare_resample();
   g_launch_stats = &stats;

@@ -220,6 +220,12 @@ class Model {
   // G.711 codes of the 16-bit PCM value (law 0 = mu-law, 1 = A-law, -1 = none) written by the resampling pass
   void set_g711(int law) { want_law_ = law; }
   void fetch_g711(unsigned char* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
+  // Lossless FLAC (kernels_flac.cu) of the last run's 16-bit PCM (a run with set_pcm16(true)): one stream per item,
+  // back to back; encode_flac() launches the encoder and copies the per-item byte offsets to the host.
+  void encode_flac();
+  long long flac_bytes() const { return flac_valid_ ? flac_off_.back() : 0; }
+  void fetch_flac(unsigned char* dst, long long capacity, int64_t* byte_offsets, int64_t* sample_offsets,
+                  int32_t* pred_dur);
   // Optional host sink for the waveform: called once the total sample count is known (after the token phase);
   // returns a pinned buffer of >= n floats.  Each frame group's audio is then copied to it on a second stream as
   // soon as the group's iSTFT is done, overlapping the device->host copy with the next group's kernels.
@@ -352,6 +358,10 @@ class Model {
   float* d_audio_ = nullptr; size_t audio_cap_ = 0;
   short* d_pcm_ = nullptr; size_t pcm_cap_ = 0; bool want_pcm_ = false, pcm_valid_ = false;   // optional 16-bit PCM twin of d_audio_
   unsigned char* d_g711_ = nullptr; size_t g711_cap_ = 0; int want_law_ = -1; bool g711_valid_ = false;  // optional G.711 twin
+  // FLAC streams of the last encode_flac(): bytes, per-item byte offsets (host), and the encoder's tables / scratch
+  unsigned char* d_flac_ = nullptr; size_t flac_cap_ = 0; bool flac_valid_ = false;
+  char* d_flac_meta_ = nullptr; size_t flac_meta_cap_ = 0;
+  std::vector<long long> flac_off_;
   // output resampling of the current run (opt.out_rate): U / D, half length H; d_taps_ holds the filter of taps_rate_
   bool resample_ = false; int rs_U_ = 1, rs_D_ = 1, rs_H_ = 0;
   float* d_taps_ = nullptr; int taps_rate_ = 0;

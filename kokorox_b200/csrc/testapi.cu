@@ -92,6 +92,37 @@ KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64
   });
 }
 
+KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
+                              uint8_t* dst, int64_t capacity, int64_t* byte_offsets) {
+  long long total = 0;
+  const int rc = run(device, [&] {
+    if (!pcm || !lens || !byte_offsets || B < 1) throw ArgError("kkx_test_flac: bad argument");
+    if (!flac_rate_ok(rate)) throw ArgError("kkx_test_flac: rejected rate");
+    std::vector<long long> soff(B + 1, 0);
+    std::vector<int> foff(B + 1, 0);
+    for (int b = 0; b < B; b++) {
+      if (lens[b] < 1) throw ArgError("kkx_test_flac: every item needs >= 1 sample");
+      soff[b + 1] = soff[b] + lens[b];
+      foff[b + 1] = foff[b] + (int)flac_frames(lens[b]);
+    }
+    const int F = foff[B];
+    DevBuf dp(pcm, (size_t)soff[B] * 2), ds(soff.data(), (B + 1) * 8), df(foff.data(), (B + 1) * 4);
+    DevBuf dio(nullptr, (B + 1) * 8), dw(nullptr, flac_work_bytes(F)), dout(nullptr, (size_t)flac_bound(B, F, soff[B]));
+    launch_flac(dp.as<short>(), ds.as<long long>(), df.as<int>(), B, F, rate, dw.p, dout.as<unsigned char>(),
+                dio.as<long long>(), 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    std::vector<long long> io(B + 1);
+    KKX_CUDA(cudaMemcpy(io.data(), dio.p, (B + 1) * 8, cudaMemcpyDeviceToHost));
+    for (int b = 0; b <= B; b++) byte_offsets[b] = io[b];
+    total = io[B];
+    if (dst) {
+      if (capacity < total) throw ArgError("kkx_test_flac: dst too small");
+      KKX_CUDA(cudaMemcpy(dst, dout.p, (size_t)total, cudaMemcpyDeviceToHost));
+    }
+  });
+  return rc == KKX_OK ? (int64_t)total : (int64_t)rc;
+}
+
 KKX_API int kkx_test_conv(int device, const float* in, int rows_in, int ldi, int Ci, const float* w,
                           const float* bias, int Co, int ks, int dil, int pad, int stride,
                           const float* pscale, const float* pshift, int pact, float pslope,

@@ -71,6 +71,9 @@ def load_library(path: Optional[str] = None):
         lib.kkx_infer_batch_g711.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), i32, P(P(u8)), P(i64), P(i32)]
         lib.kkx_release_g711.argtypes = [vp, P(u8)]
         lib.kkx_release_g711.restype = None
+        lib.kkx_infer_batch_flac.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), P(P(u8)), P(i64), P(i64), P(i32)]
+        lib.kkx_release_flac.argtypes = [vp, P(u8)]
+        lib.kkx_release_flac.restype = None
         lib.kkx_wav_header_pcm16.argtypes = [P(C.c_uint8), i64, i32]
         lib.kkx_wav_header_f32_stream.argtypes = [P(C.c_uint8), i32, i32]
         lib.kkx_encode_wav16_base64.argtypes = [P(i16), i64, i32, C.c_char_p, i64]
@@ -100,6 +103,8 @@ def load_library(path: Optional[str] = None):
         lib.kkx_test_resample_taps.argtypes = [i32, P(f32), i64]
         lib.kkx_test_resample_taps.restype = i64
         lib.kkx_test_resample.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(i16), P(u8)]
+        lib.kkx_test_flac.argtypes = [C.c_int, P(i16), i32, P(i64), i32, P(u8), i64, P(i64)]
+        lib.kkx_test_flac.restype = i64
         lib.kkx_test_attention_batch.argtypes = [C.c_int, P(f32), C.c_int, P(i32), P(i32), C.c_int, C.c_int, P(f32)]
         lib.kkx_debug_stage.argtypes = [vp, C.c_char_p, i32, P(f32), i64, P(i64), P(i64)]
         lib.kkx_debug_stage.restype = i64
@@ -507,6 +512,37 @@ class B200Koko:
         weakref.finalize(base, B200Koko._release_buffer, self, C.cast(codes, C.c_void_p).value)
         outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
         del base
+        if return_durations:
+            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
+        return outs
+
+    def infer_batch_flac(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
+                         return_durations: bool = False):
+        """Like infer_batch_pcm16, but item b comes back as one complete FLAC file (``bytes``, Content-Type
+        audio/flac) at the session's ``out_rate``, encoded on the device; decoding it gives exactly the int16 samples
+        infer_batch_pcm16 returns.  The files are copied out of the library's buffer, which is released before this
+        returns."""
+        self._require()
+        B = len(tokens)
+        if B == 0:
+            raise KkxError(-1, "empty batch")
+        lens = [len(t) for t in tokens]
+        offs = np.zeros(B + 1, dtype=np.int32)
+        offs[1:] = np.cumsum(lens)
+        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
+        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, 256))
+        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        buf = C.POINTER(C.c_uint8)()
+        boff = np.zeros(B + 1, dtype=np.int64)
+        dur = np.zeros(int(offs[-1]), dtype=np.int32)
+        self._check(self._lib.kkx_infer_batch_flac(
+            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
+            _fp(st), _fp(sp), C.byref(buf), boff.ctypes.data_as(C.POINTER(C.c_int64)), None,
+            dur.ctypes.data_as(C.POINTER(C.c_int32))))
+        try:
+            outs = [C.string_at(C.addressof(buf.contents) + int(boff[b]), int(boff[b + 1] - boff[b])) for b in range(B)]
+        finally:
+            self._lib.kkx_release_flac(self._ctx, buf)
         if return_durations:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs

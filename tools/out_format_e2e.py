@@ -5,15 +5,21 @@ comparing
   * infer_batch        at 24 kHz, f32      (the benchmark's e2e leg)
   * infer_batch_pcm16  at 16 kHz, int16    ("out_rate" 16000)
   * infer_batch_g711   at  8 kHz, mu-law   ("out_rate" 8000)
+  * infer_batch_flac   at 24 kHz, FLAC     (lossless, encoded on the device)
 
 One session switches "out_rate" before each format's warm-up (a server would hold one session per rate; those share the
 device weights), and the formats alternate over --rounds rounds so that drift on a shared host hits all of them alike.
 
     python tools/out_format_e2e.py [--batch 64] [--tokens 510] [--steps 10] [--warmup 3] [--rounds 2] [--out FILE]
 Prints one JSON object: per format the wall time per step (every round), audio seconds per step, audio-s/s and the
-device-to-host bytes per step (waveform payload + the per-token durations the call also returns).
+device-to-host bytes per step (waveform payload + the per-token durations the call also returns; for FLAC also the
+per-item byte offsets, and the payload's bytes per sample against 16-bit PCM).  After the timed rounds, one more
+FLAC step runs with kkx_profile_enable (a run of its own, since the per-launch events slow the host) and
+"flac_profile" gives the encoder kernels' device time in that step.  The compression of the random-init
+checkpoint's audio says nothing about the ratio on real-model speech.
 """
 import argparse
+import ctypes
 import json
 import os
 import subprocess
@@ -28,7 +34,13 @@ FORMATS = (   # name, out_rate, bytes per sample, per-token durations fetched by
     ("f32_24k", 24000, 4, True),
     ("pcm16_16k", 16000, 2, False),
     ("g711_ulaw_8k", 8000, 1, True),
+    ("flac_24k", 24000, None, True),   # variable: the files' byte count
 )
+FLAC_KERNELS = ("flac_analyze", "flac_scan", "flac_pack")
+
+
+def flac_samples(data: bytes) -> int:
+    return int.from_bytes(data[18:26], "big") & ((1 << 36) - 1)   # STREAMINFO total samples
 
 
 def gpu_info():
@@ -61,6 +73,8 @@ def main():
             return m.infer_batch(toks, styles, speeds)
         if name.startswith("pcm16"):
             return m.infer_batch_pcm16(toks, styles, speeds)
+        if name.startswith("flac"):
+            return m.infer_batch_flac(toks, styles, speeds)
         return m.infer_batch_g711(toks, styles, speeds, law="ulaw")
 
     res = {name: {"out_rate": rate, "wall_ms_per_step": []} for name, rate, _, _ in FORMATS}
@@ -74,19 +88,46 @@ def main():
             for _ in range(a.steps):
                 outs = call(name)
             wall = (time.perf_counter() - t0) / a.steps
-            n = sum(len(o) for o in outs)
-            del outs
             r = res[name]
+            if bps is None:
+                n = sum(flac_samples(o) for o in outs)
+                payload = sum(len(o) for o in outs)
+                r["payload_bytes_per_step"] = payload
+                r["bytes_per_sample"] = round(payload / n, 4)
+                r["of_pcm16"] = round(payload / (2 * n), 4)
+                payload += 8 * (a.batch + 1)
+            else:
+                n = sum(len(o) for o in outs)
+                payload = n * bps
+            del outs
             r["wall_ms_per_step"].append(round(wall * 1e3, 3))
             r["samples_per_step"] = n
             r["audio_s_per_step"] = n / rate
-            r["d2h_bytes_per_step"] = n * bps + (sum_n * 4 if with_dur else 0)
+            r["d2h_bytes_per_step"] = payload + (sum_n * 4 if with_dur else 0)
     for name, _, _, _ in FORMATS:
         r = res[name]
         best = min(r["wall_ms_per_step"])
         r["audio_s_per_s_best"] = round(r["audio_s_per_step"] / (best / 1e3), 1)
+    # one profiled FLAC step: per-kernel device time (event after every launch) of the run and of the encoder
+    m.set_option("out_rate", 24000)
+    m._lib.kkx_profile_enable(m._ctx, 1)
+    call("flac")
+    nbuf = m._lib.kkx_profile_json(m._ctx, None, 0)
+    buf = ctypes.create_string_buffer(int(nbuf) + 1)
+    m._lib.kkx_profile_json(m._ctx, buf, nbuf + 1)
+    m._lib.kkx_profile_enable(m._ctx, 0)
+    prof = json.loads(buf.value.decode())
+    kern = prof["kernels"]
+    enc_ms = {k: round(kern[k][1] / 1e3, 4) for k in FLAC_KERNELS}
+    step_ms = sum(v[1] for v in kern.values()) / 1e3
+    flac_profile = {"run_gpu_ms": round(prof["gpu_us"] / 1e3, 3), "step_kernels_ms": round(step_ms, 3),
+                    "encoder_ms": enc_ms, "encoder_total_ms": round(sum(enc_ms.values()), 4),
+                    "encoder_share_of_step": round(sum(enc_ms.values()) / step_ms, 5),
+                    "launches": m.get_stat("launches")}
     out = {"gpu": gpu_info(), "batch": a.batch, "tokens": a.tokens, "steps": a.steps, "warmup": a.warmup,
-           "rounds": a.rounds, "formats": res}
+           "rounds": a.rounds, "formats": res, "flac_profile": flac_profile,
+           "note": "FLAC sizes are those of the random-init checkpoint's audio; they say nothing about the "
+                   "compression ratio of real-model speech"}
     print(json.dumps(out, indent=1))
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
