@@ -260,12 +260,57 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                   0 <= m < ceil(n U / D)   (n = 600 T input samples)
  *                 accumulated in fp32 (taps designed in double, stored as fp32), one output per thread on the GPU, so
  *                 results stay bit-identical to the item's own B = 1 call.  16-bit PCM and G.711 are converted from y.
+ *   "loudness_target"  integrated-loudness target in 1/100 LUFS (e.g. -2300 = EBU R128's -23 LUFS, -1600 podcast,
+ *                 -1400 streaming); 0 (DEFAULT) = off: no kernel is added and every bit and launch is as before.
+ *                 Accepted: 0 or -7000..-500.
+ *   "true_peak_max"  true-peak ceiling in 1/100 dBTP (default -100, EBU R128's -1 dBTP); accepted -2000..0.
+ *                 For both, any other value is KKX_ERR_ARG and the session keeps its setting.  Like "out_rate", one
+ *                 setting per session, followed by every waveform entry point (kkx_infer, _batch, _batch_voices,
+ *                 _batch_pcm16, _batch_g711, _batch_flac, coalesced and kkx_submit batches, kkx_run_staged /
+ *                 kkx_fetch_staged) for runs that start after the call.  Each item (utterance) is measured and scaled
+ *                 on its own, on its 24 kHz model waveform x (n samples), before resampling and integer conversion, so
+ *                 it gets the same gain at every "out_rate":
+ *                 1. K-weighting (ITU-R BS.1770-4): two biquads designed in double at fs = 24000 with libebur128's
+ *                    analog parameters and the bilinear transform, K = tan(pi f0 / fs) -- shelf f0 =
+ *                    1681.974450955533 Hz, G = 3.999843853973347 dB, Q = 0.7071752369554196, Vb = Vh^0.4996667741545416;
+ *                    high-pass f0 = 38.13547087602444 Hz, Q = 0.5003270373238773, numerator 1, -2, 1 (at fs = 48000
+ *                    these are the standard's coefficient table); zero state at the item's first sample.
+ *                 2. Blocks of 400 ms (9600 samples) on a 100 ms hop (2400), from sample 0, whole blocks only:
+ *                    z_j = mean square of the K-weighted block, l_j = -0.691 + 10 log10 z_j.
+ *                 3. Gating: absolute gate l_j > -70; relative gate Gamma_r = -0.691 + 10 log10(mean z over the
+ *                    absolute-gated blocks) - 10; L = -0.691 + 10 log10(mean z over blocks with l_j > -70 and
+ *                    l_j > Gamma_r) (strict comparisons).  L is undefined when no block passes: items shorter than
+ *                    400 ms (fewer than 16 frames) and silence.
+ *                 4. True peak tp = max |resample_poly(x, 4, 1)| over the item, with scipy's default filter
+ *                    h = 4 firwin(81, 1/4, ("kaiser", 5.0)) and zeros outside the item; dBTP = 20 log10 tp.  (A
+ *                    deliberate deviation from the 48-tap example filter of the BS.1770 annex: the same design rule
+ *                    as "out_rate", so the measurement is reproducible with scipy alone.)
+ *                 5. Gain g = 10^((target - L) / 20); if tp g > 10^(ceiling / 20) then g = 10^(ceiling / 20) / tp
+ *                    (a static gain: no limiter, no compressor).  Undefined L: g = 1 exactly.
+ *                 6. Each returned sample is fp32(y * g), y being the sample the same run returns with the option off
+ *                    (the iSTFT sample at 24 kHz, the resampling FIR's output at other rates); PCM16, G.711 and FLAC
+ *                    follow from that value by their rules above, so an item with undefined L comes back bit-identical
+ *                    to normalisation off.  The measurement runs in fp32 on the device (the filter restarted from zero
+ *                    state 4800 samples before each 2400-sample segment, sums in double); values and bits of an item
+ *                    do not depend on its batch, frame group or pass.  Not provided: one loudness across several items
+ *                    (program loudness of a request split into chunks), lookahead limiting or compression, measurement
+ *                    at the output rate, momentary / short-term loudness and loudness range, a measure-only mode.
  * kkx_get_stat keys: "launches", "last_frames", "gpu_us", "precision", "coalesced_batches",
  * "coalesced_requests", "coalesced_largest", "async_batches", "async_requests", "frame_groups",
  * "group_first:<g>" (first item of frame group g of the last run), "weights_sessions" (sessions sharing this
- * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate". */
+ * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate", "loudness_target",
+ * "true_peak_max", "loudness_items" (items kkx_last_loudness reports now; 0 if it would fail with KKX_ERR_STATE). */
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value);
 KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "last_frames", "gpu_us" ... */
+
+/* What loudness normalisation measured and applied in the last SYNCHRONOUS call on the ctx (kkx_infer without
+ * "coalesce", kkx_infer_batch and its _voices / _pcm16 / _g711 / _flac forms, kkx_run_staged), in item order, over
+ * every pass of a "max_tokens" split.  Per item: lufs = integrated loudness L (NaN when undefined), true_peak_dbtp =
+ * 20 log10 tp of the unscaled item (-inf for silence), gain = the applied g.  Each pointer is nullable and receives
+ * `batch` floats.  KKX_ERR_STATE if no synchronous call has completed or that call ran with "loudness_target" = 0;
+ * KKX_ERR_ARG if `batch` is not that call's item count.  Coalesced callers and kkx_submit batches are normalised
+ * but not reported here (a batch of several callers has no per-caller report). */
+KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* true_peak_dbtp, float* gain);
 
 /* Per-kernel device timing of the last run (CUDA events on the library's stream, one after every
  * launch).  kkx_profile_json writes {"conv_flops": F, "gpu_us": T, "kernels": {name: [launches,

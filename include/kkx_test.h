@@ -130,6 +130,17 @@ KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64
  * and their offsets into byte_offsets [B + 1]; returns the total byte count or < 0. */
 KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
                               uint8_t* dst, int64_t capacity, int64_t* byte_offsets);
+/* Loudness normalisation (kernels_loudness.cu, kkx.h "loudness_target").
+ * kkx_test_loudness_design: host only -- the K-weighting biquads the library designs in double for sample rate fs
+ *   (kweight[10], nullable: shelf b0 b1 b2 a1 a2, then high-pass b0 b1 b2 a1 a2; a0 = 1) and the fp32 taps of the
+ *   true-peak filter (4 * firwin(81, 1/4, ("kaiser", 5.0)), at most `capacity` to tp_taps, nullable); returns the tap
+ *   count.  The library itself measures at 24 kHz only.
+ * kkx_test_loudness: B items packed back to back in x (item b has lens[b] >= 1 samples at 24 kHz) -> per item the
+ *   integrated loudness (LUFS, NaN = undefined), the true peak (dBTP) and the gain for the given target (1/100 LUFS)
+ *   and ceiling (1/100 dBTP); each output nullable.  The same three launches the model runs per frame group. */
+KKX_API int64_t kkx_test_loudness_design(double fs, double* kweight, float* tp_taps, int64_t capacity);
+KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
+                              int32_t ceiling_centi_dbtp, float* lufs, float* true_peak_dbtp, float* gain);
 KKX_API const char* kkx_test_last_error(void);
 
 #ifdef __cplusplus

@@ -63,6 +63,11 @@ struct kkx_ctx {
   int64_t next_ticket = 1;
   std::atomic<int> async_batch{64};      // most requests the worker merges into one ragged batch
   int64_t async_batches = 0, async_requests = 0;
+
+  // Loudness report of the last synchronous call (kkx_last_loudness), guarded by `mu`: 3 floats per item (LUFS, dBTP,
+  // gain), appended pass by pass; valid once the call has succeeded, `normalised` if its runs had the option on.
+  std::vector<float> loud;
+  bool loud_valid = false, loud_normalised = false;
 };
 
 static thread_local std::string g_err;
@@ -228,6 +233,17 @@ static void hand_out(kkx_ctx* ctx, float* host, size_t cap) {
 
 KKX_API void kkx_release(kkx_ctx* ctx, float* audio);
 
+// kkx_last_loudness bookkeeping of a synchronous call (caller holds ctx->mu): begin, one note per model run, done.
+// Coalesced and asynchronous batches leave the report alone.
+static void loud_begin(kkx_ctx* ctx) { ctx->loud.clear(); ctx->loud_valid = false; ctx->loud_normalised = false; }
+static void loud_note(kkx_ctx* ctx) {
+  const Model& m = *ctx->model;
+  if (!m.loudness_ran()) return;
+  ctx->loud_normalised = true;
+  ctx->loud.insert(ctx->loud.end(), m.last_loudness().begin(), m.last_loudness().end());
+}
+static void loud_done(kkx_ctx* ctx) { ctx->loud_valid = true; }
+
 // The argument contract of one utterance (kkx.h): checked before a request is queued anywhere.
 static int validate_request(const int64_t* tokens, int32_t n_tokens, const float* style256, float speed) {
   if (!tokens || !style256) { g_err = "null argument"; return KKX_ERR_ARG; }
@@ -277,12 +293,13 @@ static void recycle_pinned(kkx_ctx* ctx, float* host, size_t cap) {
 // apart from one host-side concatenation.
 static void run_batch_locked(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                              const float* styles, const float* speeds, float** host_out, size_t* cap_out,
-                             int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+                             int64_t* out_sample_offsets, int32_t* out_pred_dur, bool report = false) {
   if (batch <= 0 || !tok_offsets) throw ArgError("batch must be >= 1");
   const long long budget = ctx->max_tokens;
   if (batch == 1 || (long long)tok_offsets[batch] - tok_offsets[0] <= budget) {
     ctx->model->stage(batch, tokens, tok_offsets, styles, speeds);
     run_staged_locked(ctx, host_out, cap_out, out_sample_offsets, out_pred_dur);
+    if (report) loud_note(ctx);
     return;
   }
   if (!styles) throw ArgError("null input pointer");
@@ -299,6 +316,7 @@ static void run_batch_locked(kkx_ctx* ctx, int32_t batch, const int64_t* tokens,
       run_staged_locked(ctx, &p.host, &p.cap, so.data(),
                         out_pred_dur ? out_pred_dur + (tok_offsets[b0] - tok_offsets[0]) : nullptr);
       parts.push_back(p);
+      if (report) loud_note(ctx);
       for (int i = 0; i < b1 - b0; i++) soff[b0 + i + 1] = soff[b0] + so[i + 1];
       b0 = b1;
     }
@@ -327,7 +345,10 @@ KKX_API int kkx_infer_batch(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, 
     if (!out_audio) throw ArgError("out_audio is null");
     float* host = nullptr;
     size_t cap = 0;
-    run_batch_locked(ctx, batch, tokens, tok_offsets, styles, speeds, &host, &cap, out_sample_offsets, out_pred_dur);
+    loud_begin(ctx);
+    run_batch_locked(ctx, batch, tokens, tok_offsets, styles, speeds, &host, &cap, out_sample_offsets, out_pred_dur,
+                     true);
+    loud_done(ctx);
     hand_out(ctx, host, cap);
     *out_audio = host;
   });
@@ -455,7 +476,10 @@ KKX_API int kkx_infer_batch_voices(kkx_ctx* ctx, int32_t batch, const int64_t* t
     m.stage_voices(batch, tokens, tok_offsets, mix_offsets, voice_ids, voice_portions, style_rows, speeds);
     float* host = nullptr;
     size_t cap = 0;
+    loud_begin(ctx);
     run_staged_locked(ctx, &host, &cap, out_sample_offsets, out_pred_dur);
+    loud_note(ctx);
+    loud_done(ctx);
     hand_out(ctx, host, cap);
     *out_audio = host;
   });
@@ -472,9 +496,11 @@ KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* to
     if (!out_pcm) throw ArgError("out_pcm is null");
     Model& m = *ctx->model;
     m.stage(batch, tokens, tok_offsets, styles, speeds);
+    loud_begin(ctx);
     m.set_pcm16(true);
     try { m.run(); } catch (...) { m.set_pcm16(false); throw; }
     m.set_pcm16(false);
+    loud_note(ctx);
     const long long n = m.total_samples();
     size_t cap = 0;
     float* host = take_pinned(ctx, (size_t)(n + 1) / 2, &cap);   // n int16 = n/2 floats of the same pool
@@ -482,6 +508,7 @@ KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* to
       m.fetch_pcm16(reinterpret_cast<short*>(host), n, out_sample_offsets, out_pred_dur);
     } catch (...) { cudaFreeHost(host); throw; }
     hand_out(ctx, host, cap);
+    loud_done(ctx);
     *out_pcm = reinterpret_cast<int16_t*>(host);
   });
 }
@@ -500,9 +527,11 @@ KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tok
     if (law != 0 && law != 1) throw ArgError("law must be 0 (mu-law) or 1 (A-law), got " + std::to_string(law));
     Model& m = *ctx->model;
     m.stage(batch, tokens, tok_offsets, styles, speeds);
+    loud_begin(ctx);
     m.set_g711(law);
     try { m.run(); } catch (...) { m.set_g711(-1); throw; }
     m.set_g711(-1);
+    loud_note(ctx);
     const long long n = m.total_samples();
     size_t cap = 0;
     float* host = take_pinned(ctx, (size_t)(n + 3) / 4, &cap);   // n one-byte codes = n/4 floats of the same pool
@@ -510,6 +539,7 @@ KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tok
       m.fetch_g711(reinterpret_cast<unsigned char*>(host), n, out_sample_offsets, out_pred_dur);
     } catch (...) { cudaFreeHost(host); throw; }
     hand_out(ctx, host, cap);
+    loud_done(ctx);
     *out_codes = reinterpret_cast<uint8_t*>(host);
   });
 }
@@ -528,9 +558,11 @@ KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tok
     if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
     Model& m = *ctx->model;
     m.stage(batch, tokens, tok_offsets, styles, speeds);
+    loud_begin(ctx);
     m.set_pcm16(true);
     try { m.run(); } catch (...) { m.set_pcm16(false); throw; }
     m.set_pcm16(false);
+    loud_note(ctx);
     m.encode_flac();
     const long long n = m.flac_bytes();
     size_t cap = 0;
@@ -539,6 +571,7 @@ KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tok
       m.fetch_flac(reinterpret_cast<unsigned char*>(host), n, out_byte_offsets, out_sample_offsets, out_pred_dur);
     } catch (...) { cudaFreeHost(host); throw; }
     hand_out(ctx, host, cap);
+    loud_done(ctx);
     *out_bytes = reinterpret_cast<uint8_t*>(host);
   });
 }
@@ -768,7 +801,10 @@ KKX_API int kkx_run_staged(kkx_ctx* ctx, int64_t* out_total_samples, int64_t* ou
   if (rc) return rc;
   std::lock_guard<std::mutex> lk(ctx->mu);
   return guarded(ctx, [&] {
+    loud_begin(ctx);
     ctx->model->run();
+    loud_note(ctx);
+    loud_done(ctx);
     if (out_total_samples) *out_total_samples = ctx->model->total_samples();
     if (out_launches) *out_launches = ctx->model->stats.launches;
   });
@@ -826,6 +862,15 @@ KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
                        "32000, 44100, 48000)");
       }
       o.out_rate = (int)value;
+    } else if (k == "loudness_target") {
+      if (value != 0 && (value < -7000 || value > -500))
+        throw ArgError("loudness_target " + std::to_string(value) +
+                       " is not supported: give 1/100 LUFS in -7000..-500 (e.g. -2300 for -23 LUFS), or 0 for off");
+      o.loudness_target = (int)value;
+    } else if (k == "true_peak_max") {
+      if (value < -2000 || value > 0)
+        throw ArgError("true_peak_max " + std::to_string(value) + " is not supported: give 1/100 dBTP in -2000..0");
+      o.true_peak_max = (int)value;
     }
     else throw ArgError("unknown option: " + k);
   });
@@ -840,6 +885,9 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   if (k == "gpu_us") return (int64_t)ctx->model->last_gpu_us;
   if (k == "precision") return ctx->model->opt.precision;
   if (k == "out_rate") return ctx->model->opt.out_rate;
+  if (k == "loudness_target") return ctx->model->opt.loudness_target;
+  if (k == "true_peak_max") return ctx->model->opt.true_peak_max;
+  if (k == "loudness_items") return ctx->loud_valid && ctx->loud_normalised ? (int64_t)(ctx->loud.size() / 3) : 0;
   if (k == "coalesced_batches") return ctx->coalesced_batches;
   if (k == "coalesced_requests") return ctx->coalesced_requests;
   if (k == "coalesced_largest") return ctx->coalesced_largest;
@@ -859,6 +907,24 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
     if (k == "async_requests") return ctx->async_requests;
   }
   return -1;
+}
+
+KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* true_peak_dbtp, float* gain) {
+  int rc = check_ctx(ctx);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(ctx, [&] {
+    if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
+    if (!ctx->loud_normalised) throw StateError("the last synchronous call ran with loudness normalisation off");
+    const int64_t n = (int64_t)(ctx->loud.size() / 3);
+    if (batch != n)
+      throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
+    for (int64_t b = 0; b < n; b++) {
+      if (lufs) lufs[b] = ctx->loud[b * 3];
+      if (true_peak_dbtp) true_peak_dbtp[b] = ctx->loud[b * 3 + 1];
+      if (gain) gain[b] = ctx->loud[b * 3 + 2];
+    }
+  });
 }
 
 KKX_API int kkx_profile_enable(kkx_ctx* ctx, int enable) {

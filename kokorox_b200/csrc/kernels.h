@@ -278,12 +278,37 @@ void launch_istft(const float* cp, int ldc, const int* h_off, const int* h_len, 
 //   launch_resample: item b reads x[in_off[b] .. + in_len[b]) and writes ceil(in_len[b] U / D) samples at out_off[b]
 //                    as f32 and optionally as 16-bit PCM (trunc(clamp(y, -1, 1) * 32767)) and / or G.711 codes of that
 //                    PCM value (law 0 = mu-law, 1 = A-law); U = D = 1 with H = 0 is a pass-through (no taps).
-//                    max_out = largest per-item output length.  Profile name "resample".
+//                    max_out = largest per-item output length.  gain (nullable): every output y of item b is
+//                    fp32(y * gain[b]) (loudness normalisation); null leaves the arithmetic as it is.
+//                    Profile name "resample".
+//   poly_design:     the taps of resample_poly(x, u, d) for any u / d (the true-peak filter uses 4 / 1).
 bool resample_ratio(int out_rate, int* U, int* D);
 int resample_design(int out_rate, std::vector<float>* taps, int* U, int* D, int* H);
+int poly_design(int u, int d, std::vector<float>* taps);
 void launch_resample(const float* x, const long long* in_off, const long long* in_len, const long long* out_off,
-                     const float* taps, int U, int D, int H, float* out, short* pcm /*nullable*/,
-                     unsigned char* codes /*nullable*/, int law, int B, long long max_out, cudaStream_t st);
+                     const float* taps, int U, int D, int H, const float* gain /*nullable*/, float* out,
+                     short* pcm /*nullable*/, unsigned char* codes /*nullable*/, int law, int B, long long max_out,
+                     cudaStream_t st);
+
+// Loudness normalisation (kernels_loudness.cu, K14): ITU-R BS.1770 integrated loudness of each item's 24 kHz waveform
+// with a true-peak ceiling (kkx.h "loudness_target").
+//   loudness_design: the K-weighting biquads at fs in double (shelf b0 b1 b2 a1 a2, then high-pass b0 b1 b2 a1 a2)
+//                    and, if tp_taps is given, the 81 taps of resample_poly(x, 4, 1).
+//   LoudParams:      everything the kernels read, passed by value (fp32 biquads, the 4x taps, target and ceiling).
+//   launch_loudness: item b = x[in_off[b] .. + in_len[b]); writes lufs[b] (NaN = undefined), tp_db[b] (dBTP) and
+//                    gain[b].  energy: scratch of in_len[b] / 2400 floats per item at seg_off[b]; peak: [B] scratch.
+//                    Three launches: "loud_energy", "loud_peak", "loud_gain".
+constexpr int kLoudSeg = 2400, kLoudWarm = 4800, kTpTaps = 81;
+struct LoudParams {
+  float kw[10];
+  float tp[kTpTaps];
+  double target_lufs, ceiling_dbtp;
+};
+void loudness_design(double fs, double kw[10], std::vector<float>* tp_taps);
+LoudParams loudness_params(double target_lufs, double ceiling_dbtp);
+void launch_loudness(const float* x, const long long* in_off, const long long* in_len, const long long* seg_off,
+                     const LoudParams& P, float* energy, unsigned* peak, float* lufs, float* tp_db, float* gain, int B,
+                     long long max_len, cudaStream_t st);
 
 // Lossless FLAC of 16-bit mono PCM (kernels_flac.cu; the bitstream rules are in kkx.h, kkx_infer_batch_flac).
 //   Item b is pcm[soff[b] .. soff[b + 1]) (>= 1 sample) and has flac_frames(n_b) frames of 4096 samples; foff[b + 1]

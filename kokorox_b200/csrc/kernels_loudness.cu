@@ -1,0 +1,236 @@
+// kernels_loudness.cu -- loudness normalisation (K14): ITU-R BS.1770 integrated loudness of each utterance's 24 kHz
+// waveform, its true peak, and the static gain that brings it to the session's target under a true-peak ceiling
+// (kkx.h "loudness_target" / "true_peak_max").  The gain itself is applied by resample_kernel (kernels_signal.cu).
+//
+// Per item (n samples x at 24 kHz):
+//   loud_energy  one thread per 2400-sample segment s (the 100 ms hop): the K-weighting cascade (shelf, then
+//                high-pass) runs from zero state over x[max(0, 2400 s - 4800), 2400 (s + 1)) and the sum of squares of
+//                its last 2400 outputs is the segment's energy.  The slowest pole has radius 0.99007, so after 4800
+//                samples the dropped history weighs 0.99007^4800 ~ 1e-21: the value is the one the filter would have
+//                run serially from the item's first sample, to fp32 rounding.  A serial filter over a 510-token item
+//                (~7e5 samples) would be one long dependency chain; here it is n / 2400 chains of 7200 steps.
+//   loud_peak    the 4x polyphase FIR of resample_poly(x, 4, 1) (scipy's default Kaiser filter, zeros outside the
+//                item), one input position (4 outputs) per thread; max |y| of the item through an integer atomicMax on
+//                the float's bits (non-negative floats order like their bit patterns: exact and order-independent).
+//   loud_gain    one CTA per item: block j (400 ms = segments j .. j + 3) has z_j = sum of its 4 energies / 9600,
+//                l_j = -0.691 + 10 log10 z_j; the absolute gate (l_j > -70) and the relative gate (l_j > Gamma_r)
+//                follow BS.1770-4; sums in double in a fixed order; L, dBTP and the gain are written per item.
+// Every value is a function of the item's samples alone: an item gets the same bits in any batch, frame group or pass.
+#include "kernels.h"
+#include <math.h>
+#include <cmath>
+#include <vector>
+
+namespace kkx {
+
+// K-weighting as libebur128 designs it (analog prototypes through the bilinear transform, K = tan(pi f0 / fs)); at
+// fs = 48000 these are the BS.1770-4 table's coefficients.
+void loudness_design(double fs, double kw[10], std::vector<float>* tp_taps) {
+  {   // stage 1: high shelf
+    const double f0 = 1681.974450955533, G = 3.999843853973347, Q = 0.7071752369554196;
+    const double K = std::tan(M_PI * f0 / fs);
+    const double Vh = std::pow(10.0, G / 20.0), Vb = std::pow(Vh, 0.4996667741545416);
+    const double a0 = 1.0 + K / Q + K * K;
+    kw[0] = (Vh + Vb * K / Q + K * K) / a0;
+    kw[1] = 2.0 * (K * K - Vh) / a0;
+    kw[2] = (Vh - Vb * K / Q + K * K) / a0;
+    kw[3] = 2.0 * (K * K - 1.0) / a0;
+    kw[4] = (1.0 - K / Q + K * K) / a0;
+  }
+  {   // stage 2: high-pass (RLB); numerator 1, -2, 1 as in the standard's table
+    const double f0 = 38.13547087602444, Q = 0.5003270373238773;
+    const double K = std::tan(M_PI * f0 / fs);
+    const double a0 = 1.0 + K / Q + K * K;
+    kw[5] = 1.0; kw[6] = -2.0; kw[7] = 1.0;
+    kw[8] = 2.0 * (K * K - 1.0) / a0;
+    kw[9] = (1.0 - K / Q + K * K) / a0;
+  }
+  if (tp_taps) poly_design(4, 1, tp_taps);   // 4 * firwin(81, 1/4, ("kaiser", 5.0))
+}
+
+LoudParams loudness_params(double target_lufs, double ceiling_dbtp) {
+  LoudParams P{};
+  double kw[10];
+  std::vector<float> taps;
+  loudness_design(24000.0, kw, &taps);
+  if ((int)taps.size() != kTpTaps) throw ArgError("loudness: unexpected true-peak filter length");
+  for (int i = 0; i < 10; i++) P.kw[i] = (float)kw[i];
+  for (int i = 0; i < kTpTaps; i++) P.tp[i] = taps[i];
+  P.target_lufs = target_lufs;
+  P.ceiling_dbtp = ceiling_dbtp;
+  return P;
+}
+
+// ------------------------------------------------------------------------------------------ segment energies
+constexpr int kLeThreads = 128;
+
+// one K-weighting step (transposed direct form II, fp32 FMA in a fixed order); returns the high-pass output
+__device__ __forceinline__ float kweight_step(const LoudParams& P, float x, float& s1, float& s2, float& t1, float& t2) {
+  const float u = fmaf(P.kw[0], x, s1);
+  s1 = fmaf(P.kw[1], x, fmaf(-P.kw[3], u, s2));
+  s2 = fmaf(P.kw[2], x, -P.kw[4] * u);
+  const float y = fmaf(P.kw[5], u, t1);
+  t1 = fmaf(P.kw[6], u, fmaf(-P.kw[8], y, t2));
+  t2 = fmaf(P.kw[7], u, -P.kw[9] * y);
+  return y;
+}
+
+__global__ void __launch_bounds__(kLeThreads) loud_energy_kernel(const float* __restrict__ x,
+                                                                 const long long* __restrict__ in_off,
+                                                                 const long long* __restrict__ in_len,
+                                                                 const long long* __restrict__ seg_off, LoudParams P,
+                                                                 float* __restrict__ energy, unsigned* __restrict__ peak) {
+  const int b = blockIdx.y;
+  if (blockIdx.x == 0 && threadIdx.x == 0) peak[b] = 0u;   // loud_peak (the next launch) accumulates into it
+  const long long nseg = in_len[b] / kLoudSeg;
+  const long long s = (long long)blockIdx.x * kLeThreads + threadIdx.x;
+  if (s >= nseg) return;
+  const float* xb = x + in_off[b];
+  const long long e0 = s * kLoudSeg;
+  const long long start = e0 > kLoudWarm ? e0 - kLoudWarm : 0;
+  float s1 = 0.f, s2 = 0.f, t1 = 0.f, t2 = 0.f;
+  for (long long i = start; i < e0; i += 8) {   // warm-up: state only (lengths are multiples of 2400)
+    float v[8];
+#pragma unroll
+    for (int k = 0; k < 8; k++) v[k] = __ldg(xb + i + k);
+#pragma unroll
+    for (int k = 0; k < 8; k++) kweight_step(P, v[k], s1, s2, t1, t2);
+  }
+  float acc = 0.f;
+  for (long long i = e0; i < e0 + kLoudSeg; i += 8) {
+    float v[8];
+#pragma unroll
+    for (int k = 0; k < 8; k++) v[k] = __ldg(xb + i + k);
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+      const float y = kweight_step(P, v[k], s1, s2, t1, t2);
+      acc = fmaf(y, y, acc);
+    }
+  }
+  energy[seg_off[b] + s] = acc;
+}
+
+// ------------------------------------------------------------------------------------------ true peak
+// y[4q + p] = sum over k of x[k] h[4 (q - k) + p + 40], 0 <= 4 (q - k) + p + 40 <= 80: inputs q - 10 .. q + 10.
+constexpr int kTpThreads = 256, kTpPer = 4, kTpTile = kTpThreads * kTpPer, kTpHalo = 10;
+
+__global__ void __launch_bounds__(kTpThreads) loud_peak_kernel(const float* __restrict__ x,
+                                                               const long long* __restrict__ in_off,
+                                                               const long long* __restrict__ in_len, LoudParams P,
+                                                               unsigned* __restrict__ peak) {
+  __shared__ float s_x[kTpTile + 2 * kTpHalo];
+  const int b = blockIdx.y, t = threadIdx.x;
+  const long long n = in_len[b];
+  const long long q0 = (long long)blockIdx.x * kTpTile;
+  if (q0 >= n) return;
+  const float* xb = x + in_off[b];
+  for (int i = t; i < kTpTile + 2 * kTpHalo; i += kTpThreads) {
+    const long long k = q0 - kTpHalo + i;
+    s_x[i] = (k >= 0 && k < n) ? __ldg(xb + k) : 0.f;
+  }
+  __syncthreads();
+  float m = 0.f;
+#pragma unroll
+  for (int i = 0; i < kTpPer; i++) {
+    const int r = t + i * kTpThreads;
+    if (q0 + r >= n) break;
+    const float* w = s_x + r + kTpHalo;   // w[d] = x[q + d]
+#pragma unroll
+    for (int p = 0; p < 4; p++) {
+      float acc = 0.f;
+#pragma unroll
+      for (int d = -kTpHalo; d <= kTpHalo; d++) {   // k = q + d ascending: tap 40 + p - 4 d
+        const int j = 40 + p - 4 * d;
+        if (j >= 0 && j < kTpTaps) acc = fmaf(w[d], P.tp[j], acc);
+      }
+      m = fmaxf(m, fabsf(acc));
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((t & 31) == 0 && m > 0.f) atomicMax(peak + b, __float_as_uint(m));
+}
+
+// ------------------------------------------------------------------------------------------ gating and gain
+constexpr int kLgThreads = 256;
+
+template <class T>
+__device__ T block_sum(T v, T* red) {   // fixed-shape tree: the result depends on the thread values alone
+  const int t = threadIdx.x;
+  __syncthreads();
+  red[t] = v;
+  __syncthreads();
+  for (int h = kLgThreads / 2; h > 0; h >>= 1) {
+    if (t < h) red[t] += red[t + h];
+    __syncthreads();
+  }
+  return red[0];
+}
+
+__global__ void __launch_bounds__(kLgThreads) loud_gain_kernel(const long long* __restrict__ in_len,
+                                                               const long long* __restrict__ seg_off,
+                                                               const float* __restrict__ energy,
+                                                               const unsigned* __restrict__ peak, LoudParams P,
+                                                               float* __restrict__ lufs, float* __restrict__ tp_db,
+                                                               float* __restrict__ gain) {
+  __shared__ double red_d[kLgThreads];
+  __shared__ long long red_n[kLgThreads];
+  const int b = blockIdx.x, t = threadIdx.x;
+  const long long nblk = in_len[b] / kLoudSeg - 3;          // whole 400 ms blocks (<= 0: none)
+  const float* e = energy + seg_off[b];
+  auto level = [&](long long j, double* z) {
+    *z = ((double)e[j] + (double)e[j + 1] + (double)e[j + 2] + (double)e[j + 3]) / (4.0 * kLoudSeg);
+    return -0.691 + 10.0 * log10(*z);                       // z = 0: -inf, gated out
+  };
+  double s = 0.0;
+  long long c = 0;
+  for (long long j = t; j < nblk; j += kLgThreads) {
+    double z;
+    if (level(j, &z) > -70.0) { s += z; c++; }
+  }
+  const double s1 = block_sum(s, red_d);
+  const long long c1 = block_sum(c, red_n);
+  double L = NAN;
+  if (c1 > 0) {
+    const double rel = -0.691 + 10.0 * log10(s1 / (double)c1) - 10.0;
+    s = 0.0; c = 0;
+    for (long long j = t; j < nblk; j += kLgThreads) {
+      double z;
+      const double l = level(j, &z);
+      if (l > -70.0 && l > rel) { s += z; c++; }
+    }
+    const double s2 = block_sum(s, red_d);
+    const long long c2 = block_sum(c, red_n);
+    if (c2 > 0) L = -0.691 + 10.0 * log10(s2 / (double)c2);
+  }
+  if (t != 0) return;
+  const float tp = __uint_as_float(peak[b]);
+  double g = 1.0;
+  if (!isnan(L)) {
+    g = pow(10.0, (P.target_lufs - L) / 20.0);
+    const double cap = pow(10.0, P.ceiling_dbtp / 20.0);
+    if ((double)tp * g > cap) g = cap / (double)tp;
+  }
+  lufs[b] = (float)L;
+  tp_db[b] = (float)(20.0 * log10((double)tp));
+  gain[b] = (float)g;
+}
+
+void launch_loudness(const float* x, const long long* in_off, const long long* in_len, const long long* seg_off,
+                     const LoudParams& P, float* energy, unsigned* peak, float* lufs, float* tp_db, float* gain, int B,
+                     long long max_len, cudaStream_t st) {
+  if (g_dry_run) return;
+  if (B < 1 || B > 65535) throw ArgError("launch_loudness: batch out of range");
+  const long long max_seg = max_len / kLoudSeg;
+  const long long ge = std::max(1LL, (max_seg + kLeThreads - 1) / kLeThreads);
+  const long long gp = std::max(1LL, (max_len + kTpTile - 1) / kTpTile);
+  if (gp > 0x7FFFFFFFLL) throw ArgError("launch_loudness: grid too large");
+  loud_energy_kernel<<<dim3((unsigned)ge, B), kLeThreads, 0, st>>>(x, in_off, in_len, seg_off, P, energy, peak);
+  post_launch("loud_energy", st);
+  loud_peak_kernel<<<dim3((unsigned)gp, B), kTpThreads, 0, st>>>(x, in_off, in_len, P, peak);
+  post_launch("loud_peak", st);
+  loud_gain_kernel<<<B, kLgThreads, 0, st>>>(in_len, seg_off, energy, peak, P, lufs, tp_db, gain);
+  post_launch("loud_gain", st);
+}
+
+}  // namespace kkx

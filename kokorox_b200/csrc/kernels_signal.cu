@@ -861,6 +861,13 @@ int resample_design(int out_rate, std::vector<float>* taps, int* U, int* D, int*
     if (H) *H = 0;
     return 1;
   }
+  if (U) *U = u;
+  if (D) *D = d;
+  if (H) *H = 10 * std::max(u, d);
+  return poly_design(u, d, taps);
+}
+
+int poly_design(int u, int d, std::vector<float>* taps) {
   const int half = 10 * std::max(u, d), n = 2 * half + 1;
   // U * firwin(2H + 1, 1 / max(U, D), window = ("kaiser", 5.0)), in double: windowed sinc, normalised to unit DC gain
   const double fc = 1.0 / std::max(u, d), beta = 5.0, i0b = bessel_i0(beta);
@@ -877,9 +884,6 @@ int resample_design(int out_rate, std::vector<float>* taps, int* U, int* D, int*
     taps->resize(n);
     for (int i = 0; i < n; i++) (*taps)[i] = (float)(u * (h[i] / sum));
   }
-  if (U) *U = u;
-  if (D) *D = d;
-  if (H) *H = half;
   return n;
 }
 
@@ -907,7 +911,8 @@ __device__ __forceinline__ unsigned char g711_alaw(int p) {
 // input span its tile reads (zero outside the item) and all 2H + 1 taps in shared memory with coalesced loads.  Each
 // output sample is a function of its item alone, so results do not depend on the batch around it.  Output offsets
 // need not be multiples of 4 (at 11025 / 22050 / 44100 Hz they are not): every store is a scalar, coalesced across
-// the warp.  PASS: U = D = 1 without a filter (the G.711 codes of the 24 kHz waveform itself).
+// the warp.  PASS: U = D = 1 without a filter (the G.711 codes of the 24 kHz waveform itself).  gain (nullable): y of
+// item b becomes fp32(y * gain[b]) before any output is written; without it the arithmetic is the plain filter's.
 constexpr int kRsThreads = 256, kRsPer = 8, kRsTile = kRsThreads * kRsPer;
 __host__ __device__ inline long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 
@@ -916,6 +921,7 @@ __global__ void __launch_bounds__(kRsThreads) resample_kernel(const float* __res
                                                               const long long* __restrict__ in_len,
                                                               const long long* __restrict__ out_off,
                                                               const float* __restrict__ taps, int U, int D, int H,
+                                                              const float* __restrict__ gain,
                                                               float* __restrict__ out, short* __restrict__ pcm,
                                                               unsigned char* __restrict__ codes, int law) {
   extern __shared__ float rs_smem[];
@@ -965,6 +971,11 @@ __global__ void __launch_bounds__(kRsThreads) resample_kernel(const float* __res
       y[i] = acc;
     }
   }
+  if (gain) {   // loudness normalisation: fp32(y * g), one gain per item (kernels_loudness.cu)
+    const float g = gain[b];
+#pragma unroll
+    for (int i = 0; i < kRsPer; i++) y[i] = __fmul_rn(y[i], g);
+  }
 #pragma unroll
   for (int i = 0; i < kRsPer; i++) {
     const long long m = m0 + t + i * kRsThreads;
@@ -985,8 +996,8 @@ size_t resample_smem_bytes(int U, int D, int H) {
 }
 
 void launch_resample(const float* x, const long long* in_off, const long long* in_len, const long long* out_off,
-                     const float* taps, int U, int D, int H, float* out, short* pcm, unsigned char* codes, int law,
-                     int B, long long max_out, cudaStream_t st) {
+                     const float* taps, int U, int D, int H, const float* gain, float* out, short* pcm,
+                     unsigned char* codes, int law, int B, long long max_out, cudaStream_t st) {
   if (g_dry_run) return;
   const bool pass = U == 1 && D == 1 && H == 0;
   if (!pass && !taps) throw ArgError("launch_resample: filter taps missing");
@@ -998,9 +1009,11 @@ void launch_resample(const float* x, const long long* in_off, const long long* i
   if (smem > 48 * 1024) throw ArgError("launch_resample: filter too long for one CTA");
   dim3 g((unsigned)tiles, B);
   if (pass)
-    resample_kernel<true><<<g, kRsThreads, 0, st>>>(x, in_off, in_len, out_off, nullptr, 1, 1, 0, out, pcm, codes, law);
+    resample_kernel<true><<<g, kRsThreads, 0, st>>>(x, in_off, in_len, out_off, nullptr, 1, 1, 0, gain, out, pcm, codes,
+                                                    law);
   else
-    resample_kernel<false><<<g, kRsThreads, smem, st>>>(x, in_off, in_len, out_off, taps, U, D, H, out, pcm, codes, law);
+    resample_kernel<false><<<g, kRsThreads, smem, st>>>(x, in_off, in_len, out_off, taps, U, D, H, gain, out, pcm, codes,
+                                                        law);
   post_launch("resample", st);
 }
 

@@ -176,6 +176,7 @@ Model::~Model() {
   if (d_flac_) cudaFree(d_flac_);
   if (d_flac_meta_) cudaFree(d_flac_meta_);
   if (d_taps_) cudaFree(d_taps_);
+  if (d_loud_) cudaFree(d_loud_);
   if (d_voices_) cudaFree(d_voices_);
   if (d_noise_) cudaFree(d_noise_);
   if (h_pred_dur_) cudaFreeHost(h_pred_dur_);
@@ -870,10 +871,13 @@ void Model::fetch_flac(unsigned char* dst, long long capacity, int64_t* byte_off
   }
 }
 
-// The resampling pass of this run: off at 24 kHz unless G.711 codes are wanted (then a pass-through, U = D = 1).  The
-// taps live on the device per Model and are rebuilt only when the rate changes.
+// The resampling pass of this run: off at 24 kHz unless G.711 codes or loudness normalisation are wanted (then a
+// pass-through, U = D = 1, which applies the gain).  The taps live on the device per Model and are rebuilt only when
+// the rate changes.
 void Model::prepare_resample() {
-  resample_ = opt.out_rate != 24000 || want_law_ >= 0;
+  loud_ = opt.loudness_target != 0;
+  if (loud_) loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0);
+  resample_ = opt.out_rate != 24000 || want_law_ >= 0 || loud_;
   rs_U_ = 1; rs_D_ = 1; rs_H_ = 0;
   if (opt.out_rate == 24000) return;
   std::vector<float> taps;
@@ -976,6 +980,14 @@ void Model::run() {
     KKX_CUDA(cudaMalloc(&d_g711_, cap));
     g711_cap_ = cap;
   }
+  if (loud_ && (size_t)B_ * 3 > loud_cap_) {
+    KKX_CUDA(cudaStreamSynchronize(stream_));
+    if (d_loud_) cudaFree(d_loud_);
+    d_loud_ = nullptr; loud_cap_ = 0;
+    KKX_CUDA(cudaMalloc(&d_loud_, (size_t)B_ * 3 * sizeof(float)));
+    loud_cap_ = (size_t)B_ * 3;
+  }
+  h_loud_.clear();
   pcm_valid_ = want_pcm_;
   g711_valid_ = want_law_ >= 0;
   sink_filled_ = false;
@@ -1020,6 +1032,13 @@ void Model::run() {
     KKX_CUDA(cudaEventRecord(ev1_, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
     if (sink) { KKX_CUDA(cudaStreamSynchronize(copy_stream_)); sink_filled_ = true; }
+    if (loud_) {   // [3][B] on the device -> item-major on the host
+      std::vector<float> rows((size_t)B_ * 3);
+      KKX_CUDA(cudaMemcpy(rows.data(), d_loud_, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
+      h_loud_.resize(rows.size());
+      for (int b = 0; b < B_; b++)
+        for (int k = 0; k < 3; k++) h_loud_[(size_t)b * 3 + k] = rows[(size_t)k * B_ + b];
+    }
   } catch (...) {
     cudaStreamSynchronize(stream_);
     cudaStreamSynchronize(stream2_);

@@ -170,6 +170,10 @@ struct Options {
   int lstm_fast_gates = 1;
   // sample rate of every waveform a run returns (kkx.h "out_rate"); 24000 = the model's own rate, no resampling
   int out_rate = 24000;
+  // loudness normalisation (kkx.h): integrated-loudness target in 1/100 LUFS (0 = off) and true-peak ceiling in
+  // 1/100 dBTP
+  int loudness_target = 0;
+  int true_peak_max = -100;
 };
 
 // Device-resident weights of one checkpoint on one GPU: every layout the kernels read (fp32 SIMT, bf16 / split-TF32
@@ -234,6 +238,10 @@ class Model {
   void run();
   long long total_samples() const { return total_samples_; }
   void fetch(float* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
+  // Loudness of the last run's items (kernels_loudness.cu): true if that run normalised; then last_loudness() holds
+  // 3 B floats, per item b at 3 b: integrated loudness (LUFS, NaN = undefined), true peak (dBTP), applied gain.
+  bool loudness_ran() const { return ran_ && loud_; }
+  const std::vector<float>& last_loudness() const { return h_loud_; }
 
   void set_noise(const float* noise, long long n);
   void set_inject(const std::string& name, int item, const void* data, long long count);
@@ -366,6 +374,11 @@ class Model {
   bool resample_ = false; int rs_U_ = 1, rs_D_ = 1, rs_H_ = 0;
   float* d_taps_ = nullptr; int taps_rate_ = 0;
   void prepare_resample();
+  // loudness normalisation of the current run: d_loud_ = [3][B_] floats (lufs | dBTP | gain), h_loud_ its host copy
+  // (item-major); the gain row feeds the resampling pass
+  bool loud_ = false; LoudParams loud_par_{};
+  float* d_loud_ = nullptr; size_t loud_cap_ = 0;
+  std::vector<float> h_loud_;
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
   std::vector<long long> sample_off_;
   int* h_pred_dur_ = nullptr; size_t h_pred_dur_cap_ = 0;                  // pinned: per-row integer durations of the last run

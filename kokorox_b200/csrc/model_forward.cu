@@ -607,16 +607,30 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
   // pass reads it and writes d_audio_ at the output-rate offsets s_glob
   float* wav24 = nullptr;
   long long* d_s_len = nullptr;
-  long long max_out = 0;
+  long long max_out = 0, max_len24 = 0;
+  // loudness normalisation: per-item 2400-sample segment energies (offsets seg_off) and true-peak scratch
+  long long* d_seg_off = nullptr;
+  float* energy = nullptr;
+  unsigned* peak = nullptr;
   if (resample_) {
-    std::vector<long long> s_len(B);
+    std::vector<long long> s_len(B), seg_off(B);
+    long long nseg = 0;
     for (int b = 0; b < B; b++) {
       s_len[b] = 600LL * T[b];
       max_out = std::max(max_out, (s_len[b] * rs_U_ + rs_D_ - 1) / rs_D_);
+      max_len24 = std::max(max_len24, s_len[b]);
+      seg_off[b] = nseg;
+      nseg += s_len[b] / kLoudSeg;
     }
     wav24 = A.alloc<float>((size_t)(s_loc[B - 1] + s_len[B - 1]));
     d_s_len = A.alloc<long long>(B);
     upload(d_s_len, s_len.data(), B * sizeof(long long));
+    if (loud_) {
+      d_seg_off = A.alloc<long long>(B);
+      energy = A.alloc<float>((size_t)std::max(nseg, 1LL));
+      peak = A.alloc<unsigned>(B);
+      upload(d_seg_off, seg_off.data(), B * sizeof(long long));
+    }
   }
 
   // ---- length regulation (K4/K5)
@@ -917,8 +931,14 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
     return;
   }
   launch_istft(cp, 24, G120.d_off, G120.d_len, wav24, nullptr, d_s_loc, opt.precision == 1, B, G120.max_len, st);
-  launch_resample(wav24, d_s_loc, d_s_len, d_s_glob, d_taps_, rs_U_, rs_D_, rs_H_, d_audio_, want_pcm_ ? d_pcm_ : nullptr,
-                  want_law_ >= 0 ? d_g711_ : nullptr, want_law_ > 0 ? 1 : 0, B, max_out, st);
+  float* gain = nullptr;
+  if (loud_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (d_loud_ = lufs | dBTP | gain)
+    gain = d_loud_ + 2 * (size_t)B_ + b0;
+    launch_loudness(wav24, d_s_loc, d_s_len, d_seg_off, loud_par_, energy, peak, d_loud_ + b0, d_loud_ + B_ + b0, gain,
+                    B, max_len24, st);
+  }
+  launch_resample(wav24, d_s_loc, d_s_len, d_s_glob, d_taps_, rs_U_, rs_D_, rs_H_, gain, d_audio_,
+                  want_pcm_ ? d_pcm_ : nullptr, want_law_ >= 0 ? d_g711_ : nullptr, want_law_ > 0 ? 1 : 0, B, max_out, st);
 }
 
 }  // namespace kkx

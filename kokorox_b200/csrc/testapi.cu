@@ -83,12 +83,46 @@ KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64
     DevBuf doo(out_off.data(), B * 8), dout(nullptr, (size_t)no * 4), dpcm(nullptr, pcm ? (size_t)no * 2 : 0);
     DevBuf dcode(nullptr, codes && law >= 0 ? (size_t)no : 0);
     launch_resample(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), doo.as<long long>(),
-                    taps.empty() ? nullptr : dt.as<float>(), U, D, H, dout.as<float>(), pcm ? dpcm.as<short>() : nullptr,
+                    taps.empty() ? nullptr : dt.as<float>(), U, D, H, nullptr, dout.as<float>(), pcm ? dpcm.as<short>() : nullptr,
                     codes && law >= 0 ? dcode.as<unsigned char>() : nullptr, law > 0 ? 1 : 0, B, max_out, 0);
     KKX_CUDA(cudaDeviceSynchronize());
     KKX_CUDA(cudaMemcpy(out, dout.p, (size_t)no * 4, cudaMemcpyDeviceToHost));
     if (pcm) KKX_CUDA(cudaMemcpy(pcm, dpcm.p, (size_t)no * 2, cudaMemcpyDeviceToHost));
     if (codes && law >= 0) KKX_CUDA(cudaMemcpy(codes, dcode.p, (size_t)no, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int64_t kkx_test_loudness_design(double fs, double* kweight, float* tp_taps, int64_t capacity) {
+  if (!(fs > 0)) return KKX_ERR_ARG;
+  double kw[10];
+  std::vector<float> taps;
+  loudness_design(fs, kw, &taps);
+  if (kweight) memcpy(kweight, kw, sizeof kw);
+  if (tp_taps && capacity > 0) memcpy(tp_taps, taps.data(), (size_t)std::min<int64_t>(capacity, taps.size()) * sizeof(float));
+  return (int64_t)taps.size();
+}
+
+KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
+                              int32_t ceiling_centi_dbtp, float* lufs, float* true_peak_dbtp, float* gain) {
+  return run(device, [&] {
+    if (!x || !lens || B < 1) throw ArgError("kkx_test_loudness: bad argument");
+    std::vector<long long> in_off(B), in_len(B), seg_off(B);
+    long long ni = 0, nseg = 0, max_len = 0;
+    for (int b = 0; b < B; b++) {
+      if (lens[b] < 1) throw ArgError("kkx_test_loudness: every item needs >= 1 sample");
+      in_off[b] = ni; in_len[b] = lens[b]; seg_off[b] = nseg;
+      ni += lens[b]; nseg += lens[b] / kLoudSeg; max_len = std::max<long long>(max_len, lens[b]);
+    }
+    const LoudParams P = loudness_params(target_centi_lufs / 100.0, ceiling_centi_dbtp / 100.0);
+    DevBuf dx(x, (size_t)ni * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8), dso(seg_off.data(), B * 8);
+    DevBuf de(nullptr, (size_t)std::max(nseg, 1LL) * 4), dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4);
+    float* r = dr.as<float>();
+    launch_loudness(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), dso.as<long long>(), P, de.as<float>(),
+                    dp.as<unsigned>(), r, r + B, r + 2 * B, B, max_len, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    if (lufs) KKX_CUDA(cudaMemcpy(lufs, r, B * 4, cudaMemcpyDeviceToHost));
+    if (true_peak_dbtp) KKX_CUDA(cudaMemcpy(true_peak_dbtp, r + B, B * 4, cudaMemcpyDeviceToHost));
+    if (gain) KKX_CUDA(cudaMemcpy(gain, r + 2 * B, B * 4, cudaMemcpyDeviceToHost));
   });
 }
 

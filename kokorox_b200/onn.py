@@ -103,6 +103,10 @@ def load_library(path: Optional[str] = None):
         lib.kkx_test_resample_taps.argtypes = [i32, P(f32), i64]
         lib.kkx_test_resample_taps.restype = i64
         lib.kkx_test_resample.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(i16), P(u8)]
+        lib.kkx_last_loudness.argtypes = [vp, i32, P(f32), P(f32), P(f32)]
+        lib.kkx_test_loudness_design.argtypes = [C.c_double, P(C.c_double), P(f32), i64]
+        lib.kkx_test_loudness_design.restype = i64
+        lib.kkx_test_loudness.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(f32), P(f32)]
         lib.kkx_test_flac.argtypes = [C.c_int, P(i16), i32, P(i64), i32, P(u8), i64, P(i64)]
         lib.kkx_test_flac.restype = i64
         lib.kkx_test_attention_batch.argtypes = [C.c_int, P(f32), C.c_int, P(i32), P(i32), C.c_int, C.c_int, P(f32)]
@@ -546,6 +550,17 @@ class B200Koko:
         if return_durations:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
+
+    def last_loudness(self):
+        """What loudness normalisation (option ``loudness_target``) measured and applied in this session's last
+        synchronous call: ``(lufs, true_peak_dbtp, gain)``, three float32 arrays in item order (``lufs`` is NaN where
+        the loudness is undefined: items under 400 ms, silence).  Raises KkxError when that call ran with the option
+        off.  Coalesced and ``submit`` batches are not reported."""
+        self._require()
+        n = max(int(self._lib.kkx_get_stat(self._ctx, b"loudness_items")), 0)
+        lufs, tp, gain = (np.zeros(max(n, 1), np.float32) for _ in range(3))
+        self._check(self._lib.kkx_last_loudness(self._ctx, n, _fp(lufs), _fp(tp), _fp(gain)))
+        return lufs[:n], tp[:n], gain[:n]
 
     # -- device-resident path (bench `value`) ---------------------------------------------
     def stage(self, tokens, styles, speeds) -> None:
