@@ -24,9 +24,9 @@ struct kkx_ctx {
   std::mutex mu;  // single-flight like the reference's Mutex<Session> (ort_koko.rs:14,77-78)
   // pinned result buffers; their own lock, so that kkx_release never waits for the step `mu` is held across
   std::mutex pool_mu;
-  std::map<float*, size_t> pinned;       // audio buffers handed out -> capacity (floats)
-  std::vector<std::pair<float*, size_t>> pinned_free;  // returned buffers kept for reuse
-  size_t pinned_free_floats = 0;
+  std::map<void*, size_t> pinned;        // result buffers handed out -> capacity (bytes)
+  std::vector<std::pair<void*, size_t>> pinned_free;  // returned buffers kept for reuse
+  size_t pinned_free_bytes = 0;
   size_t pinned_hi = 0;                  // largest request so far: big buffers are sized alike so they recycle
 
   // Request coalescing (SURVEY 8f row 4): concurrent kkx_infer callers queue here; one of them becomes the
@@ -36,7 +36,7 @@ struct kkx_ctx {
     const int64_t* tokens; int32_t n; const float* style; float speed; int32_t* pred_dur;
     float* audio = nullptr; int64_t samples = 0; int rc = 0; std::string err; bool done = false;
   };
-  struct SharedBuf { float* base; size_t cap; int refs; };
+  struct SharedBuf { float* base; size_t cap; int refs; };   // cap in bytes
   std::mutex qmu;
   std::condition_variable qcv;
   std::deque<Waiter*> queue;
@@ -198,35 +198,35 @@ static int check_ctx(kkx_ctx* ctx) {
   return KKX_OK;
 }
 
-// shared tail of the infer entry points: run the staged batch and hand out a pooled pinned buffer
-static float* take_pinned(kkx_ctx* ctx, size_t need_floats, size_t* cap_out) {
-  float* host = nullptr;
+// shared tail of the infer entry points: a pooled pinned result buffer of at least `need` bytes
+static void* take_pinned(kkx_ctx* ctx, size_t need, size_t* cap_out) {
+  void* host = nullptr;
   size_t cap = 0, hi = 0;
   {
     std::lock_guard<std::mutex> pl(ctx->pool_mu);
-    hi = ctx->pinned_hi = std::max(ctx->pinned_hi, need_floats);
+    hi = ctx->pinned_hi = std::max(ctx->pinned_hi, need);
     size_t best = ctx->pinned_free.size();   // smallest buffer that fits
     for (size_t i = 0; i < ctx->pinned_free.size(); i++)
-      if (ctx->pinned_free[i].second >= need_floats &&
+      if (ctx->pinned_free[i].second >= need &&
           (best == ctx->pinned_free.size() || ctx->pinned_free[i].second < ctx->pinned_free[best].second))
         best = i;
     if (best < ctx->pinned_free.size()) {
       host = ctx->pinned_free[best].first; cap = ctx->pinned_free[best].second;
       ctx->pinned_free.erase(ctx->pinned_free.begin() + best);
-      ctx->pinned_free_floats -= cap;
+      ctx->pinned_free_bytes -= cap;
     }
   }
   if (!host) {
     // pinned allocation costs ~1 ms per MB and synchronises the device: give every request in the top size class
     // the same capacity, so a stream of similar batches reuses the pooled buffers instead of outgrowing them
-    const size_t base = need_floats >= hi / 2 ? hi : need_floats;
-    cap = std::max<size_t>(base + base / 8, 1024);
-    KKX_CUDA(cudaMallocHost(&host, cap * sizeof(float)));
+    const size_t base = need >= hi / 2 ? hi : need;
+    cap = std::max<size_t>(base + base / 8, 4096);
+    KKX_CUDA(cudaMallocHost(&host, cap));
   }
   *cap_out = cap;
   return host;
 }
-static void hand_out(kkx_ctx* ctx, float* host, size_t cap) {
+static void hand_out(kkx_ctx* ctx, void* host, size_t cap) {
   std::lock_guard<std::mutex> pl(ctx->pool_mu);
   ctx->pinned[host] = cap;
 }
@@ -262,29 +262,30 @@ static void run_staged_locked(kkx_ctx* ctx, float** host_out, size_t* cap_out, i
   Model& m = *ctx->model;
   float* host = nullptr;
   size_t cap = 0;
-  m.host_sink = [&](long long n) { host = take_pinned(ctx, (size_t)n, &cap); return host; };
+  m.host_sink = [&](long long n) { host = static_cast<float*>(take_pinned(ctx, n * sizeof(float), &cap)); return host; };
   try {
     m.run();
     m.host_sink = nullptr;
     const long long n = m.total_samples();
-    if (!host) host = take_pinned(ctx, (size_t)n, &cap);
+    if (!host) host = static_cast<float*>(take_pinned(ctx, n * sizeof(float), &cap));
     m.fetch(m.sink_filled() ? nullptr : host, n, out_sample_offsets, out_pred_dur);
   } catch (...) { m.host_sink = nullptr; if (host) cudaFreeHost(host); throw; }
   *host_out = host;
   *cap_out = cap;
 }
-static void recycle_pinned(kkx_ctx* ctx, float* host, size_t cap) {
-  float* to_free = nullptr;
+// A result buffer that came back: kept for reuse (pinned allocation costs milliseconds and synchronises the device)
+// up to 64 buffers and 1 GiB, freed otherwise.
+static void recycle_pinned(kkx_ctx* ctx, void* host, size_t cap) {
   {
     std::lock_guard<std::mutex> pl(ctx->pool_mu);
-    if (ctx->pinned_free.size() < 64 && ctx->pinned_free_floats + cap <= (size_t(1) << 28)) {
+    if (ctx->pinned_free.size() < 64 && ctx->pinned_free_bytes + cap <= (size_t(1) << 30)) {
       ctx->pinned_free.push_back({host, cap});
-      ctx->pinned_free_floats += cap;
-    } else {
-      to_free = host;
+      ctx->pinned_free_bytes += cap;
+      return;
     }
   }
-  if (to_free) cudaFreeHost(to_free);
+  if (ctx->model) cudaSetDevice(ctx->model->device());
+  cudaFreeHost(host);
 }
 
 // A call may carry any number of utterances; the device working set is bounded by running at most `max_tokens`
@@ -321,7 +322,7 @@ static void run_batch_locked(kkx_ctx* ctx, int32_t batch, const int64_t* tokens,
       b0 = b1;
     }
     size_t cap = 0;
-    float* host = take_pinned(ctx, (size_t)soff[batch], &cap);
+    float* host = static_cast<float*>(take_pinned(ctx, soff[batch] * sizeof(float), &cap));
     for (const Part& p : parts)
       memcpy(host + soff[p.b0], p.host, (size_t)(soff[p.b1] - soff[p.b0]) * sizeof(float));
     for (const Part& p : parts) recycle_pinned(ctx, p.host, p.cap);
@@ -485,6 +486,27 @@ KKX_API int kkx_infer_batch_voices(kkx_ctx* ctx, int32_t batch, const int64_t* t
   });
 }
 
+// The encoded entry points (kkx_infer_batch_pcm16 / _g711 / _flac): one pass of the staged batch with `enc`, its
+// encoded bytes in a pooled pinned buffer (caller holds ctx->mu; throws).
+static void* infer_encoded_locked(kkx_ctx* ctx, Encoding enc, int32_t batch, const int64_t* tokens,
+                                  const int32_t* tok_offsets, const float* styles, const float* speeds,
+                                  int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+  Model& m = *ctx->model;
+  m.stage(batch, tokens, tok_offsets, styles, speeds);
+  loud_begin(ctx);
+  m.run(enc);
+  loud_note(ctx);
+  const long long n = m.encoded_bytes();
+  size_t cap = 0;
+  void* host = take_pinned(ctx, (size_t)n, &cap);
+  try {
+    m.fetch_encoded(host, n, out_byte_offsets, out_sample_offsets, out_pred_dur);
+  } catch (...) { cudaFreeHost(host); throw; }
+  hand_out(ctx, host, cap);
+  loud_done(ctx);
+  return host;
+}
+
 KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                           const float* styles, const float* speeds, int16_t** out_pcm,
                           int64_t* out_sample_offsets, int32_t* out_pred_dur) {
@@ -494,22 +516,8 @@ KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* to
   std::lock_guard<std::mutex> lk(ctx->mu);
   return guarded(ctx, [&] {
     if (!out_pcm) throw ArgError("out_pcm is null");
-    Model& m = *ctx->model;
-    m.stage(batch, tokens, tok_offsets, styles, speeds);
-    loud_begin(ctx);
-    m.set_pcm16(true);
-    try { m.run(); } catch (...) { m.set_pcm16(false); throw; }
-    m.set_pcm16(false);
-    loud_note(ctx);
-    const long long n = m.total_samples();
-    size_t cap = 0;
-    float* host = take_pinned(ctx, (size_t)(n + 1) / 2, &cap);   // n int16 = n/2 floats of the same pool
-    try {
-      m.fetch_pcm16(reinterpret_cast<short*>(host), n, out_sample_offsets, out_pred_dur);
-    } catch (...) { cudaFreeHost(host); throw; }
-    hand_out(ctx, host, cap);
-    loud_done(ctx);
-    *out_pcm = reinterpret_cast<int16_t*>(host);
+    *out_pcm = static_cast<int16_t*>(infer_encoded_locked(ctx, Encoding::PCM16, batch, tokens, tok_offsets, styles,
+                                                          speeds, nullptr, out_sample_offsets, out_pred_dur));
   });
 }
 
@@ -525,22 +533,9 @@ KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tok
   return guarded(ctx, [&] {
     if (!out_codes) throw ArgError("out_codes is null");
     if (law != 0 && law != 1) throw ArgError("law must be 0 (mu-law) or 1 (A-law), got " + std::to_string(law));
-    Model& m = *ctx->model;
-    m.stage(batch, tokens, tok_offsets, styles, speeds);
-    loud_begin(ctx);
-    m.set_g711(law);
-    try { m.run(); } catch (...) { m.set_g711(-1); throw; }
-    m.set_g711(-1);
-    loud_note(ctx);
-    const long long n = m.total_samples();
-    size_t cap = 0;
-    float* host = take_pinned(ctx, (size_t)(n + 3) / 4, &cap);   // n one-byte codes = n/4 floats of the same pool
-    try {
-      m.fetch_g711(reinterpret_cast<unsigned char*>(host), n, out_sample_offsets, out_pred_dur);
-    } catch (...) { cudaFreeHost(host); throw; }
-    hand_out(ctx, host, cap);
-    loud_done(ctx);
-    *out_codes = reinterpret_cast<uint8_t*>(host);
+    *out_codes = static_cast<uint8_t*>(infer_encoded_locked(ctx, law ? Encoding::ALAW : Encoding::ULAW, batch, tokens,
+                                                            tok_offsets, styles, speeds, nullptr, out_sample_offsets,
+                                                            out_pred_dur));
   });
 }
 
@@ -556,23 +551,8 @@ KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tok
   return guarded(ctx, [&] {
     if (!out_bytes) throw ArgError("out_bytes is null");
     if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
-    Model& m = *ctx->model;
-    m.stage(batch, tokens, tok_offsets, styles, speeds);
-    loud_begin(ctx);
-    m.set_pcm16(true);
-    try { m.run(); } catch (...) { m.set_pcm16(false); throw; }
-    m.set_pcm16(false);
-    loud_note(ctx);
-    m.encode_flac();
-    const long long n = m.flac_bytes();
-    size_t cap = 0;
-    float* host = take_pinned(ctx, (size_t)(n + 3) / 4, &cap);   // n bytes = n/4 floats of the same pool
-    try {
-      m.fetch_flac(reinterpret_cast<unsigned char*>(host), n, out_byte_offsets, out_sample_offsets, out_pred_dur);
-    } catch (...) { cudaFreeHost(host); throw; }
-    hand_out(ctx, host, cap);
-    loud_done(ctx);
-    *out_bytes = reinterpret_cast<uint8_t*>(host);
+    *out_bytes = static_cast<uint8_t*>(infer_encoded_locked(ctx, Encoding::FLAC, batch, tokens, tok_offsets, styles,
+                                                            speeds, out_byte_offsets, out_sample_offsets, out_pred_dur));
   });
 }
 
@@ -759,7 +739,8 @@ KKX_API int kkx_wait(kkx_ctx* ctx, kkx_ticket ticket, float** out_audio, int64_t
 
 KKX_API void kkx_release(kkx_ctx* ctx, float* audio) {
   if (!ctx || !audio) return;
-  float* to_free = nullptr;
+  void* host = audio;
+  size_t cap = 0;
   {
     std::lock_guard<std::mutex> pl(ctx->pool_mu);
     auto vit = ctx->views.find(audio);
@@ -767,25 +748,17 @@ KKX_API void kkx_release(kkx_ctx* ctx, float* audio) {
       kkx_ctx::SharedBuf* sb = vit->second;
       ctx->views.erase(vit);
       if (--sb->refs > 0) return;
-      ctx->pinned[sb->base] = sb->cap;
-      audio = sb->base;
+      host = sb->base;
+      cap = sb->cap;
       delete sb;
-    }
-    auto it = ctx->pinned.find(audio);
-    if (it == ctx->pinned.end()) return;
-    // keep returned buffers for reuse (pinned allocation costs milliseconds and synchronises the device)
-    if (ctx->pinned_free.size() < 64 && ctx->pinned_free_floats + it->second <= (size_t(1) << 28)) {
-      ctx->pinned_free.push_back({it->first, it->second});
-      ctx->pinned_free_floats += it->second;
     } else {
-      to_free = audio;
+      auto it = ctx->pinned.find(audio);
+      if (it == ctx->pinned.end()) return;
+      cap = it->second;
+      ctx->pinned.erase(it);
     }
-    ctx->pinned.erase(it);
   }
-  if (to_free) {
-    if (ctx->model) cudaSetDevice(ctx->model->device());
-    cudaFreeHost(to_free);
-  }
+  recycle_pinned(ctx, host, cap);
 }
 
 KKX_API int kkx_stage_batch(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,

@@ -170,13 +170,7 @@ Model::~Model() {
   if (stream_) cudaStreamSynchronize(stream_);
   if (stream2_) cudaStreamSynchronize(stream2_);
   clear_graphs();
-  if (d_audio_) cudaFree(d_audio_);
-  if (d_pcm_) cudaFree(d_pcm_);
-  if (d_g711_) cudaFree(d_g711_);
-  if (d_flac_) cudaFree(d_flac_);
-  if (d_flac_meta_) cudaFree(d_flac_meta_);
   if (d_taps_) cudaFree(d_taps_);
-  if (d_loud_) cudaFree(d_loud_);
   if (d_voices_) cudaFree(d_voices_);
   if (d_noise_) cudaFree(d_noise_);
   if (h_pred_dur_) cudaFreeHost(h_pred_dur_);
@@ -768,105 +762,29 @@ void Model::stage_voices(int B, const int64_t* tokens, const int32_t* tok_offset
   staged_ = true;
 }
 
-void Model::fetch_pcm16(short* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur) {
-  if (!ran_) throw StateError("no completed run to fetch from");
-  if (!d_pcm_ || !pcm_valid_) throw ArgError("the last run did not produce 16-bit PCM");
-  fetch(nullptr, 0, sample_offsets, pred_dur);
-  if (dst) {
-    if (capacity < total_samples_) throw ArgError("pcm buffer too small");
-    KKX_CUDA(cudaMemcpyAsync(dst, d_pcm_, total_samples_ * sizeof(short), cudaMemcpyDeviceToHost, stream_));
-    KKX_CUDA(cudaStreamSynchronize(stream_));
+long long Model::encoded_bytes() const {
+  if (!ran_) return 0;
+  switch (enc_) {
+    case Encoding::PCM16: return total_samples_ * (long long)sizeof(short);
+    case Encoding::ULAW: case Encoding::ALAW: return total_samples_;
+    case Encoding::FLAC: return flac_off_[B_];
+    default: return 0;
   }
 }
 
-void Model::fetch_g711(unsigned char* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur) {
+void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
+                          int32_t* pred_dur) {
   if (!ran_) throw StateError("no completed run to fetch from");
-  if (!d_g711_ || !g711_valid_) throw ArgError("the last run did not produce G.711 codes");
-  fetch(nullptr, 0, sample_offsets, pred_dur);
-  if (dst) {
-    if (capacity < total_samples_) throw ArgError("code buffer too small");
-    KKX_CUDA(cudaMemcpyAsync(dst, d_g711_, total_samples_, cudaMemcpyDeviceToHost, stream_));
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-  }
-}
-
-void Model::encode_flac() {
-  if (!ran_) throw StateError("no completed run to encode");
-  if (!d_pcm_ || !pcm_valid_) throw ArgError("the last run did not produce 16-bit PCM");
-  KKX_CUDA(cudaSetDevice(device_));
-  flac_valid_ = false;
-  // frames per item (4096 samples each) and the device tables: sample offsets, frame prefix, item byte offsets
-  std::vector<int> foff(B_ + 1, 0);
-  for (int b = 0; b < B_; b++) {
-    const long long nf = flac_frames(sample_off_[b + 1] - sample_off_[b]);
-    if (foff[b] + nf > 0x7FFFFFFFLL) throw ArgError("batch too long for one FLAC encode");
-    foff[b + 1] = foff[b] + (int)nf;
-  }
-  const int F = foff[B_];
-  const size_t bound = (size_t)flac_bound(B_, F, total_samples_);
-  const size_t t_soff = 0, t_foff = t_soff + (((size_t)(B_ + 1) * 8 + 255) & ~size_t(255));
-  const size_t t_ioff = t_foff + (((size_t)(B_ + 1) * 4 + 255) & ~size_t(255));
-  const size_t t_work = t_ioff + (((size_t)(B_ + 1) * 8 + 255) & ~size_t(255));
-  const size_t meta = t_work + flac_work_bytes(F);
-  if (bound > flac_cap_) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_flac_) cudaFree(d_flac_);
-    d_flac_ = nullptr; flac_cap_ = 0;
-    const size_t cap = bound + bound / 4;
-    KKX_CUDA(cudaMalloc(&d_flac_, cap));
-    flac_cap_ = cap;
-  }
-  if (meta > flac_meta_cap_) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_flac_meta_) cudaFree(d_flac_meta_);
-    d_flac_meta_ = nullptr; flac_meta_cap_ = 0;
-    const size_t cap = meta + meta / 4;
-    KKX_CUDA(cudaMalloc(&d_flac_meta_, cap));
-    flac_meta_cap_ = cap;
-  }
-  long long* d_soff = reinterpret_cast<long long*>(d_flac_meta_ + t_soff);
-  int* d_foff = reinterpret_cast<int*>(d_flac_meta_ + t_foff);
-  long long* d_ioff = reinterpret_cast<long long*>(d_flac_meta_ + t_ioff);
-  KKX_CUDA(cudaMemcpyAsync(d_soff, sample_off_.data(), (size_t)(B_ + 1) * 8, cudaMemcpyHostToDevice, stream_));
-  KKX_CUDA(cudaMemcpyAsync(d_foff, foff.data(), (size_t)(B_ + 1) * 4, cudaMemcpyHostToDevice, stream_));
-  // the encoder's launches count in "launches" and appear in kkx_profile_json beside the run's kernels
-  g_launch_stats = &stats;
-  const size_t e0 = stats.n_events;
-  if (stats.profile) {   // a new start event; the name keeps names[i] = launch between events[i] and [i + 1]
-    cudaEventRecord(stats.next_event(), stream_);
-    stats.names.push_back("(host)");
-  }
-  try {
-    launch_flac(d_pcm_, d_soff, d_foff, B_, F, opt.out_rate, d_flac_meta_ + t_work, d_flac_, d_ioff, stream_);
-    flac_off_.assign(B_ + 1, 0);
-    KKX_CUDA(cudaMemcpyAsync(flac_off_.data(), d_ioff, (size_t)(B_ + 1) * 8, cudaMemcpyDeviceToHost, stream_));
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-  } catch (...) {
-    cudaStreamSynchronize(stream_);
-    g_launch_stats = nullptr;
-    throw;
-  }
-  if (stats.profile)
-    for (size_t i = e0; i + 1 < stats.n_events && i < stats.names.size(); i++) {
-      float dt = 0.f;
-      cudaEventElapsedTime(&dt, stats.events[i], stats.events[i + 1]);
-      auto& e = prof_[stats.names[i]];
-      e.first += 1; e.second += dt * 1e3;
-    }
-  g_launch_stats = nullptr;
-  flac_valid_ = true;
-}
-
-void Model::fetch_flac(unsigned char* dst, long long capacity, int64_t* byte_offsets, int64_t* sample_offsets,
-                       int32_t* pred_dur) {
-  if (!ran_) throw StateError("no completed run to fetch from");
-  if (!flac_valid_) throw ArgError("the last run was not FLAC-encoded");
+  if (enc_ == Encoding::F32) throw ArgError("the last run produced no encoded output");
   fetch(nullptr, 0, sample_offsets, pred_dur);
   if (byte_offsets)
-    for (int b = 0; b <= B_; b++) byte_offsets[b] = flac_off_[b];
+    for (int b = 0; b <= B_; b++)
+      byte_offsets[b] = enc_ == Encoding::FLAC ? flac_off_[b] : sample_off_[b] * (enc_ == Encoding::PCM16 ? 2 : 1);
   if (dst) {
-    if (capacity < flac_off_[B_]) throw ArgError("FLAC buffer too small");
-    KKX_CUDA(cudaMemcpyAsync(dst, d_flac_, (size_t)flac_off_[B_], cudaMemcpyDeviceToHost, stream_));
+    const long long n = encoded_bytes();
+    if (capacity_bytes < n) throw ArgError("output buffer too small");
+    KKX_CUDA(cudaMemcpyAsync(dst, enc_ == Encoding::FLAC ? flacA_.base() : twinA_.base(), (size_t)n,
+                             cudaMemcpyDeviceToHost, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
   }
 }
@@ -877,7 +795,7 @@ void Model::fetch_flac(unsigned char* dst, long long capacity, int64_t* byte_off
 void Model::prepare_resample() {
   loud_ = opt.loudness_target != 0;
   if (loud_) loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0);
-  resample_ = opt.out_rate != 24000 || want_law_ >= 0 || loud_;
+  resample_ = opt.out_rate != 24000 || enc_ == Encoding::ULAW || enc_ == Encoding::ALAW || loud_;
   rs_U_ = 1; rs_D_ = 1; rs_H_ = 0;
   if (opt.out_rate == 24000) return;
   std::vector<float> taps;
@@ -905,17 +823,25 @@ void Model::fetch(float* dst, long long capacity, int64_t* sample_offsets, int32
   }
   if (dst) {
     if (capacity < total_samples_) throw ArgError("audio buffer too small");
-    KKX_CUDA(cudaMemcpyAsync(dst, d_audio_, total_samples_ * sizeof(float), cudaMemcpyDeviceToHost, stream_));
+    KKX_CUDA(cudaMemcpyAsync(dst, audioA_.base(), total_samples_ * sizeof(float), cudaMemcpyDeviceToHost, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
   }
 }
 
+// A grow-only output buffer, reset for the run; when it is too small the stream must be done with the old one.
+void Model::grow(Arena& a, size_t bytes) {
+  a.reset();
+  if (bytes <= a.capacity()) return;
+  KKX_CUDA(cudaStreamSynchronize(stream_));
+  a.reserve(bytes + bytes / 4);
+}
+
 // ============================================================================ forward
-void Model::run() {
+void Model::run(Encoding enc) {
   if (!staged_ || B_ <= 0) throw StateError("no batch staged");
   KKX_CUDA(cudaSetDevice(device_));
   ran_ = false;
-  flac_valid_ = false;
+  enc_ = enc;
   use_lane(0);
   prepare_resample();
   g_launch_stats = &stats;
@@ -956,43 +882,44 @@ void Model::run() {
   sample_off_[B_] = ns;
   total_samples_ = ns;
   last_frames = tot;
-  if ((size_t)total_samples_ > audio_cap_) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_audio_) cudaFree(d_audio_);
-    d_audio_ = nullptr; audio_cap_ = 0;
-    const size_t cap = (size_t)total_samples_ + (size_t)total_samples_ / 4;
-    KKX_CUDA(cudaMalloc(&d_audio_, cap * sizeof(float)));
-    audio_cap_ = cap;
+  grow(audioA_, (size_t)total_samples_ * sizeof(float));
+  r.audio = audioA_.alloc<float>(total_samples_);
+  if (enc != Encoding::F32) {
+    const size_t bytes = (size_t)total_samples_ * (enc == Encoding::ULAW || enc == Encoding::ALAW ? 1 : sizeof(short));
+    grow(twinA_, bytes);
+    r.twin = twinA_.alloc_bytes(bytes);
   }
-  if (want_pcm_ && (size_t)total_samples_ > pcm_cap_) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_pcm_) cudaFree(d_pcm_);
-    d_pcm_ = nullptr; pcm_cap_ = 0;
-    const size_t cap = (size_t)total_samples_ + (size_t)total_samples_ / 4;
-    KKX_CUDA(cudaMalloc(&d_pcm_, cap * sizeof(short)));
-    pcm_cap_ = cap;
+  if (loud_) {
+    grow(loudA_, (size_t)B_ * 3 * sizeof(float));
+    r.loud = loudA_.alloc<float>((size_t)B_ * 3);
   }
-  if (want_law_ >= 0 && (size_t)total_samples_ > g711_cap_) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_g711_) cudaFree(d_g711_);
-    d_g711_ = nullptr; g711_cap_ = 0;
-    const size_t cap = (size_t)total_samples_ + (size_t)total_samples_ / 4;
-    KKX_CUDA(cudaMalloc(&d_g711_, cap));
-    g711_cap_ = cap;
-  }
-  if (loud_ && (size_t)B_ * 3 > loud_cap_) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_loud_) cudaFree(d_loud_);
-    d_loud_ = nullptr; loud_cap_ = 0;
-    KKX_CUDA(cudaMalloc(&d_loud_, (size_t)B_ * 3 * sizeof(float)));
-    loud_cap_ = (size_t)B_ * 3;
+  // FLAC: the encoder's tables -- sample offsets, frames per item (4096 samples each) as a prefix, item byte offsets
+  // -- and its output, ready before the forward pass so that the encoder follows it without a host round trip
+  struct { int F = 0; long long *soff = nullptr, *ioff = nullptr; int* foff = nullptr; void* work = nullptr;
+           unsigned char* out = nullptr; } fl;
+  if (enc == Encoding::FLAC) {
+    std::vector<int> foff(B_ + 1, 0);
+    for (int b = 0; b < B_; b++) {
+      const long long nf = flac_frames(sample_off_[b + 1] - sample_off_[b]);
+      if (foff[b] + nf > 0x7FFFFFFFLL) throw ArgError("batch too long for one FLAC encode");
+      foff[b + 1] = foff[b] + (int)nf;
+    }
+    fl.F = foff[B_];
+    const size_t bound = (size_t)flac_bound(B_, fl.F, total_samples_);
+    grow(flacA_, bound);
+    fl.out = flacA_.alloc<unsigned char>(bound);
+    grow(flacTabA_, 3 * ((size_t)(B_ + 1) * sizeof(long long) + 256) + flac_work_bytes(fl.F));
+    fl.soff = flacTabA_.alloc<long long>(B_ + 1);
+    fl.foff = flacTabA_.alloc<int>(B_ + 1);
+    fl.ioff = flacTabA_.alloc<long long>(B_ + 1);
+    fl.work = flacTabA_.alloc_bytes(flac_work_bytes(fl.F));
+    upload(fl.soff, sample_off_.data(), (size_t)(B_ + 1) * sizeof(long long));
+    upload(fl.foff, foff.data(), (size_t)(B_ + 1) * sizeof(int));
   }
   h_loud_.clear();
-  pcm_valid_ = want_pcm_;
-  g711_valid_ = want_law_ >= 0;
   sink_filled_ = false;
   float* sink = (host_sink && !debug_) ? host_sink(total_samples_) : nullptr;
-  // (both streams are idle here: the previous run synchronised them, and d_audio_ was sized above)
+  // (both streams are idle here: the previous run synchronised them, and the outputs were sized above)
   try {
     int b0 = 0;
     while (b0 < B_) {
@@ -1025,16 +952,23 @@ void Model::run() {
         KKX_CUDA(cudaEventRecord(ev_grp_, stream_));
         KKX_CUDA(cudaStreamWaitEvent(copy_stream_, ev_grp_, 0));
         if (s1 > s0)
-          KKX_CUDA(cudaMemcpyAsync(sink + s0, d_audio_ + s0, (size_t)(s1 - s0) * sizeof(float), cudaMemcpyDeviceToHost, copy_stream_));
+          KKX_CUDA(cudaMemcpyAsync(sink + s0, r.audio + s0, (size_t)(s1 - s0) * sizeof(float), cudaMemcpyDeviceToHost, copy_stream_));
       }
       b0 = b1;
     }
     KKX_CUDA(cudaEventRecord(ev1_, stream_));
+    if (enc == Encoding::FLAC) {
+      launch_flac(static_cast<const short*>(r.twin), fl.soff, fl.foff, B_, fl.F, opt.out_rate, fl.work, fl.out, fl.ioff,
+                  stream_);
+      flac_off_.assign(B_ + 1, 0);
+      KKX_CUDA(cudaMemcpyAsync(flac_off_.data(), fl.ioff, (size_t)(B_ + 1) * sizeof(long long),
+                               cudaMemcpyDeviceToHost, stream_));
+    }
     KKX_CUDA(cudaStreamSynchronize(stream_));
     if (sink) { KKX_CUDA(cudaStreamSynchronize(copy_stream_)); sink_filled_ = true; }
     if (loud_) {   // [3][B] on the device -> item-major on the host
       std::vector<float> rows((size_t)B_ * 3);
-      KKX_CUDA(cudaMemcpy(rows.data(), d_loud_, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
+      KKX_CUDA(cudaMemcpy(rows.data(), r.loud, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
       h_loud_.resize(rows.size());
       for (int b = 0; b < B_; b++)
         for (int k = 0; k < 3; k++) h_loud_[(size_t)b * 3 + k] = rows[(size_t)k * B_ + b];

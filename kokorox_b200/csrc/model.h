@@ -205,6 +205,10 @@ constexpr float kMinSpeed = 0.1f, kMaxSpeed = 10.f;   // dur per token <= 50 / s
 constexpr int kMaxItemFrames = 65536;                  // one utterance: <= 27 min of audio (120*T+1 rows fit int32;
                                                        // at out_rate 48000: 1 200 samples per frame, 7.9e7 per utterance)
 
+// What a run returns besides the f32 waveform, which every run writes: its 16-bit PCM twin, the G.711 codes of that
+// PCM (mu-law / A-law), or one FLAC stream per item encoded from it (kkx.h).
+enum class Encoding { F32, PCM16, ULAW, ALAW, FLAC };
+
 class Model {
  public:
   Model(const std::string& weights_path, int device);
@@ -219,25 +223,21 @@ class Model {
   void load_voices(const float* table, int n_voices);
   void stage_voices(int B, const int64_t* tokens, const int32_t* tok_offsets, const int32_t* mix_offsets,
                     const int32_t* voice_ids, const float* portions, const int32_t* style_rows, const float* speeds);
-  void set_pcm16(bool on) { want_pcm_ = on; }
-  void fetch_pcm16(short* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
-  // G.711 codes of the 16-bit PCM value (law 0 = mu-law, 1 = A-law, -1 = none) written by the resampling pass
-  void set_g711(int law) { want_law_ = law; }
-  void fetch_g711(unsigned char* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
-  // Lossless FLAC (kernels_flac.cu) of the last run's 16-bit PCM (a run with set_pcm16(true)): one stream per item,
-  // back to back; encode_flac() launches the encoder and copies the per-item byte offsets to the host.
-  void encode_flac();
-  long long flac_bytes() const { return flac_valid_ ? flac_off_.back() : 0; }
-  void fetch_flac(unsigned char* dst, long long capacity, int64_t* byte_offsets, int64_t* sample_offsets,
-                  int32_t* pred_dur);
   // Optional host sink for the waveform: called once the total sample count is known (after the token phase);
   // returns a pinned buffer of >= n floats.  Each frame group's audio is then copied to it on a second stream as
   // soon as the group's iSTFT is done, overlapping the device->host copy with the next group's kernels.
   std::function<float*(long long)> host_sink;
   bool sink_filled() const { return sink_filled_; }
-  void run();
+  // A FLAC run launches the encoder (kernels_flac.cu) after the forward pass: gpu_us does not include it.
+  void run(Encoding enc = Encoding::F32);
   long long total_samples() const { return total_samples_; }
+  // The f32 waveform of the last run, whatever its encoding.
   void fetch(float* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
+  // The encoded output of the last run (ArgError after an F32 run): 2 bytes per sample for PCM16, 1 for G.711, the
+  // FLAC streams back to back.  byte_offsets [B + 1] locate each item's bytes.
+  long long encoded_bytes() const;
+  void fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
+                     int32_t* pred_dur);
   // Loudness of the last run's items (kernels_loudness.cu): true if that run normalised; then last_loudness() holds
   // 3 B floats, per item b at 3 b: integrated loudness (LUFS, NaN = undefined), true peak (dBTP), applied gain.
   bool loudness_ran() const { return ran_ && loud_; }
@@ -270,6 +270,9 @@ class Model {
     int* total = nullptr;      // [B]     T_b
     std::vector<int> T;        // frames per item (host)
     Level styL;                // one item of B rows (style FC GEMMs)
+    float* audio = nullptr;    // [total_samples_] the f32 waveform at the output rate
+    void* twin = nullptr;      // its 16-bit PCM (PCM16, FLAC) or G.711 (ULAW, ALAW) twin
+    float* loud = nullptr;     // [3][B] lufs | dBTP | gain of loudness normalisation; the gain feeds the resampling
   };
   // Linear / Conv1d on the precision-critical path: split-TF32 tensor cores when precision==1 and
   // the weight has a TcW32, fp32 SIMT otherwise.
@@ -362,22 +365,18 @@ class Model {
   std::vector<int> tok_len_;
   int* d_ids_ = nullptr; float* d_styles_ = nullptr; float* d_speeds_ = nullptr;
   Level tokL_;
-  // outputs
-  float* d_audio_ = nullptr; size_t audio_cap_ = 0;
-  short* d_pcm_ = nullptr; size_t pcm_cap_ = 0; bool want_pcm_ = false, pcm_valid_ = false;   // optional 16-bit PCM twin of d_audio_
-  unsigned char* d_g711_ = nullptr; size_t g711_cap_ = 0; int want_law_ = -1; bool g711_valid_ = false;  // optional G.711 twin
-  // FLAC streams of the last encode_flac(): bytes, per-item byte offsets (host), and the encoder's tables / scratch
-  unsigned char* d_flac_ = nullptr; size_t flac_cap_ = 0; bool flac_valid_ = false;
-  char* d_flac_meta_ = nullptr; size_t flac_meta_cap_ = 0;
+  // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC streams, their
+  // per-item byte offsets (host) and the encoder's tables and scratch
+  Encoding enc_ = Encoding::F32;
+  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_;
   std::vector<long long> flac_off_;
+  void grow(Arena& a, size_t bytes);
   // output resampling of the current run (opt.out_rate): U / D, half length H; d_taps_ holds the filter of taps_rate_
   bool resample_ = false; int rs_U_ = 1, rs_D_ = 1, rs_H_ = 0;
   float* d_taps_ = nullptr; int taps_rate_ = 0;
   void prepare_resample();
-  // loudness normalisation of the current run: d_loud_ = [3][B_] floats (lufs | dBTP | gain), h_loud_ its host copy
-  // (item-major); the gain row feeds the resampling pass
+  // loudness normalisation of the current run; h_loud_ = the host copy of Run::loud (item-major)
   bool loud_ = false; LoudParams loud_par_{};
-  float* d_loud_ = nullptr; size_t loud_cap_ = 0;
   std::vector<float> h_loud_;
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
   std::vector<long long> sample_off_;

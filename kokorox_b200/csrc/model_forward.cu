@@ -604,7 +604,7 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
   upload(d_s_loc, s_loc.data(), B * sizeof(long long));
   upload(d_s_glob, s_glob.data(), B * sizeof(long long));
   // output resampling: the iSTFT writes the group's 24 kHz audio here (group-local offsets s_loc), the resampling
-  // pass reads it and writes d_audio_ at the output-rate offsets s_glob
+  // pass reads it and writes r.audio at the output-rate offsets s_glob
   float* wav24 = nullptr;
   long long* d_s_len = nullptr;
   long long max_out = 0, max_len24 = 0;
@@ -926,19 +926,21 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
     launch_conv_f32(c, st);
   }
   capture("conv_post", cp, 24, 0, 22, G120, b0);
+  const bool law = enc_ == Encoding::ULAW || enc_ == Encoding::ALAW;
+  short* pcm = enc_ == Encoding::PCM16 || enc_ == Encoding::FLAC ? static_cast<short*>(r.twin) : nullptr;
   if (!resample_) {
-    launch_istft(cp, 24, G120.d_off, G120.d_len, d_audio_, want_pcm_ ? d_pcm_ : nullptr, d_s_glob, opt.precision == 1, B, G120.max_len, st);
+    launch_istft(cp, 24, G120.d_off, G120.d_len, r.audio, pcm, d_s_glob, opt.precision == 1, B, G120.max_len, st);
     return;
   }
   launch_istft(cp, 24, G120.d_off, G120.d_len, wav24, nullptr, d_s_loc, opt.precision == 1, B, G120.max_len, st);
   float* gain = nullptr;
-  if (loud_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (d_loud_ = lufs | dBTP | gain)
-    gain = d_loud_ + 2 * (size_t)B_ + b0;
-    launch_loudness(wav24, d_s_loc, d_s_len, d_seg_off, loud_par_, energy, peak, d_loud_ + b0, d_loud_ + B_ + b0, gain,
+  if (loud_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
+    gain = r.loud + 2 * (size_t)B_ + b0;
+    launch_loudness(wav24, d_s_loc, d_s_len, d_seg_off, loud_par_, energy, peak, r.loud + b0, r.loud + B_ + b0, gain,
                     B, max_len24, st);
   }
-  launch_resample(wav24, d_s_loc, d_s_len, d_s_glob, d_taps_, rs_U_, rs_D_, rs_H_, gain, d_audio_,
-                  want_pcm_ ? d_pcm_ : nullptr, want_law_ >= 0 ? d_g711_ : nullptr, want_law_ > 0 ? 1 : 0, B, max_out, st);
+  launch_resample(wav24, d_s_loc, d_s_len, d_s_glob, d_taps_, rs_U_, rs_D_, rs_H_, gain, r.audio, pcm,
+                  law ? static_cast<unsigned char*>(r.twin) : nullptr, enc_ == Encoding::ALAW ? 1 : 0, B, max_out, st);
 }
 
 }  // namespace kkx

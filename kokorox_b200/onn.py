@@ -274,6 +274,35 @@ class B200Koko:
         if not self._ctx.value:
             raise KkxError(-5, "Session is not initialized.")  # ort_koko.rs:88-90
 
+    @staticmethod
+    def _pack(tokens, styles, speeds):
+        """A ragged batch as the C ABI takes it: (B, flat int64 tokens, int32 offsets [B + 1], styles [B, 256] -- None
+        when ``styles`` is None -- and f32 speeds [B])."""
+        B = len(tokens)
+        if B == 0:
+            raise KkxError(-1, "empty batch")
+        offs = np.zeros(B + 1, dtype=np.int32)
+        offs[1:] = np.cumsum([len(t) for t in tokens])
+        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
+        st = None
+        if styles is not None:
+            st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(-1))
+            if st.size != B * 256:
+                raise KkxError(-1, f"style must have 256 values, got {st.size / B:g}")
+            st = st.reshape(B, 256)
+        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        return B, flat, offs, st, sp
+
+    def _adopt(self, ptr, offsets):
+        """Zero-copy: item b of a library-owned result buffer as the view [offsets[b], offsets[b + 1]) (the reference
+        copies its output twice, ort_koko.rs:85 + koko.rs:1179).  The buffer goes back to the library's pool
+        (kkx_release) when the last view is garbage-collected; the views keep this session alive until then."""
+        base = np.ctypeslib.as_array(ptr, shape=(max(int(offsets[-1]), 1),))
+        with self._count_lock:
+            self._outstanding += 1
+        weakref.finalize(base, B200Koko._release_buffer, self, C.cast(ptr, C.c_void_p).value)
+        return [base[int(offsets[b]):int(offsets[b + 1])] for b in range(len(offsets) - 1)]
+
     # -- the reference entry point --------------------------------------------------------
     def infer(self, tokens: Sequence[Sequence[int]], styles: Sequence[Sequence[float]],
               speed: float) -> np.ndarray:
@@ -301,11 +330,7 @@ class B200Koko:
                                  C.c_float(speed), C.byref(audio), C.byref(ns),
                                  dur.ctypes.data_as(C.POINTER(C.c_int32)))
         self._check(rc)
-        out = np.ctypeslib.as_array(audio, shape=(max(int(ns.value), 1),))
-        with self._count_lock:
-            self._outstanding += 1
-        weakref.finalize(out, B200Koko._release_buffer, self, C.cast(audio, C.c_void_p).value)
-        out = out[:int(ns.value)]
+        out = self._adopt(audio, (0, ns.value))[0]
         return (out, dur[:tk.size]) if return_durations else out
 
     # -- asynchronous form (kkx_submit / kkx_poll / kkx_wait): sentence k+1 synthesises while k is being sent
@@ -343,11 +368,7 @@ class B200Koko:
         dur = np.zeros(max(n, 1), dtype=np.int32)
         self._check(self._lib.kkx_wait(self._ctx, int(ticket), C.byref(audio), C.byref(ns),
                                        dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        out = np.ctypeslib.as_array(audio, shape=(max(int(ns.value), 1),))
-        with self._count_lock:
-            self._outstanding += 1
-        weakref.finalize(out, B200Koko._release_buffer, self, C.cast(audio, C.c_void_p).value)
-        out = out[:int(ns.value)]
+        out = self._adopt(audio, (0, ns.value))[0]
         return (out, dur[:n]) if return_durations else out
 
     def infer_batch(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
@@ -355,17 +376,7 @@ class B200Koko:
         """Ragged batch of independent utterances (kkx_infer_batch).  Returns a list of 1-D f32
         arrays (and the per-item integer frame durations if asked)."""
         self._require()
-        B = len(tokens)
-        if B == 0:
-            raise KkxError(-1, "empty batch")
-        lens = [len(t) for t in tokens]
-        offs = np.zeros(B + 1, dtype=np.int32)
-        offs[1:] = np.cumsum(lens)
-        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
-        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, -1))
-        if st.shape[1] != 256:
-            raise KkxError(-1, f"style must have 256 values, got {st.shape[1]}")
-        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
         audio = C.POINTER(C.c_float)()
         soff = np.zeros(B + 1, dtype=np.int64)
         dur = np.zeros(int(offs[-1]), dtype=np.int32)
@@ -374,17 +385,7 @@ class B200Koko:
             offs.ctypes.data_as(C.POINTER(C.c_int32)), _fp(st), _fp(sp), C.byref(audio),
             soff.ctypes.data_as(C.POINTER(C.c_int64)), dur.ctypes.data_as(C.POINTER(C.c_int32)))
         self._check(rc)
-        total = int(soff[-1])
-        # Zero-copy: the waveforms are views into the library-owned pinned buffer the D2H copy landed in
-        # (the reference copies its output twice, ort_koko.rs:85 + koko.rs:1179).  The buffer goes back to
-        # the library's pool (kkx_release) when the last view is garbage-collected; the views keep this
-        # session alive until then.
-        base = np.ctypeslib.as_array(audio, shape=(max(total, 1),))
-        with self._count_lock:
-            self._outstanding += 1
-        weakref.finalize(base, B200Koko._release_buffer, self, C.cast(audio, C.c_void_p).value)
-        outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
-        del base
+        outs = self._adopt(audio, soff)
         if return_durations:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
@@ -425,11 +426,7 @@ class B200Koko:
         """koko.rs:1161-1180 for a ragged batch: item b uses voice / mix ``style_names[b]`` at table row
         ``len(tokens[b]) - 2`` (the un-padded token count); styles are mixed on the device."""
         self._require()
-        B = len(tokens)
-        lens = [len(t) for t in tokens]
-        offs = np.zeros(B + 1, dtype=np.int32)
-        offs[1:] = np.cumsum(lens)
-        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
+        B, flat, offs, _, sp = self._pack(tokens, None, speeds)
         moff = np.zeros(B + 1, dtype=np.int32)
         vids, pors = [], []
         for b, name in enumerate(style_names):
@@ -439,8 +436,7 @@ class B200Koko:
             moff[b + 1] = len(vids)
         vids = np.asarray(vids, dtype=np.int32)
         pors = np.asarray(pors, dtype=np.float32)
-        rows = np.asarray([n - 2 for n in lens], dtype=np.int32)
-        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        rows = np.asarray([len(t) - 2 for t in tokens], dtype=np.int32)
         audio = C.POINTER(C.c_float)()
         soff = np.zeros(B + 1, dtype=np.int64)
         dur = np.zeros(int(offs[-1]), dtype=np.int32)
@@ -448,13 +444,7 @@ class B200Koko:
         self._check(self._lib.kkx_infer_batch_voices(
             self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), ip(offs), ip(moff), ip(vids), _fp(pors),
             ip(rows), _fp(sp), C.byref(audio), soff.ctypes.data_as(C.POINTER(C.c_int64)), ip(dur)))
-        total = int(soff[-1])
-        base = np.ctypeslib.as_array(audio, shape=(max(total, 1),))
-        with self._count_lock:
-            self._outstanding += 1
-        weakref.finalize(base, B200Koko._release_buffer, self, C.cast(audio, C.c_void_p).value)
-        outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
-        del base
+        outs = self._adopt(audio, soff)
         if return_durations:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
@@ -463,26 +453,13 @@ class B200Koko:
         """Like infer_batch, but returns int16 PCM (trunc(clamp(s,-1,1)*32767), kokorox-websocket lib.rs:699-703),
         converted inside the iSTFT kernel; the device->host copy is half the size."""
         self._require()
-        B = len(tokens)
-        lens = [len(t) for t in tokens]
-        offs = np.zeros(B + 1, dtype=np.int32)
-        offs[1:] = np.cumsum(lens)
-        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
-        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, 256))
-        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
         pcm = C.POINTER(C.c_int16)()
         soff = np.zeros(B + 1, dtype=np.int64)
         self._check(self._lib.kkx_infer_batch_pcm16(
             self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
             _fp(st), _fp(sp), C.byref(pcm), soff.ctypes.data_as(C.POINTER(C.c_int64)), None))
-        total = int(soff[-1])
-        base = np.ctypeslib.as_array(pcm, shape=(max(total, 1),))
-        with self._count_lock:
-            self._outstanding += 1
-        weakref.finalize(base, B200Koko._release_buffer, self, C.cast(pcm, C.c_void_p).value)
-        outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
-        del base
-        return outs
+        return self._adopt(pcm, soff)
 
     def infer_batch_g711(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float], law: str = "ulaw",
                          return_durations: bool = False):
@@ -493,15 +470,7 @@ class B200Koko:
         laws = {"ulaw": 0, "alaw": 1}
         if law not in laws:
             raise KkxError(-1, f"law must be 'ulaw' or 'alaw', got {law!r}")
-        B = len(tokens)
-        if B == 0:
-            raise KkxError(-1, "empty batch")
-        lens = [len(t) for t in tokens]
-        offs = np.zeros(B + 1, dtype=np.int32)
-        offs[1:] = np.cumsum(lens)
-        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
-        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, 256))
-        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
         codes = C.POINTER(C.c_uint8)()
         soff = np.zeros(B + 1, dtype=np.int64)
         dur = np.zeros(int(offs[-1]), dtype=np.int32)
@@ -509,13 +478,7 @@ class B200Koko:
             self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
             _fp(st), _fp(sp), laws[law], C.byref(codes), soff.ctypes.data_as(C.POINTER(C.c_int64)),
             dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        total = int(soff[-1])
-        base = np.ctypeslib.as_array(codes, shape=(max(total, 1),))
-        with self._count_lock:
-            self._outstanding += 1
-        weakref.finalize(base, B200Koko._release_buffer, self, C.cast(codes, C.c_void_p).value)
-        outs = [base[int(soff[b]):int(soff[b + 1])] for b in range(B)]
-        del base
+        outs = self._adopt(codes, soff)
         if return_durations:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
@@ -527,15 +490,7 @@ class B200Koko:
         infer_batch_pcm16 returns.  The files are copied out of the library's buffer, which is released before this
         returns."""
         self._require()
-        B = len(tokens)
-        if B == 0:
-            raise KkxError(-1, "empty batch")
-        lens = [len(t) for t in tokens]
-        offs = np.zeros(B + 1, dtype=np.int32)
-        offs[1:] = np.cumsum(lens)
-        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
-        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, 256))
-        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
         buf = C.POINTER(C.c_uint8)()
         boff = np.zeros(B + 1, dtype=np.int64)
         dur = np.zeros(int(offs[-1]), dtype=np.int32)
@@ -565,12 +520,7 @@ class B200Koko:
     # -- device-resident path (bench `value`) ---------------------------------------------
     def stage(self, tokens, styles, speeds) -> None:
         self._require()
-        B = len(tokens)
-        offs = np.zeros(B + 1, dtype=np.int32)
-        offs[1:] = np.cumsum([len(t) for t in tokens])
-        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, dtype=np.int64).reshape(-1) for t in tokens]))
-        st = np.ascontiguousarray(np.asarray(styles, dtype=np.float32).reshape(B, 256))
-        sp = np.ascontiguousarray(np.asarray(speeds, dtype=np.float32).reshape(B))
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
         self._check(self._lib.kkx_stage_batch(self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)),
                                               offs.ctypes.data_as(C.POINTER(C.c_int32)), _fp(st), _fp(sp)))
         self._staged = (B, int(offs[-1]))

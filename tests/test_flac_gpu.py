@@ -131,6 +131,32 @@ def test_other_outputs_unchanged_after_flac(model, weights_path):
     assert flac_launches == want_pcm_launches + 3   # the encoder's three kernels
 
 
+@pytest.mark.parametrize("first", ("pcm16", "ulaw", "alaw"))
+def test_f32_unchanged_after_encoded_output(model, weights_path, first):
+    # the encoding belongs to one call: the next f32 call runs the launches and returns the bits of a fresh session,
+    # and the encoded call's own f32 waveform stays fetchable
+    from kokorox_b200.onn import B200Koko
+    toks, styles, speeds = _batch(seed=45)
+    fresh = B200Koko.new(weights_path)
+    try:
+        want = [a.copy() for a in fresh.infer_batch(toks, styles, speeds)]
+        want_launches = fresh.get_stat("launches")
+    finally:
+        fresh.close()
+    model.stage(toks, styles, speeds)
+    if first == "pcm16":
+        model.infer_batch_pcm16(toks, styles, speeds)
+    else:
+        model.infer_batch_g711(toks, styles, speeds, law=first)
+    wav, soff, _ = model.fetch_staged(sum(len(a) for a in want))
+    for b in range(len(want)):
+        assert np.array_equal(wav[soff[b]:soff[b + 1]], want[b])
+    got = model.infer_batch(toks, styles, speeds)
+    assert model.get_stat("launches") == want_launches
+    for a, b in zip(got, want):
+        assert np.array_equal(a, b)
+
+
 def test_profile_names_the_encoder_kernels(model):
     import json
     toks, styles, speeds = _batch(seed=60)
@@ -157,3 +183,17 @@ def test_null_outputs_are_argument_errors(model):
     files = model.infer_batch_flac(toks, styles, speeds)
     pcm = model.infer_batch_pcm16(toks, styles, speeds)
     assert np.array_equal(flac_decode_ref(files[0])[0], pcm[0])
+
+
+def test_bad_batches_are_argument_errors(model):
+    from kokorox_b200.onn import KkxError
+    toks, styles, speeds = _batch(2, seed=85)
+    short = np.asarray(styles, np.float32).reshape(2, 256)[:, :255]
+    for f in (model.infer_batch, model.infer_batch_pcm16, model.infer_batch_g711, model.infer_batch_flac, model.stage):
+        for args in (([], [], []), (toks, short, speeds)):
+            with pytest.raises(KkxError) as e:
+                f(*args)
+            assert e.value.code == -1, f.__name__
+    with pytest.raises(KkxError) as e:
+        model.infer_batch_voices([], [], [])
+    assert e.value.code == -1

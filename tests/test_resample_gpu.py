@@ -238,6 +238,28 @@ def test_default_rate_is_unchanged(model, weights_path):
         assert np.array_equal(a, b)
 
 
+def test_encoded_launches_at_default_rate(model):
+    # at 24 kHz without loudness normalisation the iSTFT writes the 16-bit PCM itself; G.711 codes come from the
+    # resampling pass in pass-through mode, one launch per frame group
+    toks, styles, speeds = _batch(seed=95)
+    model.set_option("max_frames", 300)
+    try:
+        model.infer_batch(toks, styles, speeds)
+        f32 = model.get_stat("launches")
+        groups = model.get_stat("frame_groups")
+        model.infer_batch_pcm16(toks, styles, speeds)
+        pcm16 = model.get_stat("launches")
+        g711 = []
+        for law in ("ulaw", "alaw"):
+            model.infer_batch_g711(toks, styles, speeds, law=law)
+            g711.append(model.get_stat("launches"))
+    finally:
+        model.set_option("max_frames", 49152)
+    assert groups >= 2
+    assert pcm16 == f32
+    assert g711 == [f32 + groups] * 2
+
+
 def test_rejected_rates_keep_the_previous_rate(model, rate):
     from kokorox_b200.onn import KkxError
     rate(16000)
