@@ -193,6 +193,52 @@ KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tok
                                  int64_t* out_sample_offsets /* [batch + 1], nullable */, int32_t* out_pred_dur);
 KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes);
 
+/* kkx_infer_programs: one output per PROGRAM instead of one per item, for a request that was split into chunks (the
+ *   reference splits text into chunks of at most 500 tokens, koko.rs:781-783, runs one infer per chunk and joins the
+ *   audio with extend_from_slice, koko.rs:947-1191; its OpenAI server and `file --merge` return one file per request).
+ *   Program k is the run of consecutive items [program_offsets[k], program_offsets[k+1]).  Items take their inputs
+ *   as in kkx_infer_batch.  Let x_k be the concatenation, in item order, of the 24 kHz model waveforms of program k's
+ *   items -- each exactly what kkx_infer_batch returns for the item at "out_rate" 24000 with loudness off -- so x_k
+ *   has n_k = sum of 600 T_b samples.  The program is then treated as one utterance of waveform x_k:
+ *   1. Loudness (when "loudness_target" != 0): rules 1-5 of "loudness_target" below apply to x_k as one signal: the
+ *      K-weighting starts from zero state at x_k's first sample and runs across the joins, the 400 ms blocks start
+ *      at x_k's sample 0, gating is over all of x_k's blocks, the true peak is that of resample_poly(x_k, 4, 1);
+ *      one gain g_k for the whole program.
+ *   2. Rate: y_k = resample_poly(x_k, U, D) under the "out_rate" rule, with zeros outside x_k, ceil(n_k U / D)
+ *      samples (at 24000, y_k = x_k).
+ *   3. Samples: each returned sample is fp32(y * g_k); PCM16, G.711 and FLAC follow from that value by their rules
+ *      above.  FLAC is one file per program under the kkx_infer_batch_flac rules, with n = the program's sample count.
+ *   4. Purity: a program's output depends on its own items only -- not on its position in the call, on the other
+ *      programs, or on how "max_frames" splits the items into frame groups (a program may span several groups).
+ *   5. Identity: a program of one item returns exactly what the entry point of that encoding returns for that item
+ *      (bits, FLAC bytes and the loudness report).  At 24000 with loudness off, an F32 or PCM16 program is the
+ *      bit-exact concatenation of its items' outputs (the reference's extend_from_slice).
+ *   encoding: KKX_ENC_F32 (4 bytes per sample), _PCM16 (2), _ULAW / _ALAW (1, G.711 as kkx_infer_batch_g711), _FLAC.
+ *   Program k's output is bytes [out_byte_offsets[k], out_byte_offsets[k+1]) of *out_bytes (offsets in bytes for every
+ *   encoding); out_sample_offsets (nullable, [n_programs + 1]) in output-rate samples; out_pred_dur (nullable) is
+ *   indexed like tokens.  One pass (no "max_tokens" split).  Afterwards kkx_last_loudness and the "loudness_items"
+ *   stat report per program (their batch is n_programs).  A FLAC program holds at most 2^36 - 1 samples (the
+ *   STREAMINFO field; longer is KKX_ERR_ARG).  Release the buffer with kkx_release_programs.
+ *   KKX_ERR_ARG, with the session left as it was, for: a null out_bytes or out_byte_offsets; n_programs outside
+ *   1..batch; program_offsets null, not starting at 0, not ending at batch, or not strictly increasing (no empty
+ *   program); encoding outside 0..4.
+ *   Not provided: pauses, cross-fades or silence trimming at the joins (the reference joins chunks as they are);
+ *   programs through kkx_infer, coalescing, kkx_submit, kkx_infer_batch_voices or kkx_run_staged; a "max_tokens" split
+ *   of a program call; streaming a program before its last item is done; MP3 or Opus. */
+#define KKX_ENC_F32 0   /* f32 samples, 4 bytes each */
+#define KKX_ENC_PCM16 1
+#define KKX_ENC_ULAW 2
+#define KKX_ENC_ALAW 3
+#define KKX_ENC_FLAC 4
+KKX_API int kkx_infer_programs(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                               const float* styles, const float* speeds,
+                               int32_t n_programs, const int32_t* program_offsets /* [n_programs + 1] */,
+                               int32_t encoding, void** out_bytes,
+                               int64_t* out_byte_offsets /* [n_programs + 1], required */,
+                               int64_t* out_sample_offsets /* [n_programs + 1], nullable */,
+                               int32_t* out_pred_dur /* nullable, indexed like tokens */);
+KKX_API void kkx_release_programs(kkx_ctx* ctx, void* bytes);
+
 /* ---- output containers (host-side byte work after the pcm16 / f32 result; no GPU involved, no ctx needed).
  * kkx_wav_header_pcm16: the 44-byte RIFF/WAVE header of the WebSocket server's `encode_audio`
  *   (kokorox-websocket/src/lib.rs:707-731): PCM format 1, mono, 16 bit, sizes filled in from n_samples.
@@ -253,8 +299,9 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                 point (kkx_infer, _batch, _batch_voices, _batch_pcm16, _batch_g711, kkx_wait and coalesced / async
  *                 batches, kkx_run_staged / kkx_fetch_staged) for runs that start after the call; every sample count
  *                 and offset is then in output-rate samples.  One rate per session (sessions of one file share the
- *                 device weights, so a server holds one session per rate).  Each utterance is resampled on its own,
- *                 with zeros outside it, exactly as scipy.signal.resample_poly(x, U, D) with its defaults:
+ *                 device weights, so a server holds one session per rate).  Each utterance (item, or program of
+ *                 kkx_infer_programs) is resampled on its own, with zeros outside it, exactly as
+ *                 scipy.signal.resample_poly(x, U, D) with its defaults:
  *                   H = 10 max(U, D),  h = U * firwin(2H + 1, 1 / max(U, D), window = ("kaiser", 5.0))
  *                   y[m] = sum over k ascending, 0 <= k < n, 0 <= mD - kU + H <= 2H, of x[k] * h[mD - kU + H],
  *                   0 <= m < ceil(n U / D)   (n = 600 T input samples)
@@ -267,9 +314,9 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                 For both, any other value is KKX_ERR_ARG and the session keeps its setting.  Like "out_rate", one
  *                 setting per session, followed by every waveform entry point (kkx_infer, _batch, _batch_voices,
  *                 _batch_pcm16, _batch_g711, _batch_flac, coalesced and kkx_submit batches, kkx_run_staged /
- *                 kkx_fetch_staged) for runs that start after the call.  Each item (utterance) is measured and scaled
- *                 on its own, on its 24 kHz model waveform x (n samples), before resampling and integer conversion, so
- *                 it gets the same gain at every "out_rate":
+ *                 kkx_fetch_staged, kkx_infer_programs) for runs that start after the call.  Each item (utterance), or
+ *                 program of kkx_infer_programs, is measured and scaled on its own, on its 24 kHz model waveform x
+ *                 (n samples), before resampling and integer conversion, so it gets the same gain at every "out_rate":
  *                 1. K-weighting (ITU-R BS.1770-4): two biquads designed in double at fs = 24000 with libebur128's
  *                    analog parameters and the bilinear transform, K = tan(pi f0 / fs) -- shelf f0 =
  *                    1681.974450955533 Hz, G = 3.999843853973347 dB, Q = 0.7071752369554196, Vb = Vh^0.4996667741545416;
@@ -292,20 +339,22 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                    follow from that value by their rules above, so an item with undefined L comes back bit-identical
  *                    to normalisation off.  The measurement runs in fp32 on the device (the filter restarted from zero
  *                    state 4800 samples before each 2400-sample segment, sums in double); values and bits of an item
- *                    do not depend on its batch, frame group or pass.  Not provided: one loudness across several items
- *                    (program loudness of a request split into chunks), lookahead limiting or compression, measurement
+ *                    do not depend on its batch, frame group or pass.  One loudness across several items (program
+ *                    loudness of a request split into chunks) is kkx_infer_programs.  Not provided: lookahead
+ *                    limiting or compression, measurement
  *                    at the output rate, momentary / short-term loudness and loudness range, a measure-only mode.
  * kkx_get_stat keys: "launches", "last_frames", "gpu_us", "precision", "coalesced_batches",
  * "coalesced_requests", "coalesced_largest", "async_batches", "async_requests", "frame_groups",
  * "group_first:<g>" (first item of frame group g of the last run), "weights_sessions" (sessions sharing this
  * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate", "loudness_target",
- * "true_peak_max", "loudness_items" (items kkx_last_loudness reports now; 0 if it would fail with KKX_ERR_STATE). */
+ * "true_peak_max", "loudness_items" (items -- programs after kkx_infer_programs -- kkx_last_loudness reports now; 0
+ * if it would fail with KKX_ERR_STATE). */
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value);
 KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "last_frames", "gpu_us" ... */
 
 /* What loudness normalisation measured and applied in the last SYNCHRONOUS call on the ctx (kkx_infer without
  * "coalesce", kkx_infer_batch and its _voices / _pcm16 / _g711 / _flac forms, kkx_run_staged), in item order, over
- * every pass of a "max_tokens" split.  Per item: lufs = integrated loudness L (NaN when undefined), true_peak_dbtp =
+ * every pass of a "max_tokens" split; after kkx_infer_programs, in program order (one entry per program).  Per item: lufs = integrated loudness L (NaN when undefined), true_peak_dbtp =
  * 20 log10 tp of the unscaled item (-inf for silence), gain = the applied g.  Each pointer is nullable and receives
  * `batch` floats.  KKX_ERR_STATE if no synchronous call has completed or that call ran with "loudness_target" = 0;
  * KKX_ERR_ARG if `batch` is not that call's item count.  Coalesced callers and kkx_submit batches are normalised

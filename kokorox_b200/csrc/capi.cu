@@ -486,15 +486,17 @@ KKX_API int kkx_infer_batch_voices(kkx_ctx* ctx, int32_t batch, const int64_t* t
   });
 }
 
-// The encoded entry points (kkx_infer_batch_pcm16 / _g711 / _flac): one pass of the staged batch with `enc`, its
-// encoded bytes in a pooled pinned buffer (caller holds ctx->mu; throws).
+// The encoded entry points (kkx_infer_batch_pcm16 / _g711 / _flac, kkx_infer_programs): one pass of the staged batch
+// with `enc` and the program table (empty: one item per program), its bytes in a pooled pinned buffer (caller holds
+// ctx->mu; throws).
 static void* infer_encoded_locked(kkx_ctx* ctx, Encoding enc, int32_t batch, const int64_t* tokens,
                                   const int32_t* tok_offsets, const float* styles, const float* speeds,
-                                  int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+                                  int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur,
+                                  const std::vector<int>& programs = {}) {
   Model& m = *ctx->model;
   m.stage(batch, tokens, tok_offsets, styles, speeds);
   loud_begin(ctx);
-  m.run(enc);
+  m.run(enc, programs);
   loud_note(ctx);
   const long long n = m.encoded_bytes();
   size_t cap = 0;
@@ -557,6 +559,31 @@ KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tok
 }
 
 KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes) { kkx_release(ctx, reinterpret_cast<float*>(bytes)); }
+
+KKX_API int kkx_infer_programs(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                               const float* styles, const float* speeds, int32_t n_programs,
+                               const int32_t* program_offsets, int32_t encoding, void** out_bytes,
+                               int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+  int rc = check_ctx(ctx);
+  if (rc) return rc;
+  if (out_bytes) *out_bytes = nullptr;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(ctx, [&] {
+    // every check before the batch is staged: a rejected call leaves the session as it was
+    if (!out_bytes) throw ArgError("out_bytes is null");
+    if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
+    if (encoding < KKX_ENC_F32 || encoding > KKX_ENC_FLAC)
+      throw ArgError("encoding must be in 0..4 (KKX_ENC_F32 .. KKX_ENC_FLAC), got " + std::to_string(encoding));
+    if (batch < 1) throw ArgError("batch must be >= 1");
+    check_programs(batch, n_programs, program_offsets);
+    static const Encoding enc[] = {Encoding::F32, Encoding::PCM16, Encoding::ULAW, Encoding::ALAW, Encoding::FLAC};
+    *out_bytes = infer_encoded_locked(ctx, enc[encoding], batch, tokens, tok_offsets, styles, speeds, out_byte_offsets,
+                                      out_sample_offsets, out_pred_dur,
+                                      std::vector<int>(program_offsets, program_offsets + n_programs + 1));
+  });
+}
+
+KKX_API void kkx_release_programs(kkx_ctx* ctx, void* bytes) { kkx_release(ctx, static_cast<float*>(bytes)); }
 
 // ---- output containers: host-side byte work (little-endian host assumed, as everywhere in this library)
 static void put_u16(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }

@@ -762,29 +762,37 @@ void Model::stage_voices(int B, const int64_t* tokens, const int32_t* tok_offset
   staged_ = true;
 }
 
+void check_programs(int B, int P, const int32_t* p) {
+  if (P < 1 || P > B) throw ArgError("n_programs must be in 1.." + std::to_string(B) + " (got " + std::to_string(P) + ")");
+  if (!p) throw ArgError("program_offsets is null");
+  if (p[0] != 0 || p[P] != B) throw ArgError("program_offsets must start at 0 and end at the batch size");
+  for (int k = 0; k < P; k++)
+    if (p[k + 1] <= p[k]) throw ArgError("program_offsets must be strictly increasing (no empty program)");
+}
+
+namespace {
+long long bytes_per_sample(Encoding e) {
+  return e == Encoding::F32 ? sizeof(float) : e == Encoding::ULAW || e == Encoding::ALAW ? 1 : sizeof(short);
+}
+}  // namespace
+
 long long Model::encoded_bytes() const {
   if (!ran_) return 0;
-  switch (enc_) {
-    case Encoding::PCM16: return total_samples_ * (long long)sizeof(short);
-    case Encoding::ULAW: case Encoding::ALAW: return total_samples_;
-    case Encoding::FLAC: return flac_off_[B_];
-    default: return 0;
-  }
+  return enc_ == Encoding::FLAC ? flac_off_[n_prog()] : total_samples_ * bytes_per_sample(enc_);
 }
 
 void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
                           int32_t* pred_dur) {
   if (!ran_) throw StateError("no completed run to fetch from");
-  if (enc_ == Encoding::F32) throw ArgError("the last run produced no encoded output");
   fetch(nullptr, 0, sample_offsets, pred_dur);
   if (byte_offsets)
-    for (int b = 0; b <= B_; b++)
-      byte_offsets[b] = enc_ == Encoding::FLAC ? flac_off_[b] : sample_off_[b] * (enc_ == Encoding::PCM16 ? 2 : 1);
+    for (int k = 0; k <= n_prog(); k++)
+      byte_offsets[k] = enc_ == Encoding::FLAC ? flac_off_[k] : sample_off_[k] * bytes_per_sample(enc_);
   if (dst) {
     const long long n = encoded_bytes();
     if (capacity_bytes < n) throw ArgError("output buffer too small");
-    KKX_CUDA(cudaMemcpyAsync(dst, enc_ == Encoding::FLAC ? flacA_.base() : twinA_.base(), (size_t)n,
-                             cudaMemcpyDeviceToHost, stream_));
+    const void* src = enc_ == Encoding::FLAC ? flacA_.base() : enc_ == Encoding::F32 ? audioA_.base() : twinA_.base();
+    KKX_CUDA(cudaMemcpyAsync(dst, src, (size_t)n, cudaMemcpyDeviceToHost, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
   }
 }
@@ -812,10 +820,11 @@ void Model::prepare_resample() {
 }
 
 void Model::fetch(float* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur) {
-  if (!ran_ || B_ <= 0 || (int)sample_off_.size() != B_ + 1) throw StateError("no completed run to fetch from");
+  if (!ran_ || B_ <= 0 || n_prog() < 1 || (int)sample_off_.size() != n_prog() + 1)
+    throw StateError("no completed run to fetch from");
   KKX_CUDA(cudaSetDevice(device_));
   if (sample_offsets)
-    for (int b = 0; b <= B_; b++) sample_offsets[b] = sample_off_[b];
+    for (int k = 0; k <= n_prog(); k++) sample_offsets[k] = sample_off_[k];
   if (pred_dur) {
     size_t k = 0;
     for (int b = 0; b < B_; b++)
@@ -837,11 +846,19 @@ void Model::grow(Arena& a, size_t bytes) {
 }
 
 // ============================================================================ forward
-void Model::run(Encoding enc) {
+void Model::run(Encoding enc, const std::vector<int>& programs) {
   if (!staged_ || B_ <= 0) throw StateError("no batch staged");
+  if (!programs.empty()) check_programs(B_, (int)programs.size() - 1, programs.data());
   KKX_CUDA(cudaSetDevice(device_));
   ran_ = false;
   enc_ = enc;
+  if (programs.empty()) {
+    prog_.resize(B_ + 1);
+    for (int b = 0; b <= B_; b++) prog_[b] = b;
+  } else {
+    prog_ = programs;
+  }
+  const int P = n_prog();
   use_lane(0);
   prepare_resample();
   g_launch_stats = &stats;
@@ -871,69 +888,81 @@ void Model::run(Encoding enc) {
     throw;
   }
 
-  // frame-phase groups under the frame budget; sample counts at the output rate: item b has ceil(600 T_b U / D)
-  sample_off_.assign(B_ + 1, 0);
-  long long tot = 0, ns = 0;
+  // Items lie back to back in the run's 24 kHz waveform (600 T_b samples each), so a program is contiguous there.
+  // Sample counts at the output rate are per program: program k of n_k samples at 24 kHz has ceil(n_k U / D).
+  s24_off_.assign(B_ + 1, 0);
+  long long tot = 0;
   for (int b = 0; b < B_; b++) {
-    sample_off_[b] = ns;
     tot += r.T[b];
-    ns += (600LL * r.T[b] * rs_U_ + rs_D_ - 1) / rs_D_;
+    s24_off_[b + 1] = s24_off_[b] + 600LL * r.T[b];
   }
-  sample_off_[B_] = ns;
-  total_samples_ = ns;
+  sample_off_.assign(P + 1, 0);
+  for (int k = 0; k < P; k++) {
+    const long long n24 = s24_off_[prog_[k + 1]] - s24_off_[prog_[k]];
+    sample_off_[k + 1] = sample_off_[k] + (n24 * rs_U_ + rs_D_ - 1) / rs_D_;
+  }
+  total_samples_ = sample_off_[P];
   last_frames = tot;
   grow(audioA_, (size_t)total_samples_ * sizeof(float));
   r.audio = audioA_.alloc<float>(total_samples_);
   if (enc != Encoding::F32) {
-    const size_t bytes = (size_t)total_samples_ * (enc == Encoding::ULAW || enc == Encoding::ALAW ? 1 : sizeof(short));
+    const size_t bytes = (size_t)total_samples_ * bytes_per_sample(enc);
     grow(twinA_, bytes);
     r.twin = twinA_.alloc_bytes(bytes);
   }
-  if (loud_) {
-    grow(loudA_, (size_t)B_ * 3 * sizeof(float));
-    r.loud = loudA_.alloc<float>((size_t)B_ * 3);
+  if (resample_) {
+    grow(wav24A_, (size_t)s24_off_[B_] * sizeof(float));
+    r.wav24 = wav24A_.alloc<float>(s24_off_[B_]);
   }
-  // FLAC: the encoder's tables -- sample offsets, frames per item (4096 samples each) as a prefix, item byte offsets
-  // -- and its output, ready before the forward pass so that the encoder follows it without a host round trip
+  if (loud_) {
+    grow(loudA_, (size_t)P * 3 * sizeof(float));
+    r.loud = loudA_.alloc<float>((size_t)P * 3);
+  }
+  // FLAC: the encoder's tables -- sample offsets, frames per program (4096 samples each) as a prefix, program byte
+  // offsets -- and its output, ready before the forward pass so that the encoder follows it without a host round trip
   struct { int F = 0; long long *soff = nullptr, *ioff = nullptr; int* foff = nullptr; void* work = nullptr;
            unsigned char* out = nullptr; } fl;
   if (enc == Encoding::FLAC) {
-    std::vector<int> foff(B_ + 1, 0);
-    for (int b = 0; b < B_; b++) {
-      const long long nf = flac_frames(sample_off_[b + 1] - sample_off_[b]);
-      if (foff[b] + nf > 0x7FFFFFFFLL) throw ArgError("batch too long for one FLAC encode");
-      foff[b + 1] = foff[b] + (int)nf;
+    std::vector<int> foff(P + 1, 0);
+    for (int k = 0; k < P; k++) {
+      const long long n = sample_off_[k + 1] - sample_off_[k];
+      if (n > kMaxFlacSamples) throw ArgError("program too long for one FLAC stream (2^36 - 1 samples at most)");
+      const long long nf = flac_frames(n);
+      if (foff[k] + nf > 0x7FFFFFFFLL) throw ArgError("batch too long for one FLAC encode");
+      foff[k + 1] = foff[k] + (int)nf;
     }
-    fl.F = foff[B_];
-    const size_t bound = (size_t)flac_bound(B_, fl.F, total_samples_);
+    fl.F = foff[P];
+    const size_t bound = (size_t)flac_bound(P, fl.F, total_samples_);
     grow(flacA_, bound);
     fl.out = flacA_.alloc<unsigned char>(bound);
-    grow(flacTabA_, 3 * ((size_t)(B_ + 1) * sizeof(long long) + 256) + flac_work_bytes(fl.F));
-    fl.soff = flacTabA_.alloc<long long>(B_ + 1);
-    fl.foff = flacTabA_.alloc<int>(B_ + 1);
-    fl.ioff = flacTabA_.alloc<long long>(B_ + 1);
+    grow(flacTabA_, 3 * ((size_t)(P + 1) * sizeof(long long) + 256) + flac_work_bytes(fl.F));
+    fl.soff = flacTabA_.alloc<long long>(P + 1);
+    fl.foff = flacTabA_.alloc<int>(P + 1);
+    fl.ioff = flacTabA_.alloc<long long>(P + 1);
     fl.work = flacTabA_.alloc_bytes(flac_work_bytes(fl.F));
-    upload(fl.soff, sample_off_.data(), (size_t)(B_ + 1) * sizeof(long long));
-    upload(fl.foff, foff.data(), (size_t)(B_ + 1) * sizeof(int));
+    upload(fl.soff, sample_off_.data(), (size_t)(P + 1) * sizeof(long long));
+    upload(fl.foff, foff.data(), (size_t)(P + 1) * sizeof(int));
   }
   h_loud_.clear();
   sink_filled_ = false;
   float* sink = (host_sink && !debug_) ? host_sink(total_samples_) : nullptr;
   // (both streams are idle here: the previous run synchronised them, and the outputs were sized above)
   try {
-    int b0 = 0;
+    int b0 = 0, k0 = 0;
     while (b0 < B_) {
       int b1 = b0; long long fr = 0;
       // at most 512 items per group: the fused generator kernels keep per-item tables in shared memory, and a
       // batch must take the same code path as a single call (results are bit-identical either way)
       while (b1 < B_ && b1 - b0 < 512 && (b1 == b0 || fr + r.T[b1] <= opt.max_frames)) { fr += r.T[b1]; b1++; }
       group_first_.push_back(b0);
+      int k1 = k0;   // programs [k0, k1) end in this group
+      while (k1 < P && prog_[k1 + 1] <= b1) k1++;
       // size the arena with a dry run of the same allocation sequence (no launches, no copies)
       frA_.reset();
       frA_.set_virtual(true);
       g_dry_run = true;
       try {
-        frame_phase(r, b0, b1, true);
+        frame_phase(r, b0, b1, k0, k1, true);
       } catch (...) {
         g_dry_run = false; frA_.set_virtual(false);
         throw;
@@ -946,32 +975,33 @@ void Model::run(Encoding enc) {
         frA_.reserve(need + need / 8 + (1 << 20));
       }
       frA_.reset();
-      frame_phase(r, b0, b1, false);
-      if (sink) {   // this group's audio goes to the host while the next group computes
-        const long long s0 = sample_off_[b0], s1 = sample_off_[b1];
+      frame_phase(r, b0, b1, k0, k1, false);
+      if (sink && k1 > k0) {   // the programs this group completed go to the host while the next group computes
+        const long long s0 = sample_off_[k0], s1 = sample_off_[k1];
         KKX_CUDA(cudaEventRecord(ev_grp_, stream_));
         KKX_CUDA(cudaStreamWaitEvent(copy_stream_, ev_grp_, 0));
         if (s1 > s0)
           KKX_CUDA(cudaMemcpyAsync(sink + s0, r.audio + s0, (size_t)(s1 - s0) * sizeof(float), cudaMemcpyDeviceToHost, copy_stream_));
       }
       b0 = b1;
+      k0 = k1;
     }
     KKX_CUDA(cudaEventRecord(ev1_, stream_));
     if (enc == Encoding::FLAC) {
-      launch_flac(static_cast<const short*>(r.twin), fl.soff, fl.foff, B_, fl.F, opt.out_rate, fl.work, fl.out, fl.ioff,
+      launch_flac(static_cast<const short*>(r.twin), fl.soff, fl.foff, P, fl.F, opt.out_rate, fl.work, fl.out, fl.ioff,
                   stream_);
-      flac_off_.assign(B_ + 1, 0);
-      KKX_CUDA(cudaMemcpyAsync(flac_off_.data(), fl.ioff, (size_t)(B_ + 1) * sizeof(long long),
+      flac_off_.assign(P + 1, 0);
+      KKX_CUDA(cudaMemcpyAsync(flac_off_.data(), fl.ioff, (size_t)(P + 1) * sizeof(long long),
                                cudaMemcpyDeviceToHost, stream_));
     }
     KKX_CUDA(cudaStreamSynchronize(stream_));
     if (sink) { KKX_CUDA(cudaStreamSynchronize(copy_stream_)); sink_filled_ = true; }
-    if (loud_) {   // [3][B] on the device -> item-major on the host
-      std::vector<float> rows((size_t)B_ * 3);
+    if (loud_) {   // [3][P] on the device -> program-major on the host
+      std::vector<float> rows((size_t)P * 3);
       KKX_CUDA(cudaMemcpy(rows.data(), r.loud, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
       h_loud_.resize(rows.size());
-      for (int b = 0; b < B_; b++)
-        for (int k = 0; k < 3; k++) h_loud_[(size_t)b * 3 + k] = rows[(size_t)k * B_ + b];
+      for (int k = 0; k < P; k++)
+        for (int j = 0; j < 3; j++) h_loud_[(size_t)k * 3 + j] = rows[(size_t)j * P + k];
     }
   } catch (...) {
     cudaStreamSynchronize(stream_);

@@ -204,6 +204,13 @@ class WeightSet {
 constexpr float kMinSpeed = 0.1f, kMaxSpeed = 10.f;   // dur per token <= 50 / speed <= 500 frames
 constexpr int kMaxItemFrames = 65536;                  // one utterance: <= 27 min of audio (120*T+1 rows fit int32;
                                                        // at out_rate 48000: 1 200 samples per frame, 7.9e7 per utterance)
+// A program (kkx_infer_programs) has no frame cap of its own: its sample offsets, lengths and segment indices are 64-bit
+// in every kernel that reads them.  Its FLAC stream counts samples in STREAMINFO's 36-bit field.
+constexpr long long kMaxFlacSamples = (1LL << 36) - 1;
+
+// A program table: item offsets p[0 .. P] of P runs of consecutive items, p[0] = 0, p[P] = B, strictly increasing.
+// Throws ArgError otherwise.
+void check_programs(int B, int P, const int32_t* p);
 
 // What a run returns besides the f32 waveform, which every run writes: its 16-bit PCM twin, the G.711 codes of that
 // PCM (mu-law / A-law), or one FLAC stream per item encoded from it (kkx.h).
@@ -229,17 +236,20 @@ class Model {
   std::function<float*(long long)> host_sink;
   bool sink_filled() const { return sink_filled_; }
   // A FLAC run launches the encoder (kernels_flac.cu) after the forward pass: gpu_us does not include it.
-  void run(Encoding enc = Encoding::F32);
+  // programs: the run's program table (check_programs, P + 1 item offsets); every output -- sample offsets, the
+  // encoded bytes, FLAC streams, loudness -- is per program, a program being one utterance whose 24 kHz waveform is
+  // the concatenation of its items' (kkx.h, kkx_infer_programs).  Empty = one item per program.
+  void run(Encoding enc = Encoding::F32, const std::vector<int>& programs = {});
   long long total_samples() const { return total_samples_; }
-  // The f32 waveform of the last run, whatever its encoding.
+  // The f32 waveform of the last run, whatever its encoding; sample_offsets [P + 1] per program.
   void fetch(float* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
-  // The encoded output of the last run (ArgError after an F32 run): 2 bytes per sample for PCM16, 1 for G.711, the
-  // FLAC streams back to back.  byte_offsets [B + 1] locate each item's bytes.
+  // The output of the last run in its encoding: 4 bytes per sample for F32, 2 for PCM16, 1 for G.711, the FLAC
+  // streams back to back.  byte_offsets [P + 1] locate each program's bytes.
   long long encoded_bytes() const;
   void fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
                      int32_t* pred_dur);
-  // Loudness of the last run's items (kernels_loudness.cu): true if that run normalised; then last_loudness() holds
-  // 3 B floats, per item b at 3 b: integrated loudness (LUFS, NaN = undefined), true peak (dBTP), applied gain.
+  // Loudness of the last run's programs (kernels_loudness.cu): true if that run normalised; then last_loudness()
+  // holds 3 P floats, per program k at 3 k: integrated loudness (LUFS, NaN = undefined), true peak (dBTP), gain.
   bool loudness_ran() const { return ran_ && loud_; }
   const std::vector<float>& last_loudness() const { return h_loud_; }
 
@@ -272,7 +282,8 @@ class Model {
     Level styL;                // one item of B rows (style FC GEMMs)
     float* audio = nullptr;    // [total_samples_] the f32 waveform at the output rate
     void* twin = nullptr;      // its 16-bit PCM (PCM16, FLAC) or G.711 (ULAW, ALAW) twin
-    float* loud = nullptr;     // [3][B] lufs | dBTP | gain of loudness normalisation; the gain feeds the resampling
+    float* loud = nullptr;     // [3][P] lufs | dBTP | gain of loudness normalisation; the gain feeds the resampling
+    float* wav24 = nullptr;    // resampling pass only: the run's 24 kHz waveform, item b at s24_off_[b]
   };
   // Linear / Conv1d on the precision-critical path: split-TF32 tensor cores when precision==1 and
   // the weight has a TcW32, fp32 SIMT otherwise.
@@ -316,7 +327,8 @@ class Model {
   void token_issue(Run& r);          // every token-rate launch + the D2H of frame counts / durations (no sync)
   void token_finish(Run& r);         // sync, read T_b, validate
   size_t token_arena_bytes() const;
-  void frame_phase(Run& r, int b0, int b1, bool dry);
+  // items [b0, b1); programs [k0, k1) are those whose last item is in the group (post-processed after it)
+  void frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry);
   void adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ldx, const Level& Lin,
                  const Level& Lout, const float* sty, int sld, float* out, int ldo, int ocol,
                  bool dry);
@@ -368,18 +380,23 @@ class Model {
   // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC streams, their
   // per-item byte offsets (host) and the encoder's tables and scratch
   Encoding enc_ = Encoding::F32;
-  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_;
+  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_, wav24A_;
   std::vector<long long> flac_off_;
+  // program table of the current run (P + 1 item offsets); s24_off_ [B + 1]: each item's offset in the run's 24 kHz
+  // waveform, where a program is contiguous
+  std::vector<int> prog_;
+  std::vector<long long> s24_off_;
+  int n_prog() const { return (int)prog_.size() - 1; }
   void grow(Arena& a, size_t bytes);
   // output resampling of the current run (opt.out_rate): U / D, half length H; d_taps_ holds the filter of taps_rate_
   bool resample_ = false; int rs_U_ = 1, rs_D_ = 1, rs_H_ = 0;
   float* d_taps_ = nullptr; int taps_rate_ = 0;
   void prepare_resample();
-  // loudness normalisation of the current run; h_loud_ = the host copy of Run::loud (item-major)
+  // loudness normalisation of the current run; h_loud_ = the host copy of Run::loud (program-major)
   bool loud_ = false; LoudParams loud_par_{};
   std::vector<float> h_loud_;
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
-  std::vector<long long> sample_off_;
+  std::vector<long long> sample_off_;                                      // [P + 1] at the output rate
   int* h_pred_dur_ = nullptr; size_t h_pred_dur_cap_ = 0;                  // pinned: per-row integer durations of the last run
   int* h_T_ = nullptr; size_t h_T_cap_ = 0;                                // pinned: frames per item
   long long total_samples_ = 0;

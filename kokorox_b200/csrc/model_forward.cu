@@ -565,7 +565,7 @@ void Model::arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L,
 
 // ------------------------------------------------------------------------------------------
 // Frame phase for items [b0, b1): length regulation, F0/N, decoder, generator, iSTFT.
-void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
+void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   use_lane(0);
   cudaStream_t st = stream_;
   Arena& A = frA_;
@@ -586,50 +586,56 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
   const int* cum = r.cum + (size_t)b0 * 512;
   const float* sty_pro = r.sty_pro + (size_t)b0 * W.sty_pro_n;
   const float* sty_dec = r.sty_dec + (size_t)b0 * W.sty_dec_n;
-  // curve (F0 / N) offsets: element offsets == FR2 row offsets (ld 1); phase offsets; sample offsets
+  // curve (F0 / N) offsets: element offsets == FR2 row offsets (ld 1); phase offsets; group-local sample offsets of
+  // the harmonic source (s_loc); each item's offset in the run's 24 kHz waveform (s24)
   std::vector<int> ph_off(B);
-  std::vector<long long> s_loc(B), s_glob(B);
+  std::vector<long long> s_loc(B);
   {
     int po = 0; long long so = 0;
     for (int b = 0; b < B; b++) {
       ph_off[b] = po; po += 9 * T2[b];
       s_loc[b] = so; so += 600LL * T[b];
-      s_glob[b] = sample_off_[b0 + b];
     }
   }
   int* d_ph_off = A.alloc<int>(B);
   long long* d_s_loc = A.alloc<long long>(B);
-  long long* d_s_glob = A.alloc<long long>(B);
+  long long* d_s24 = A.alloc<long long>(B);
   upload(d_ph_off, ph_off.data(), B * sizeof(int));
   upload(d_s_loc, s_loc.data(), B * sizeof(long long));
-  upload(d_s_glob, s_glob.data(), B * sizeof(long long));
-  // output resampling: the iSTFT writes the group's 24 kHz audio here (group-local offsets s_loc), the resampling
-  // pass reads it and writes r.audio at the output-rate offsets s_glob
-  float* wav24 = nullptr;
-  long long* d_s_len = nullptr;
+  upload(d_s24, s24_off_.data() + b0, B * sizeof(long long));
+  // output resampling: the iSTFT writes each item into r.wav24 at its run-wide offset, so that a program is one
+  // contiguous span there; once a program's last item is done (programs [k0, k1) here) the resampling pass reads
+  // the span (p_in, p_len) and writes r.audio at the program's output-rate offset (p_out)
+  const int K = k1 - k0;
+  long long *d_p_in = nullptr, *d_p_len = nullptr, *d_p_out = nullptr;
   long long max_out = 0, max_len24 = 0;
-  // loudness normalisation: per-item 2400-sample segment energies (offsets seg_off) and true-peak scratch
+  // loudness normalisation: per-program 2400-sample segment energies (offsets seg_off) and true-peak scratch
   long long* d_seg_off = nullptr;
   float* energy = nullptr;
   unsigned* peak = nullptr;
-  if (resample_) {
-    std::vector<long long> s_len(B), seg_off(B);
+  if (resample_ && K > 0) {
+    std::vector<long long> p_in(K), p_len(K), p_out(K), seg_off(K);
     long long nseg = 0;
-    for (int b = 0; b < B; b++) {
-      s_len[b] = 600LL * T[b];
-      max_out = std::max(max_out, (s_len[b] * rs_U_ + rs_D_ - 1) / rs_D_);
-      max_len24 = std::max(max_len24, s_len[b]);
-      seg_off[b] = nseg;
-      nseg += s_len[b] / kLoudSeg;
+    for (int k = 0; k < K; k++) {
+      p_in[k] = s24_off_[prog_[k0 + k]];
+      p_len[k] = s24_off_[prog_[k0 + k + 1]] - p_in[k];
+      p_out[k] = sample_off_[k0 + k];
+      max_out = std::max(max_out, sample_off_[k0 + k + 1] - p_out[k]);
+      max_len24 = std::max(max_len24, p_len[k]);
+      seg_off[k] = nseg;
+      nseg += p_len[k] / kLoudSeg;
     }
-    wav24 = A.alloc<float>((size_t)(s_loc[B - 1] + s_len[B - 1]));
-    d_s_len = A.alloc<long long>(B);
-    upload(d_s_len, s_len.data(), B * sizeof(long long));
+    d_p_in = A.alloc<long long>(K);
+    d_p_len = A.alloc<long long>(K);
+    d_p_out = A.alloc<long long>(K);
+    upload(d_p_in, p_in.data(), K * sizeof(long long));
+    upload(d_p_len, p_len.data(), K * sizeof(long long));
+    upload(d_p_out, p_out.data(), K * sizeof(long long));
     if (loud_) {
-      d_seg_off = A.alloc<long long>(B);
+      d_seg_off = A.alloc<long long>(K);
       energy = A.alloc<float>((size_t)std::max(nseg, 1LL));
-      peak = A.alloc<unsigned>(B);
-      upload(d_seg_off, seg_off.data(), B * sizeof(long long));
+      peak = A.alloc<unsigned>(K);
+      upload(d_seg_off, seg_off.data(), K * sizeof(long long));
     }
   }
 
@@ -928,19 +934,22 @@ void Model::frame_phase(Run& r, int b0, int b1, bool dry) {
   capture("conv_post", cp, 24, 0, 22, G120, b0);
   const bool law = enc_ == Encoding::ULAW || enc_ == Encoding::ALAW;
   short* pcm = enc_ == Encoding::PCM16 || enc_ == Encoding::FLAC ? static_cast<short*>(r.twin) : nullptr;
-  if (!resample_) {
-    launch_istft(cp, 24, G120.d_off, G120.d_len, r.audio, pcm, d_s_glob, opt.precision == 1, B, G120.max_len, st);
+  if (!resample_) {   // the output is the 24 kHz waveform: program layout == item layout
+    launch_istft(cp, 24, G120.d_off, G120.d_len, r.audio, pcm, d_s24, opt.precision == 1, B, G120.max_len, st);
     return;
   }
-  launch_istft(cp, 24, G120.d_off, G120.d_len, wav24, nullptr, d_s_loc, opt.precision == 1, B, G120.max_len, st);
+  launch_istft(cp, 24, G120.d_off, G120.d_len, r.wav24, nullptr, d_s24, opt.precision == 1, B, G120.max_len, st);
+  if (K == 0) return;   // every program of this group goes on into the next
+  const int P = n_prog();
   float* gain = nullptr;
   if (loud_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
-    gain = r.loud + 2 * (size_t)B_ + b0;
-    launch_loudness(wav24, d_s_loc, d_s_len, d_seg_off, loud_par_, energy, peak, r.loud + b0, r.loud + B_ + b0, gain,
-                    B, max_len24, st);
+    gain = r.loud + 2 * (size_t)P + k0;
+    launch_loudness(r.wav24, d_p_in, d_p_len, d_seg_off, loud_par_, energy, peak, r.loud + k0, r.loud + P + k0, gain,
+                    K, max_len24, st);
   }
-  launch_resample(wav24, d_s_loc, d_s_len, d_s_glob, d_taps_, rs_U_, rs_D_, rs_H_, gain, r.audio, pcm,
-                  law ? static_cast<unsigned char*>(r.twin) : nullptr, enc_ == Encoding::ALAW ? 1 : 0, B, max_out, st);
+  // grids span the longest program (64-bit sample indices); CTAs past a shorter program's end return at once
+  launch_resample(r.wav24, d_p_in, d_p_len, d_p_out, d_taps_, rs_U_, rs_D_, rs_H_, gain, r.audio, pcm,
+                  law ? static_cast<unsigned char*>(r.twin) : nullptr, enc_ == Encoding::ALAW ? 1 : 0, K, max_out, st);
 }
 
 }  // namespace kkx

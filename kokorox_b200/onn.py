@@ -74,6 +74,10 @@ def load_library(path: Optional[str] = None):
         lib.kkx_infer_batch_flac.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), P(P(u8)), P(i64), P(i64), P(i32)]
         lib.kkx_release_flac.argtypes = [vp, P(u8)]
         lib.kkx_release_flac.restype = None
+        lib.kkx_infer_programs.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), i32, P(i32), i32, P(vp), P(i64),
+                                           P(i64), P(i32)]
+        lib.kkx_release_programs.argtypes = [vp, vp]
+        lib.kkx_release_programs.restype = None
         lib.kkx_wav_header_pcm16.argtypes = [P(C.c_uint8), i64, i32]
         lib.kkx_wav_header_f32_stream.argtypes = [P(C.c_uint8), i32, i32]
         lib.kkx_encode_wav16_base64.argtypes = [P(i16), i64, i32, C.c_char_p, i64]
@@ -506,9 +510,47 @@ class B200Koko:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
 
+    # encoding name -> (KKX_ENC_* code, element type of the returned arrays; None = one ``bytes`` per program)
+    _ENCODINGS = {"f32": (0, C.c_float), "pcm16": (1, C.c_int16), "ulaw": (2, C.c_uint8), "alaw": (3, C.c_uint8),
+                  "flac": (4, None)}
+
+    def infer_programs(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
+                       program_offsets: Sequence[int], encoding: str = "f32", return_durations: bool = False):
+        """One output per program (kkx_infer_programs): program k is items [program_offsets[k],
+        program_offsets[k + 1]), synthesised as ONE utterance whose 24 kHz waveform is the concatenation of its items'
+        -- the chunks of one long request, as koko.rs splits and joins them.  Loudness, resampling and FLAC apply to
+        the program as a whole.  ``encoding``: "f32" / "pcm16" / "ulaw" / "alaw" give one float32 / int16 / uint8
+        array per program (views into a library-owned buffer, released like infer_batch's), "flac" one ``bytes`` file
+        per program."""
+        self._require()
+        if encoding not in self._ENCODINGS:
+            raise KkxError(-1, f"encoding must be one of {sorted(self._ENCODINGS)}, got {encoding!r}")
+        code, ctype = self._ENCODINGS[encoding]
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
+        prog = np.ascontiguousarray(np.asarray(program_offsets, dtype=np.int32).reshape(-1))
+        P = max(prog.size - 1, 0)
+        buf = C.c_void_p()
+        boff = np.zeros(P + 1, dtype=np.int64)
+        dur = np.zeros(int(offs[-1]), dtype=np.int32)
+        self._check(self._lib.kkx_infer_programs(
+            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
+            _fp(st), _fp(sp), P, prog.ctypes.data_as(C.POINTER(C.c_int32)), code, C.byref(buf),
+            boff.ctypes.data_as(C.POINTER(C.c_int64)), None, dur.ctypes.data_as(C.POINTER(C.c_int32))))
+        if ctype is None:
+            try:
+                outs = [C.string_at(buf.value + int(boff[k]), int(boff[k + 1] - boff[k])) for k in range(P)]
+            finally:
+                self._lib.kkx_release_programs(self._ctx, buf)
+        else:
+            outs = self._adopt(C.cast(buf, C.POINTER(ctype)), boff // C.sizeof(ctype))
+        if return_durations:
+            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
+        return outs
+
     def last_loudness(self):
         """What loudness normalisation (option ``loudness_target``) measured and applied in this session's last
-        synchronous call: ``(lufs, true_peak_dbtp, gain)``, three float32 arrays in item order (``lufs`` is NaN where
+        synchronous call: ``(lufs, true_peak_dbtp, gain)``, three float32 arrays in item order -- program order after
+        ``infer_programs`` -- (``lufs`` is NaN where
         the loudness is undefined: items under 400 ms, silence).  Raises KkxError when that call ran with the option
         off.  Coalesced and ``submit`` batches are not reported."""
         self._require()
