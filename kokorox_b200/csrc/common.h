@@ -36,9 +36,9 @@ struct StateError : std::runtime_error {   // call sequence error (nothing stage
     }                                                                                       \
   } while (0)
 
-// Kernel-variant switches read from the environment exist only in experiment builds (-DKKX_EXPERIMENTS, e.g.
-// KKX_NVCC_EXTRA=-DKKX_EXPERIMENTS python -m kokorox_b200.build --force): the production library always takes the
-// measured-best path, so no environment variable can change which kernel runs or what it computes.
+// Diagnostic switches read from the environment (role cycle counters, perf-experiment masks) exist only in experiment
+// builds (-DKKX_EXPERIMENTS, e.g. KKX_NVCC_EXTRA=-DKKX_EXPERIMENTS python -m kokorox_b200.build --force): in the
+// production library no environment variable can change which kernel runs or what it computes.
 #ifdef KKX_EXPERIMENTS
 inline bool env_flag(const char* name, bool dflt) {
   const char* e = getenv(name);
@@ -189,8 +189,8 @@ struct Level {
   int* d_off = nullptr;  // device copies
   int* d_len = nullptr;
   // prefix sums (B+1) of the per-item tile counts for 128- and 256-row tiles (persistent kernels)
-  int* d_tiles128 = nullptr; int* d_tiles256 = nullptr; int* d_tiles512 = nullptr;
-  int ntiles128 = 0, ntiles256 = 0, ntiles512 = 0;
+  int* d_tiles128 = nullptr; int* d_tiles256 = nullptr;
+  int ntiles128 = 0, ntiles256 = 0;
 };
 
 constexpr int kGapRows = 32;  // >= largest conv halo (k=11, dil=5 -> 25)

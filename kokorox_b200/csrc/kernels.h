@@ -41,9 +41,10 @@ struct TcConvArgs {
   const void* tmB = nullptr;
   const void* tmA2 = nullptr; // split-TF32 mode: the "lo" planes
   const void* tmB2 = nullptr;
-  const void* tmB_c = nullptr;   // split-TF32 cluster mode: weight maps with half-height boxes (BN/2 rows)
-  const void* tmB2_c = nullptr;
-  int cluster = 1;               // CTAs per cluster along M sharing each weight tile by TMA multicast (1 or 2)
+  const void* tmB_c = nullptr;   // weight maps with half-height boxes: a CTA's half of the weight tile in the CTA-pair
+  const void* tmB2_c = nullptr;  // kernels, and the 64-wide tiles of the small-problem split-precision kernel
+  int debug = 0;  // KKX_TC_DEBUG bit mask (perf experiments): 1 skip global stores, 2 skip MMA issue, 4 skip TMEM loads
+                  // (placed here, it keeps wscale / eact 8-byte aligned: the epilogue reads them with one 64-bit load)
   int tf32 = 0;               // 1 = split-precision operands (hi / lo planes), nprod products (3 or 4)
   int nprod = 3;
   int f16 = 0;                // split planes are fp16 (2 B, 64 K-elements per 128-byte span) instead of tf32-in-fp32:
@@ -77,8 +78,7 @@ struct TcConvArgs {
   int nphase = 1;
   int phase_pad[10] = {0};
   int phase_oro[10] = {0};
-  int phase_loop = 0;            // Co = 128 only: one CTA per m-tile loops over the phases (conv_tc_multi_kernel<.., PH>)
-  int debug = 0;  // KKX_TC_DEBUG bit mask (perf experiments): 1 skip global stores, 2 skip MMA issue, 4 skip TMEM loads
+  int phase_loop = 0;            // Co = 128 only: one CTA per m-tile loops over the phases (conv_tc_multi_kernel)
 };
 void launch_conv_tc(const TcConvArgs& a, cudaStream_t st);
 // true when launch_conv_tc will run the CTA-pair kernel for these arguments (the only kernel that honours out_hi / out_lo)
@@ -126,7 +126,7 @@ struct ArbConvArgs {
   const void* tmB = nullptr;                           // host pointer to the weight CUtensorMap (bf16 [C][ks*C], box [C,64])
   int C = 0, ks = 1, dil = 1, pad = 0;
   const int* off = nullptr; const int* len = nullptr;  // Level (device)
-  const int* tile_start = nullptr;                     // [B+1] prefix sum of ceil(len/arb_tile_rows(C, ks))
+  const int* tile_start = nullptr;                     // [B+1] prefix sum of ceil(len/arb_tile_rows(C))
   int B = 1; int total_tiles = 0; long long sum_m = 0;
   const float* bias = nullptr;
   __nv_bfloat16* out_bf16 = nullptr;                   // y (+res) as bf16, unscaled (nullable)
@@ -143,7 +143,7 @@ struct ArbConvArgs {
   // zero-padded to C output channels, fp32 output [rows, ldo] of the first `cout` channels, no statistics
   int post = 0, cout = 0, ldo = 0; float slope = 0.f;
 };
-int arb_tile_rows(int C, int ks);   // rows per persistent-kernel tile for this shape (128, 256 or 512)
+int arb_tile_rows(int C);   // rows per persistent-kernel tile: 256 at C = 128 (transposed accumulator), 128 at C = 256
 bool arb_conv_supported(int C, int ks, int dil, int B);
 void launch_arb_conv(const ArbConvArgs& a, cudaStream_t st);
 

@@ -61,14 +61,21 @@ constexpr int kArbMaxB = 512;
 //     coalesced across the warp (32 channels = 128 contiguous bytes per row), so the epilogue needs no smem
 //     transpose and no barrier, the bias is a per-thread scalar, and the AdaIN statistics are plain
 //     per-thread sums (no shuffles); the freed smem holds a third operand slot.
-template <int BN, int MSUB, bool T>
+// C = 256 keeps rows as M: 128-row tiles with a smem-transposed epilogue.  At C = 128 the transposed accumulator and the
+// branch-free operand transform together took arb_conv from 104 to 93 ms per B = 64 step against rows as M
+// (profiles/r1_step_b64_fused_v9_detail.txt).  512-row tiles at C = 128 (two 128x256 MMAs per weight tile, halving the
+// weight re-streaming; the two accumulators fill TMEM, so the epilogue no longer overlaps the next tile's MMAs) were no
+// net win on 5.7 M rows: conv1 k7 1.40 -> 1.25 ms, conv1 k11 unchanged, conv2 k7 / k11 1.65 -> 1.81 / 1.81 -> 2.19 ms.
+template <int BN>
 struct ArbCfg {
+  static constexpr bool T = BN == 128;                      // transposed accumulator
+  static constexpr int MSUB = T ? 2 : 1;                    // 128-row sub-tiles per tile
   static constexpr int KCH = BN / 64;                       // 64-channel chunks
   static constexpr int RA = MSUB * 128 + 56;                // rows per A slot (halo <= 2*25, 8-row granule)
   static constexpr uint32_t A_SLOT = RA * 128;              // bytes (multiple of 1024)
-  static constexpr int NA = (BN == 128 && (!T || MSUB == 4)) ? 2 : 3;   // A slots
+  static constexpr int NA = 3;                              // A slots
   static constexpr uint32_t B_STAGE = BN * 128;             // bytes
-  static constexpr int NB = (T && MSUB == 4) ? 4 : (BN == 128) ? 6 : 3;   // B stages
+  static constexpr int NB = T ? 6 : 3;                      // B stages
   static constexpr int PITCH = 36;                          // floats per staged epilogue row
   static constexpr uint32_t STG = T ? 0 : 2 * 128 * PITCH * 4;   // one transpose buffer per epilogue group
   static constexpr uint32_t STAT = 4 * BN * 2 * 4;          // per-quadrant column sums
@@ -115,20 +122,16 @@ struct TileCur {
 // iteration moves 10 B: conv1 reads bf16 x (SB = 1), conv2 reads the bf16 residual and writes either the next bf16 x
 // (SB = 1) or -- last iteration -- the fp32 block output (SB = 2).  The AdaIN statistics still come from the fp32
 // accumulator, before any rounding.
-template <int BN, int MSUB, bool CONV2, bool T, bool POST = false, int SB = 0, bool PB = false>
+template <int BN, bool CONV2, bool POST = false, int SB = 0, bool PB = false>
 __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_constant__ CUtensorMap tmB, ArbConvArgs a) {
+  using Cfg = ArbCfg<BN>;
+  constexpr bool T = Cfg::T;
+  constexpr int MSUB = Cfg::MSUB;
   static_assert(SB == 0 || (!POST && (CONV2 || SB == 1)), "stream-bf16 variants: conv1 SB=1, conv2 SB=1 (bf16 out) / SB=2 (fp32 out)");
-  static_assert(!PB || (T && !CONV2 && !POST && SB == 0 && MSUB == 2), "balanced-producer variant: conv1, transposed accumulator, fp32 input");
+  static_assert(!PB || (T && !CONV2 && !POST && SB == 0), "balanced-producer variant: conv1, transposed accumulator, fp32 input");
   constexpr bool XIN_BF = CONV2 || SB != 0;          // element type of the operand the producers read
   constexpr bool OUT_BF = !CONV2 || SB == 1;         // epilogue writes bf16 (conv1 always; conv2 when the stream stays bf16)
-  static_assert(!T || (BN == 128 && (MSUB == 2 || MSUB == 4)), "transposed mode: C = 128, 256- or 512-row tiles");
-  static_assert(!POST || (T && !CONV2 && MSUB == 2), "post variant: transposed accumulator, fp32 input");
-  // T with MSUB = 4 (k >= 7): 512-row tiles, i.e. TWO 128x256 MMAs per weight tile.  The k = 7 / 11 convs are
-  // bound by what an SM can ingest from L2 (the weight set is re-streamed for every tile: 352 KB per tile at
-  // k = 11); doubling the rows per weight tile halves that.  The two accumulators fill TMEM, so the epilogue
-  // of tile i no longer overlaps the MMAs of tile i+1 (the producers still run ahead) -- measured: not a net win
-  // (see arb_variant), kept as an opt-in variant.
-  constexpr int NBUF = (T && MSUB == 4) ? 1 : 2;
+  static_assert(!POST || (T && !CONV2), "post variant: transposed accumulator, fp32 input");
   // Warp split between epilogue and operand producers (14 warps besides TMA and MMA): 8 + 6.  A 4 + 10 split for
   // conv1 in transposed mode (trivial epilogue, producer-bound) was measured: no gain (1.14 / 1.35 / 1.61 ms vs
   // 1.20 / 1.29 / 1.63 ms at k = 3 / 7 / 11) -- the producers are limited by the shared-memory port they share
@@ -140,7 +143,6 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
   constexpr int NPW = PB ? 8 : 14 - NEW;                    // producer warps
   constexpr int kProdThreads = NPW * 32;
   constexpr int kProdRows = kProdThreads / 8;               // rows per producer pass (24 or 32: multiples of 8)
-  using Cfg = ArbCfg<BN, MSUB, T>;
   constexpr int KCH = Cfg::KCH, NA = Cfg::NA, NB = Cfg::NB, PITCH = Cfg::PITCH;
   constexpr int MT = MSUB * 128;
   extern __shared__ uint8_t smem_raw[];
@@ -230,8 +232,8 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
       for (int tile = t_begin; tile < t_end; tile++, ti++) {
         const int rem = s_len[cur.b] - cur.mt * MT;         // rows of this item left from the tile start
         (void)rem;
-        const int buf = NBUF == 2 ? (ti & 1) : 0;
-        mbar_wait(tempty(buf), (NBUF == 2 ? (((uint32_t)(ti >> 1)) & 1u) : ((uint32_t)ti & 1u)) ^ 1u);
+        const int buf = ti & 1;
+        mbar_wait(tempty(buf), (((uint32_t)(ti >> 1)) & 1u) ^ 1u);
         tc_fence_after();
         TICK(0);
 #pragma unroll 1
@@ -253,15 +255,11 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
             if (T) {
               // D[co, row] += W[co, k] * Act[row + tap*dil, k]: weights = M operand, 256 rows = N operand
               constexpr uint32_t idescT = umma_idesc_bf16(128, 256);
-              const uint64_t wd = bd;
+              const uint64_t xd = umma_desc_sw128(slot + (uint32_t)(tap * dil) * 128u);
+              const uint32_t td = tmem_base + (uint32_t)(buf * 256);
 #pragma unroll
-              for (int s2 = 0; s2 < MSUB / 2; s2++) {
-                const uint64_t xd = umma_desc_sw128(slot + (uint32_t)(s2 * 256 + tap * dil) * 128u);
-                const uint32_t td = tmem_base + (uint32_t)(buf * 256 + s2 * 256);
-#pragma unroll
-                for (int k = 0; k < 4; k++)
-                  if (!ARB_DBG(a, 8)) umma_bf16(td, wd + (uint64_t)(2 * k), xd + (uint64_t)(2 * k), idescT, (c | tap | k) ? 1u : 0u);
-              }
+              for (int k = 0; k < 4; k++)
+                if (!ARB_DBG(a, 8)) umma_bf16(td, bd + (uint64_t)(2 * k), xd + (uint64_t)(2 * k), idescT, (c | tap | k) ? 1u : 0u);
             } else {
 #pragma unroll
               for (int sub = 0; sub < MSUB; sub++) {
@@ -337,12 +335,12 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
       const int b = cur.b;
       const int L = s_len[b], off = s_off[b];
       const int m0 = cur.mt * MT;
-      const int buf = NBUF == 2 ? (ti & 1) : 0;
+      const int buf = ti & 1;
       cur.next(s_ts);                       // cur now names the NEXT tile (prefetch target)
       const bool has_next = tile + 1 < t_end;
       const int nL = has_next ? s_len[cur.b] : 0, noff = has_next ? s_off[cur.b] : 0, nm0 = cur.mt * MT;
       TICK(8);
-      mbar_wait(tfull(buf), NBUF == 2 ? (((uint32_t)(ti >> 1)) & 1u) : ((uint32_t)ti & 1u));
+      mbar_wait(tfull(buf), ((uint32_t)(ti >> 1)) & 1u);
       tc_fence_after();
       TICK(0);
       float2 s2 = make_float2(0.f, 0.f), q2 = s2;
@@ -752,32 +750,21 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
   }
 }
 
-template <int BN, int MSUB, bool CONV2, bool T, bool POST = false, int SB = 0, bool PB = false>
+template <int BN, bool CONV2, bool POST = false, int SB = 0, bool PB = false>
 void launch_arb_t(const ArbConvArgs& a, cudaStream_t st) {
-  using Cfg = ArbCfg<BN, MSUB, T>;
+  using Cfg = ArbCfg<BN>;
   static DevOnce once;
   int dev = 0;
   cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(arb_conv_kernel<BN, MSUB, CONV2, T, POST, SB, PB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM)); });
+  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(arb_conv_kernel<BN, CONV2, POST, SB, PB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM)); });
   const int nsm = device_sm_count(dev);
   const int grid = a.total_tiles < nsm ? a.total_tiles : nsm;
-  arb_conv_kernel<BN, MSUB, CONV2, T, POST, SB, PB><<<grid, kArbThreads, Cfg::SMEM, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmB), a);
+  arb_conv_kernel<BN, CONV2, POST, SB, PB><<<grid, kArbThreads, Cfg::SMEM, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmB), a);
 }
 
 }  // namespace
 
-// kernel variant per shape: 0 = rows as M (C = 256, or C = 128 with KKX_ARB_NOT=1), 1 = transposed with 256-row
-// tiles, 2 = transposed with 512-row tiles (k >= 7: halves the weight re-streaming the k = 7/11 convs are bound by)
-static int arb_variant(int C, int ks) {
-  static const bool no_t = env_flag("KKX_ARB_NOT", false);
-  // 512-row tiles measured on B200 (5.7 M rows): conv1 k7 1.40 -> 1.25 ms, conv1 k11 unchanged, conv2 k7 / k11
-  // 1.65 -> 1.81 / 1.81 -> 2.19 ms (losing the epilogue/MMA overlap costs more than the halved weight stream
-  // saves; ncu shows the tensor pipe already 75 % active at k = 11).  Opt-in: KKX_ARB_512=1.
-  static const bool use_512 = env_flag("KKX_ARB_512", false);
-  if (C != 128 || no_t) return 0;
-  return (ks >= 7 && use_512) ? 2 : 1;
-}
-int arb_tile_rows(int C, int ks) { return C == 128 ? (arb_variant(C, ks) == 2 ? 512 : 256) : 128; }
+int arb_tile_rows(int C) { return (C == 128 ? ArbCfg<128>::MSUB : ArbCfg<256>::MSUB) * 128; }
 
 bool arb_conv_supported(int C, int ks, int dil, int B) {
   return (C == 128 || C == 256) && ks >= 1 && dil >= 1 && dil * (ks - 1) <= 50 && (ks & 1) && B <= kArbMaxB;
@@ -792,7 +779,7 @@ void launch_arb_conv(const ArbConvArgs& a, cudaStream_t st) {
         a.ldo < a.cout || !(a.slope > 0.f && a.slope < 1.f))
       throw ArgError("launch_arb_conv: unsupported post-conv arguments");
     if (g_launch_stats) g_launch_stats->conv_flops += 2.0 * (double)a.sum_m * a.C * a.cout * a.ks;
-    launch_arb_t<128, 2, false, true, true>(a, st);
+    launch_arb_t<128, false, true>(a, st);
     post_launch("post_conv", st);
     return;
   }
@@ -802,13 +789,11 @@ void launch_arb_conv(const ArbConvArgs& a, cudaStream_t st) {
   if (conv2 ? (!a.in_bf16 || (a.out_f32 != nullptr) == (a.out_bf16 != nullptr) || (a.out_bf16 && (!a.res_bf16 || a.accumulate)))
             : (!a.out_bf16 || a.out_f32 || a.accumulate || a.res_bf16))
     throw ArgError("launch_arb_conv: unsupported input/output combination");
-  const int variant = arb_variant(a.C, a.ks);
 #ifdef KKX_EXPERIMENTS
   static const int dbg = env_int("KKX_ARB_DBG", 0);
   if (dbg && !a.debug) { ArbConvArgs d = a; d.debug = dbg; launch_arb_conv(d, st); return; }
 #endif
   const bool stream_bf = conv2 ? a.res_bf16 != 0 : a.in_bf16 != 0;
-  if (stream_bf && !(variant == 1 || a.C == 256)) throw ArgError("launch_arb_conv: the bf16 stream needs the default kernel variants");
   if (g_launch_stats) {
     const double fl = 2.0 * (double)a.sum_m * a.C * a.C * a.ks;
     g_launch_stats->conv_flops += fl;
@@ -819,27 +804,20 @@ void launch_arb_conv(const ArbConvArgs& a, cudaStream_t st) {
   }
   if (stream_bf) {
     if (a.C == 128) {
-      if (!conv2) launch_arb_t<128, 2, false, true, false, 1>(a, st);
-      else if (a.out_bf16) launch_arb_t<128, 2, true, true, false, 1>(a, st);
-      else launch_arb_t<128, 2, true, true, false, 2>(a, st);
+      if (!conv2) launch_arb_t<128, false, false, 1>(a, st);
+      else if (a.out_bf16) launch_arb_t<128, true, false, 1>(a, st);
+      else launch_arb_t<128, true, false, 2>(a, st);
     } else {
-      if (!conv2) launch_arb_t<256, 1, false, false, false, 1>(a, st);
-      else if (a.out_bf16) launch_arb_t<256, 1, true, false, false, 1>(a, st);
-      else launch_arb_t<256, 1, true, false, false, 2>(a, st);
+      if (!conv2) launch_arb_t<256, false, false, 1>(a, st);
+      else if (a.out_bf16) launch_arb_t<256, true, false, 1>(a, st);
+      else launch_arb_t<256, true, false, 2>(a, st);
     }
-  } else if (variant == 2) {
-    if (a.in_bf16) launch_arb_t<128, 4, true, true>(a, st); else launch_arb_t<128, 4, false, true>(a, st);
-  } else if (variant == 1) {
+  } else if (a.C == 128) {
     // conv1: 4 epilogue + 8 producer warps, two producer warps on every scheduler -- measured against 8 + 6 on one box
     // (profiles/r2_arb_balanced_producers_v32.txt): k = 3 1.45 -> 1.15 ms, k = 7 1.50 -> 1.25 ms, k = 11 unchanged
-    static const bool pb = env_flag("KKX_ARB_PB", true);
-    if (a.in_bf16) launch_arb_t<128, 2, true, true>(a, st);
-    else if (pb) launch_arb_t<128, 2, false, true, false, 0, true>(a, st);
-    else launch_arb_t<128, 2, false, true>(a, st);
-  } else if (a.C == 128) {
-    if (a.in_bf16) launch_arb_t<128, 2, true, false>(a, st); else launch_arb_t<128, 2, false, false>(a, st);
+    if (a.in_bf16) launch_arb_t<128, true>(a, st); else launch_arb_t<128, false, false, 0, true>(a, st);
   } else {
-    if (a.in_bf16) launch_arb_t<256, 1, true, false>(a, st); else launch_arb_t<256, 1, false, false>(a, st);
+    if (a.in_bf16) launch_arb_t<256, true>(a, st); else launch_arb_t<256, false>(a, st);
   }
   if (g_launch_stats && g_launch_stats->profile && g_launch_stats->detail) {
     char nm[96]; snprintf(nm, sizeof nm, "arb_conv[c%d k%d d%d %s%s m%lld]", a.C, a.ks, a.dil, conv2 ? "conv2" : "conv1", stream_bf ? " sb" : "", a.sum_m);

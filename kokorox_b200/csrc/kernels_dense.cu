@@ -398,97 +398,8 @@ void launch_copy_row(float* u, int C, int dst_row, int src_row, const int* off, 
 }
 
 // ------------------------------------------------------------------------------------------
-// ALBERT self-attention (12 heads x 64), flash-style online softmax in fp32.
-// Block = 8 warps, 32 query rows (4 per warp); keys/values streamed in chunks of 64 via smem.
-__global__ void __launch_bounds__(256) attention_kernel(const float* __restrict__ qkv,
-                                                        float* __restrict__ ctx, const int* off,
-                                                        const int* len) {
-  __shared__ float Ks[64][65];
-  __shared__ float Vs[64][64];
-  __shared__ float Qs[32][64];
-  const int b = blockIdx.z, h = blockIdx.y;
-  const int N = len[b];
-  const int q0 = blockIdx.x * 32;
-  if (q0 >= N) return;
-  const size_t base = (size_t)off[b];
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  for (int i = tid; i < 32 * 64; i += 256) {
-    const int r = i >> 6, d = i & 63;
-    Qs[r][d] = (q0 + r < N) ? qkv[(base + q0 + r) * 2304 + h * 64 + d] : 0.f;
-  }
-  float m[4], l[4], o0[4], o1[4];
-#pragma unroll
-  for (int r = 0; r < 4; r++) { m[r] = -INFINITY; l[r] = 0.f; o0[r] = 0.f; o1[r] = 0.f; }
-
-  for (int k0 = 0; k0 < N; k0 += 64) {
-    __syncthreads();
-    for (int i = tid; i < 64 * 64; i += 256) {
-      const int j = i >> 6, d = i & 63;
-      const bool ok = k0 + j < N;
-      Ks[j][d] = ok ? qkv[(base + k0 + j) * 2304 + 768 + h * 64 + d] : 0.f;
-      Vs[j][d] = ok ? qkv[(base + k0 + j) * 2304 + 1536 + h * 64 + d] : 0.f;
-    }
-    __syncthreads();
-    float s0[4] = {0.f, 0.f, 0.f, 0.f}, s1[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll 8
-    for (int d = 0; d < 64; d++) {
-      const float ka = Ks[lane][d], kb = Ks[lane + 32][d];
-#pragma unroll
-      for (int r = 0; r < 4; r++) {
-        const float qv = Qs[warp * 4 + r][d];
-        s0[r] = fmaf(qv, ka, s0[r]);
-        s1[r] = fmaf(qv, kb, s1[r]);
-      }
-    }
-    const bool v0 = k0 + lane < N, v1 = k0 + lane + 32 < N;
-    float pr0[4], pr1[4];
-#pragma unroll
-    for (int r = 0; r < 4; r++) {
-      const float a0 = v0 ? s0[r] * 0.125f : -INFINITY;
-      const float a1 = v1 ? s1[r] * 0.125f : -INFINITY;
-      float cm = fmaxf(a0, a1);
-#pragma unroll
-      for (int o = 16; o; o >>= 1) cm = fmaxf(cm, __shfl_xor_sync(0xffffffffu, cm, o));
-      const float mn = fmaxf(m[r], cm);
-      const float p0 = expf(a0 - mn), p1 = expf(a1 - mn);
-      float ps = p0 + p1;
-#pragma unroll
-      for (int o = 16; o; o >>= 1) ps += __shfl_xor_sync(0xffffffffu, ps, o);
-      const float corr = expf(m[r] - mn);
-      l[r] = l[r] * corr + ps;
-      o0[r] *= corr; o1[r] *= corr;
-      m[r] = mn;
-      pr0[r] = p0;
-      pr1[r] = p1;
-    }
-#pragma unroll 4
-    for (int j = 0; j < 32; j++) {
-      const float va = Vs[j][lane], vb = Vs[j][lane + 32];
-      const float vc = Vs[j + 32][lane], vd = Vs[j + 32][lane + 32];
-#pragma unroll
-      for (int r = 0; r < 4; r++) {
-        const float pa = __shfl_sync(0xffffffffu, pr0[r], j);
-        const float pb = __shfl_sync(0xffffffffu, pr1[r], j);
-        o0[r] = fmaf(pa, va, o0[r]);
-        o1[r] = fmaf(pa, vb, o1[r]);
-        o0[r] = fmaf(pb, vc, o0[r]);
-        o1[r] = fmaf(pb, vd, o1[r]);
-      }
-    }
-  }
-#pragma unroll
-  for (int r = 0; r < 4; r++) {
-    const int q = q0 + warp * 4 + r;
-    if (q < N) {
-      const float inv = 1.0f / l[r];
-      ctx[(base + q) * 768 + h * 64 + lane] = o0[r] * inv;
-      ctx[(base + q) * 768 + h * 64 + lane + 32] = o1[r] * inv;
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// Tensor-core variant: flash attention with split-TF32 ("3xTF32") products on mma.sync m16n8k8, which
+// ALBERT self-attention (12 heads x 64), flash-style online softmax in fp32, with split-TF32 ("3xTF32") products on
+// mma.sync m16n8k8, which
 // keeps fp32-grade accuracy (this path feeds the duration predictor, whose integer durations must match
 // the fp32 oracle bit-exactly) at several times the fp32 SIMT rate.  Attention is ~0.5 % of the model's
 // FLOPs, with d = 64 and N <= 512: the warp-level MMA with register fragments fits it better than a
@@ -665,26 +576,20 @@ __global__ void __launch_bounds__(NW * 32) attention_tc_kernel(const float* __re
 void launch_attention(const float* qkv, float* ctx, const int* off, const int* len, int B,
                       int max_len, cudaStream_t st) {
   if (g_dry_run) return;
-  static const bool simt = env_flag("KKX_ATT_SIMT", false);
-  if (simt) {
-    dim3 g((max_len + 31) / 32, 12, B);
-    attention_kernel<<<g, 256, 0, st>>>(qkv, ctx, off, len);
+  constexpr int smem = 4 * 64 * kAttLd * 4;
+  static DevOnce once;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  once.run(dev, [] {
+    KKX_CUDA(cudaFuncSetAttribute(attention_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    KKX_CUDA(cudaFuncSetAttribute(attention_tc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  });
+  if (max_len > 64) {   // 128 query rows per CTA: the K/V staging (load + tf32 split) is amortised over twice the MMAs
+    dim3 g((max_len + 127) / 128, 12, B);
+    attention_tc_kernel<8><<<g, 256, smem, st>>>(qkv, ctx, off, len);
   } else {
-    constexpr int smem = 4 * 64 * kAttLd * 4;
-    static DevOnce once;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    once.run(dev, [] {
-      KKX_CUDA(cudaFuncSetAttribute(attention_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      KKX_CUDA(cudaFuncSetAttribute(attention_tc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    });
-    if (max_len > 64) {   // 128 query rows per CTA: the K/V staging (load + tf32 split) is amortised over twice the MMAs
-      dim3 g((max_len + 127) / 128, 12, B);
-      attention_tc_kernel<8><<<g, 256, smem, st>>>(qkv, ctx, off, len);
-    } else {
-      dim3 g((max_len + 63) / 64, 12, B);
-      attention_tc_kernel<4><<<g, 128, smem, st>>>(qkv, ctx, off, len);
-    }
+    dim3 g((max_len + 63) / 64, 12, B);
+    attention_tc_kernel<4><<<g, 128, smem, st>>>(qkv, ctx, off, len);
   }
   post_launch("attention", st);
 }

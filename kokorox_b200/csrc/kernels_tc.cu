@@ -101,10 +101,9 @@ __device__ __forceinline__ float gelu_new_f(float v) {
 // pair of tf32-exact fp32 planes (hi, lo = a - hi), D += Ahi*Bhi + Alo*Bhi + Ahi*Blo [+ Alo*Blo] on
 // kind::tf32, which recovers ~fp32 accuracy on the tensor cores for the precision-critical
 // predictor path (ALBERT -> durations, F0/N).
-// CL > 1 (split-TF32 GEMMs): a cluster of CL CTAs along M shares every weight (B) tile -- each CTA fetches
-// 1/CL of its rows and multicasts them to all CTAs of the cluster, which cuts the L2->SM operand traffic
-// these GEMMs are bound by (4 fp32 planes per stage) by 25 % at CL = 2.
-template <int BN, int STAGES, int MODE, int CL>
+// Clusters of 2 CTAs along M sharing each weight tile by TMA multicast were measured not faster for the
+// split-TF32 GEMMs (13.9 vs 12.4 ms for the 12 QKV GEMMs).
+template <int BN, int STAGES, int MODE>
 __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                                                       const __grid_constant__ CUtensorMap tmB,
                                                       const __grid_constant__ CUtensorMap tmA2,
@@ -134,20 +133,14 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
   const int b = blockIdx.z;
   const int mlen = a.m_len[b];
   // phase-fused launches put (phase, n-tile) on grid.x and the m-tile on grid.y
-  const bool fused = MODE == 0 && CL == 1 && a.nphase > 1;
+  const bool fused = MODE == 0 && a.nphase > 1;
   const int bx = fused ? blockIdx.y : blockIdx.x, by = fused ? blockIdx.x : blockIdx.y;
   const int m0 = bx * 128;
-  if (CL == 1) {
-    if (m0 >= mlen) return;  // CTA-uniform
-  } else {
-    if ((int)(blockIdx.x / CL) * CL * 128 >= mlen) return;  // cluster-uniform: a CTA past the end still feeds its peers
-  }
+  if (m0 >= mlen) return;  // CTA-uniform
   const int ntn = (a.Co + BN - 1) / BN;
   const int ph = fused ? by / ntn : 0;
   const int c_pad = fused ? a.phase_pad[ph] : a.pad;
   const int c_oro = fused ? a.phase_oro[ph] : a.oro;
-  const uint32_t crank = CL > 1 ? cluster_ctarank() : 0u;
-  constexpr uint16_t cmask = (uint16_t)((1u << CL) - 1u);
   const int n0 = (fused ? by - ph * ntn : by) * BN;
   const int wrow0 = ph * a.Co + n0;          // row of this tile in the (phase-stacked) weight map
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -161,7 +154,7 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
       asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA2) : "memory");
       asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB2) : "memory");
     }
-    for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), CL); }
+    for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     mbar_init(tfull_bar, 1);
     if (MODE) for (int j = 0; j < 3; j++) { mbar_init(bfull_bar(j), 1); mbar_init(bempty_bar(j), 4); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -173,7 +166,6 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();   // peers' barriers exist before any multicast / remote arrive can land
   tc_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
@@ -185,7 +177,7 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
       for (int it = 0; it < num_k; it++) {
         const int s = it % STAGES;
         const uint32_t ph = (uint32_t)(it / STAGES) & 1u;
-        mbar_wait(empty_bar(s), ph ^ 1u);   // CL > 1: every CTA of the cluster has drained this stage
+        mbar_wait(empty_bar(s), ph ^ 1u);
         TCT(0);
         const int tap = it / kchunks, c0 = (it - tap * kchunks) * KE;
         const uint32_t sa = base + s * STAGE_BYTES;
@@ -194,17 +186,8 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
         mbar_expect_tx(full_bar(s), STAGE_BYTES - (skipA2 ? A_BYTES : 0) - (skipB2 ? B_BYTES : 0));
         tma_load_2d(sa, &tmA, c0, row0 + tap * a.dil, full_bar(s));
         if (MODE && !skipA2) tma_load_2d(sa + A_BYTES, &tmA2, c0, row0 + tap * a.dil, full_bar(s));
-        if (CL == 1) {
-          tma_load_2d(sa + PLANES * A_BYTES, &tmB, tap * a.Cpad + c0, wrow0, full_bar(s));
-          if (MODE && !skipB2) tma_load_2d(sa + 2 * A_BYTES + B_BYTES, &tmB2, tap * a.Cpad + c0, wrow0, full_bar(s));
-        } else {
-          // this CTA's 1/CL of the weight rows (tmB / tmB2 have BN/CL-row boxes), multicast to the whole cluster
-          constexpr uint32_t SUB = (BN / CL) * 128;
-          tma_load_2d_mc(sa + PLANES * A_BYTES + crank * SUB, &tmB, tap * a.Cpad + c0, n0 + (int)crank * (BN / CL),
-                         full_bar(s), cmask);
-          if (MODE) tma_load_2d_mc(sa + 2 * A_BYTES + B_BYTES + crank * SUB, &tmB2, tap * a.Cpad + c0,
-                                   n0 + (int)crank * (BN / CL), full_bar(s), cmask);
-        }
+        tma_load_2d(sa + PLANES * A_BYTES, &tmB, tap * a.Cpad + c0, wrow0, full_bar(s));
+        if (MODE && !skipB2) tma_load_2d(sa + 2 * A_BYTES + B_BYTES, &tmB2, tap * a.Cpad + c0, wrow0, full_bar(s));
         TCT(1);
       }
       TCT_FLUSH(0, 2);
@@ -249,8 +232,7 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
           }
           if ((it & cs) == cs || it == num_k - 1) umma_commit(bfull_bar(j));  // chain complete
         }
-        if (CL == 1) umma_commit(empty_bar(s));  // frees the smem stage when these MMAs have read it
-        else umma_commit_mc(empty_bar(s), cmask);   // ... in every CTA of the cluster (they all write into it)
+        umma_commit(empty_bar(s));  // frees the smem stage when these MMAs have read it
         TCT(2);
       }
       umma_commit(tfull_bar);       // accumulator complete
@@ -380,7 +362,6 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();   // no CTA exits while a peer can still arrive on its barriers
   if (warp == 1) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
@@ -388,15 +369,13 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
 }
 
 // ------------------------------------------------------------------------------------------
-// Multi-tile variant (bf16): one CTA walks TPC consecutive 128-row tiles of one item.  The TMA/MMA
-// pipeline runs straight across tile boundaries and alternates between two TMEM accumulators, so
-// the epilogue of tile i (TMEM -> smem transpose -> global) overlaps the main loop of tile i+1, and
-// barrier init / TMEM allocation / descriptor prefetch are paid once per TPC tiles.
-// PH (phase-fused ConvTranspose1d, a.nphase two-tap phase convs): the CTA's "tiles" are the PHASES of ONE 128-row m-tile
-// (same activation rows, phase p's weights at rows [p*Co, (p+1)*Co) of the stacked map, output rows m*ors + phase_oro[p]):
-// barrier init / TMEM allocation / descriptor prefetch are paid once per a.nphase tiles, each phase's epilogue runs under
-// the next phase's loads and MMAs, and the activation tile of the later phases comes out of L2.
-template <int BN, int STAGES, int TPC, bool PH = false>
+// Phase-loop variant (bf16, phase-fused ConvTranspose1d with a.nphase two-tap phase convs): one CTA walks the PHASES of
+// ONE 128-row m-tile as consecutive tiles (same activation rows, phase p's weights at rows [p*Co, (p+1)*Co) of the
+// stacked map, output rows m*ors + phase_oro[p]).  The TMA/MMA pipeline runs straight across the phases and alternates
+// between two TMEM accumulators, so the epilogue of one phase (TMEM -> smem transpose -> global) runs under the next
+// phase's loads and MMAs, barrier init / TMEM allocation / descriptor prefetch are paid once per a.nphase tiles, and the
+// activation tile of the later phases comes out of L2.
+template <int BN, int STAGES>
 __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constant__ CUtensorMap tmA,
                                                             const __grid_constant__ CUtensorMap tmB,
                                                             TcConvArgs a) {
@@ -415,9 +394,9 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
 
   const int b = blockIdx.z;
   const int mlen = a.m_len[b];
-  const int m_base = PH ? blockIdx.x * 128 : blockIdx.x * (128 * TPC);
-  if (m_base >= mlen) return;  // CTA-uniform
-  const int ntiles = PH ? a.nphase : min(TPC, (mlen - m_base + 127) >> 7);
+  const int m0 = blockIdx.x * 128;
+  if (m0 >= mlen) return;  // CTA-uniform
+  const int ntiles = a.nphase;
   const int n0 = blockIdx.y * BN;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int kchunks = a.Cpad >> 6;
@@ -445,8 +424,8 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
     if (lane == 0) {
       int g = 0;
       for (int ti = 0; ti < ntiles; ti++) {
-        const int row0 = PH ? a.in_off[b] + m_base - a.phase_pad[ti] : a.in_off[b] + m_base + ti * 128 - a.pad;
-        const int wrow = PH ? ti * a.Co + n0 : n0;
+        const int row0 = a.in_off[b] + m0 - a.phase_pad[ti];
+        const int wrow = ti * a.Co + n0;
         for (int it = 0; it < num_k; it++, g++) {
           const int s = g % STAGES;
           const uint32_t ph = (uint32_t)(g / STAGES) & 1u;
@@ -493,8 +472,7 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
     const int c4 = (t & 7) << 2;
     int chunk_ctr = 0;
     for (int ti = 0; ti < ntiles; ti++) {
-      const int m0 = PH ? m_base : m_base + ti * 128;
-      const int oro = PH ? a.phase_oro[ti] : a.oro;
+      const int oro = a.phase_oro[ti];
       const int acc = ti & 1;
       auto fetch = [&](int c, float4* rv) {
         const int n = n0 + c + c4;
@@ -1038,9 +1016,8 @@ static void launch_gemm32p(const TcConvArgs& a, cudaStream_t st) {
   const int total = a.ntiles_m * ((a.Co + 127) / 128);
   const int grid = total < nsm ? total : nsm;
   TcConvArgs b = a;
-  static const int l2mb = env_int("KKX_TC_GROUP_MB", 24);
   const long long per_tile = 128LL * a.Cpad * (a.f16 ? 4 : 8);       // bytes of hi+lo planes of one m-tile
-  long long gm = (long long)l2mb * 1000000LL / (per_tile > 0 ? per_tile : 1);
+  long long gm = 24LL * 1000000LL / (per_tile > 0 ? per_tile : 1);
   if (gm < 8) gm = 8;
   if (gm > a.ntiles_m) gm = a.ntiles_m;
   b.group_m = (int)gm;
@@ -1069,17 +1046,20 @@ static void launch_gemm32p(const TcConvArgs& a, cudaStream_t st) {
 //     warps the accumulator ring was not drained for ~8 k cycles per tile and the MMA warp spent 13 of its 36 Mcycles
 //     per step waiting for a ring slot.)
 constexpr int kG2Stages = 3;
-// threads: TMA warp, MMA warp, 8 drain warps, NFIN final warps (6: 16 warps x 128 registers fill the register file --
-// registers are granted in steps of 32 per thread, so 18 warps would get 96; 4 is kept for A/B runs in experiment builds)
-constexpr int g2_threads(int nfin) { return (2 + 8 + nfin) * 32; }
+// final warps: 16 warps x 128 registers fill the register file (registers are granted in steps of 32 per thread, so 18
+// warps would get 96).  4 final warps measured slower: the GELU + plane split of the FFN GEMM (128 tanh per lane and
+// tile) and the transposed V pass of the QKV GEMM took longer than the tile's MMAs (ncu: tensor pipe 29 % / 38 % active
+// against 52 % for the plain GEMMs); the 89 split-precision GEMMs of a B = 64 step 25.7-25.8 ms against 23.3-23.9 ms
+// with 6 (profiles/r2_gemm_final_warps_ab_v29.txt).
+constexpr int kG2Fin = 6;
+constexpr int kG2Threads = (2 + 8 + kG2Fin) * 32;   // TMA warp, MMA warp, 8 drain warps, the final warps
 constexpr uint32_t kG2A = 128 * 128, kG2Bh = 64 * 128, kG2Stage = 2 * (kG2A + kG2Bh);
 constexpr uint32_t kG2Stg = 128 * 128 * 4;
 constexpr int kG2Smem = kG2Stages * (int)kG2Stage + (int)kG2Stg + 20 * 8 + 16 + 1024;
-template <int NFIN>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(g2_threads(NFIN), 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kG2Threads, 1)
 gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmBh,
                 const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB2h, TcConvArgs a) {
-  constexpr int BN = 128, STAGES = kG2Stages;
+  constexpr int BN = 128, STAGES = kG2Stages, NFIN = kG2Fin;
   constexpr int KE = 64;                                   // K elements per 128-byte span (fp16 planes); one chain per stage
   constexpr int NEPI = 8;
   extern __shared__ uint8_t smem_raw[];
@@ -1414,32 +1394,23 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   }
 }
 
-template <int NFIN>
-static void launch_gemm32p2_t(const TcConvArgs& a, cudaStream_t st) {
+static void launch_gemm32p2(const TcConvArgs& a, cudaStream_t st) {
   static DevOnce once;
   int dev = 0;
   cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(gemm32p2_kernel<NFIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, kG2Smem)); });
+  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(gemm32p2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kG2Smem)); });
   const int nsm = device_sm_count(dev);
   const int total = ((a.ntiles_m + 1) / 2) * ((a.Co + 127) / 128);
   int npairs = nsm / 2;
   if (npairs > total) npairs = total;
   TcConvArgs b = a;
-  static const int l2mb = env_int("KKX_TC_GROUP_MB", 24);
   const long long per_tile = 128LL * a.Cpad * 4;                      // bytes of the hi + lo planes of one m-tile
-  long long gm = (long long)l2mb * 1000000LL / (per_tile > 0 ? per_tile : 1);
+  long long gm = 24LL * 1000000LL / (per_tile > 0 ? per_tile : 1);
   if (gm < 8) gm = 8;
   if (gm > a.ntiles_m) gm = a.ntiles_m;
   b.group_m = (int)gm;
-  gemm32p2_kernel<NFIN><<<2 * npairs, g2_threads(NFIN), kG2Smem, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmA), *reinterpret_cast<const CUtensorMap*>(a.tmB_c),
-                                                                 *reinterpret_cast<const CUtensorMap*>(a.tmA2), *reinterpret_cast<const CUtensorMap*>(a.tmB2_c), b);
-}
-static void launch_gemm32p2(const TcConvArgs& a, cudaStream_t st) {
-  // 6 final warps: with 4, the GELU + plane split of the FFN GEMM (128 tanh per lane and tile) and the transposed V
-  // pass of the QKV GEMM took longer than the tile's MMAs (ncu: tensor pipe 29 % / 38 % active against 52 % for the
-  // plain GEMMs)
-  static const bool fin4 = env_flag("KKX_G2_FIN4", false);
-  if (fin4) launch_gemm32p2_t<4>(a, st); else launch_gemm32p2_t<6>(a, st);
+  gemm32p2_kernel<<<2 * npairs, kG2Threads, kG2Smem, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmA), *reinterpret_cast<const CUtensorMap*>(a.tmB_c),
+                                                         *reinterpret_cast<const CUtensorMap*>(a.tmA2), *reinterpret_cast<const CUtensorMap*>(a.tmB2_c), b);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1613,7 +1584,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
 // true when launch_conv_tc runs the bf16 CTA-pair kernel for these arguments (tmB_c: the weight map with 128-row boxes)
 static bool conv_tc_takes_pair_bf16(const TcConvArgs& a, int nsm) {
-  if (a.tf32 || !a.pair || !a.tmB_c || a.cluster > 1) return false;
+  if (a.tf32 || !a.pair || !a.tmB_c) return false;
   if (a.Co < 256 || a.Co % 256 != 0 || !a.tile_start || a.ntiles_m < 2) return false;
   return (long long)((a.ntiles_m + 1) / 2) * (a.Co / 256) * (a.nphase > 1 ? a.nphase : 1) >= nsm / 2;     // at least one tile per pair
 }
@@ -1638,50 +1609,39 @@ static void launch_conv_pair_t(const TcConvArgs& a, cudaStream_t st) {
 }
 static void launch_conv_pair(const TcConvArgs& a, cudaStream_t st) { launch_conv_pair_t<256>(a, st); }
 
-template <int BN, int STAGES, int TPC, bool PH = false>
+template <int BN, int STAGES>
 static void launch_tc_multi(const TcConvArgs& a, cudaStream_t st) {
   constexpr int smem = STAGES * (128 * 128 + BN * 128) + 2 * 128 * 36 * 4 + (2 * STAGES + 4) * 8 + 16 + 1024;
   static DevOnce once;
   int dev = 0;
   cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_tc_multi_kernel<BN, STAGES, TPC, PH>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
-  dim3 g(PH ? (a.max_m + 127) / 128 : (a.max_m + 128 * TPC - 1) / (128 * TPC), (a.Co + BN - 1) / BN, a.B);
-  conv_tc_multi_kernel<BN, STAGES, TPC, PH><<<g, 192, smem, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmA),
-                                                                 *reinterpret_cast<const CUtensorMap*>(a.tmB), a);
+  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_tc_multi_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
+  dim3 g((a.max_m + 127) / 128, (a.Co + BN - 1) / BN, a.B);
+  conv_tc_multi_kernel<BN, STAGES><<<g, 192, smem, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmA),
+                                                         *reinterpret_cast<const CUtensorMap*>(a.tmB), a);
 }
 
-template <int BN, int STAGES, int MODE, int CL = 1>
+template <int BN, int STAGES, int MODE>
 static void launch_tc(const TcConvArgs& a, cudaStream_t st) {
   constexpr int PLANES = MODE ? 2 : 1;
   constexpr int smem = STAGES * PLANES * (128 * 128 + BN * 128) + (2 * STAGES + 7) * 8 + 16 + 1024;
   static DevOnce once;
   int dev = 0;
   cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BN, STAGES, MODE, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
-  const unsigned gx = (unsigned)(((a.max_m + 127) / 128 + CL - 1) / CL * CL);
+  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BN, STAGES, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
+  const unsigned gx = (unsigned)((a.max_m + 127) / 128);
   dim3 g(gx, (a.Co + BN - 1) / BN, a.B);
-  if (MODE == 0 && CL == 1 && a.nphase > 1) g = dim3((unsigned)(a.nphase * ((a.Co + BN - 1) / BN)), gx, a.B);
+  if (MODE == 0 && a.nphase > 1) g = dim3((unsigned)(a.nphase * ((a.Co + BN - 1) / BN)), gx, a.B);
   const CUtensorMap* mA = reinterpret_cast<const CUtensorMap*>(a.tmA);
-  const CUtensorMap* mB = reinterpret_cast<const CUtensorMap*>(CL > 1 ? a.tmB_c : a.tmB);
+  const CUtensorMap* mB = reinterpret_cast<const CUtensorMap*>(a.tmB);
   const CUtensorMap* mA2 = reinterpret_cast<const CUtensorMap*>(a.tmA2 ? a.tmA2 : a.tmA);
-  const CUtensorMap* mB2 = reinterpret_cast<const CUtensorMap*>(CL > 1 ? a.tmB2_c : (a.tmB2 ? a.tmB2 : a.tmB));
-  if (CL == 1) {
-    conv_tc_kernel<BN, STAGES, MODE, CL><<<g, 192, smem, st>>>(*mA, *mB, *mA2, *mB2, a);
-  } else {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = g; cfg.blockDim = dim3(192, 1, 1); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    KKX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BN, STAGES, MODE, CL>, *mA, *mB, *mA2, *mB2, a));
-  }
+  const CUtensorMap* mB2 = reinterpret_cast<const CUtensorMap*>(a.tmB2 ? a.tmB2 : a.tmB);
+  conv_tc_kernel<BN, STAGES, MODE><<<g, 192, smem, st>>>(*mA, *mB, *mA2, *mB2, a);
 }
 
 bool conv_tc_takes_pair(const TcConvArgs& a) {
   if (!(a.tf32 && a.f16 && a.pair && a.nprod == 3 && a.tmA2 && a.tmB2 && a.tmB_c && a.tmB2_c)) return false;
-  if (!(a.Co > 64 && a.cluster < 2 && a.tile_start && a.ntiles_m >= 2)) return false;
-  if (!env_flag("KKX_TC_PERSIST", true)) return false;
+  if (!(a.Co > 64 && a.tile_start && a.ntiles_m >= 2)) return false;
   if (a.force_kernel == 0) {   // small problems take the 64-wide single-tile kernel (see launch_conv_tc)
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1706,8 +1666,6 @@ void launch_conv_tc(const TcConvArgs& a0, cudaStream_t st) {
   if (a.nphase > 1 && (a.tf32 || a.nphase > 10 || a.Co % tc_box_n(a.Co) != 0)) throw ArgError("launch_conv_tc: unsupported phase-fused shape");
   if (a.tf32) {
     // split-TF32: 4 operand planes per stage (64 KB at BN=128) -> 3 stages, one CTA per SM
-    static const bool bn64 = env_flag("KKX_TC_BN64", false);
-    static const bool persist = env_flag("KKX_TC_PERSIST", true);
     // Small problems (one utterance): fewer 128-wide tiles than SMs -> 64-wide single-tile CTAs fill twice as many
     // SMs and shorten the latency-bound launch (B=1, 510 tokens: 3.4 -> 2.8 ms over the 74 GEMMs of a step).  The
     // per-element accumulation order is the same in both kernels, so results do not depend on the choice.
@@ -1715,53 +1673,36 @@ void launch_conv_tc(const TcConvArgs& a0, cudaStream_t st) {
     cudaGetDevice(&cur_dev);
     const int nsm = device_sm_count(cur_dev);
     const long long tiles128 = (long long)(a.ntiles_m > 0 ? a.ntiles_m : (a.sum_m + 127) / 128) * ((a.Co + 127) / 128);
-    const bool small = tiles128 < nsm && a.tmB_c && a.tmB2_c && a.cluster < 2 && a.force_kernel == 0;
+    const bool small = tiles128 < nsm && a.tmB_c && a.tmB2_c && a.force_kernel == 0;
     if (a.Co > 64 && small) {
       TcConvArgs b = a; b.tmB = a.tmB_c; b.tmB2 = a.tmB2_c;
       launch_tc<64, 4, 1>(b, st);
-    } else if (a.Co > 64 && persist && a.cluster < 2 && a.tile_start && a.ntiles_m > 0 && a.tmA2 && a.tmB2) {
+    } else if (a.Co > 64 && a.tile_start && a.ntiles_m > 0 && a.tmA2 && a.tmB2) {
       // CTA pairs (cta_group::2) for the split-FP16 planes when the weight maps with 64-row boxes exist
       if (conv_tc_takes_pair(a)) launch_gemm32p2(a, st);
       else launch_gemm32p(a, st);
     }
-    else if (a.Co > 64 && a.cluster == 2 && a.tmB_c && a.tmB2_c) launch_tc<128, 3, 1, 2>(a, st);
-    else if (a.Co > 64 && !(bn64 && a.tmB_c)) launch_tc<128, 3, 1>(a, st);
-    else if (a.Co > 64) {   // experiment: 64-wide tiles (4 stages of 48 KB) with the half-height weight boxes
-      TcConvArgs b = a; b.tmB = a.tmB_c; b.tmB2 = a.tmB2_c;
-      launch_tc<64, 4, 1>(b, st);
-    } else launch_tc<64, 4, 1>(a, st);
+    else if (a.Co > 64) launch_tc<128, 3, 1>(a, st);
+    else launch_tc<64, 4, 1>(a, st);
     if (g_launch_stats && g_launch_stats->profile && g_launch_stats->detail) {
       char nm[96]; snprintf(nm, sizeof nm, "conv_tc_tf32x3[ci%d co%d k%d m%lld]", a.Ci, a.Co, a.ks, a.sum_m);
       post_launch(nm, st);
     } else post_launch("conv_tc_tf32x3", st);
     return;
   }
-  // Multi-tile CTAs (pipeline runs across tiles, double-buffered TMEM accumulators).  Measured on
-  // B200: NOT faster than 2-3 co-resident single-tile CTAs (202 vs 182 ms per B=64 step) -- the
-  // kernel is bound by L2->SM operand traffic (A re-fetched per tap, B per tile), not by prologue /
-  // epilogue serialisation (KKX_TC_DEBUG experiments, profiles/r1_conv_tc_experiments.txt).  Kept
-  // opt-in (KKX_TC_MULTI=1) as the base for the halo-reuse kernel.
-  static const bool multi_ok = env_flag("KKX_TC_MULTI", false);
-  const long long tiles = (a.sum_m + 127) / 128 * ((a.Co + 127) / 128);
-  if (multi_ok && a.nphase <= 1 && tiles >= 4 * 2 * 148 && a.Co > 64) {
-    if (a.Co > 128) launch_tc_multi<256, 2, 4>(a, st);   // 96 + 37 KB smem, 512 TMEM cols: 1 CTA/SM
-    else launch_tc_multi<128, 2, 4>(a, st);              // 64 + 37 KB smem, 256 TMEM cols: 2 CTAs/SM
-    if (g_launch_stats && g_launch_stats->profile && g_launch_stats->detail) {
-      char nm[96]; snprintf(nm, sizeof nm, "conv_tc[ci%d co%d k%d m%lld]", a.Ci, a.Co, a.ks, a.sum_m);
-      post_launch(nm, st);
-    } else post_launch("conv_tc", st);
-    return;
-  }
   // smem per CTA ~97 KB in every configuration -> two CTAs per SM, so one tile's epilogue overlaps
   // the other's TMA/MMA main loop (TMEM: 2 x 256 columns = the whole 512-column file)
+  // Multi-tile CTAs (4 tiles per CTA, pipeline across tiles, double-buffered TMEM accumulators) measured slower than
+  // 2-3 co-resident single-tile CTAs: 202 vs 182 ms per B=64 step.  The kernel is bound by L2->SM operand traffic
+  // (A re-fetched per tap, B per tile), not by prologue / epilogue serialisation (profiles/r1_conv_tc_experiments.txt).
   int pdev = 0;
   cudaGetDevice(&pdev);
   if (a.phase_loop == 3 && conv_phase_resident_ok(a)) {
     launch_conv_phase_resident(a, st);     // stage-1 up-sampling of a batch: persistent CTAs with one phase's weights resident
   } else if (a.nphase > 1 && a.Co == 128 && a.phase_loop && !a.res && !a.accumulate) {
     // one CTA loops over the phases of its m-tile (2 stages: two CTAs per SM; 3: one)
-    if (a.phase_loop == 2) launch_tc_multi<128, 3, 1, true>(a, st);
-    else launch_tc_multi<128, 2, 1, true>(a, st);
+    if (a.phase_loop == 2) launch_tc_multi<128, 3>(a, st);
+    else launch_tc_multi<128, 2>(a, st);
   }
   else if (conv_tc_takes_pair_bf16(a, device_sm_count(pdev))) launch_conv_pair(a, st);   // wide convs of big batches: CTA pairs
   else if (a.Co > 128) launch_tc<256, 2, 0>(a, st);

@@ -530,7 +530,6 @@ void WeightSet::load(const WeightFile& wf) {
   UPS(G + "ups.0.weight", 512, 256, 20, 10, W.ups0, W.tups0, W.tups0_all); W.ups0_b = U(G + "ups.0.bias");
   UPS(G + "ups.1.weight", 256, 128, 12, 6, W.ups1, W.tups1, W.tups1_all); W.ups1_b = U(G + "ups.1.bias");
   W.post_w = CW(G + "conv_post.weight", 22, 128, 7); W.post_b = U(G + "conv_post.bias");
-  W.t_post = make_tc(convCoKsCi(wf, G + "conv_post.weight", 22, 128, 7), 22, 7, 128);
   {
     std::vector<float> wp = convCoKsCi(wf, G + "conv_post.weight", 22, 128, 7);
     wp.resize((size_t)128 * 7 * 128, 0.f);                 // rows 22..127 are zero
@@ -603,20 +602,19 @@ Level Model::make_level(const std::vector<int>& lens, Arena& A, int first_off) {
     L.sum_len += lens[b];
   }
   L.rows = (int)o;
-  // one device block, one upload: off[B] len[B] tiles128[B+1] tiles256[B+1] tiles512[B+1]
-  const size_t n = (size_t)5 * L.B + 3;
+  // one device block, one upload: off[B] len[B] tiles128[B+1] tiles256[B+1]
+  const size_t n = (size_t)4 * L.B + 2;
   int* d = A.alloc<int>(n);
   L.d_off = d; L.d_len = d + L.B;
-  L.d_tiles128 = d + 2 * L.B; L.d_tiles256 = L.d_tiles128 + L.B + 1; L.d_tiles512 = L.d_tiles256 + L.B + 1;
+  L.d_tiles128 = d + 2 * L.B; L.d_tiles256 = L.d_tiles128 + L.B + 1;
   std::vector<int> h(n, 0);
-  int* t128 = h.data() + 2 * L.B; int* t256 = t128 + L.B + 1; int* t512 = t256 + L.B + 1;
+  int* t128 = h.data() + 2 * L.B; int* t256 = t128 + L.B + 1;
   for (int b = 0; b < L.B; b++) {
     h[b] = L.off[b]; h[L.B + b] = lens[b];
     t128[b + 1] = t128[b] + (lens[b] + 127) / 128;
     t256[b + 1] = t256[b] + (lens[b] + 255) / 256;
-    t512[b + 1] = t512[b] + (lens[b] + 511) / 512;
   }
-  L.ntiles128 = t128[L.B]; L.ntiles256 = t256[L.B]; L.ntiles512 = t512[L.B];
+  L.ntiles128 = t128[L.B]; L.ntiles256 = t256[L.B];
   upload(d, h.data(), n * sizeof(int));
   return L;
 }

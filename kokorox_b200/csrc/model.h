@@ -65,7 +65,7 @@ struct TcW32 {
   float* hi = nullptr; float* lo = nullptr;
   alignas(64) unsigned char tm_hi[128];
   alignas(64) unsigned char tm_lo[128];
-  alignas(64) unsigned char tm_hi_c[128];   // half-height boxes for the 2-CTA multicast GEMM (Co > 64 only)
+  alignas(64) unsigned char tm_hi_c[128];   // half-height boxes (64 rows) for the 64-wide small-problem tiles (Co > 64 only)
   alignas(64) unsigned char tm_lo_c[128];
   bool has_c = false;
   int Cpad = 0, Ci = 0, Co = 0, ks = 0;
@@ -117,7 +117,7 @@ struct Weights {
   std::vector<float*> ups0, ups1;  // per-phase [2][Ci][Co]
   std::vector<TcW> tups0, tups1;   // per-phase bf16 [Co][2][Ci]
   TcW tups0_all, tups1_all;        // the phases stacked along Co (phase-fused launch): [s*Co][2][Ci]
-  TcW t_post, t_nc0, t_nc1, t_asr; // conv_post, noise_convs (nc0 as an im2col GEMM, K = 12*22), asr_res
+  TcW t_nc0, t_nc1, t_asr;         // noise_convs (nc0 as an im2col GEMM, K = 12*22), asr_res
   float *ups0_b, *ups1_b, *post_w, *post_b;
   TcW t_post_arb; float* post_b128 = nullptr;   // conv_post zero-padded to 128 output channels for the fused kernel
   // style FC tables (all AdaIN / AdaLN fcs of one style half concatenated)

@@ -102,10 +102,7 @@ void Model::gemm(const Level& Lin, const Level& Lm, const float* in, int ldi, in
       make_tmap_f32(tA, split_hi_, w32->Cpad, Lin.rows, w32->Cpad, 128);
       make_tmap_f32(tA2, split_lo_, w32->Cpad, Lin.rows, w32->Cpad, 128);
       a.tmB = w32->tm_hi; a.tmB2 = w32->tm_lo;
-      // 2-CTA clusters with TMA-multicast weight tiles: measured on B200 NOT faster (13.9 vs 12.4 ms for the 12 qkv
-      // GEMMs); opt-in in experiment builds (KKX_TC_CLUSTER=1)
-      static const bool cl_ok = env_flag("KKX_TC_CLUSTER", false);
-      if (w32->has_c) { a.tmB_c = w32->tm_hi_c; a.tmB2_c = w32->tm_lo_c; a.cluster = cl_ok ? 2 : 1; }
+      if (w32->has_c) { a.tmB_c = w32->tm_hi_c; a.tmB2_c = w32->tm_lo_c; }
     }
     a.tmA = tA; a.tmA2 = tA2; a.tf32 = 1; a.nprod = 3; a.eact = eact;
     a.Cpad = w32->Cpad; a.Ci = K; a.Co = N; a.ks = ks; a.dil = 1; a.pad = pad;
@@ -463,7 +460,7 @@ void Model::adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ld
 // AdaINResBlock1 (A.9): three (AdaIN -> Snake -> dilated conv -> AdaIN -> Snake -> conv) + residual
 // iterations.  Reads x, uses xw/t1 as work buffers, writes (or accumulates) oscale * result to out.
 bool Model::use_stream_bf16(int C, int k, int B) const {
-  return opt.precision == 1 && opt.stream_bf16 && arb_conv_supported(C, k, 5, B) && arb_tile_rows(C, k) == (C == 128 ? 256 : 128);
+  return opt.precision == 1 && opt.stream_bf16 && arb_conv_supported(C, k, 5, B);
 }
 
 void Model::arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L, const float* sty,
@@ -480,15 +477,14 @@ void Model::arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L,
   const float* cur = x;
   const bool tc = opt.precision == 1;
   void* abuf = tc ? A.alloc_bytes((size_t)L.rows * w.t1[0].Cpad * 2) : nullptr;
-  static const bool fused_ok = env_flag("KKX_ARB_FUSED", true);
-  if (tc && fused_ok && arb_conv_supported(C, k, 5, B)) {
+  if (tc) {
     // fused path (kernels_arb.cu): AdaIN + Snake inside the conv kernel, bf16 intermediate, column
     // statistics for the next AdaIN from the conv epilogues -- one colstats pass per res-block
     ArbConvArgs base;
     base.C = C; base.ks = k; base.off = L.d_off; base.len = L.d_len; base.B = B; base.sum_m = L.sum_len;
-    const int trows = arb_tile_rows(C, k);
-    base.tile_start = trows == 512 ? L.d_tiles512 : trows == 256 ? L.d_tiles256 : L.d_tiles128;
-    base.total_tiles = trows == 512 ? L.ntiles512 : trows == 256 ? L.ntiles256 : L.ntiles128;
+    const bool t256 = arb_tile_rows(C) == 256;
+    base.tile_start = t256 ? L.d_tiles256 : L.d_tiles128;
+    base.total_tiles = t256 ? L.ntiles256 : L.ntiles128;
     base.scale = sc; base.shift = sh; base.nchunk = nch;
     // bf16 residual stream: x0 arrives as bf16 (from the caller's add_rows_stats, or copied by the statistics pass
     // below), x1 / x2 live in `xw` as bf16 and the block output leaves in fp32
@@ -532,20 +528,6 @@ void Model::arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L,
   for (int j = 0; j < 3; j++) {
     launch_colstats(cur, C, C, part, L.d_off, L.d_len, B, L.max_len, st);
     launch_adain_coef(part, C, L.max_len, L.d_len, sty, sld, w.s1[j], 1e-5f, sc, sh, B, st);
-    if (tc) {
-      const int cp = w.t1[j].Cpad;
-      launch_apply_bf16(cur, C, C, sc, sh, ACT_SNAKE, 0.f, w.a1[j], abuf, cp, L.rows, L.d_off, L.d_len, B, L.max_len, st);
-      tc_conv(A, abuf, L.rows, w.t1[j], dil[j], dil[j] * (k - 1) / 2, L, L, w.b1[j], t1, C, 0, L, 1, 0, nullptr, 0,
-              nullptr, 0, 1.f, false);
-      launch_colstats(t1, C, C, part, L.d_off, L.d_len, B, L.max_len, st);
-      launch_adain_coef(part, C, L.max_len, L.d_len, sty, sld, w.s2[j], 1e-5f, sc, sh, B, st);
-      launch_apply_bf16(t1, C, C, sc, sh, ACT_SNAKE, 0.f, w.a2[j], abuf, cp, L.rows, L.d_off, L.d_len, B, L.max_len, st);
-      float* dst = (j == 2) ? out : xw;
-      tc_conv(A, abuf, L.rows, w.t2[j], 1, (k - 1) / 2, L, L, w.b2[j], dst, C, 0, L, 1, 0, cur, C, &L, 0,
-              j == 2 ? oscale : 1.f, j == 2 && accumulate);
-      cur = dst;
-      continue;
-    }
     ConvArgs c1 = gemm_args(L, cur, C, C, w.w1[j], w.b1[j], C, t1, C, 0);
     c1.ks = k; c1.dil = dil[j]; c1.pad = dil[j] * (k - 1) / 2;
     c1.pscale = sc; c1.pshift = sh; c1.pld = C; c1.pact = ACT_SNAKE; c1.palpha = w.a1[j];
@@ -912,8 +894,7 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
 
   // ---- head (K11)
   float* cp = A.alloc<float>((size_t)G120.rows * 24);
-  static const bool post_fused = env_flag("KKX_POST_FUSED", true);
-  if (opt.precision == 1 && post_fused && arb_conv_supported(128, 7, 1, B)) {
+  if (opt.precision == 1) {
     // fused: LeakyReLU in the operand producer, all 7 taps from one activation tile (kernels_arb.cu, POST)
     ArbConvArgs pc;
     pc.C = 128; pc.ks = 7; pc.dil = 1; pc.pad = 3; pc.off = G120.d_off; pc.len = G120.d_len; pc.B = B;
@@ -921,11 +902,6 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     pc.x = acc1; pc.in_bf16 = 0; pc.tmB = W.t_post_arb.tmap; pc.bias = W.post_b128;
     pc.out_f32 = cp; pc.post = 1; pc.cout = 22; pc.ldo = 24; pc.slope = 0.01f;
     launch_arb_conv(pc, st);
-  } else if (opt.precision == 1) {
-    void* pb = A.alloc_bytes((size_t)G120.rows * 128 * 2);
-    launch_apply_bf16(acc1, 128, 128, nullptr, nullptr, ACT_LRELU, 0.01f, nullptr, pb, 128, G120.rows, G120.d_off,
-                      G120.d_len, B, G120.max_len, st);
-    tc_conv(A, pb, G120.rows, W.t_post, 1, 3, G120, G120, W.post_b, cp, 24, 0, G120, 1, 0, nullptr, 0, nullptr, 0, 1.f, false);
   } else {
     ConvArgs c = gemm_args(G120, acc1, 128, 128, W.post_w, W.post_b, 22, cp, 24, 0);
     c.ks = 7; c.pad = 3; c.pact = ACT_LRELU; c.pslope = 0.01f;

@@ -29,13 +29,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const void* tmap, int 
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1) : "memory");
 }
-// multicast variant: the box lands at the same smem offset in every CTA of `mask`, and completes tx bytes on
-// the mbarrier at the same offset in each of them
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const void* tmap, int c0, int c1, uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(dst), "l"(tmap), "r"(bar), "r"(c0), "r"(c1), "h"(mask) : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -86,11 +79,6 @@ __device__ __forceinline__ void umma_split(uint32_t tmem_d, uint64_t adesc, uint
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// arrive on the mbarrier at this offset in every CTA of `mask` once the MMAs issued so far have completed
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask) : "memory");
 }
 
 // ---- CTA pairs (cta_group::2): two CTAs of a cluster run ONE tcgen05.mma of M = 256; each supplies its own 128 rows

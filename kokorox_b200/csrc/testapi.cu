@@ -516,7 +516,7 @@ static int arb_conv_test(int device, const float* x, int B, const int* lens, int
     if (!arb_conv_supported(C, ks, dil, B)) throw ArgError("kkx_test_arb_conv: unsupported shape");
     // ragged Level layout with NaN-filled gap rows: the kernel must never consume a gap row
     std::vector<int> off(B), tiles(B + 1, 0);
-    const int MT = arb_tile_rows(C, ks);
+    const int MT = arb_tile_rows(C);
     int o = kGapRows, maxL = 0; long long sumL = 0;
     for (int b = 0; b < B; b++) {
       off[b] = o; o = (o + lens[b] + kGapRows + 7) & ~7;

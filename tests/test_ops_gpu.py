@@ -517,9 +517,9 @@ def test_split_fp16_gemm_kernels_are_bit_identical(lib, L, Ci, Co, k, eact, use_
 
 
 @pytest.mark.parametrize("Cc,k,dil", [(128, 3, 1), (128, 11, 5), (256, 7, 3)])
-def test_tc_conv_multi_tile_kernel(lib, Cc, k, dil):
-    # large enough (>= 1184 tiles) to take the multi-tile / double-buffered-TMEM kernel, with a ragged
-    # tail (L not a multiple of 128*4), residual, scale and accumulate fused in the epilogue
+def test_tc_conv_large_ragged_fused_epilogue(lib, Cc, k, dil):
+    # a large conv (>= 1184 128-row tiles) on the single-tile kernel with a ragged tail (L not a multiple of 128)
+    # and residual, scale and accumulate fused in the epilogue
     L = 128 * 4 * 300 + 77 if Cc == 128 else 128 * 4 * 150 + 205
     x, w, b = rnd(L, Cc, seed=31), rnd(Cc, Cc, k, seed=32, scale=1 / np.sqrt(Cc * k)), rnd(Cc, seed=33)
     res, init = rnd(L, Cc, seed=34), rnd(L, Cc, seed=35)
