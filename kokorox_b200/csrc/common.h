@@ -53,7 +53,7 @@ inline bool env_flag(const char*, bool dflt) { return dflt; }
 inline int env_int(const char*, int dflt) { return dflt; }
 #endif
 
-// One-time per-device setup (cudaFuncSetAttribute for a kernel's dynamic shared memory): two sessions on two
+// One-time per-device setup (a kernel's dynamic shared-memory limit, constant tables): two sessions on two
 // threads may reach a launcher's first use together, so the flag is a std::once_flag per device, not a bool.
 struct DevOnce {
   std::once_flag flag[64];
@@ -61,6 +61,17 @@ struct DevOnce {
     if (dev >= 0 && dev < 64) std::call_once(flag[dev], fn); else fn();
   }
 };
+// Call before launching `Kernel` with `bytes` of dynamic shared memory: raises the kernel's limit to `bytes` once per
+// device and returns the current device; a failure throws CudaError.  The template argument is the kernel itself, not
+// its type, so each kernel has its own once-state (conv_tc_kernel<128,3,1> and <64,4,1> share one function type).
+template <auto Kernel>
+int prepare_smem_launch(int bytes) {
+  static DevOnce once;
+  int dev = 0;
+  KKX_CUDA(cudaGetDevice(&dev));
+  once.run(dev, [bytes] { KKX_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes)); });
+  return dev;
+}
 inline int device_sm_count(int dev) {
   static std::atomic<int> cache[64];
   if (dev < 0 || dev >= 64) return 148;

@@ -174,22 +174,19 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
   for (int i = threadIdx.x; i < B; i += kArbThreads) { s_len[i] = a.len[i]; s_off[i] = a.off[i]; }
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
+    prefetch_tmap(&tmB);
     for (int s = 0; s < NA; s++) { mbar_init(fullA(s), kProdThreads / 32); mbar_init(emptyA(s), 1); }
     for (int s = 0; s < NB; s++) { mbar_init(fullB(s), 1); mbar_init(emptyB(s), 1); }
     for (int j = 0; j < 2; j++) { mbar_init(tfull(j), 1); mbar_init(tempty(j), NEW); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(tmem_slot, 512u);
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   // contiguous tile range of this CTA (neighbouring tiles share halo rows and, mostly, the item)
   const int t_begin = (int)(((long long)a.total_tiles * blockIdx.x) / gridDim.x);
@@ -352,7 +349,7 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * 256 + eg * RW + ch * 32), v);
         if (ch == NCHK - 1) {      // last TMEM read of this tile by this warp
           tc_fence_before();
-          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tempty(buf)) : "memory");
+          if (lane == 0) mbar_arrive(tempty(buf));
         }
         TICK(1);
         if (CONV2 && !OUT_BF) {
@@ -504,7 +501,7 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
           tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)((buf * MSUB + sub) * BN + n - c4), v);
           if (e == E - 1) {   // last TMEM read of this tile: hand the accumulators back
             tc_fence_before();
-            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tempty(buf)) : "memory");
+            if (lane == 0) mbar_arrive(tempty(buf));
           }
           TICK(1);
           asm volatile("bar.sync %0, 128;" ::"r"(bar_id) : "memory");   // staging buffer drained by the previous iteration
@@ -718,7 +715,7 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
       if (++s_g == ngc) {
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(fullA(sa)) : "memory");
+        if (lane == 0) mbar_arrive(fullA(sa));
         s_g = 0; gA++;
         if (++s_c == KCH) { s_c = 0; sc_.next(s_ts); }
       }
@@ -746,17 +743,14 @@ __global__ void __launch_bounds__(kArbThreads, 1) arb_conv_kernel(const __grid_c
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc<1>(tmem_base, 512u);
   }
 }
 
 template <int BN, bool CONV2, bool POST = false, int SB = 0, bool PB = false>
 void launch_arb_t(const ArbConvArgs& a, cudaStream_t st) {
   using Cfg = ArbCfg<BN>;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(arb_conv_kernel<BN, CONV2, POST, SB, PB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM)); });
+  const int dev = prepare_smem_launch<arb_conv_kernel<BN, CONV2, POST, SB, PB>>((int)Cfg::SMEM);
   const int nsm = device_sm_count(dev);
   const int grid = a.total_tiles < nsm ? a.total_tiles : nsm;
   arb_conv_kernel<BN, CONV2, POST, SB, PB><<<grid, kArbThreads, Cfg::SMEM, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmB), a);

@@ -62,12 +62,6 @@ __device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, ui
       "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
       ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
 }
-// v (already scaled) -> fp16 hi = rn(v), lo = rn(v - hi); returned as raw 16-bit patterns
-__device__ __forceinline__ void split_h(float v, uint32_t& hi, uint32_t& lo) {
-  const __half h = __float2half_rn(v);
-  hi = __half_as_ushort(h);
-  lo = __half_as_ushort(__float2half_rn(v - __half2float(h)));
-}
 constexpr float kQScale = 2.0f;          // 16 * (1/8): the 1/sqrt(64) of the scores folded in, exact
 constexpr float kKVScale = 16.0f;
 constexpr float kPScale = 4096.0f;
@@ -93,9 +87,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* v) {
       : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 
 constexpr int kVtPitch = 512;          // keys per V^T row (ALBERT max_position_embeddings)
 
@@ -128,8 +119,8 @@ __global__ void __launch_bounds__(256) attn_prep_kernel(const float* __restrict_
     uint32_t w[4][8];   // qh ql kh kl
 #pragma unroll
     for (int e = 0; e < 8; e++) {
-      split_h(q[e] * kQScale, w[0][e], w[1][e]);
-      split_h(k[e] * kKVScale, w[2][e], w[3][e]);
+      split_f16(q[e] * kQScale, w[0][e], w[1][e]);
+      split_f16(k[e] * kKVScale, w[2][e], w[3][e]);
     }
     __half* dst[4] = {qh, ql, kh, kl};
 #pragma unroll
@@ -140,7 +131,7 @@ __global__ void __launch_bounds__(256) attn_prep_kernel(const float* __restrict_
 #pragma unroll
   for (int e = 0; e < 8; e++) {
     uint32_t hi, lo;
-    split_h(v[e] * kKVScale, hi, lo);
+    split_f16(v[e] * kKVScale, hi, lo);
     s_h[c8 + e][r] = (unsigned short)hi;
     s_l[c8 + e][r] = (unsigned short)lo;
   }
@@ -216,9 +207,9 @@ __global__ void __launch_bounds__(kAttnThreads, 1) attn_umma_kernel(const __grid
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmQh) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmKh) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmVh) : "memory");
+    prefetch_tmap(&tmQh);
+    prefetch_tmap(&tmKh);
+    prefetch_tmap(&tmVh);
     for (int s = 0; s < NST; s++) {
       mbar_init(fullk_bar(s), 1); mbar_init(emptyk_bar(s), 1); mbar_init(fullv_bar(s), 1); mbar_init(emptyv_bar(s), 1);
     }
@@ -227,18 +218,15 @@ __global__ void __launch_bounds__(kAttnThreads, 1) attn_umma_kernel(const __grid
       mbar_init(pfull_bar(s), 8); mbar_init(ofull_bar(s), 1); mbar_init(ofree_bar(s), 8);
       mbar_init(qfull_bar(s), 1); mbar_init(qfree_bar(s), 1);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(tmem_slot, 512u);
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -494,7 +482,7 @@ __global__ void __launch_bounds__(kAttnThreads, 1) attn_umma_kernel(const __grid
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc<1>(tmem_base, 512u);
   }
 }
 }  // namespace
@@ -533,10 +521,7 @@ void launch_attention_umma(const float* qkv, float* scratch, float* ctx, const i
   __half* qh = static_cast<__half*>(pl[0]); __half* ql = static_cast<__half*>(pl[1]);
   __half* kh = static_cast<__half*>(pl[2]); __half* kl = static_cast<__half*>(pl[3]);
   __half* vth = static_cast<__half*>(pl[4]); __half* vtl = static_cast<__half*>(pl[5]);
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(attn_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttnSmem)); });
+  const int dev = prepare_smem_launch<attn_umma_kernel>(kAttnSmem);
   if (!planes_ready) {
     dim3 gp((((max_len + 63) & ~63) + 31) / 32, 12, B);
     attn_prep_kernel<<<gp, 256, 0, st>>>(qkv, qh, ql, kh, kl, vth, vtl, off, len);

@@ -5,6 +5,7 @@
 #include "kernels.h"
 #include <cuda_fp16.h>
 #include <math.h>
+#include "tc_ptx.cuh"
 
 namespace kkx {
 
@@ -169,11 +170,11 @@ __global__ void __launch_bounds__(256) layernorm_kernel(LnArgs a) {
     if (ada) v = (1.0f + ada[c]) * v + ada[C + c];
     if (a.slope != 1.f) v = v > 0.f ? v : v * a.slope;
     o[c] = v;
-    if (a.pl_hi) {   // operand planes for the next split-FP16 GEMM (same arithmetic as apply_f16x2_kernel)
-      const float sv = fminf(fmaxf(v * kSplitF16Scale, -65504.f), 65504.f);
-      const __half hi = __float2half_rn(sv);
-      static_cast<__half*>(a.pl_hi)[row * a.pl_ld + c] = hi;
-      static_cast<__half*>(a.pl_lo)[row * a.pl_ld + c] = __float2half_rn(sv - __half2float(hi));
+    if (a.pl_hi) {   // operand planes for the next split-FP16 GEMM
+      uint32_t hi, lo;
+      split_f16_operand(v, hi, lo);
+      static_cast<uint16_t*>(a.pl_hi)[row * a.pl_ld + c] = (uint16_t)hi;
+      static_cast<uint16_t*>(a.pl_lo)[row * a.pl_ld + c] = (uint16_t)lo;
     }
   }
 }
@@ -232,20 +233,12 @@ __global__ void __launch_bounds__(256) layernorm_vec_kernel(LnArgs a) {
       for (int k = 0; k < 4; k++) e[k] = e[k] > 0.f ? e[k] : e[k] * a.slope;
     }
     *reinterpret_cast<float4*>(o + c) = make_float4(e[0], e[1], e[2], e[3]);
-    if (a.pl_hi) {   // operand planes for the next split-FP16 GEMM (same arithmetic as apply_f16x2_kernel)
-      __half hi[4], lo[4];
+    if (a.pl_hi) {   // operand planes for the next split-FP16 GEMM
+      uint32_t hi[4], lo[4];
 #pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const float sv = fminf(fmaxf(e[k] * kSplitF16Scale, -65504.f), 65504.f);
-        hi[k] = __float2half_rn(sv);
-        lo[k] = __float2half_rn(sv - __half2float(hi[k]));
-      }
-      const __half2 h01 = __halves2half2(hi[0], hi[1]), h23 = __halves2half2(hi[2], hi[3]);
-      const __half2 l01 = __halves2half2(lo[0], lo[1]), l23 = __halves2half2(lo[2], lo[3]);
-      *reinterpret_cast<uint2*>(static_cast<__half*>(a.pl_hi) + row * a.pl_ld + c) =
-          make_uint2(*reinterpret_cast<const uint32_t*>(&h01), *reinterpret_cast<const uint32_t*>(&h23));
-      *reinterpret_cast<uint2*>(static_cast<__half*>(a.pl_lo) + row * a.pl_ld + c) =
-          make_uint2(*reinterpret_cast<const uint32_t*>(&l01), *reinterpret_cast<const uint32_t*>(&l23));
+      for (int k = 0; k < 4; k++) split_f16_operand(e[k], hi[k], lo[k]);
+      *reinterpret_cast<uint2*>(static_cast<uint16_t*>(a.pl_hi) + row * a.pl_ld + c) = make_uint2(hi[0] | (hi[1] << 16), hi[2] | (hi[3] << 16));
+      *reinterpret_cast<uint2*>(static_cast<uint16_t*>(a.pl_lo) + row * a.pl_ld + c) = make_uint2(lo[0] | (lo[1] << 16), lo[2] | (lo[3] << 16));
     }
   }
 }
@@ -577,17 +570,12 @@ void launch_attention(const float* qkv, float* ctx, const int* off, const int* l
                       int max_len, cudaStream_t st) {
   if (g_dry_run) return;
   constexpr int smem = 4 * 64 * kAttLd * 4;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] {
-    KKX_CUDA(cudaFuncSetAttribute(attention_tc_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    KKX_CUDA(cudaFuncSetAttribute(attention_tc_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  });
   if (max_len > 64) {   // 128 query rows per CTA: the K/V staging (load + tf32 split) is amortised over twice the MMAs
+    prepare_smem_launch<attention_tc_kernel<8>>(smem);
     dim3 g((max_len + 127) / 128, 12, B);
     attention_tc_kernel<8><<<g, 256, smem, st>>>(qkv, ctx, off, len);
   } else {
+    prepare_smem_launch<attention_tc_kernel<4>>(smem);
     dim3 g((max_len + 63) / 64, 12, B);
     attention_tc_kernel<4><<<g, 128, smem, st>>>(qkv, ctx, off, len);
   }
@@ -891,13 +879,8 @@ static void launch_lstm_cluster(const float* xproj, const float* whhT, float* ou
                                 const int* off, const int* len, int B, cudaStream_t st, int fast) {
   const size_t smem = (size_t)(2 * G * kHItem + 2 * G * 128) * sizeof(float) + 16;
   auto kern = fast ? lstm_cluster_kernel<G, true> : lstm_cluster_kernel<G, false>;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [smem] {
-    KKX_CUDA(cudaFuncSetAttribute(lstm_cluster_kernel<G, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    KKX_CUDA(cudaFuncSetAttribute(lstm_cluster_kernel<G, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  });
+  if (fast) prepare_smem_launch<lstm_cluster_kernel<G, true>>((int)smem);
+  else prepare_smem_launch<lstm_cluster_kernel<G, false>>((int)smem);
   const int groups = (B + G - 1) / G;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(8 * groups, 2, 1);

@@ -509,11 +509,8 @@ void launch_flac(const short* pcm, const long long* soff, const int* foff, int B
   FlacFrame* frames = static_cast<FlacFrame*>(work);
   long long* frame_off = reinterpret_cast<long long*>(reinterpret_cast<char*>(work) +
                                                       (((size_t)F * sizeof(FlacFrame) + 255) & ~size_t(255)));
-  static DevOnce once;
-  int dev = 0;
-  KKX_CUDA(cudaGetDevice(&dev));
   const size_t smem = analyze_smem();
-  once.run(dev, [&] { cudaFuncSetAttribute(flac_analyze_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); });
+  prepare_smem_launch<flac_analyze_kernel>((int)smem);
   flac_analyze_kernel<<<F, kThreads, smem, st>>>(pcm, soff, foff, B, rate, frames);
   post_launch("flac_analyze", st);
   flac_scan_kernel<<<1, 1024, 0, st>>>(frames, foff, B, F, frame_off, item_off);

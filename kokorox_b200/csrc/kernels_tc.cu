@@ -92,6 +92,35 @@ __device__ __forceinline__ float gelu_new_f(float v) {
   return 0.5f * v * (1.0f + tanhf(u));
 }
 
+// ---- fp32 output epilogue of every kernel below.  Which kernel runs depends on the batch, so all of them finish an
+// accumulator with these helpers: the same inputs give the same bits whatever the batch composition.  A thread handles
+// columns n .. n+3 of one output row; `vec` (a.vec4 && n + 3 < Co) makes that one 16-byte access, otherwise only the
+// columns below Co are touched.
+// bias / residual / accumulate operand; columns >= Co read as 0
+__device__ __forceinline__ float4 epi_load4(const float* p, int n, int Co, bool vec) {
+  if (vec) return *reinterpret_cast<const float4*>(p);
+  float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
+  r.x = p[0]; if (n + 1 < Co) r.y = p[1]; if (n + 2 < Co) r.z = p[2]; if (n + 3 < Co) r.w = p[3];
+  return r;
+}
+// (acc * wscale + bias), GELU if eact says so, then (+ res) * oscale.  Without a residual res is 0: the + 0.f stays,
+// it turns -0 into +0.
+__device__ __forceinline__ float4 epi_math4(float4 o, float wscale, float4 bias, int eact, float4 res, float oscale) {
+  o.x = fmaf(o.x, wscale, bias.x); o.y = fmaf(o.y, wscale, bias.y); o.z = fmaf(o.z, wscale, bias.z); o.w = fmaf(o.w, wscale, bias.w);
+  if (eact == ACT_GELU_NEW) { o.x = gelu_new_f(o.x); o.y = gelu_new_f(o.y); o.z = gelu_new_f(o.z); o.w = gelu_new_f(o.w); }
+  o.x = (o.x + res.x) * oscale; o.y = (o.y + res.y) * oscale; o.z = (o.z + res.z) * oscale; o.w = (o.w + res.w) * oscale;
+  return o;
+}
+// adds what is already stored when `accumulate`, then stores
+__device__ __forceinline__ void epi_store4(float* p, float4 o, int n, int Co, bool vec, bool accumulate) {
+  if (accumulate) { const float4 pv = epi_load4(p, n, Co, vec); o.x += pv.x; o.y += pv.y; o.z += pv.z; o.w += pv.w; }
+  if (vec) {
+    *reinterpret_cast<float4*>(p) = o;
+  } else {
+    p[0] = o.x; if (n + 1 < Co) p[1] = o.y; if (n + 2 < Co) p[2] = o.z; if (n + 3 < Co) p[3] = o.w;
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // The kernel.  One 128 x BN output tile per CTA.  6 warps:
 //   warp 0  TMA producer (one elected lane)        warp 1  TMEM alloc + MMA issuer (one lane)
@@ -148,27 +177,24 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
   const int num_k = a.ks * kchunks;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
     if (MODE) {
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA2) : "memory");
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB2) : "memory");
+      prefetch_tmap(&tmA2);
+      prefetch_tmap(&tmB2);
     }
     for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     mbar_init(tfull_bar, 1);
     if (MODE) for (int j = 0; j < 3; j++) { mbar_init(bfull_bar(j), 1); mbar_init(bempty_bar(j), 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(tmem_slot, TMEM_COLS);
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -276,7 +302,7 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
           }
         }
         tc_fence_before();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bempty_bar(j)) : "memory");
+        if (lane == 0) mbar_arrive(bempty_bar(j));
         TCT(1);
       }
     }
@@ -297,12 +323,8 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
       for (int i = 0; i < 8; i++) {
         const int mm = m0 + (t >> 3) + 16 * i;
         rv[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.res && n < a.Co && mm < mlen) {
-          const int orow = mm * a.ors + c_oro;
-          const float* rp = a.res + ((size_t)(res_off + (orow >> a.res_shift)) * a.ldr + a.rcol + n);
-          if (vec) rv[i] = *reinterpret_cast<const float4*>(rp);
-          else { rv[i].x = rp[0]; if (n + 1 < a.Co) rv[i].y = rp[1]; if (n + 2 < a.Co) rv[i].z = rp[2]; if (n + 3 < a.Co) rv[i].w = rp[3]; }
-        }
+        if (a.res && n < a.Co && mm < mlen)
+          rv[i] = epi_load4(a.res + ((size_t)(res_off + ((mm * a.ors + c_oro) >> a.res_shift)) * a.ldr + a.rcol + n), n, a.Co, vec);
       }
     };
     float4 rv[8];
@@ -327,32 +349,14 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
       const int n = n0 + c + c4;
       if (n < a.Co) {
         const bool vec = a.vec4 && (n + 3 < a.Co);
-        float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.bias) {
-          if (vec) bb = *reinterpret_cast<const float4*>(a.bias + n);
-          else { bb.x = a.bias[n]; if (n + 1 < a.Co) bb.y = a.bias[n + 1]; if (n + 2 < a.Co) bb.z = a.bias[n + 2]; if (n + 3 < a.Co) bb.w = a.bias[n + 3]; }
-        }
+        const float4 bb = a.bias ? epi_load4(a.bias + n, n, a.Co, vec) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
         for (int i = 0; i < 8; i++) {
           const int row = (t >> 3) + 16 * i;
           const int mm = m0 + row;
           if (mm >= mlen || TC_DBG(a, 1)) continue;
-          float4 o = *reinterpret_cast<const float4*>(buf + row * PITCH + c4);
-          o.x = fmaf(o.x, a.wscale, bb.x); o.y = fmaf(o.y, a.wscale, bb.y); o.z = fmaf(o.z, a.wscale, bb.z); o.w = fmaf(o.w, a.wscale, bb.w);
-          if (a.eact == ACT_GELU_NEW) { o.x = gelu_new_f(o.x); o.y = gelu_new_f(o.y); o.z = gelu_new_f(o.z); o.w = gelu_new_f(o.w); }
-          o.x = (o.x + rv[i].x) * a.oscale; o.y = (o.y + rv[i].y) * a.oscale;
-          o.z = (o.z + rv[i].z) * a.oscale; o.w = (o.w + rv[i].w) * a.oscale;
-          float* op = a.out + ((size_t)(out_off + mm * a.ors + c_oro) * a.ldo + a.ocol + n);
-          if (vec) {
-            if (a.accumulate) { const float4 pvv = *reinterpret_cast<const float4*>(op); o.x += pvv.x; o.y += pvv.y; o.z += pvv.z; o.w += pvv.w; }
-            *reinterpret_cast<float4*>(op) = o;
-          } else {
-            if (a.accumulate) { o.x += op[0]; if (n + 1 < a.Co) o.y += op[1]; if (n + 2 < a.Co) o.z += op[2]; if (n + 3 < a.Co) o.w += op[3]; }
-            op[0] = o.x;
-            if (n + 1 < a.Co) op[1] = o.y;
-            if (n + 2 < a.Co) op[2] = o.z;
-            if (n + 3 < a.Co) op[3] = o.w;
-          }
+          const float4 o = epi_math4(*reinterpret_cast<const float4*>(buf + row * PITCH + c4), a.wscale, bb, a.eact, rv[i], a.oscale);
+          epi_store4(a.out + ((size_t)(out_off + mm * a.ors + c_oro) * a.ldo + a.ocol + n), o, n, a.Co, vec, a.accumulate);
         }
       }
       if (MODE == 0 && c + 32 < BN) fetch(c + 32, rv);   // in flight during the next chunk's TMEM->smem hop
@@ -364,7 +368,7 @@ __global__ void __launch_bounds__(192) conv_tc_kernel(const __grid_constant__ CU
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    tmem_dealloc<1>(tmem_base, TMEM_COLS);
   }
 }
 
@@ -403,22 +407,19 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
   const int num_k = a.ks * kchunks;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
     for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int j = 0; j < 2; j++) { mbar_init(tfull_bar(j), 1); mbar_init(tempty_bar(j), 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"((uint32_t)(2 * BN)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(tmem_slot, (uint32_t)(2 * BN));
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -481,12 +482,8 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
         for (int i = 0; i < 8; i++) {
           const int mm = m0 + (t >> 3) + 16 * i;
           rv[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (a.res && n < a.Co && mm < mlen) {
-            const int orow = mm * a.ors + oro;
-            const float* rp = a.res + ((size_t)(res_off + (orow >> a.res_shift)) * a.ldr + a.rcol + n);
-            if (vec) rv[i] = *reinterpret_cast<const float4*>(rp);
-            else { rv[i].x = rp[0]; if (n + 1 < a.Co) rv[i].y = rp[1]; if (n + 2 < a.Co) rv[i].z = rp[2]; if (n + 3 < a.Co) rv[i].w = rp[3]; }
-          }
+          if (a.res && n < a.Co && mm < mlen)
+            rv[i] = epi_load4(a.res + ((size_t)(res_off + ((mm * a.ors + oro) >> a.res_shift)) * a.ldr + a.rcol + n), n, a.Co, vec);
         }
       };
       float4 rv[8];
@@ -499,7 +496,7 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN + c), v);
         if (c + 32 >= BN) {   // last TMEM read of this tile: hand the accumulator back to the MMA warp
           tc_fence_before();
-          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tempty_bar(acc)) : "memory");
+          if (lane == 0) mbar_arrive(tempty_bar(acc));
         }
         float* buf = stage_f + (chunk_ctr & 1) * (128 * PITCH);
         chunk_ctr++;
@@ -510,32 +507,14 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
         const int n = n0 + c + c4;
         if (n < a.Co) {
           const bool vec = a.vec4 && (n + 3 < a.Co);
-          float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (a.bias) {
-            if (vec) bb = *reinterpret_cast<const float4*>(a.bias + n);
-            else { bb.x = a.bias[n]; if (n + 1 < a.Co) bb.y = a.bias[n + 1]; if (n + 2 < a.Co) bb.z = a.bias[n + 2]; if (n + 3 < a.Co) bb.w = a.bias[n + 3]; }
-          }
+          const float4 bb = a.bias ? epi_load4(a.bias + n, n, a.Co, vec) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
           for (int i = 0; i < 8; i++) {
             const int row = (t >> 3) + 16 * i;
             const int mm = m0 + row;
             if (mm >= mlen || TC_DBG(a, 1)) continue;
-            float4 o = *reinterpret_cast<const float4*>(buf + row * PITCH + c4);
-            o.x = fmaf(o.x, a.wscale, bb.x); o.y = fmaf(o.y, a.wscale, bb.y); o.z = fmaf(o.z, a.wscale, bb.z); o.w = fmaf(o.w, a.wscale, bb.w);
-            if (a.eact == ACT_GELU_NEW) { o.x = gelu_new_f(o.x); o.y = gelu_new_f(o.y); o.z = gelu_new_f(o.z); o.w = gelu_new_f(o.w); }
-            o.x = (o.x + rv[i].x) * a.oscale; o.y = (o.y + rv[i].y) * a.oscale;
-            o.z = (o.z + rv[i].z) * a.oscale; o.w = (o.w + rv[i].w) * a.oscale;
-            float* op = a.out + ((size_t)(out_off + mm * a.ors + oro) * a.ldo + a.ocol + n);
-            if (vec) {
-              if (a.accumulate) { const float4 pvv = *reinterpret_cast<const float4*>(op); o.x += pvv.x; o.y += pvv.y; o.z += pvv.z; o.w += pvv.w; }
-              *reinterpret_cast<float4*>(op) = o;
-            } else {
-              if (a.accumulate) { o.x += op[0]; if (n + 1 < a.Co) o.y += op[1]; if (n + 2 < a.Co) o.z += op[2]; if (n + 3 < a.Co) o.w += op[3]; }
-              op[0] = o.x;
-              if (n + 1 < a.Co) op[1] = o.y;
-              if (n + 2 < a.Co) op[2] = o.z;
-              if (n + 3 < a.Co) op[3] = o.w;
-            }
+            const float4 o = epi_math4(*reinterpret_cast<const float4*>(buf + row * PITCH + c4), a.wscale, bb, a.eact, rv[i], a.oscale);
+            epi_store4(a.out + ((size_t)(out_off + mm * a.ors + oro) * a.ldo + a.ocol + n), o, n, a.Co, vec, a.accumulate);
           }
         }
         if (c + 32 < BN) fetch(c + 32, rv);
@@ -546,7 +525,7 @@ __global__ void __launch_bounds__(192) conv_tc_multi_kernel(const __grid_constan
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN)) : "memory");
+    tmem_dealloc<1>(tmem_base, (uint32_t)(2 * BN));
   }
 }
 
@@ -596,23 +575,20 @@ __global__ void __launch_bounds__(192) conv_phase_resident_kernel(const __grid_c
   };
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
     for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int j = 0; j < 2; j++) { mbar_init(tfull_bar(j), 1); mbar_init(tempty_bar(j), 4); }
     mbar_init(wfull_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"((uint32_t)(2 * BN)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(tmem_slot, (uint32_t)(2 * BN));
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   if (warp == 0) {
     if (lane == 0 && t_begin < t_end) {
@@ -682,7 +658,7 @@ __global__ void __launch_bounds__(192) conv_phase_resident_kernel(const __grid_c
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN + c), v);
         if (c + 32 >= BN) {   // last TMEM read of this tile: hand the accumulator back to the MMA warp
           tc_fence_before();
-          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tempty_bar(acc)) : "memory");
+          if (lane == 0) mbar_arrive(tempty_bar(acc));
         }
         float* buf = stage_f + (chunk_ctr & 1) * (128 * PITCH);
         chunk_ctr++;
@@ -690,18 +666,16 @@ __global__ void __launch_bounds__(192) conv_phase_resident_kernel(const __grid_c
         for (int j = 0; j < 32; j += 4)
           *reinterpret_cast<uint4*>(buf + et * PITCH + j) = make_uint4(v[j], v[j + 1], v[j + 2], v[j + 3]);
         asm volatile("bar.sync 1, 128;" ::: "memory");
-        const int n = c + c4;
-        float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.bias) bb = *reinterpret_cast<const float4*>(a.bias + n);
+        const int n = c + c4;       // Co == BN, vec4, no residual, activation or accumulate (conv_phase_resident_ok)
+        const float4 bb = a.bias ? epi_load4(a.bias + n, n, BN, true) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
         for (int i = 0; i < 8; i++) {
           const int row = (t >> 3) + 16 * i;
           const int mm = m0 + row;
           if (mm >= mlen) continue;
-          float4 o = *reinterpret_cast<const float4*>(buf + row * PITCH + c4);
-          o.x = fmaf(o.x, a.wscale, bb.x); o.y = fmaf(o.y, a.wscale, bb.y); o.z = fmaf(o.z, a.wscale, bb.z); o.w = fmaf(o.w, a.wscale, bb.w);
-          o.x = (o.x + 0.f) * a.oscale; o.y = (o.y + 0.f) * a.oscale; o.z = (o.z + 0.f) * a.oscale; o.w = (o.w + 0.f) * a.oscale;
-          *reinterpret_cast<float4*>(a.out + ((size_t)(out_off + mm * a.ors + oro) * a.ldo + a.ocol + n)) = o;
+          const float4 o = epi_math4(*reinterpret_cast<const float4*>(buf + row * PITCH + c4), a.wscale, bb, ACT_NONE,
+                                     make_float4(0.f, 0.f, 0.f, 0.f), a.oscale);
+          epi_store4(a.out + ((size_t)(out_off + mm * a.ors + oro) * a.ldo + a.ocol + n), o, n, BN, true, false);
         }
       }
     }
@@ -710,7 +684,7 @@ __global__ void __launch_bounds__(192) conv_phase_resident_kernel(const __grid_c
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN)) : "memory");
+    tmem_dealloc<1>(tmem_base, (uint32_t)(2 * BN));
   }
 }
 static bool conv_phase_resident_ok(const TcConvArgs& a) {
@@ -719,10 +693,7 @@ static bool conv_phase_resident_ok(const TcConvArgs& a) {
 }
 static void launch_conv_phase_resident(const TcConvArgs& a, cudaStream_t st) {
   constexpr int smem = 8 * 128 * 128 + kUpsStages * 128 * 128 + 2 * 128 * 36 * 4 + (2 * kUpsStages + 5) * 8 + 16 + 1024;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_phase_resident_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
+  const int dev = prepare_smem_launch<conv_phase_resident_kernel>(smem);
   const int per_phase = std::max(1, std::min(device_sm_count(dev) / a.nphase, a.ntiles_m));
   dim3 g(per_phase, a.nphase, 1);
   conv_phase_resident_kernel<<<g, 192, smem, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmA),
@@ -750,45 +721,22 @@ __device__ __forceinline__ void gemm32_final(const TcConvArgs& a, float* scr, co
     const int n = n0 + hh * 64 + blk * 32 + cq * 4;
     if (n < a.Co) {
       const bool vec = a.vec4 && (n + 3 < a.Co);
-      float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (bias) {
-        if (vec) bb = *reinterpret_cast<const float4*>(bias + n);
-        else { bb.x = bias[n]; if (n + 1 < a.Co) bb.y = bias[n + 1]; if (n + 2 < a.Co) bb.z = bias[n + 2]; if (n + 3 < a.Co) bb.w = bias[n + 3]; }
-      }
+      const float4 bb = bias ? epi_load4(bias + n, n, a.Co, vec) : make_float4(0.f, 0.f, 0.f, 0.f);
       float4 rv[8];
 #pragma unroll
       for (int i = 0; i < 8; i++) {
         rv[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         const int mm = m0 + q * 32 + rq + 4 * i;
-        if (a.res && mm < mlen) {
-          const float* rp = a.res + ((size_t)(res_row0 + ((mm * a.ors + oro) >> a.res_shift)) * a.ldr + a.rcol) + n;
-          if (vec) rv[i] = *reinterpret_cast<const float4*>(rp);
-          else { rv[i].x = rp[0]; if (n + 1 < a.Co) rv[i].y = rp[1]; if (n + 2 < a.Co) rv[i].z = rp[2]; if (n + 3 < a.Co) rv[i].w = rp[3]; }
-        }
+        if (a.res && mm < mlen)
+          rv[i] = epi_load4(a.res + ((size_t)(res_row0 + ((mm * a.ors + oro) >> a.res_shift)) * a.ldr + a.rcol) + n, n, a.Co, vec);
       }
 #pragma unroll
       for (int i = 0; i < 8; i++) {
         const int r = rq + 4 * i;
         const int mm = m0 + q * 32 + r;
         if (mm >= mlen) continue;
-        const float4 v = *reinterpret_cast<const float4*>(scr + r * 32 + ((cq ^ (r & 7)) << 2));
-        float4 o;
-        o.x = fmaf(v.x, a.wscale, bb.x); o.y = fmaf(v.y, a.wscale, bb.y);
-        o.z = fmaf(v.z, a.wscale, bb.z); o.w = fmaf(v.w, a.wscale, bb.w);
-        if (a.eact == ACT_GELU_NEW) { o.x = gelu_new_f(o.x); o.y = gelu_new_f(o.y); o.z = gelu_new_f(o.z); o.w = gelu_new_f(o.w); }
-        o.x = (o.x + rv[i].x) * a.oscale; o.y = (o.y + rv[i].y) * a.oscale;
-        o.z = (o.z + rv[i].z) * a.oscale; o.w = (o.w + rv[i].w) * a.oscale;
-        float* op = a.out + ((size_t)(out_row0 + mm * a.ors + oro) * a.ldo + a.ocol) + n;
-        if (vec) {
-          if (a.accumulate) { const float4 pvv = *reinterpret_cast<const float4*>(op); o.x += pvv.x; o.y += pvv.y; o.z += pvv.z; o.w += pvv.w; }
-          *reinterpret_cast<float4*>(op) = o;
-        } else {
-          if (a.accumulate) { o.x += op[0]; if (n + 1 < a.Co) o.y += op[1]; if (n + 2 < a.Co) o.z += op[2]; if (n + 3 < a.Co) o.w += op[3]; }
-          op[0] = o.x;
-          if (n + 1 < a.Co) op[1] = o.y;
-          if (n + 2 < a.Co) op[2] = o.z;
-          if (n + 3 < a.Co) op[3] = o.w;
-        }
+        const float4 o = epi_math4(*reinterpret_cast<const float4*>(scr + r * 32 + ((cq ^ (r & 7)) << 2)), a.wscale, bb, a.eact, rv[i], a.oscale);
+        epi_store4(a.out + ((size_t)(out_row0 + mm * a.ors + oro) * a.ldo + a.ocol) + n, o, n, a.Co, vec, a.accumulate);
       }
     }
     __syncwarp();
@@ -836,25 +784,22 @@ __global__ void __launch_bounds__(kGemm32pThreads, 1) gemm32p_kernel(const __gri
   const int total = ntm * ((a.Co + BN - 1) / BN);
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA2) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB2) : "memory");
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmB);
+    prefetch_tmap(&tmA2);
+    prefetch_tmap(&tmB2);
     for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int j = 0; j < 3; j++) { mbar_init(bfull_bar(j), 1); mbar_init(bempty_bar(j), NEPI); }
     mbar_init(sfull_bar, 1); mbar_init(sfree_bar, NEPI);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tmem_alloc<1>(tmem_slot, 512u);
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   // tile -> (n-tile, item, m-tile); tile_start is the prefix sum of ceil(m_len / 128) over the items
   // Order: groups of `gm` consecutive m-tiles whose operand planes (~48 MB) stay L2-resident while all the
@@ -976,7 +921,7 @@ __global__ void __launch_bounds__(kGemm32pThreads, 1) gemm32p_kernel(const __gri
           for (int e = 0; e < 64; e++) racc[e] += __uint_as_float(v[e]);
         }
         tc_fence_before();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bempty_bar(j)) : "memory");
+        if (lane == 0) mbar_arrive(bempty_bar(j));
         TCT(1);
       }
       gc += nchains;
@@ -990,7 +935,7 @@ __global__ void __launch_bounds__(kGemm32pThreads, 1) gemm32p_kernel(const __gri
         for (int e = 0; e < 64; e++) racc[e] = __uint_as_float(v[e]) + racc[e];   // same order as the single-tile kernel
       }
       tc_fence_before();
-      if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(sfree_bar) : "memory");   // TMEM is free again
+      if (lane == 0) mbar_arrive(sfree_bar);   // TMEM is free again
 
       // ---- the rest runs while the next tile's pipeline is already going (see gemm32_final)
       gemm32_final(a, scr_f + (warp - 2) * 1024, racc, b, m0, n0, hh, q, lane, mlen, a.oro, a.bias);
@@ -1002,16 +947,13 @@ __global__ void __launch_bounds__(kGemm32pThreads, 1) gemm32p_kernel(const __gri
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc<1>(tmem_base, 512u);
   }
 }
 
 static void launch_gemm32p(const TcConvArgs& a, cudaStream_t st) {
   constexpr int smem = 3 * 4 * 128 * 128 + 8 * 4096 + 14 * 8 + 16 + 1024;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(gemm32p_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
+  const int dev = prepare_smem_launch<gemm32p_kernel>(smem);
   const int nsm = device_sm_count(dev);
   const int total = a.ntiles_m * ((a.Co + 127) / 128);
   const int grid = total < nsm ? total : nsm;
@@ -1085,26 +1027,23 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   const int npairs = gridDim.x >> 1, pair = blockIdx.x >> 1;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmBh) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA2) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmB2h) : "memory");
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmBh);
+    prefetch_tmap(&tmA2);
+    prefetch_tmap(&tmB2h);
     for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int j = 0; j < 3; j++) { mbar_init(bfull_bar(j), 1); mbar_init(bempty_bar(j), 2 * NEPI); }
     mbar_init(sfull_bar, 1); mbar_init(sfree_bar, 2 * NEPI);
     mbar_init(gfull_bar, NEPI); mbar_init(gfree_bar, NFIN);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {   // the same warp of both CTAs
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2>(tmem_slot, 512u);
   }
   tc_fence_before();
   cluster_sync_all();      // barriers of both CTAs initialised, TMEM of both allocated, before any cross-CTA traffic
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   // pair-tile -> (n-tile, this CTA's m-tile); groups of gm2 consecutive m-tile PAIRS stay L2-resident while all their
   // n-tiles are computed (same idea as gemm32p_kernel)
@@ -1246,7 +1185,7 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             make_float4(racc[4 * c], racc[4 * c + 1], racc[4 * c + 2], racc[4 * c + 3]);
       }
       __syncwarp();
-      if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(gfull_bar) : "memory");
+      if (lane == 0) mbar_arrive(gfull_bar);
       TCT(3);
     }
     TCT_FLUSH(8, 4);
@@ -1262,11 +1201,7 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const int n = n0 + lane * 4;
       const bool ncol = n < a.Co;
       const bool vec = a.vec4 && (n + 3 < a.Co);
-      float4 bb = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (a.bias && ncol) {
-        if (vec) bb = *reinterpret_cast<const float4*>(a.bias + n);
-        else { bb.x = a.bias[n]; if (n + 1 < a.Co) bb.y = a.bias[n + 1]; if (n + 2 < a.Co) bb.z = a.bias[n + 2]; if (n + 3 < a.Co) bb.w = a.bias[n + 3]; }
-      }
+      const float4 bb = a.bias && ncol ? epi_load4(a.bias + n, n, a.Co, vec) : make_float4(0.f, 0.f, 0.f, 0.f);
       const int out_row0 = a.out_off[b];
       const int res_row0 = a.res ? a.res_off[b] : 0;
       constexpr int RB = 4;                                    // rows per batch: residual loads of a batch are issued together
@@ -1276,11 +1211,7 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         for (int i = 0; i < RB; i++) {
           rv[i] = make_float4(0.f, 0.f, 0.f, 0.f);
           const int mm = m0 + fw + NFIN * (i0 + i);
-          if (a.res && ncol && mm < mlen && fw + NFIN * (i0 + i) < 128) {
-            const float* rp = res_ptr(mm);
-            if (vec) rv[i] = *reinterpret_cast<const float4*>(rp);
-            else { rv[i].x = rp[0]; if (n + 1 < a.Co) rv[i].y = rp[1]; if (n + 2 < a.Co) rv[i].z = rp[2]; if (n + 3 < a.Co) rv[i].w = rp[3]; }
-          }
+          if (a.res && ncol && mm < mlen && fw + NFIN * (i0 + i) < 128) rv[i] = epi_load4(res_ptr(mm), n, a.Co, vec);
         }
       };
       float4 rv[RB];
@@ -1291,29 +1222,29 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         // fp16 hi / lo of 16 v, zero-filled to a multiple of 64 keys).  The staged tile is read by columns instead: warp fw
         // takes every NFIN-th dim of the tile, a lane one token, so every store covers 32 consecutive keys (64 bytes).
         const int NR = (mlen + 63) & ~63;
-        __half* const vth = static_cast<__half*>(a.attn_pl[4]);
-        __half* const vtl = static_cast<__half*>(a.attn_pl[5]);
+        uint16_t* const vth = static_cast<uint16_t*>(a.attn_pl[4]);
+        uint16_t* const vtl = static_cast<uint16_t*>(a.attn_pl[5]);
 #pragma unroll 1
         for (int cl = fw; cl < 128; cl += NFIN) {                // column inside the tile
           const int cv = n0 - 1536 + cl;                       // V column: head * 64 + d
           const float bias_c = a.bias ? a.bias[n0 + cl] : 0.f;
-          __half* const vh = vth + ((size_t)b * 768 + cv) * 512 + m0;
-          __half* const vl = vtl + ((size_t)b * 768 + cv) * 512 + m0;
+          uint16_t* const vh = vth + ((size_t)b * 768 + cv) * 512 + m0;
+          uint16_t* const vl = vtl + ((size_t)b * 768 + cv) * 512 + m0;
           const int chunk = cl >> 2, e4 = cl & 3;
 #pragma unroll
           for (int tg = 0; tg < 4; tg++) {
             const int r = tg * 32 + lane;                      // token inside the tile
             if (m0 + r < NR) {
               const float raw = stg_f[r * 128 + (((chunk & ~7) | ((chunk ^ r) & 7)) << 2) + e4];
-              const float sv = (m0 + r < mlen ? fmaf(raw, a.wscale, bias_c) : 0.f) * 16.0f;
-              const __half hi = __float2half_rn(sv);
-              vh[r] = hi;
-              vl[r] = __float2half_rn(sv - __half2float(hi));
+              uint32_t hi, lo;
+              split_f16((m0 + r < mlen ? fmaf(raw, a.wscale, bias_c) : 0.f) * 16.0f, hi, lo);
+              vh[r] = (uint16_t)hi;
+              vl[r] = (uint16_t)lo;
             }
           }
         }
         __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(gfree_bar) : "memory");
+        if (lane == 0) mbar_arrive(gfree_bar);
         continue;
       }
 #pragma unroll 1
@@ -1326,18 +1257,13 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         }
         if (i0 + RB >= (128 + NFIN - 1) / NFIN) {             // last read of the staged tile
           __syncwarp();
-          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(gfree_bar) : "memory");
+          if (lane == 0) mbar_arrive(gfree_bar);
         }
 #pragma unroll
         for (int i = 0; i < RB; i++) {
           const int mm = m0 + fw + NFIN * (i0 + i);
           if (mm >= mlen || !ncol || fw + NFIN * (i0 + i) >= 128) continue;
-          float4 o;
-          o.x = fmaf(v[i].x, a.wscale, bb.x); o.y = fmaf(v[i].y, a.wscale, bb.y);
-          o.z = fmaf(v[i].z, a.wscale, bb.z); o.w = fmaf(v[i].w, a.wscale, bb.w);
-          if (a.eact == ACT_GELU_NEW) { o.x = gelu_new_f(o.x); o.y = gelu_new_f(o.y); o.z = gelu_new_f(o.z); o.w = gelu_new_f(o.w); }
-          o.x = (o.x + rv[i].x) * a.oscale; o.y = (o.y + rv[i].y) * a.oscale;
-          o.z = (o.z + rv[i].z) * a.oscale; o.w = (o.w + rv[i].w) * a.oscale;
+          const float4 o = epi_math4(v[i], a.wscale, bb, a.eact, rv[i], a.oscale);
           const size_t orow = (size_t)(out_row0 + mm * a.ors + a.oro);
           if (a.attn_pl[0]) {   // QKV projection, Q and K columns: fp16 hi / lo planes of 2 q (= 16 q / sqrt(64)) and 16 k
             const bool isq = n0 < 768;
@@ -1345,12 +1271,7 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             const float e4[4] = {o.x, o.y, o.z, o.w};
             uint32_t hw[4], lw[4];
 #pragma unroll
-            for (int e = 0; e < 4; e++) {
-              const float sv = e4[e] * sc_;
-              const __half hi = __float2half_rn(sv);
-              hw[e] = __half_as_ushort(hi);
-              lw[e] = __half_as_ushort(__float2half_rn(sv - __half2float(hi)));
-            }
+            for (int e = 0; e < 4; e++) split_f16(e4[e] * sc_, hw[e], lw[e]);
             const size_t pidx = orow * 768 + (size_t)(isq ? n : n - 768);
             *reinterpret_cast<uint2*>(static_cast<__half*>(a.attn_pl[isq ? 0 : 2]) + pidx) = make_uint2(hw[0] | (hw[1] << 16), hw[2] | (hw[3] << 16));
             *reinterpret_cast<uint2*>(static_cast<__half*>(a.attn_pl[isq ? 1 : 3]) + pidx) = make_uint2(lw[0] | (lw[1] << 16), lw[2] | (lw[3] << 16));
@@ -1360,27 +1281,12 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             const float e4[4] = {o.x, o.y, o.z, o.w};
             uint32_t hw[4], lw[4];
 #pragma unroll
-            for (int e = 0; e < 4; e++) {
-              const float sv = fminf(fmaxf(e4[e] * kSplitF16Scale, -65504.f), 65504.f);
-              const __half hi = __float2half_rn(sv);
-              hw[e] = __half_as_ushort(hi);
-              lw[e] = __half_as_ushort(__float2half_rn(sv - __half2float(hi)));
-            }
+            for (int e = 0; e < 4; e++) split_f16_operand(e4[e], hw[e], lw[e]);
             *reinterpret_cast<uint2*>(static_cast<__half*>(a.out_hi) + orow * a.out_pl_ld + n) = make_uint2(hw[0] | (hw[1] << 16), hw[2] | (hw[3] << 16));
             *reinterpret_cast<uint2*>(static_cast<__half*>(a.out_lo) + orow * a.out_pl_ld + n) = make_uint2(lw[0] | (lw[1] << 16), lw[2] | (lw[3] << 16));
             if (!a.out) continue;
           }
-          float* op = a.out + (orow * a.ldo + a.ocol) + n;
-          if (vec) {
-            if (a.accumulate) { const float4 pvv = *reinterpret_cast<const float4*>(op); o.x += pvv.x; o.y += pvv.y; o.z += pvv.z; o.w += pvv.w; }
-            *reinterpret_cast<float4*>(op) = o;
-          } else {
-            if (a.accumulate) { o.x += op[0]; if (n + 1 < a.Co) o.y += op[1]; if (n + 2 < a.Co) o.z += op[2]; if (n + 3 < a.Co) o.w += op[3]; }
-            op[0] = o.x;
-            if (n + 1 < a.Co) op[1] = o.y;
-            if (n + 2 < a.Co) op[2] = o.z;
-            if (n + 3 < a.Co) op[3] = o.w;
-          }
+          epi_store4(a.out + (orow * a.ldo + a.ocol) + n, o, n, a.Co, vec, a.accumulate);
         }
         if (i0 + RB < (128 + NFIN - 1) / NFIN) load_res(i0 + RB, rv);
       }
@@ -1390,15 +1296,12 @@ gemm32p2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   cluster_sync_all();      // nobody leaves (or frees TMEM) while the peer may still signal it or the pair-MMAs read its smem
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc<2>(tmem_base, 512u);
   }
 }
 
 static void launch_gemm32p2(const TcConvArgs& a, cudaStream_t st) {
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(gemm32p2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kG2Smem)); });
+  const int dev = prepare_smem_launch<gemm32p2_kernel>(kG2Smem);
   const int nsm = device_sm_count(dev);
   const int total = ((a.ntiles_m + 1) / 2) * ((a.Co + 127) / 128);
   int npairs = nsm / 2;
@@ -1462,22 +1365,19 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   const int npairs = gridDim.x >> 1, pair = blockIdx.x >> 1;
 
   if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmA) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmBh) : "memory");
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmBh);
     for (int s = 0; s < STAGES; s++) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
     for (int j = 0; j < 2; j++) { mbar_init(tfull_bar(j), 1); mbar_init(tempty_bar(j), 2 * NEPI); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    mbar_init_fence();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    tmem_alloc<2>(tmem_slot, 512u);
   }
   tc_fence_before();
   cluster_sync_all();
   tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot) : "memory");
+  const uint32_t tmem_base = tmem_base_of(tmem_slot);
 
   const int gm2 = a.group_m > 1 ? (a.group_m >> 1) : 1;
   // tile -> (item, m-tile of this CTA, phase, first output channel); n-tiles (all phases) are the outer loop inside a
@@ -1578,7 +1478,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   cluster_sync_all();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+    tmem_dealloc<2>(tmem_base, 512u);
   }
 }
 
@@ -1591,10 +1491,7 @@ static bool conv_tc_takes_pair_bf16(const TcConvArgs& a, int nsm) {
 
 template <int BN>
 static void launch_conv_pair_t(const TcConvArgs& a, cudaStream_t st) {
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_pair_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, CpCfg<BN>::SMEM)); });
+  const int dev = prepare_smem_launch<conv_pair_kernel<BN>>(CpCfg<BN>::SMEM);
   const int nsm = device_sm_count(dev);
   const int total = ((a.ntiles_m + 1) / 2) * (a.Co / BN) * (a.nphase > 1 ? a.nphase : 1);
   int npairs = nsm / 2;
@@ -1612,10 +1509,7 @@ static void launch_conv_pair(const TcConvArgs& a, cudaStream_t st) { launch_conv
 template <int BN, int STAGES>
 static void launch_tc_multi(const TcConvArgs& a, cudaStream_t st) {
   constexpr int smem = STAGES * (128 * 128 + BN * 128) + 2 * 128 * 36 * 4 + (2 * STAGES + 4) * 8 + 16 + 1024;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_tc_multi_kernel<BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
+  prepare_smem_launch<conv_tc_multi_kernel<BN, STAGES>>(smem);
   dim3 g((a.max_m + 127) / 128, (a.Co + BN - 1) / BN, a.B);
   conv_tc_multi_kernel<BN, STAGES><<<g, 192, smem, st>>>(*reinterpret_cast<const CUtensorMap*>(a.tmA),
                                                          *reinterpret_cast<const CUtensorMap*>(a.tmB), a);
@@ -1625,10 +1519,7 @@ template <int BN, int STAGES, int MODE>
 static void launch_tc(const TcConvArgs& a, cudaStream_t st) {
   constexpr int PLANES = MODE ? 2 : 1;
   constexpr int smem = STAGES * PLANES * (128 * 128 + BN * 128) + (2 * STAGES + 7) * 8 + 16 + 1024;
-  static DevOnce once;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  once.run(dev, [] { KKX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BN, STAGES, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); });
+  prepare_smem_launch<conv_tc_kernel<BN, STAGES, MODE>>(smem);
   const unsigned gx = (unsigned)((a.max_m + 127) / 128);
   dim3 g(gx, (a.Co + BN - 1) / BN, a.B);
   if (MODE == 0 && a.nphase > 1) g = dim3((unsigned)(a.nphase * ((a.Co + BN - 1) / BN)), gx, a.B);
@@ -2064,19 +1955,11 @@ __global__ void __launch_bounds__(256) apply_f16x2_kernel(const float* __restric
         } else v[e] = 0.f;
       }
     }
-    __half hi[4], lo[4];
+    uint32_t hi[4], lo[4];
 #pragma unroll
-    for (int e = 0; e < 4; e++) {
-      const float s = fminf(fmaxf(v[e] * kSplitF16Scale, -65504.f), 65504.f);
-      hi[e] = __float2half_rn(s);
-      lo[e] = __float2half_rn(s - __half2float(hi[e]));
-    }
-    *reinterpret_cast<uint2*>(out_hi + (size_t)r * Cpad + c) =
-        make_uint2((uint32_t)__half_as_ushort(hi[0]) | ((uint32_t)__half_as_ushort(hi[1]) << 16),
-                   (uint32_t)__half_as_ushort(hi[2]) | ((uint32_t)__half_as_ushort(hi[3]) << 16));
-    *reinterpret_cast<uint2*>(out_lo + (size_t)r * Cpad + c) =
-        make_uint2((uint32_t)__half_as_ushort(lo[0]) | ((uint32_t)__half_as_ushort(lo[1]) << 16),
-                   (uint32_t)__half_as_ushort(lo[2]) | ((uint32_t)__half_as_ushort(lo[3]) << 16));
+    for (int e = 0; e < 4; e++) split_f16_operand(v[e], hi[e], lo[e]);
+    *reinterpret_cast<uint2*>(out_hi + (size_t)r * Cpad + c) = make_uint2(hi[0] | (hi[1] << 16), hi[2] | (hi[3] << 16));
+    *reinterpret_cast<uint2*>(out_lo + (size_t)r * Cpad + c) = make_uint2(lo[0] | (lo[1] << 16), lo[2] | (lo[3] << 16));
   }
 }
 float split_f16_host(const float* w, size_t n, unsigned short* hi, unsigned short* lo) {
@@ -2092,11 +1975,10 @@ float split_f16_host(const float* w, size_t n, unsigned short* hi, unsigned shor
   if (s < -60) s = -60;
   const float up = ldexpf(1.f, s);
   for (size_t i = 0; i < n; i++) {
-    const float v = w[i] * up;         // exact (power of two)
-    const __half h = __float2half_rn(v);
-    const __half l = __float2half_rn(v - __half2float(h));
-    hi[i] = __half_as_ushort(h);
-    lo[i] = __half_as_ushort(l);
+    uint32_t h, l;
+    split_f16(w[i] * up, h, l);        // the scaling is exact (power of two)
+    hi[i] = (unsigned short)h;
+    lo[i] = (unsigned short)l;
   }
   return ldexpf(1.f, -s);
 }

@@ -1,16 +1,41 @@
 // tc_ptx.cuh -- raw-PTX device helpers shared by the tcgen05 kernels (mbarrier, TMA, UMMA
-// descriptors, tcgen05.mma / commit / ld).  sm_100a only.
+// descriptors, tcgen05.mma / commit / ld / alloc) and the split-FP16 operand encoding.  sm_100a only.
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
+#include "kernels.h"
 
 namespace kkx {
 
+// fp16 hi = rn(v), lo = rn(v - hi) of an already scaled v, as raw 16-bit patterns.  Every split-FP16 plane (activation
+// operands, weights, attention Q / K / V^T) is encoded here, so a value gives the same planes whichever kernel wrote them.
+__host__ __device__ __forceinline__ void split_f16(float v, uint32_t& hi, uint32_t& lo) {
+  const __half h = __float2half_rn(v);
+  hi = __half_as_ushort(h);
+  lo = __half_as_ushort(__float2half_rn(v - __half2float(h)));
+}
+// GEMM activation operand: kSplitF16Scale * v, saturated at the fp16 range, then split (the GEMM epilogue divides by
+// kSplitF16Scale again through its wscale)
+__device__ __forceinline__ void split_f16_operand(float v, uint32_t& hi, uint32_t& lo) {
+  split_f16(fminf(fmaxf(v * kSplitF16Scale, -65504.f), 65504.f), hi, lo);
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+__device__ __forceinline__ void prefetch_tmap(const void* p) { asm volatile("prefetch.tensormap [%0];" ::"l"(p) : "memory"); }
 
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
+}
+// after the barrier inits of a CTA: make them visible to the async proxy (TMA, tcgen05.commit) and to the cluster
+__device__ __forceinline__ void mbar_init_fence() {
+  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
@@ -40,6 +65,32 @@ __device__ __forceinline__ void cluster_sync_all() {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+
+// TMEM of a CTA (CG = 1) or of a CTA pair (CG = 2, the same warp of both CTAs): one whole warp allocates `cols`
+// columns, writes the base address to the shared-memory word `slot` and gives up the right to allocate more; the
+// other warps read the base after the CTA (cluster) barrier that follows.
+template <int CG>
+__device__ __forceinline__ void tmem_alloc(uint32_t slot, uint32_t cols) {
+  static_assert(CG == 1 || CG == 2, "cta_group is 1 or 2");
+  if constexpr (CG == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(cols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  } else {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(cols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+  }
+}
+__device__ __forceinline__ uint32_t tmem_base_of(uint32_t slot) {
+  uint32_t base;
+  asm volatile("ld.shared.b32 %0, [%1];" : "=r"(base) : "r"(slot) : "memory");
+  return base;
+}
+template <int CG>
+__device__ __forceinline__ void tmem_dealloc(uint32_t base, uint32_t cols) {
+  static_assert(CG == 1 || CG == 2, "cta_group is 1 or 2");
+  if constexpr (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols) : "memory");
+  else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(cols) : "memory");
+}
 
 // SM100 shared-memory matrix descriptor, K-major, SWIZZLE_128B: start>>4 | LBO(1)<<16 | SBO(1024B>>4)<<32 |
 // version 1 <<46 | layout SWIZZLE_128B (2) << 61
