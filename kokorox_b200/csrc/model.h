@@ -212,6 +212,30 @@ constexpr long long kMaxFlacSamples = (1LL << 36) - 1;
 // Throws ArgError otherwise.
 void check_programs(int B, int P, const int32_t* p);
 
+// Optional parts of a Model::gemm / Model::tc_conv launch, set by name; the defaults are a plain Linear (a k = 1 conv).
+// The fields mean what they mean in ConvArgs (kernels.h): taps ks at input rows m + tap * dil - pad, output row
+// m * ors + oro, epilogue activation eact, residual res (rows of Lres, shifted right by res_shift), scale oscale.
+// tc_conv takes its taps from the weight and has neither the prologue nor the operand planes.
+struct ConvOpt {
+  int eact = ACT_NONE;
+  int ks = 1, dil = 1, pad = 0;
+  int ors = 1, oro = 0;
+  // prologue on the input operand: pact(x * pscale[b, c] + pshift[b, c]), LeakyReLU slope pslope
+  const float* pscale = nullptr; const float* pshift = nullptr; int pact = ACT_NONE; float pslope = 0.f;
+  const float* res = nullptr; int ldr = 0; const Level* Lres = nullptr; int res_shift = 0;
+  float oscale = 1.f;
+  // Operand planes handed from producer to consumer without the fp32 round trip (gemm, split-FP16 path only):
+  //   in_hi / in_lo   the input already exists as fp16 hi / lo planes [Lin.rows, Cpad of the weight] (written by the
+  //                   LayerNorm before, or by the GEMM before): no apply pass;
+  //   out_hi / out_lo ask the GEMM to leave its result as planes [rows, out_ld] for the next GEMM INSTEAD of the fp32
+  //                   output; honoured only by the CTA-pair kernel -- gemm returns whether it happened (otherwise the
+  //                   fp32 output was written as usual);
+  //   attn_scratch    the same for the QKV projection and the planes of launch_attention_umma.
+  const void* in_hi = nullptr; const void* in_lo = nullptr;
+  void* out_hi = nullptr; void* out_lo = nullptr; int out_ld = 0;
+  float* attn_scratch = nullptr;
+};
+
 // What a run returns besides the f32 waveform, which every run writes: its 16-bit PCM twin, the G.711 codes of that
 // PCM (mu-law / A-law), or one FLAC stream per item encoded from it (kkx.h).
 enum class Encoding { F32, PCM16, ULAW, ALAW, FLAC };
@@ -286,24 +310,10 @@ class Model {
     float* wav24 = nullptr;    // resampling pass only: the run's 24 kHz waveform, item b at s24_off_[b]
   };
   // Linear / Conv1d on the precision-critical path: split-TF32 tensor cores when precision==1 and
-  // the weight has a TcW32, fp32 SIMT otherwise.
-  // Operand planes handed from producer to consumer without the fp32 round trip (split-FP16 path only):
-  //   in_hi / in_lo   the input already exists as fp16 hi / lo planes [Lin.rows, Cpad of the weight] (written by the
-  //                   LayerNorm before, or by the GEMM before): no apply pass;
-  //   out_hi / out_lo ask the GEMM to leave its result as planes [rows, out_ld] for the next GEMM INSTEAD of the fp32
-  //                   output; honoured only by the CTA-pair kernel -- `out_done` tells the caller whether it happened
-  //                   (otherwise the fp32 output was written as usual);
-  //   attn_scratch    the same for the QKV projection and the planes of launch_attention_umma.
-  struct GemmPlanes {
-    const void* in_hi = nullptr; const void* in_lo = nullptr;
-    void* out_hi = nullptr; void* out_lo = nullptr; int out_ld = 0; bool out_done = false;
-    float* attn_scratch = nullptr;   // QKV projection: leave the result as the attention kernel's operand planes (same rule)
-  };
-  void gemm(const Level& Lin, const Level& Lm, const float* in, int ldi, int K, const float* w, const TcW32* w32,
-            const float* bias, int N, float* out, int ldo, int ocol, int eact = ACT_NONE, int ks = 1,
-            int pad = 0, const float* pscale = nullptr, const float* pshift = nullptr, int pact = ACT_NONE,
-            float pslope = 0.f, const float* res = nullptr, int ldr = 0, const Level* Lres = nullptr,
-            int res_shift = 0, float oscale = 1.f, GemmPlanes* pl = nullptr);
+  // the weight has a TcW32, fp32 SIMT otherwise.  Returns true when the result went to the operand planes of `o`
+  // instead of `out`.
+  bool gemm(const Level& Lin, const Level& Lm, const float* in, int ldi, int K, const float* w, const TcW32* w32,
+            const float* bias, int N, float* out, int ldo, int ocol, const ConvOpt& o = ConvOpt());
   bool planes_ok() const { return opt.precision == 1 && opt.split_f16 && opt.fuse_planes; }
   float* split_hi_ = nullptr; float* split_lo_ = nullptr; size_t split_cap_ = 0;  // scratch planes (floats) of the current lane
   // Two execution lanes: lane 0 = stream_, lane 1 = stream2_ (forked branches of small batches).  cur_ is the stream
@@ -319,23 +329,30 @@ class Model {
   void fork_lane1();   // lane 1 starts after everything issued so far on lane 0
   void join_lane1();   // lane 0 continues after everything issued so far on lane 1
   bool can_fork(int B) const { return B <= opt.fork_max_batch && !debug_ && !stats.profile && !stats.check_each; }
-  void tc_conv(Arena& A, const void* abuf, int rows_total, const TcW& w, int dil, int pad, const Level& Lin,
-               const Level& Lm, const float* bias, float* out, int ldo, int ocol, const Level& Lout, int ors,
-               int oro, const float* res, int ldr, const Level* Lres, int res_shift, float oscale,
-               bool accumulate);
+  // bf16 tensor-core conv of the operand buffer `abuf` [rows_total, w.Cpad]
+  void tc_conv(const void* abuf, int rows_total, const TcW& w, const Level& Lin, const Level& Lm, const float* bias,
+               float* out, int ldo, int ocol, const Level& Lout, const ConvOpt& o = ConvOpt());
   void token_phase(Run& r);          // graph replay or eager issue, then the one host sync of the call
   void token_issue(Run& r);          // every token-rate launch + the D2H of frame counts / durations (no sync)
   void token_finish(Run& r);         // sync, read T_b, validate
   size_t token_arena_bytes() const;
   // items [b0, b1); programs [k0, k1) are those whose last item is in the group (post-processed after it)
   void frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry);
-  void adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ldx, const Level& Lin,
-                 const Level& Lout, const float* sty, int sld, float* out, int ldo, int ocol,
-                 bool dry);
-  void arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L, const float* sty,
-           int sld, float* xw, float* t1, float* out, float oscale, bool accumulate,
-           const float* part_x = nullptr, const void* x_bf16 = nullptr);
+  void adain_blk(Arena& A, const AdaBlkW& w, const float* x, int ldx, const Level& Lin, const Level& Lout,
+                 const float* sty, int sld, float* out, int ldo, int ocol);
+  void arb(Arena& A, const ArbW& w, const float* x, const Level& L, const float* sty, int sld, float* xw, float* t1,
+           float* out, float oscale, bool accumulate, const float* part_x = nullptr, const void* x_bf16 = nullptr);
   bool use_stream_bf16(int C, int k, int B) const;
+  // generator up-sampling: ConvTranspose1d(Ci, Co, k = 2s, stride s, padding s/2) of LeakyReLU(0.1)(x), x [Lin rows,
+  // Ci] -> out [Lout rows, Co], as s two-tap phase convs whose output rows are shifted by `shift`.  w_all: the phases
+  // stacked (one launch for all); w_tc / w32: one bf16 / fp32 weight per phase.  No phase-fused launch when `dry`.
+  void upsample(Arena& A, const float* x, const Level& Lin, float* out, const Level& Lout, int s, int shift,
+                const TcW& w_all, const std::vector<TcW>& w_tc, const std::vector<float*>& w32, const float* bias,
+                bool dry);
+  // generator stage after its up-sampling: x += x_source xs, then acc = the mean of the three res-blocks w[0..2] of x
+  // (sty: the items' decoder-side style parameters; xw / t: the res-blocks' work buffers)
+  void res_stage(Arena& A, const ArbW* w, float* x, const float* xs, const Level& L, const float* sty, float* xw,
+                 float* t, float* acc);
   // first_off: row offset of item 0 (kGapRows for activations; 0 for the per-item style tables)
   Level make_level(const std::vector<int>& lens, Arena& A, int first_off = kGapRows);
   // copy `bytes` of host data to device memory through the pinned staging arena (true async copy on stream_)

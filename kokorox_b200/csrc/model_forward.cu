@@ -30,6 +30,19 @@ ConvArgs gemm_args(const Level& L, const float* in, int ldi, int K, const float*
   a.out = out; a.ldo = ldo; a.ocol = ocol; a.out_off = L.d_off;
   return a;
 }
+// what every tensor-core launch fills alike: input rows of item b from Lin, output rows m of Lm stored at the rows of
+// Lout, epilogue and residual
+TcConvArgs tc_args(const Level& Lin, const Level& Lm, const Level& Lout, const float* bias, float* out, int ldo, int ocol,
+                   const ConvOpt& o) {
+  TcConvArgs a;
+  a.eact = o.eact; a.dil = o.dil; a.pad = o.pad;
+  a.in_off = Lin.d_off; a.m_len = Lm.d_len; a.max_m = Lm.max_len; a.B = Lm.B; a.sum_m = Lm.sum_len;
+  a.tile_start = Lm.d_tiles128; a.ntiles_m = Lm.ntiles128;
+  a.bias = bias; a.out = out; a.ldo = ldo; a.ocol = ocol; a.out_off = Lout.d_off; a.ors = o.ors; a.oro = o.oro;
+  a.res = o.res; a.ldr = o.ldr; a.res_off = o.Lres ? o.Lres->d_off : nullptr; a.res_shift = o.res_shift;
+  a.oscale = o.oscale;
+  return a;
+}
 }  // namespace
 
 void arb_timing_dump() {
@@ -53,81 +66,70 @@ void arb_timing_dump() {
   }
 }
 
-void Model::tc_conv(Arena& A, const void* abuf, int rows_total, const TcW& w, int dil, int pad, const Level& Lin,
-                    const Level& Lm, const float* bias, float* out, int ldo, int ocol, const Level& Lout, int ors,
-                    int oro, const float* res, int ldr, const Level* Lres, int res_shift, float oscale,
-                    bool accumulate) {
-  (void)A;
+void Model::tc_conv(const void* abuf, int rows_total, const TcW& w, const Level& Lin, const Level& Lm, const float* bias,
+                    float* out, int ldo, int ocol, const Level& Lout, const ConvOpt& o) {
   alignas(64) unsigned char tmA[128];
   if (g_dry_run) return;
   make_tmap_bf16(tmA, abuf, w.Cpad, rows_total, w.Cpad, 128);
-  TcConvArgs a;
+  TcConvArgs a = tc_args(Lin, Lm, Lout, bias, out, ldo, ocol, o);
   a.tmA = tmA; a.tmB = w.tmap;
-  a.Cpad = w.Cpad; a.Ci = w.Ci; a.Co = w.Co; a.ks = w.ks; a.dil = dil; a.pad = pad;
-  a.in_off = Lin.d_off; a.m_len = Lm.d_len; a.max_m = Lm.max_len; a.B = Lm.B; a.sum_m = Lm.sum_len;
-  a.bias = bias; a.out = out; a.ldo = ldo; a.ocol = ocol; a.out_off = Lout.d_off; a.ors = ors; a.oro = oro;
-  a.res = res; a.ldr = ldr; a.rcol = 0; a.res_off = Lres ? Lres->d_off : nullptr; a.res_shift = res_shift;
-  a.oscale = oscale; a.accumulate = accumulate ? 1 : 0;
+  a.Cpad = w.Cpad; a.Ci = w.Ci; a.Co = w.Co; a.ks = w.ks;
   if (opt.conv_pair && w.pair_map(w.Co)) {      // CTA-pair kernel (taken when the batch gives every pair a tile)
-    a.tmB_c = w.pair_map(w.Co); a.pair = 1; a.tile_start = Lm.d_tiles128; a.ntiles_m = Lm.ntiles128;
+    a.tmB_c = w.pair_map(w.Co); a.pair = 1;
   }
   launch_conv_tc(a, cur_);
 }
 
-void Model::gemm(const Level& Lin, const Level& Lm, const float* in, int ldi, int K, const float* w, const TcW32* w32,
-                 const float* bias, int N, float* out, int ldo, int ocol, int eact, int ks, int pad,
-                 const float* pscale, const float* pshift, int pact, float pslope, const float* res, int ldr,
-                 const Level* Lres, int res_shift, float oscale, GemmPlanes* pl) {
+bool Model::gemm(const Level& Lin, const Level& Lm, const float* in, int ldi, int K, const float* w, const TcW32* w32,
+                 const float* bias, int N, float* out, int ldo, int ocol, const ConvOpt& o) {
   cudaStream_t st = cur_;
-  if (pl) pl->out_done = false;
   if (opt.precision == 1 && w32 && w32->hi && split_hi_ && (size_t)Lin.rows * w32->Cpad <= split_cap_) {
-    if (g_dry_run) return;
+    if (g_dry_run) return false;
     const bool f16 = opt.split_f16 && w32->h_hi;
     alignas(64) unsigned char tA[128], tA2[128];
-    TcConvArgs a;
+    TcConvArgs a = tc_args(Lin, Lm, Lm, bias, out, ldo, ocol, o);
     if (f16) {
-      const bool planes_in = pl && pl->in_hi && pl->in_lo && !pscale && pact == ACT_NONE && ks == 1;
+      const bool planes_in = o.in_hi && o.in_lo && !o.pscale && o.pact == ACT_NONE && o.ks == 1;
       // the scratch planes hold 2-byte elements in this mode (half of the fp32-sized buffers is used)
       if (!planes_in)
-        launch_apply_f16x2(in, ldi, K, pscale, pshift, pact, pslope, split_hi_, split_lo_, w32->Cpad, Lin.rows,
+        launch_apply_f16x2(in, ldi, K, o.pscale, o.pshift, o.pact, o.pslope, split_hi_, split_lo_, w32->Cpad, Lin.rows,
                            Lin.d_off, Lin.d_len, Lin.B, Lin.max_len, st);
-      make_tmap_f16(tA, planes_in ? pl->in_hi : split_hi_, w32->Cpad, Lin.rows, w32->Cpad, 128);
-      make_tmap_f16(tA2, planes_in ? pl->in_lo : split_lo_, w32->Cpad, Lin.rows, w32->Cpad, 128);
+      make_tmap_f16(tA, planes_in ? o.in_hi : split_hi_, w32->Cpad, Lin.rows, w32->Cpad, 128);
+      make_tmap_f16(tA2, planes_in ? o.in_lo : split_lo_, w32->Cpad, Lin.rows, w32->Cpad, 128);
       a.tmB = w32->tm16_hi; a.tmB2 = w32->tm16_lo; a.f16 = 1;
       a.wscale = w32->wscale16 / kSplitF16Scale;
       if (w32->has_c) { a.tmB_c = w32->tm16_hi_c; a.tmB2_c = w32->tm16_lo_c; a.pair = opt.gemm_pair; }
     } else {
-      launch_apply_tf32(in, ldi, K, pscale, pshift, pact, pslope, split_hi_, split_lo_, w32->Cpad, Lin.rows,
+      launch_apply_tf32(in, ldi, K, o.pscale, o.pshift, o.pact, o.pslope, split_hi_, split_lo_, w32->Cpad, Lin.rows,
                         Lin.d_off, Lin.d_len, Lin.B, Lin.max_len, st);
       make_tmap_f32(tA, split_hi_, w32->Cpad, Lin.rows, w32->Cpad, 128);
       make_tmap_f32(tA2, split_lo_, w32->Cpad, Lin.rows, w32->Cpad, 128);
       a.tmB = w32->tm_hi; a.tmB2 = w32->tm_lo;
       if (w32->has_c) { a.tmB_c = w32->tm_hi_c; a.tmB2_c = w32->tm_lo_c; }
     }
-    a.tmA = tA; a.tmA2 = tA2; a.tf32 = 1; a.nprod = 3; a.eact = eact;
-    a.Cpad = w32->Cpad; a.Ci = K; a.Co = N; a.ks = ks; a.dil = 1; a.pad = pad;
-    a.in_off = Lin.d_off; a.m_len = Lm.d_len; a.max_m = Lm.max_len; a.B = Lm.B; a.sum_m = Lm.sum_len;
-    a.bias = bias; a.out = out; a.ldo = ldo; a.ocol = ocol; a.out_off = Lm.d_off;
-    a.res = res; a.ldr = ldr; a.res_off = Lres ? Lres->d_off : nullptr; a.res_shift = res_shift; a.oscale = oscale;
+    a.tmA = tA; a.tmA2 = tA2; a.tf32 = 1; a.nprod = 3;
+    a.Cpad = w32->Cpad; a.Ci = K; a.Co = N; a.ks = o.ks;
     if (long long* tim = arb_timing_buf()) a.timing = tim + 100;   // diagnostics: slots 100..111
-    a.tile_start = Lm.d_tiles128; a.ntiles_m = Lm.ntiles128;
-    if (pl && pl->out_hi && pl->out_lo && f16 && N % 4 == 0 && pl->out_ld >= N && ocol == 0 && conv_tc_takes_pair(a)) {
-      a.out_hi = pl->out_hi; a.out_lo = pl->out_lo; a.out_pl_ld = pl->out_ld; a.out = nullptr;
-      pl->out_done = true;
-    } else if (pl && pl->attn_scratch && f16 && N == 2304 && eact == ACT_NONE && !res && oscale == 1.f && conv_tc_takes_pair(a)) {
-      attention_umma_planes(pl->attn_scratch, Lm.rows, Lm.B, a.attn_pl);
+    bool planes_out = false;
+    if (o.out_hi && o.out_lo && f16 && N % 4 == 0 && o.out_ld >= N && ocol == 0 && conv_tc_takes_pair(a)) {
+      a.out_hi = o.out_hi; a.out_lo = o.out_lo; a.out_pl_ld = o.out_ld; a.out = nullptr;
+      planes_out = true;
+    } else if (o.attn_scratch && f16 && N == 2304 && o.eact == ACT_NONE && !o.res && o.oscale == 1.f && conv_tc_takes_pair(a)) {
+      attention_umma_planes(o.attn_scratch, Lm.rows, Lm.B, a.attn_pl);
       a.out = nullptr;
-      pl->out_done = true;
+      planes_out = true;
     }
     launch_conv_tc(a, st);
-    return;
+    return planes_out;
   }
   ConvArgs c = gemm_args(Lm, in, ldi, K, w, bias, N, out, ldo, ocol);
   c.in_off = Lin.d_off; c.in_len = Lin.d_len;
-  c.ks = ks; c.pad = pad; c.eact = eact;
-  c.pscale = pscale; c.pshift = pshift; c.pld = K; c.pact = pact; c.pslope = pslope;
-  c.res = res; c.ldr = ldr; c.res_off = Lres ? Lres->d_off : nullptr; c.res_shift = res_shift; c.oscale = oscale;
+  c.ks = o.ks; c.dil = o.dil; c.pad = o.pad; c.ors = o.ors; c.oro = o.oro; c.eact = o.eact;
+  c.pscale = o.pscale; c.pshift = o.pshift; c.pld = K; c.pact = o.pact; c.pslope = o.pslope;
+  c.res = o.res; c.ldr = o.ldr; c.res_off = o.Lres ? o.Lres->d_off : nullptr; c.res_shift = o.res_shift;
+  c.oscale = o.oscale;
   launch_conv_f32(c, st);
+  return false;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -248,8 +250,10 @@ void Model::token_issue(Run& r) {
   auto text_encoder = [&] {
     cudaStream_t ts = cur_;
     launch_embed_rows(d_ids_, W.temb, 512, ta, 512, L.d_off, L.d_len, B, L.max_len, ts);
+    ConvOpt k5;
+    k5.ks = 5; k5.pad = 2;
     for (int i = 0; i < 3; i++) {
-      gemm(L, L, ta, 512, 512, W.tcnn_w[i], &W.t_tcnn[i], W.tcnn_b[i], 512, tb, 512, 0, ACT_NONE, 5, 2);
+      gemm(L, L, ta, 512, 512, W.tcnn_w[i], &W.t_tcnn[i], W.tcnn_b[i], 512, tb, 512, 0, k5);
       LnArgs ln;
       ln.x = tb; ln.ldx = 512; ln.w = W.tln_g[i]; ln.b = W.tln_b[i]; ln.eps = 1e-5f; ln.slope = 0.2f;
       ln.out = ta; ln.ldo = 512; ln.off = L.d_off; ln.len = L.d_len; ln.B = B; ln.max_len = L.max_len;
@@ -286,12 +290,11 @@ void Model::token_issue(Run& r) {
                       L.max_len, st);
   gemm(L, L, e, 128, 128, W.map_w, &W.t_map, W.map_b, 768, h, 768, 0);
   for (int layer = 0; layer < 12; layer++) {
-    GemmPlanes gq;
-    if (h_planes) { gq.in_hi = p768h; gq.in_lo = p768l; }
-    if (pl_ok && att_scratch) gq.attn_scratch = att_scratch;   // Q/8, K, V^T planes straight from the GEMM's final warps
-    gemm(L, L, h, 768, 768, W.qkv_w, &W.t_qkv, W.qkv_b, 2304, qkv, 2304, 0, ACT_NONE, 1, 0, nullptr, nullptr, ACT_NONE, 0.f,
-         nullptr, 0, nullptr, 0, 1.f, &gq);
-    if (att_scratch) launch_attention_umma(qkv, att_scratch, ctx, L.d_off, L.d_len, B, L.max_len, L.rows, st, gq.out_done);
+    ConvOpt oq;
+    if (h_planes) { oq.in_hi = p768h; oq.in_lo = p768l; }
+    if (pl_ok && att_scratch) oq.attn_scratch = att_scratch;   // Q/8, K, V^T planes straight from the GEMM's final warps
+    const bool qkv_planes = gemm(L, L, h, 768, 768, W.qkv_w, &W.t_qkv, W.qkv_b, 2304, qkv, 2304, 0, oq);
+    if (att_scratch) launch_attention_umma(qkv, att_scratch, ctx, L.d_off, L.d_len, B, L.max_len, L.rows, st, qkv_planes);
     else launch_attention(qkv, ctx, L.d_off, L.d_len, B, L.max_len, st);
     gemm(L, L, ctx, 768, 768, W.dense_w, &W.t_dense, W.dense_b, 768, tmp, 768, 0);
     LnArgs ln;
@@ -300,14 +303,13 @@ void Model::token_issue(Run& r) {
     ln.max_len = L.max_len; ln.C = 768;
     if (pl_ok) { ln.pl_hi = p768h; ln.pl_lo = p768l; ln.pl_ld = 768; }      // h1 as planes for the FFN GEMM
     launch_layernorm(ln, st);
-    GemmPlanes gf;
-    if (pl_ok) { gf.in_hi = p768h; gf.in_lo = p768l; gf.out_hi = p2048h; gf.out_lo = p2048l; gf.out_ld = 2048; }
-    gemm(L, L, h1, 768, 768, W.ffn_w, &W.t_ffn, W.ffn_b, 2048, ff, 2048, 0, ACT_GELU_NEW, 1, 0, nullptr, nullptr, ACT_NONE, 0.f,
-         nullptr, 0, nullptr, 0, 1.f, &gf);
-    GemmPlanes go;
-    if (gf.out_done) { go.in_hi = p2048h; go.in_lo = p2048l; }              // gelu(ffn) exists only as planes
-    gemm(L, L, ff, 2048, 2048, W.ffo_w, &W.t_ffo, W.ffo_b, 768, tmp, 768, 0, ACT_NONE, 1, 0, nullptr, nullptr, ACT_NONE, 0.f,
-         nullptr, 0, nullptr, 0, 1.f, &go);
+    ConvOpt of;
+    of.eact = ACT_GELU_NEW;
+    if (pl_ok) { of.in_hi = p768h; of.in_lo = p768l; of.out_hi = p2048h; of.out_lo = p2048l; of.out_ld = 2048; }
+    const bool ff_planes = gemm(L, L, h1, 768, 768, W.ffn_w, &W.t_ffn, W.ffn_b, 2048, ff, 2048, 0, of);
+    ConvOpt oo;
+    if (ff_planes) { oo.in_hi = p2048h; oo.in_lo = p2048l; }                // gelu(ffn) exists only as planes
+    gemm(L, L, ff, 2048, 2048, W.ffo_w, &W.t_ffo, W.ffo_b, 768, tmp, 768, 0, oo);
     ln.x = tmp; ln.res = h1; ln.w = W.full_lnw; ln.b = W.full_lnb; ln.out = h;
     launch_layernorm(ln, st);                                                 // h (+ its planes for the next QKV / bert_encoder)
     h_planes = pl_ok;
@@ -320,10 +322,9 @@ void Model::token_issue(Run& r) {
   float* xp = A.alloc<float>(R * 2048);
   float* lo = A.alloc<float>(R * 512);
   {
-    GemmPlanes gb;
-    if (h_planes) { gb.in_hi = p768h; gb.in_lo = p768l; }
-    gemm(L, L, h, 768, 768, W.benc_w, &W.t_benc, W.benc_b, 512, xa, 640, 0, ACT_NONE, 1, 0, nullptr, nullptr, ACT_NONE, 0.f,
-         nullptr, 0, nullptr, 0, 1.f, &gb);
+    ConvOpt ob;
+    if (h_planes) { ob.in_hi = p768h; ob.in_lo = p768l; }
+    gemm(L, L, h, 768, 768, W.benc_w, &W.t_benc, W.benc_b, 512, xa, 640, 0, ob);
   }
   capture("d_en", xa, 640, 0, 512, L, 0);
   launch_bcast_cols(d_styles_, 256, 128, 128, xa, 640, 512, L.d_off, L.d_len, B, L.max_len, st);
@@ -389,10 +390,8 @@ void Model::token_finish(Run& r) {
 
 // ------------------------------------------------------------------------------------------
 // AdainResBlk1d (A.6).  x [Lin rows, ci] -> out [Lout rows, co] (Lout = 2*Lin when upsampling).
-void Model::adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ldx, const Level& Lin,
-                      const Level& Lout, const float* sty, int sld, float* out, int ldo, int ocol,
-                      bool dry) {
-  (void)r; (void)dry;
+void Model::adain_blk(Arena& A, const AdaBlkW& w, const float* x, int ldx, const Level& Lin, const Level& Lout,
+                      const float* sty, int sld, float* out, int ldo, int ocol) {
   cudaStream_t st = cur_;
   const int B = Lin.B;
   const int nch_in = (Lin.max_len + kStatRows - 1) / kStatRows;
@@ -406,6 +405,10 @@ void Model::adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ld
 
   launch_colstats(x, ldx, w.ci, part, Lin.d_off, Lin.d_len, B, Lin.max_len, st);
   launch_adain_coef(part, w.ci, Lin.max_len, Lin.d_len, sty, sld, w.sty1, 1e-5f, sc1, sh1, B, st);
+  ConvOpt k3;   // conv1 and conv2
+  k3.ks = 3; k3.pad = 1;
+  ConvOpt o2 = k3;   // conv2 adds the shortcut (x or its 1x1 conv) and scales the sum by 1/sqrt(2)
+  o2.res = x; o2.ldr = ldx; o2.Lres = &Lin; o2.res_shift = w.up ? 1 : 0; o2.oscale = 0.70710678118654752440f;
   if (opt.precision == 1 && w.t1.w) {
     // tensor-core path: bf16 operands produced by the apply kernels, tcgen05 convs, fp32 results
     const int cpi = w.t1.Cpad, cpo = w.t2.Cpad;
@@ -416,23 +419,21 @@ void Model::adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ld
     else
       launch_apply_bf16(x, ldx, w.ci, sc1, sh1, ACT_LRELU, 0.2f, nullptr, a1, cpi, Lin.rows, Lin.d_off,
                         Lin.d_len, B, Lin.max_len, st);
-    tc_conv(A, a1, Lout.rows, w.t1, 1, 1, Lout, Lout, w.b1, t, w.co, 0, Lout, 1, 0, nullptr, 0, nullptr, 0, 1.f, false);
+    tc_conv(a1, Lout.rows, w.t1, Lout, Lout, w.b1, t, w.co, 0, Lout, k3);
     launch_colstats(t, w.co, w.co, part, Lout.d_off, Lout.d_len, B, Lout.max_len, st);
     launch_adain_coef(part, w.co, Lout.max_len, Lout.d_len, sty, sld, w.sty2, 1e-5f, sc2, sh2, B, st);
     void* a2 = A.alloc_bytes((size_t)Lout.rows * cpo * 2);
     launch_apply_bf16(t, w.co, w.co, sc2, sh2, ACT_LRELU, 0.2f, nullptr, a2, cpo, Lout.rows, Lout.d_off,
                       Lout.d_len, B, Lout.max_len, st);
-    const float* scp = x; int ldsc = ldx;
     if (w.w1x1) {
       void* a3 = A.alloc_bytes((size_t)Lin.rows * cpi * 2);
       float* s = A.alloc<float>((size_t)Lin.rows * w.co);
       launch_apply_bf16(x, ldx, w.ci, nullptr, nullptr, ACT_NONE, 0.f, nullptr, a3, cpi, Lin.rows, Lin.d_off,
                         Lin.d_len, B, Lin.max_len, st);
-      tc_conv(A, a3, Lin.rows, w.t1x1, 1, 0, Lin, Lin, nullptr, s, w.co, 0, Lin, 1, 0, nullptr, 0, nullptr, 0, 1.f, false);
-      scp = s; ldsc = w.co;
+      tc_conv(a3, Lin.rows, w.t1x1, Lin, Lin, nullptr, s, w.co, 0, Lin);
+      o2.res = s; o2.ldr = w.co;
     }
-    tc_conv(A, a2, Lout.rows, w.t2, 1, 1, Lout, Lout, w.b2, out, ldo, ocol, Lout, 1, 0, scp, ldsc, &Lin,
-            w.up ? 1 : 0, 0.70710678118654752440f, false);
+    tc_conv(a2, Lout.rows, w.t2, Lout, Lout, w.b2, out, ldo, ocol, Lout, o2);
     return;
   }
   // fp32-grade path (SIMT fp32, or split-TF32 tensor cores for the F0/N predictor blocks)
@@ -440,21 +441,22 @@ void Model::adain_blk(Run& r, Arena& A, const AdaBlkW& w, const float* x, int ld
     float* p = A.alloc<float>((size_t)Lout.rows * w.ci);
     launch_pool_up(x, ldx, sc1, sh1, 0.2f, w.poolw, w.poolb, w.ci, p, w.ci, Lin.d_off, Lin.d_len,
                    Lout.d_off, B, Lin.max_len, st);
-    gemm(Lout, Lout, p, w.ci, w.ci, w.w1, &w.s1, w.b1, w.co, t, w.co, 0, ACT_NONE, 3, 1);
+    gemm(Lout, Lout, p, w.ci, w.ci, w.w1, &w.s1, w.b1, w.co, t, w.co, 0, k3);
   } else {
-    gemm(Lin, Lin, x, ldx, w.ci, w.w1, &w.s1, w.b1, w.co, t, w.co, 0, ACT_NONE, 3, 1, sc1, sh1, ACT_LRELU, 0.2f);
+    ConvOpt o1 = k3;
+    o1.pscale = sc1; o1.pshift = sh1; o1.pact = ACT_LRELU; o1.pslope = 0.2f;
+    gemm(Lin, Lin, x, ldx, w.ci, w.w1, &w.s1, w.b1, w.co, t, w.co, 0, o1);
   }
   launch_colstats(t, w.co, w.co, part, Lout.d_off, Lout.d_len, B, Lout.max_len, st);
   launch_adain_coef(part, w.co, Lout.max_len, Lout.d_len, sty, sld, w.sty2, 1e-5f, sc2, sh2, B, st);
 
-  const float* sc = x; int ldsc = ldx;
   if (w.w1x1) {
     float* s = A.alloc<float>((size_t)Lin.rows * w.co);
     gemm(Lin, Lin, x, ldx, w.ci, w.w1x1, &w.s1x1, nullptr, w.co, s, w.co, 0);
-    sc = s; ldsc = w.co;
+    o2.res = s; o2.ldr = w.co;
   }
-  gemm(Lout, Lout, t, w.co, w.co, w.w2, &w.s2, w.b2, w.co, out, ldo, ocol, ACT_NONE, 3, 1, sc2, sh2, ACT_LRELU, 0.2f,
-       sc, ldsc, &Lin, w.up ? 1 : 0, 0.70710678118654752440f);
+  o2.pscale = sc2; o2.pshift = sh2; o2.pact = ACT_LRELU; o2.pslope = 0.2f;
+  gemm(Lout, Lout, t, w.co, w.co, w.w2, &w.s2, w.b2, w.co, out, ldo, ocol, o2);
 }
 
 // AdaINResBlock1 (A.9): three (AdaIN -> Snake -> dilated conv -> AdaIN -> Snake -> conv) + residual
@@ -463,10 +465,8 @@ bool Model::use_stream_bf16(int C, int k, int B) const {
   return opt.precision == 1 && opt.stream_bf16 && arb_conv_supported(C, k, 5, B);
 }
 
-void Model::arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L, const float* sty,
-                int sld, float* xw, float* t1, float* out, float oscale, bool accumulate, const float* part_x,
-                const void* x_bf16) {
-  (void)r;
+void Model::arb(Arena& A, const ArbW& w, const float* x, const Level& L, const float* sty, int sld, float* xw,
+                float* t1, float* out, float oscale, bool accumulate, const float* part_x, const void* x_bf16) {
   cudaStream_t st = cur_;
   const int B = L.B, C = w.c, k = w.k;
   const int nch = (L.max_len + kStatRows - 1) / kStatRows;
@@ -543,6 +543,70 @@ void Model::arb(Run& r, Arena& A, const ArbW& w, const float* x, const Level& L,
     launch_conv_f32(c2, st);
     cur = dst;
   }
+}
+
+// Phase ph of the up-sampling conv reads input rows m + q0 - tap (q0 = ph < s/2) and writes output row
+// s*m + q0*s + ph - s/2 + shift.
+void Model::upsample(Arena& A, const float* x, const Level& Lin, float* out, const Level& Lout, int s, int shift,
+                     const TcW& w_all, const std::vector<TcW>& w_tc, const std::vector<float*>& w32, const float* bias,
+                     bool dry) {
+  cudaStream_t st = cur_;
+  const int Ci = w_all.Ci, Co = w_all.Co;
+  void* xbf = nullptr;
+  if (opt.precision == 1) {
+    xbf = A.alloc_bytes((size_t)Lin.rows * w_all.Cpad * 2);
+    launch_apply_bf16(x, Ci, Ci, nullptr, nullptr, ACT_LRELU, 0.1f, nullptr, xbf, w_all.Cpad, Lin.rows, Lin.d_off,
+                      Lin.d_len, Lin.B, Lin.max_len, st);
+  }
+  ConvOpt o;
+  o.dil = -1; o.ors = s;
+  if (opt.precision == 1 && opt.fuse_phases && !dry) {   // all s phases in one launch
+    alignas(64) unsigned char tmA[128];
+    make_tmap_bf16(tmA, xbf, w_all.Cpad, Lin.rows, w_all.Cpad, 128);
+    TcConvArgs a = tc_args(Lin, Lin, Lout, bias, out, Co, 0, o);
+    a.tmA = tmA; a.tmB = w_all.tmap;
+    a.Cpad = w_all.Cpad; a.Ci = Ci; a.Co = Co; a.ks = 2;
+    a.nphase = s; a.phase_loop = opt.ups_phase_loop;
+    for (int ph = 0; ph < s; ph++) {
+      const int q0 = ph < s / 2 ? 1 : 0;
+      a.phase_pad[ph] = -q0; a.phase_oro[ph] = q0 * s + ph - s / 2 + shift;
+    }
+    if (opt.conv_pair && w_all.pair_map(Co)) { a.tmB_c = w_all.pair_map(Co); a.pair = 1; }
+    launch_conv_tc(a, st);
+    return;
+  }
+  for (int ph = 0; ph < s; ph++) {
+    const int q0 = ph < s / 2 ? 1 : 0;
+    o.pad = -q0; o.oro = q0 * s + ph - s / 2 + shift;
+    if (opt.precision == 1) {
+      tc_conv(xbf, Lin.rows, w_tc[ph], Lin, Lin, bias, out, Co, 0, Lout, o);
+      continue;
+    }
+    ConvArgs c = gemm_args(Lin, x, Ci, Ci, w32[ph], bias, Co, out, Co, 0);
+    c.out_off = Lout.d_off;
+    c.ks = 2; c.dil = o.dil; c.pad = o.pad; c.ors = o.ors; c.oro = o.oro;
+    c.pact = ACT_LRELU; c.pslope = 0.1f;
+    launch_conv_f32(c, st);
+  }
+}
+
+void Model::res_stage(Arena& A, const ArbW* w, float* x, const float* xs, const Level& L, const float* sty, float* xw,
+                      float* t, float* acc) {
+  cudaStream_t st = cur_;
+  const int C = w[0].c;
+  float* px = nullptr;
+  void* xb = nullptr;
+  if (opt.precision == 1) {   // x += x_source and the statistics of the sum (input of three res-blocks) in one pass
+    px = A.alloc<float>((size_t)L.B * ((L.max_len + kStatRows - 1) / kStatRows) * 2 * C);
+    // (bf16 residual stream: the sum is written once, as the bf16 x all three res-blocks read)
+    bool sb = true;
+    for (int j = 0; j < 3; j++) sb = sb && use_stream_bf16(C, w[j].k, L.B);
+    xb = sb ? A.alloc_bytes((size_t)L.rows * C * 2) : nullptr;
+    launch_add_rows_stats(x, xs, x, C, px, L.d_off, L.d_len, L.B, L.max_len, st, xb);
+  } else {
+    launch_add_rows(x, xs, x, C, L.d_off, L.d_len, L.B, L.max_len, st);
+  }
+  for (int j = 0; j < 3; j++) arb(A, w[j], x, L, sty, W.sty_dec_n, xw, t, acc, 1.0f / 3.0f, j > 0, px, xb);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -668,9 +732,9 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     float* y0 = A.alloc<float>((size_t)FR.rows * 512);
     float* y1 = A.alloc<float>((size_t)FR2.rows * 256);
     float* y2 = A.alloc<float>((size_t)FR2.rows * 256);
-    adain_blk(r, A, blk[0], shd, 512, FR, FR, sty_pro, W.sty_pro_n, y0, 512, 0, dry);
-    adain_blk(r, A, blk[1], y0, 512, FR, FR2, sty_pro, W.sty_pro_n, y1, 256, 0, dry);
-    adain_blk(r, A, blk[2], y1, 256, FR2, FR2, sty_pro, W.sty_pro_n, y2, 256, 0, dry);
+    adain_blk(A, blk[0], shd, 512, FR, FR, sty_pro, W.sty_pro_n, y0, 512, 0);
+    adain_blk(A, blk[1], y0, 512, FR, FR2, sty_pro, W.sty_pro_n, y1, 256, 0);
+    adain_blk(A, blk[2], y1, 256, FR2, FR2, sty_pro, W.sty_pro_n, y2, 256, 0);
     curves[k] = A.alloc<float>(FR2.rows);
     launch_conv_f32(gemm_args(FR2, y2, 256, 256, k == 0 ? W.f0proj_w : W.nproj_w,
                               k == 0 ? W.f0proj_b : W.nproj_b, 1, curves[k], 1, 0), cur_);
@@ -732,14 +796,14 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     void* col = A.alloc_bytes((size_t)G20.rows * W.t_nc0.Cpad * 2);
     launch_im2col_bf16(har, 24, 22, 12, 6, 3, col, W.t_nc0.Cpad, G20.rows, G120.d_off, G120.d_len, G20.d_off,
                        G20.d_len, B, G20.max_len, st1);
-    tc_conv(A, col, G20.rows, W.t_nc0, 1, 0, G20, G20, W.nc0_b, xs0, 256, 0, G20, 1, 0, nullptr, 0, nullptr, 0, 1.f, false);
+    tc_conv(col, G20.rows, W.t_nc0, G20, G20, W.nc0_b, xs0, 256, 0, G20);
   } else {
     ConvArgs c = gemm_args(G20, har, 24, 22, W.nc0_w, W.nc0_b, 256, xs0, 256, 0);
     c.in_off = G120.d_off; c.in_len = G120.d_len;
     c.ks = 12; c.stride = 6; c.pad = 3;
     launch_conv_f32(c, st1);
   }
-  arb(r, A, W.nres[0], xs0, G20, sty_dec, W.sty_dec_n, w0, t0, xs0, 1.f, false);
+  arb(A, W.nres[0], xs0, G20, sty_dec, W.sty_dec_n, w0, t0, xs0, 1.f, false);
   capture("gen.x_source.0", xs0, 256, 0, 256, G20, b0);
   // (stage-1 buffers; the stage-1 noise branch is part of the same lane)
   float* xs1 = A.alloc<float>(n120);
@@ -758,11 +822,11 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     void* hb = A.alloc_bytes((size_t)G120.rows * W.t_nc1.Cpad * 2);
     launch_apply_bf16(har, 24, 22, nullptr, nullptr, ACT_NONE, 0.f, nullptr, hb, W.t_nc1.Cpad, G120.rows, G120.d_off,
                       G120.d_len, B, G120.max_len, st1);
-    tc_conv(A, hb, G120.rows, W.t_nc1, 1, 0, G120, G120, W.nc1_b, xs1, 128, 0, G120, 1, 0, nullptr, 0, nullptr, 0, 1.f, false);
+    tc_conv(hb, G120.rows, W.t_nc1, G120, G120, W.nc1_b, xs1, 128, 0, G120);
   } else {
     launch_conv_f32(gemm_args(G120, har, 24, 22, W.nc1_w, W.nc1_b, 128, xs1, 128, 0), st1);
   }
-  arb(r, A, W.nres[1], xs1, G120, sty_dec, W.sty_dec_n, w1, t1, xs1, 1.f, false, pxs1);
+  arb(A, W.nres[1], xs1, G120, sty_dec, W.sty_dec_n, w1, t1, xs1, 1.f, false, pxs1);
   capture("gen.x_source.1", xs1, 128, 0, 128, G120, b0);
   use_lane(0);
 
@@ -771,125 +835,34 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   float* xB = A.alloc<float>((size_t)FR.rows * 1096);
   launch_curve_conv(f0, FR2.d_off, FR2.d_len, W.f0conv_w, W.f0conv_b, x514, 520, 512, FR.d_off, FR.d_len, B, FR.max_len, st);
   launch_curve_conv(nc, FR2.d_off, FR2.d_len, W.nconv_w, W.nconv_b, x514, 520, 513, FR.d_off, FR.d_len, B, FR.max_len, st);
-  adain_blk(r, A, W.enc, x514, 520, FR, FR, sty_dec, W.sty_dec_n, xA, 1096, 0, dry);
+  adain_blk(A, W.enc, x514, 520, FR, FR, sty_dec, W.sty_dec_n, xA, 1096, 0);
   capture("dec.encode", xA, 1096, 0, 1024, FR, b0);
   launch_conv_f32(gemm_args(FR, x514, 520, 512, W.asr_w, W.asr_b, 64, xA, 1096, 1024), st);
   launch_copy_cols(x514, 520, 512, xA, 1096, 1088, 2, FR.d_off, FR.d_len, B, FR.max_len, st);
   launch_copy_cols(xA, 1096, 1024, xB, 1096, 1024, 66, FR.d_off, FR.d_len, B, FR.max_len, st);
   float* dcur = xA; float* dnxt = xB;
   for (int i = 0; i < 3; i++) {
-    adain_blk(r, A, W.dec[i], dcur, 1096, FR, FR, sty_dec, W.sty_dec_n, dnxt, 1096, 0, dry);
+    adain_blk(A, W.dec[i], dcur, 1096, FR, FR, sty_dec, W.sty_dec_n, dnxt, 1096, 0);
     std::swap(dcur, dnxt);
     capture(("dec.decode." + std::to_string(i)).c_str(), dcur, 1096, 0, 1024, FR, b0);
   }
   float* y = A.alloc<float>((size_t)FR2.rows * 512);
-  adain_blk(r, A, W.dec[3], dcur, 1096, FR, FR2, sty_dec, W.sty_dec_n, y, 512, 0, dry);
+  adain_blk(A, W.dec[3], dcur, 1096, FR, FR2, sty_dec, W.sty_dec_n, y, 512, 0);
   capture("dec.decode.3", y, 512, 0, 512, FR2, b0);
 
-  void* ybf = nullptr;
-  if (opt.precision == 1) {
-    ybf = A.alloc_bytes((size_t)FR2.rows * 512 * 2);
-    launch_apply_bf16(y, 512, 512, nullptr, nullptr, ACT_LRELU, 0.1f, nullptr, ybf, 512, FR2.rows, FR2.d_off,
-                      FR2.d_len, B, FR2.max_len, st);
-  }
-  if (opt.precision == 1 && opt.fuse_phases && !dry) {
-    // all 10 phases in one launch: phase p reads rows (m + q0 - tap), writes output row 10 m + q0*10 + p - 5
-    alignas(64) unsigned char tmA[128];
-    make_tmap_bf16(tmA, ybf, W.tups0_all.Cpad, FR2.rows, W.tups0_all.Cpad, 128);
-    TcConvArgs a;
-    a.tmA = tmA; a.tmB = W.tups0_all.tmap;
-    a.Cpad = W.tups0_all.Cpad; a.Ci = W.tups0_all.Ci; a.Co = 256; a.ks = 2; a.dil = -1;
-    a.in_off = FR2.d_off; a.m_len = FR2.d_len; a.max_m = FR2.max_len; a.B = B; a.sum_m = FR2.sum_len;
-    a.bias = W.ups0_b; a.out = x0; a.ldo = 256; a.ocol = 0; a.out_off = G20.d_off; a.ors = 10;
-    a.nphase = 10;
-    for (int ph = 0; ph < 10; ph++) { const int q0 = ph < 5 ? 1 : 0; a.phase_pad[ph] = -q0; a.phase_oro[ph] = q0 * 10 + ph - 5; }
-    if (opt.conv_pair && W.tups0_all.pair_map(256)) {
-      a.tmB_c = W.tups0_all.pair_map(256); a.pair = 1; a.tile_start = FR2.d_tiles128; a.ntiles_m = FR2.ntiles128;
-    }
-    launch_conv_tc(a, st);
-  } else
-  for (int ph = 0; ph < 10; ph++) {  // ConvTranspose1d(512,256,k20,s10,p5) as 10 two-tap phase convs
-    const int q0 = ph < 5 ? 1 : 0;
-    if (opt.precision == 1) {
-      tc_conv(A, ybf, FR2.rows, W.tups0[ph], -1, -q0, FR2, FR2, W.ups0_b, x0, 256, 0, G20, 10, q0 * 10 + ph - 5,
-              nullptr, 0, nullptr, 0, 1.f, false);
-      continue;
-    }
-    ConvArgs c = gemm_args(FR2, y, 512, 512, W.ups0[ph], W.ups0_b, 256, x0, 256, 0);
-    c.out_off = G20.d_off;
-    c.ks = 2; c.dil = -1; c.pad = -q0; c.stride = 1;
-    c.ors = 10; c.oro = q0 * 10 + ph - 5;
-    c.pact = ACT_LRELU; c.pslope = 0.1f;
-    launch_conv_f32(c, st);
-  }
+  // ---- generator stage 0: ConvTranspose1d(512, 256, k20, s10, p5), res-blocks
+  upsample(A, y, FR2, x0, G20, 10, 0, W.tups0_all, W.tups0, W.ups0, W.ups0_b, dry);
   if (fork) join_lane1();
   capture("gen.ups.0", x0, 256, 0, 256, G20, b0);
-  {
-    float* px = nullptr;
-    void* xb = nullptr;
-    if (opt.precision == 1) {   // x0 += x_source and the statistics of the sum (input of three res-blocks) in one pass
-      px = A.alloc<float>((size_t)B * ((G20.max_len + kStatRows - 1) / kStatRows) * 2 * 256);
-      // (bf16 residual stream: the sum is written once, as the bf16 x0 all three res-blocks read)
-      const bool sb0 = use_stream_bf16(256, 3, B) && use_stream_bf16(256, 7, B) && use_stream_bf16(256, 11, B);
-      xb = sb0 ? A.alloc_bytes((size_t)G20.rows * 256 * 2) : nullptr;
-      launch_add_rows_stats(x0, xs0, x0, 256, px, G20.d_off, G20.d_len, B, G20.max_len, st, xb);
-    } else {
-      launch_add_rows(x0, xs0, x0, 256, G20.d_off, G20.d_len, B, G20.max_len, st);
-    }
-    for (int j = 0; j < 3; j++)
-      arb(r, A, W.res[j], x0, G20, sty_dec, W.sty_dec_n, w0, t0, acc0, 1.0f / 3.0f, j > 0, px, xb);
-  }
+  res_stage(A, W.res, x0, xs0, G20, sty_dec, w0, t0, acc0);
   capture("gen.stage.0", acc0, 256, 0, 256, G20, b0);
 
-  // ---- generator stage 1 (120T+1 rows, 128 ch)
-  void* abf = nullptr;
-  if (opt.precision == 1) {
-    abf = A.alloc_bytes((size_t)G20.rows * 256 * 2);
-    launch_apply_bf16(acc0, 256, 256, nullptr, nullptr, ACT_LRELU, 0.1f, nullptr, abf, 256, G20.rows, G20.d_off,
-                      G20.d_len, B, G20.max_len, st);
-  }
-  if (opt.precision == 1 && opt.fuse_phases && !dry) {
-    alignas(64) unsigned char tmA[128];
-    make_tmap_bf16(tmA, abf, W.tups1_all.Cpad, G20.rows, W.tups1_all.Cpad, 128);
-    TcConvArgs a;
-    a.tmA = tmA; a.tmB = W.tups1_all.tmap;
-    a.Cpad = W.tups1_all.Cpad; a.Ci = W.tups1_all.Ci; a.Co = 128; a.ks = 2; a.dil = -1;
-    a.in_off = G20.d_off; a.m_len = G20.d_len; a.max_m = G20.max_len; a.B = B; a.sum_m = G20.sum_len;
-    a.bias = W.ups1_b; a.out = x1; a.ldo = 128; a.ocol = 0; a.out_off = G120.d_off; a.ors = 6;
-    a.nphase = 6; a.phase_loop = opt.ups_phase_loop; a.tile_start = G20.d_tiles128; a.ntiles_m = G20.ntiles128;
-    for (int ph = 0; ph < 6; ph++) { const int q0 = ph < 3 ? 1 : 0; a.phase_pad[ph] = -q0; a.phase_oro[ph] = q0 * 6 + ph - 3 + 1; }
-    launch_conv_tc(a, st);
-  } else
-  for (int ph = 0; ph < 6; ph++) {  // ConvTranspose1d(256,128,k12,s6,p3) + ReflectionPad1d((1,0))
-    const int q0 = ph < 3 ? 1 : 0;
-    if (opt.precision == 1) {
-      tc_conv(A, abf, G20.rows, W.tups1[ph], -1, -q0, G20, G20, W.ups1_b, x1, 128, 0, G120, 6, q0 * 6 + ph - 3 + 1,
-              nullptr, 0, nullptr, 0, 1.f, false);
-      continue;
-    }
-    ConvArgs c = gemm_args(G20, acc0, 256, 256, W.ups1[ph], W.ups1_b, 128, x1, 128, 0);
-    c.out_off = G120.d_off;
-    c.ks = 2; c.dil = -1; c.pad = -q0; c.stride = 1;
-    c.ors = 6; c.oro = q0 * 6 + ph - 3 + 1;
-    c.pact = ACT_LRELU; c.pslope = 0.1f;
-    launch_conv_f32(c, st);
-  }
+  // ---- generator stage 1 (120T+1 rows, 128 ch): ConvTranspose1d(256, 128, k12, s6, p3) + ReflectionPad1d((1, 0)),
+  // res-blocks
+  upsample(A, acc0, G20, x1, G120, 6, 1, W.tups1_all, W.tups1, W.ups1, W.ups1_b, dry);
   launch_copy_row(x1, 128, 0, 2, G120.d_off, B, st);
   capture("gen.ups.1", x1, 128, 0, 128, G120, b0);
-  {
-    float* px = nullptr;
-    void* xb = nullptr;
-    if (opt.precision == 1) {
-      px = A.alloc<float>((size_t)B * ((G120.max_len + kStatRows - 1) / kStatRows) * 2 * 128);
-      const bool sb1 = use_stream_bf16(128, 3, B) && use_stream_bf16(128, 7, B) && use_stream_bf16(128, 11, B);
-      xb = sb1 ? A.alloc_bytes((size_t)G120.rows * 128 * 2) : nullptr;
-      launch_add_rows_stats(x1, xs1, x1, 128, px, G120.d_off, G120.d_len, B, G120.max_len, st, xb);
-    } else {
-      launch_add_rows(x1, xs1, x1, 128, G120.d_off, G120.d_len, B, G120.max_len, st);
-    }
-    for (int j = 0; j < 3; j++)
-      arb(r, A, W.res[3 + j], x1, G120, sty_dec, W.sty_dec_n, w1, t1, acc1, 1.0f / 3.0f, j > 0, px, xb);
-  }
+  res_stage(A, W.res + 3, x1, xs1, G120, sty_dec, w1, t1, acc1);
   capture("gen.stage.1", acc1, 128, 0, 128, G120, b0);
 
   // ---- head (K11)
