@@ -340,15 +340,51 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                    to normalisation off.  The measurement runs in fp32 on the device (the filter restarted from zero
  *                    state 4800 samples before each 2400-sample segment, sums in double); values and bits of an item
  *                    do not depend on its batch, frame group or pass.  One loudness across several items (program
- *                    loudness of a request split into chunks) is kkx_infer_programs.  Not provided: lookahead
- *                    limiting or compression, measurement
- *                    at the output rate, momentary / short-term loudness and loudness range, a measure-only mode.
+ *                    loudness of a request split into chunks) is kkx_infer_programs.  Rule 5 caps the gain, so an
+ *                    item whose peak-to-loudness ratio exceeds ceiling - target comes back quieter than the target;
+ *                    "limiter" reaches it.  Not provided: compression, measurement at the output rate, momentary /
+ *                    short-term loudness and loudness range, a measure-only mode.
+ *   "limiter"     lookahead true-peak limiter: 0 (DEFAULT) = off, every bit, byte and launch as without it; 1 = on.
+ *                 Any other value is KKX_ERR_ARG and the session keeps its setting.  One setting per session, followed
+ *                 by the same entry points as "loudness_target" for runs that start after the call.  It works on each
+ *                 item's (program's) 24 kHz model waveform x (n samples), before resampling and integer conversion,
+ *                 with or without "loudness_target".  c = 10^(C / 20), C = "true_peak_max" / 100.  Fixed constants:
+ *                 lookahead Ha = 120 samples (5 ms), FIR guard Hb = 10 (the half-support of the 4x true-peak filter),
+ *                 largest reduction Rmax = 12 dB, release slope s = 0.0025 dB per sample (60 dB/s), release window
+ *                 W = Rmax / s = 4800 samples.
+ *                 1. Static gain: g = 10^((T - L) / 20) when "loudness_target" T != 0 and L is defined, else g = 1;
+ *                    instead of rule 5's cap, if tp g > c 10^(Rmax / 20) then g = c 10^(Rmax / 20) / tp (tp of rule 4;
+ *                    this cap applies also when L is undefined or T = 0).
+ *                 2. Detector: p[i] = max over j = 0..3 of |u[4 i + j]|, u = resample_poly(x, 4, 1) with rule 4's
+ *                    filter and zeros outside the item; q[i] = min(0, C - 20 log10(g p[i])), q = 0 where p = 0 and
+ *                    outside [0, n).
+ *                 3. Hold: h[i] = min over k in [-Hb, Ha + Hb] of q[i + k].
+ *                 4. Release: e[i] = min(0, min over m in [i - W, i] of (h[m] + (i - m) s)) -- a linear-in-dB recovery
+ *                    without a recurrence (h >= -Rmax makes older terms >= 0), so tiles of an item are computed
+ *                    independently.
+ *                 5. Attack: G[i] = mean over k = 0..Ha of 10^(e[i - k] / 20), e = 0 before the first sample; G = 1.0
+ *                    exactly where e is 0 throughout the window.  Every gain within Hb of a detected peak is at most
+ *                    that peak's required gain.
+ *                 6. v[i] = fp32(x[i] fp32(g G[i])).
+ *                 7. Trim: tp_v = max |resample_poly(v, 4, 1)|, t = min(1, c / tp_v).
+ *                 8. y = v resampled under the "out_rate" rule; each returned sample is fp32(y t).  PCM16, G.711 and
+ *                    FLAC follow from that value by their rules.
+ *                 Consequences: the 24 kHz-domain output has true peak <= c to fp32 rounding, so PCM16, G.711 and FLAC
+ *                 never clip; an item the limiter does not touch (G = 1, t = 1) is bit-identical at 24000 to the
+ *                 limiter-off run with the same g (with loudness off: a silent item, or one whose true peak is under the
+ *                 ceiling, is bit-identical to the plain output); an item's (program's) bits do not depend on its
+ *                 batch, frame group, "max_tokens" pass, coalescing or kkx_submit.  kkx_last_loudness keeps reporting
+ *                 L and dBTP of the input and gain = g of step 1.  Device work: the loudness launches (three, also
+ *                 when "loudness_target" is 0; loud_peak writes p), then "lim_envelope", "loud_peak" on v and
+ *                 "lim_trim" -- 3 launches more than loudness alone per frame group that completes a program (6 more
+ *                 than plain output when "loudness_target" is 0; a resampling pass runs also at 24000).
+ *                 Not provided: compression, a limiter at the output rate, user-set lookahead / release / Rmax.
  * kkx_get_stat keys: "launches", "last_frames", "gpu_us", "precision", "coalesced_batches",
  * "coalesced_requests", "coalesced_largest", "async_batches", "async_requests", "frame_groups",
  * "group_first:<g>" (first item of frame group g of the last run), "weights_sessions" (sessions sharing this
  * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate", "loudness_target",
  * "true_peak_max", "loudness_items" (items -- programs after kkx_infer_programs -- kkx_last_loudness reports now; 0
- * if it would fail with KKX_ERR_STATE). */
+ * if it would fail with KKX_ERR_STATE), "limiter", "limiter_items" (the same for kkx_last_limiter). */
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value);
 KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "last_frames", "gpu_us" ... */
 
@@ -360,6 +396,12 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "las
  * KKX_ERR_ARG if `batch` is not that call's item count.  Coalesced callers and kkx_submit batches are normalised
  * but not reported here (a batch of several callers has no per-caller report). */
 KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* true_peak_dbtp, float* gain);
+
+/* What the limiter ("limiter" = 1) did in the last SYNCHRONOUS call, with kkx_last_loudness's scope, order and errors
+ * (KKX_ERR_STATE when that call ran with the limiter off).  Per item (program): max_reduction_db =
+ * -20 log10(t min over i of G[i]) (>= 0; 0 = untouched), true_peak_dbtp = 20 log10(t tp_v), the output's true peak.
+ * Each pointer is nullable and receives `batch` floats. */
+KKX_API int kkx_last_limiter(kkx_ctx* ctx, int32_t batch, float* max_reduction_db, float* true_peak_dbtp);
 
 /* Per-kernel device timing of the last run (CUDA events on the library's stream, one after every
  * launch).  kkx_profile_json writes {"conv_flops": F, "gpu_us": T, "kernels": {name: [launches,

@@ -141,6 +141,13 @@ KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const i
 KKX_API int64_t kkx_test_loudness_design(double fs, double* kweight, float* tp_taps, int64_t capacity);
 KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
                               int32_t ceiling_centi_dbtp, float* lufs, float* true_peak_dbtp, float* gain);
+/* Lookahead true-peak limiter (kernels_loudness.cu, kkx.h "limiter"), on B items packed as for kkx_test_loudness, with
+ * the given target (1/100 LUFS, 0 = no normalisation) and ceiling (1/100 dBTP).  Per item: gain = the static g of
+ * step 1, t = the trim of step 7, max_reduction_db and true_peak_dbtp = the kkx_last_limiter report; per sample
+ * (packed like x): G = the smoothed gain of step 5 and v = the limited waveform of step 6.  Every pointer is nullable. */
+KKX_API int kkx_test_limiter(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
+                             int32_t ceiling_centi_dbtp, float* gain, float* G, float* v, float* t,
+                             float* max_reduction_db, float* true_peak_dbtp);
 KKX_API const char* kkx_test_last_error(void);
 
 #ifdef __cplusplus

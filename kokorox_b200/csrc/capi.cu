@@ -68,6 +68,9 @@ struct kkx_ctx {
   // gain), appended pass by pass; valid once the call has succeeded, `normalised` if its runs had the option on.
   std::vector<float> loud;
   bool loud_valid = false, loud_normalised = false;
+  // Limiter report of the same call (kkx_last_limiter), kept alongside: 2 floats per item (max reduction dB, dBTP).
+  std::vector<float> lim;
+  bool lim_ran = false;
 };
 
 static thread_local std::string g_err;
@@ -233,11 +236,18 @@ static void hand_out(kkx_ctx* ctx, void* host, size_t cap) {
 
 KKX_API void kkx_release(kkx_ctx* ctx, float* audio);
 
-// kkx_last_loudness bookkeeping of a synchronous call (caller holds ctx->mu): begin, one note per model run, done.
-// Coalesced and asynchronous batches leave the report alone.
-static void loud_begin(kkx_ctx* ctx) { ctx->loud.clear(); ctx->loud_valid = false; ctx->loud_normalised = false; }
+// kkx_last_loudness / kkx_last_limiter bookkeeping of a synchronous call (caller holds ctx->mu): begin, one note per
+// model run, done.  Coalesced and asynchronous batches leave the reports alone.
+static void loud_begin(kkx_ctx* ctx) {
+  ctx->loud.clear(); ctx->loud_valid = false; ctx->loud_normalised = false;
+  ctx->lim.clear(); ctx->lim_ran = false;
+}
 static void loud_note(kkx_ctx* ctx) {
   const Model& m = *ctx->model;
+  if (m.limiter_ran()) {
+    ctx->lim_ran = true;
+    ctx->lim.insert(ctx->lim.end(), m.last_limiter().begin(), m.last_limiter().end());
+  }
   if (!m.loudness_ran()) return;
   ctx->loud_normalised = true;
   ctx->loud.insert(ctx->loud.end(), m.last_loudness().begin(), m.last_loudness().end());
@@ -871,6 +881,10 @@ KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
       if (value < -2000 || value > 0)
         throw ArgError("true_peak_max " + std::to_string(value) + " is not supported: give 1/100 dBTP in -2000..0");
       o.true_peak_max = (int)value;
+    } else if (k == "limiter") {
+      if (value != 0 && value != 1)
+        throw ArgError("limiter " + std::to_string(value) + " is not supported: give 0 (off) or 1 (on)");
+      o.limiter = (int)value;
     }
     else throw ArgError("unknown option: " + k);
   });
@@ -888,6 +902,8 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   if (k == "loudness_target") return ctx->model->opt.loudness_target;
   if (k == "true_peak_max") return ctx->model->opt.true_peak_max;
   if (k == "loudness_items") return ctx->loud_valid && ctx->loud_normalised ? (int64_t)(ctx->loud.size() / 3) : 0;
+  if (k == "limiter") return ctx->model->opt.limiter;
+  if (k == "limiter_items") return ctx->loud_valid && ctx->lim_ran ? (int64_t)(ctx->lim.size() / 2) : 0;
   if (k == "coalesced_batches") return ctx->coalesced_batches;
   if (k == "coalesced_requests") return ctx->coalesced_requests;
   if (k == "coalesced_largest") return ctx->coalesced_largest;
@@ -923,6 +939,23 @@ KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* t
       if (lufs) lufs[b] = ctx->loud[b * 3];
       if (true_peak_dbtp) true_peak_dbtp[b] = ctx->loud[b * 3 + 1];
       if (gain) gain[b] = ctx->loud[b * 3 + 2];
+    }
+  });
+}
+
+KKX_API int kkx_last_limiter(kkx_ctx* ctx, int32_t batch, float* max_reduction_db, float* true_peak_dbtp) {
+  int rc = check_ctx(ctx);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(ctx, [&] {
+    if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
+    if (!ctx->lim_ran) throw StateError("the last synchronous call ran with the limiter off");
+    const int64_t n = (int64_t)(ctx->lim.size() / 2);
+    if (batch != n)
+      throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
+    for (int64_t b = 0; b < n; b++) {
+      if (max_reduction_db) max_reduction_db[b] = ctx->lim[b * 2];
+      if (true_peak_dbtp) true_peak_dbtp[b] = ctx->lim[b * 2 + 1];
     }
   });
 }

@@ -297,18 +297,32 @@ void launch_resample(const float* x, const long long* in_off, const long long* i
 //   LoudParams:      everything the kernels read, passed by value (fp32 biquads, the 4x taps, target and ceiling).
 //   launch_loudness: item b = x[in_off[b] .. + in_len[b]); writes lufs[b] (NaN = undefined), tp_db[b] (dBTP) and
 //                    gain[b].  energy: scratch of in_len[b] / 2400 floats per item at seg_off[b]; peak: [B] scratch.
-//                    Three launches: "loud_energy", "loud_peak", "loud_gain".
+//                    Three launches: "loud_energy", "loud_peak", "loud_gain".  pmax (nullable, indexed like x): the
+//                    limiter's detector p[i] = max over j of |u[4 i + j]| of the true-peak filter's output u.
+//   loudness_params(limiter = true): the gain is the limiter's step 1 (kkx.h "limiter"): normalised only when the
+//                    target is not 0, and capped at Rmax above the ceiling whether or not L is defined.
+//   launch_limiter:  after launch_loudness with pmax, on the same items: v (indexed like x) = the limited waveform,
+//                    G (nullable, indexed like x) = the smoothed gain, and per item t[b] (the static trim),
+//                    red_db[b] (max reduction, dB) and out_db[b] (the output's true peak, dBTP).  acc: [2 B] scratch.
+//                    Three launches: "lim_envelope", "loud_peak" (on v), "lim_trim".
 constexpr int kLoudSeg = 2400, kLoudWarm = 4800, kTpTaps = 81;
+// limiter constants (kkx.h "limiter"): lookahead, FIR guard, largest reduction (dB), release slope (dB per sample)
+constexpr int kLimHa = 120, kLimHb = 10, kLimW = 4800;
+constexpr double kLimRmax = 12.0, kLimSlope = 0.0025;
 struct LoudParams {
   float kw[10];
   float tp[kTpTaps];
   double target_lufs, ceiling_dbtp;
+  int normalise = 1, limiter = 0;   // limiter: cap at ceiling + kLimRmax, also when L is undefined
 };
 void loudness_design(double fs, double kw[10], std::vector<float>* tp_taps);
-LoudParams loudness_params(double target_lufs, double ceiling_dbtp);
+LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter = false);
 void launch_loudness(const float* x, const long long* in_off, const long long* in_len, const long long* seg_off,
                      const LoudParams& P, float* energy, unsigned* peak, float* lufs, float* tp_db, float* gain, int B,
-                     long long max_len, cudaStream_t st);
+                     long long max_len, cudaStream_t st, float* pmax = nullptr);
+void launch_limiter(const float* x, const float* pmax, const long long* in_off, const long long* in_len,
+                    const LoudParams& P, const float* gain, float* v, float* G, unsigned* acc, float* t, float* red_db,
+                    float* out_db, int B, long long max_len, cudaStream_t st);
 
 // Lossless FLAC of 16-bit mono PCM (kernels_flac.cu; the bitstream rules are in kkx.h, kkx_infer_batch_flac).
 //   Item b is pcm[soff[b] .. soff[b + 1]) (>= 1 sample) and has flac_frames(n_b) frames of 4096 samples; foff[b + 1]

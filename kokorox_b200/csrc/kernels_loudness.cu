@@ -1,6 +1,7 @@
 // kernels_loudness.cu -- loudness normalisation (K14): ITU-R BS.1770 integrated loudness of each utterance's 24 kHz
 // waveform, its true peak, and the static gain that brings it to the session's target under a true-peak ceiling
-// (kkx.h "loudness_target" / "true_peak_max").  The gain itself is applied by resample_kernel (kernels_signal.cu).
+// (kkx.h "loudness_target" / "true_peak_max"), and the lookahead true-peak limiter (kkx.h "limiter", at the end of
+// this file).  The gains themselves are applied by resample_kernel (kernels_signal.cu).
 //
 // Per item (n samples x at 24 kHz):
 //   loud_energy  one thread per 2400-sample segment s (the 100 ms hop): the K-weighting cascade (shelf, then
@@ -48,7 +49,7 @@ void loudness_design(double fs, double kw[10], std::vector<float>* tp_taps) {
   if (tp_taps) poly_design(4, 1, tp_taps);   // 4 * firwin(81, 1/4, ("kaiser", 5.0))
 }
 
-LoudParams loudness_params(double target_lufs, double ceiling_dbtp) {
+LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter) {
   LoudParams P{};
   double kw[10];
   std::vector<float> taps;
@@ -58,6 +59,8 @@ LoudParams loudness_params(double target_lufs, double ceiling_dbtp) {
   for (int i = 0; i < kTpTaps; i++) P.tp[i] = taps[i];
   P.target_lufs = target_lufs;
   P.ceiling_dbtp = ceiling_dbtp;
+  P.normalise = limiter ? target_lufs != 0.0 : 1;   // a limiter session may run without a loudness target
+  P.limiter = limiter ? 1 : 0;
   return P;
 }
 
@@ -117,7 +120,7 @@ constexpr int kTpThreads = 256, kTpPer = 4, kTpTile = kTpThreads * kTpPer, kTpHa
 __global__ void __launch_bounds__(kTpThreads) loud_peak_kernel(const float* __restrict__ x,
                                                                const long long* __restrict__ in_off,
                                                                const long long* __restrict__ in_len, LoudParams P,
-                                                               unsigned* __restrict__ peak) {
+                                                               unsigned* __restrict__ peak, float* __restrict__ pmax) {
   __shared__ float s_x[kTpTile + 2 * kTpHalo];
   const int b = blockIdx.y, t = threadIdx.x;
   const long long n = in_len[b];
@@ -135,6 +138,7 @@ __global__ void __launch_bounds__(kTpThreads) loud_peak_kernel(const float* __re
     const int r = t + i * kTpThreads;
     if (q0 + r >= n) break;
     const float* w = s_x + r + kTpHalo;   // w[d] = x[q + d]
+    float mq = 0.f;
 #pragma unroll
     for (int p = 0; p < 4; p++) {
       float acc = 0.f;
@@ -143,8 +147,10 @@ __global__ void __launch_bounds__(kTpThreads) loud_peak_kernel(const float* __re
         const int j = 40 + p - 4 * d;
         if (j >= 0 && j < kTpTaps) acc = fmaf(w[d], P.tp[j], acc);
       }
-      m = fmaxf(m, fabsf(acc));
+      mq = fmaxf(mq, fabsf(acc));
     }
+    if (pmax) pmax[in_off[b] + q0 + r] = mq;   // the limiter's detector p[q]
+    m = fmaxf(m, mq);
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
@@ -206,9 +212,9 @@ __global__ void __launch_bounds__(kLgThreads) loud_gain_kernel(const long long* 
   if (t != 0) return;
   const float tp = __uint_as_float(peak[b]);
   double g = 1.0;
-  if (!isnan(L)) {
-    g = pow(10.0, (P.target_lufs - L) / 20.0);
-    const double cap = pow(10.0, P.ceiling_dbtp / 20.0);
+  if (P.normalise && !isnan(L)) g = pow(10.0, (P.target_lufs - L) / 20.0);
+  if (P.limiter || !isnan(L)) {   // rule 5's cap; the limiter's sits Rmax higher and always applies (kkx.h "limiter")
+    const double cap = pow(10.0, (P.ceiling_dbtp + (P.limiter ? kLimRmax : 0.0)) / 20.0);
     if ((double)tp * g > cap) g = cap / (double)tp;
   }
   lufs[b] = (float)L;
@@ -218,7 +224,7 @@ __global__ void __launch_bounds__(kLgThreads) loud_gain_kernel(const long long* 
 
 void launch_loudness(const float* x, const long long* in_off, const long long* in_len, const long long* seg_off,
                      const LoudParams& P, float* energy, unsigned* peak, float* lufs, float* tp_db, float* gain, int B,
-                     long long max_len, cudaStream_t st) {
+                     long long max_len, cudaStream_t st, float* pmax) {
   if (g_dry_run) return;
   if (B < 1 || B > 65535) throw ArgError("launch_loudness: batch out of range");
   const long long max_seg = max_len / kLoudSeg;
@@ -227,10 +233,179 @@ void launch_loudness(const float* x, const long long* in_off, const long long* i
   if (gp > 0x7FFFFFFFLL) throw ArgError("launch_loudness: grid too large");
   loud_energy_kernel<<<dim3((unsigned)ge, B), kLeThreads, 0, st>>>(x, in_off, in_len, seg_off, P, energy, peak);
   post_launch("loud_energy", st);
-  loud_peak_kernel<<<dim3((unsigned)gp, B), kTpThreads, 0, st>>>(x, in_off, in_len, P, peak);
+  loud_peak_kernel<<<dim3((unsigned)gp, B), kTpThreads, 0, st>>>(x, in_off, in_len, P, peak, pmax);
   post_launch("loud_peak", st);
   loud_gain_kernel<<<B, kLgThreads, 0, st>>>(in_len, seg_off, energy, peak, P, lufs, tp_db, gain);
   post_launch("loud_gain", st);
+}
+
+// ------------------------------------------------------------------------------------------ lookahead limiter
+// kkx.h "limiter", steps 2-7.  lim_envelope: one CTA per tile of kLimTile output samples of one item, anchored at the
+// item's sample 0; it stages the detector p (loud_peak's pmax) over the tile plus the reach of the rule -- Ha + W + Hb
+// samples to the left (box, release, hold), Ha + Hb to the right -- and computes in shared memory
+//   q  the required reduction (dB) per sample, 0 outside the item;
+//   h  the hold, a sliding minimum of q over Ha + 2 Hb + 1 samples, by doubling (min over 2, 4, .., 128, then two
+//      overlapping 128-windows);
+//   e  the release, min(0, r s + prefix-min over m <= r of (h[m] - m s)) with tile-relative r: terms older than W
+//      are >= 0 (h >= -Rmax), so the prefix from the tile's left edge gives the windowed minimum of the rule;
+//   G  the mean of 10^(e / 20) over Ha + 1 samples, as 1 - (window sum of the deficits 1 - 10^(e / 20)) / (Ha + 1);
+//      the deficits are summed as 2^25-scaled integers (a prefix sum modulo 2^32; the window sum is < 121 * 2^25 <
+//      2^32), so the sum is exact and independent of the scan's order, and a window of zero deficits gives G = 1.0.
+// Every value is a function of the item and the tile's position in it: an item's bits do not depend on its batch.
+// v = fp32(x fp32(g G)); the largest window deficit of the item (i.e. its smallest G) goes through an integer
+// atomicMax.  loud_peak then measures v, and lim_trim turns that into t and the report.
+constexpr int kLimThreads = 512, kLimTile = 8192;
+constexpr int kLimL = kLimHa + kLimW + kLimHb;                  // q starts L samples left of the tile
+constexpr int kLimSq = kLimTile + kLimL + kLimHa + kLimHb;      // q over [-L, T + Ha + Hb)
+constexpr int kLimSh = kLimTile + kLimHa + kLimW;               // h over [-Ha - W, T)
+constexpr int kLimSd = kLimTile + kLimHa;                       // deficits over [-Ha, T)
+constexpr int kLimHold = kLimHa + 2 * kLimHb + 1;               // 141-sample hold window
+constexpr float kLimS = (float)kLimSlope;
+constexpr float kLimDefScale = 33554432.f;                      // 2^25
+constexpr float kLimBoxScale = 1.f / ((kLimHa + 1) * 33554432.f);
+static_assert(kLimHold > 128 && kLimHold <= 256, "the hold combines two 128-sample windows");
+static_assert((double)(kLimHa + 1) * 33554432.0 < 4294967296.0, "window sum of the scaled deficits must fit 32 bits");
+
+__device__ __forceinline__ float lim_gain_of(unsigned w) {   // G of a window sum of scaled deficits
+  return __fsub_rn(1.f, __fmul_rn(__uint2float_rn(w), kLimBoxScale));
+}
+
+// inclusive scan of a[0 .. S) in shared memory with an exact, associative and commutative op (min, modular add);
+// contiguous runs per thread, then the run totals across the block
+template <class T, class Op>
+__device__ void lim_scan(T* a, int S, T id, Op op, T* wt) {
+  const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  const int c = (S + kLimThreads - 1) / kLimThreads;
+  const int lo = min(t * c, S), hi = min(lo + c, S);
+  T acc = id;
+  for (int j = lo; j < hi; j++) { acc = op(acc, a[j]); a[j] = acc; }
+  T v = acc;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const T u = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v = op(u, v);
+  }
+  if (lane == 31) wt[wid] = v;
+  __syncthreads();
+  if (wid == 0) {
+    T w = lane < kLimThreads / 32 ? wt[lane] : id;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const T u = __shfl_up_sync(0xffffffffu, w, o);
+      if (lane >= o) w = op(u, w);
+    }
+    if (lane < kLimThreads / 32) wt[lane] = w;
+  }
+  __syncthreads();
+  T ex = __shfl_up_sync(0xffffffffu, v, 1);
+  if (lane == 0) ex = id;
+  const T carry = wid > 0 ? op(wt[wid - 1], ex) : ex;
+  for (int j = lo; j < hi; j++) a[j] = op(carry, a[j]);
+  __syncthreads();
+}
+
+struct LimMin { __device__ float operator()(float a, float b) const { return fminf(a, b); } };
+struct LimAdd { __device__ unsigned operator()(unsigned a, unsigned b) const { return a + b; } };
+
+__global__ void __launch_bounds__(kLimThreads) lim_envelope_kernel(const float* __restrict__ x,
+                                                                   const float* __restrict__ pmax,
+                                                                   const long long* __restrict__ in_off,
+                                                                   const long long* __restrict__ in_len, float C,
+                                                                   const float* __restrict__ gain,
+                                                                   float* __restrict__ v, float* __restrict__ G,
+                                                                   unsigned* __restrict__ acc) {
+  extern __shared__ float lim_smem[];
+  __shared__ float wtf[kLimThreads / 32];
+  __shared__ unsigned wtu[kLimThreads / 32];
+  float* fa = lim_smem;
+  float* fb = lim_smem + kLimSq;
+  const int b = blockIdx.y, t = threadIdx.x;
+  const long long n = in_len[b];
+  const long long i0 = (long long)blockIdx.x * kLimTile;
+  if (i0 >= n) return;
+  const long long off = in_off[b];
+  const float g = gain[b];
+  // step 2: q[j] at sample i0 - L + j
+  for (int j = t; j < kLimSq; j += kLimThreads) {
+    const long long i = i0 - kLimL + j;
+    const float p = (i >= 0 && i < n) ? __ldg(pmax + off + i) : 0.f;
+    fa[j] = p > 0.f ? fminf(0.f, C - 20.f * log10f(g * p)) : 0.f;
+  }
+  __syncthreads();
+  // step 3: after the doubling passes src[j] = min of q over [j, j + 127]; h[j] (sample i0 - Ha - W + j) = min of q
+  // over [j, j + Ha + 2 Hb], i.e. over samples [i - Hb, i + Ha + Hb]
+  float* src = fa;
+  float* dst = fb;
+  for (int d = 1; d < 128; d <<= 1) {
+    for (int j = t; j < kLimSq; j += kLimThreads) dst[j] = j + d < kLimSq ? fminf(src[j], src[j + d]) : src[j];
+    __syncthreads();
+    float* tmp = src; src = dst; dst = tmp;
+  }
+  float* h = dst;
+  for (int j = t; j < kLimSh; j += kLimThreads)
+    h[j] = __fsub_rn(fminf(src[j], src[j + kLimHold - 128]), __fmul_rn((float)(j - kLimHa - kLimW), kLimS));
+  __syncthreads();
+  // step 4: prefix minimum of h[m] - m s (tile-relative m), then e[r] = min(0, r s + that)
+  lim_scan(h, kLimSh, INFINITY, LimMin(), wtf);
+  unsigned* du = reinterpret_cast<unsigned*>(src);   // src is free now
+  for (int j = t; j < kLimSd; j += kLimThreads) {
+    const int r = j - kLimHa;
+    float e = fminf(0.f, __fadd_rn(__fmul_rn((float)r, kLimS), h[r + kLimHa + kLimW]));
+    if (i0 + r < 0) e = 0.f;   // e = 0 before the item's first sample
+    du[j] = __float2uint_rn(__fmul_rn(__fsub_rn(1.f, exp10f(0.05f * e)), kLimDefScale));
+  }
+  __syncthreads();
+  // step 5: window sums of the deficits over [r - Ha, r] (exact modulo 2^32); step 6: v
+  lim_scan(du, kLimSd, 0u, LimAdd(), wtu);
+  unsigned wmax = 0u;
+  for (int r = t; r < kLimTile; r += kLimThreads) {
+    const long long i = i0 + r;
+    if (i >= n) break;
+    const unsigned w = du[r + kLimHa] - (r > 0 ? du[r - 1] : 0u);
+    const float Gi = lim_gain_of(w);
+    v[off + i] = __fmul_rn(__ldg(x + off + i), __fmul_rn(g, Gi));
+    if (G) G[off + i] = Gi;
+    wmax = max(wmax, w);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) wmax = max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
+  if ((t & 31) == 0 && wmax > 0u) atomicMax(acc + gridDim.y + b, wmax);
+}
+
+// step 7 and the report, one thread per item: acc[b] = bits of v's true peak, acc[B + b] = largest window deficit
+__global__ void lim_trim_kernel(const unsigned* __restrict__ acc, double ceiling_dbtp, int B, float* __restrict__ t,
+                                float* __restrict__ red_db, float* __restrict__ out_db) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const double c = pow(10.0, ceiling_dbtp / 20.0);
+  const float tpv = __uint_as_float(acc[b]);
+  const float tb = (double)tpv > c ? (float)(c / (double)tpv) : 1.f;
+  const float gmin = lim_gain_of(acc[B + b]);
+  t[b] = tb;
+  red_db[b] = (float)(0.0 - 20.0 * log10((double)tb * (double)gmin));
+  out_db[b] = (float)(20.0 * log10((double)tb * (double)tpv));
+}
+
+size_t lim_smem_bytes() { return (size_t)2 * kLimSq * sizeof(float); }
+
+void launch_limiter(const float* x, const float* pmax, const long long* in_off, const long long* in_len,
+                    const LoudParams& P, const float* gain, float* v, float* G, unsigned* acc, float* t, float* red_db,
+                    float* out_db, int B, long long max_len, cudaStream_t st) {
+  if (g_dry_run) return;
+  if (B < 1 || B > 65535) throw ArgError("launch_limiter: batch out of range");
+  const long long tiles = std::max(1LL, (max_len + kLimTile - 1) / kLimTile);
+  const long long gp = std::max(1LL, (max_len + kTpTile - 1) / kTpTile);
+  if (gp > 0x7FFFFFFFLL) throw ArgError("launch_limiter: grid too large");
+  const int smem = (int)lim_smem_bytes();
+  prepare_smem_launch<lim_envelope_kernel>(smem);
+  KKX_CUDA(cudaMemsetAsync(acc, 0, (size_t)2 * B * sizeof(unsigned), st));
+  lim_envelope_kernel<<<dim3((unsigned)tiles, B), kLimThreads, smem, st>>>(x, pmax, in_off, in_len,
+                                                                            (float)P.ceiling_dbtp, gain, v, G, acc);
+  post_launch("lim_envelope", st);
+  loud_peak_kernel<<<dim3((unsigned)gp, B), kTpThreads, 0, st>>>(v, in_off, in_len, P, acc, nullptr);
+  post_launch("loud_peak", st);
+  lim_trim_kernel<<<(B + 127) / 128, 128, 0, st>>>(acc, P.ceiling_dbtp, B, t, red_db, out_db);
+  post_launch("lim_trim", st);
 }
 
 }  // namespace kkx

@@ -795,13 +795,14 @@ void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_off
   }
 }
 
-// The resampling pass of this run: off at 24 kHz unless G.711 codes or loudness normalisation are wanted (then a
-// pass-through, U = D = 1, which applies the gain).  The taps live on the device per Model and are rebuilt only when
+// The resampling pass of this run: off at 24 kHz unless G.711 codes, loudness normalisation or the limiter are wanted
+// (then a pass-through, U = D = 1, which applies the gain).  The taps live on the device per Model and are rebuilt only when
 // the rate changes.
 void Model::prepare_resample() {
   loud_ = opt.loudness_target != 0;
-  if (loud_) loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0);
-  resample_ = opt.out_rate != 24000 || enc_ == Encoding::ULAW || enc_ == Encoding::ALAW || loud_;
+  lim_ = opt.limiter != 0;
+  if (loud_ || lim_) loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0, lim_);
+  resample_ = opt.out_rate != 24000 || enc_ == Encoding::ULAW || enc_ == Encoding::ALAW || loud_ || lim_;
   rs_U_ = 1; rs_D_ = 1; rs_H_ = 0;
   if (opt.out_rate == 24000) return;
   std::vector<float> taps;
@@ -912,9 +913,16 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
     grow(wav24A_, (size_t)s24_off_[B_] * sizeof(float));
     r.wav24 = wav24A_.alloc<float>(s24_off_[B_]);
   }
-  if (loud_) {
+  if (loud_ || lim_) {
     grow(loudA_, (size_t)P * 3 * sizeof(float));
     r.loud = loudA_.alloc<float>((size_t)P * 3);
+  }
+  if (lim_) {
+    grow(limA_, (size_t)P * 3 * sizeof(float));
+    r.lim = limA_.alloc<float>((size_t)P * 3);
+    grow(limWavA_, (size_t)s24_off_[B_] * 2 * sizeof(float) + 256);   // two arrays, the second 256-byte aligned
+    r.lim_p = limWavA_.alloc<float>(s24_off_[B_]);
+    r.lim_v = limWavA_.alloc<float>(s24_off_[B_]);
   }
   // FLAC: the encoder's tables -- sample offsets, frames per program (4096 samples each) as a prefix, program byte
   // offsets -- and its output, ready before the forward pass so that the encoder follows it without a host round trip
@@ -942,6 +950,7 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
     upload(fl.foff, foff.data(), (size_t)(P + 1) * sizeof(int));
   }
   h_loud_.clear();
+  h_lim_.clear();
   sink_filled_ = false;
   float* sink = (host_sink && !debug_) ? host_sink(total_samples_) : nullptr;
   // (both streams are idle here: the previous run synchronised them, and the outputs were sized above)
@@ -1000,6 +1009,13 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
       h_loud_.resize(rows.size());
       for (int k = 0; k < P; k++)
         for (int j = 0; j < 3; j++) h_loud_[(size_t)k * 3 + j] = rows[(size_t)j * P + k];
+    }
+    if (lim_) {    // report rows 1, 2 of [3][P] -> program-major on the host
+      std::vector<float> rows((size_t)P * 2);
+      KKX_CUDA(cudaMemcpy(rows.data(), r.lim + P, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
+      h_lim_.resize(rows.size());
+      for (int k = 0; k < P; k++)
+        for (int j = 0; j < 2; j++) h_lim_[(size_t)k * 2 + j] = rows[(size_t)j * P + k];
     }
   } catch (...) {
     cudaStreamSynchronize(stream_);

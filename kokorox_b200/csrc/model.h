@@ -174,6 +174,8 @@ struct Options {
   // 1/100 dBTP
   int loudness_target = 0;
   int true_peak_max = -100;
+  // lookahead true-peak limiter (kkx.h "limiter"): 0 = off, 1 = on
+  int limiter = 0;
 };
 
 // Device-resident weights of one checkpoint on one GPU: every layout the kernels read (fp32 SIMT, bf16 / split-TF32
@@ -276,6 +278,10 @@ class Model {
   // holds 3 P floats, per program k at 3 k: integrated loudness (LUFS, NaN = undefined), true peak (dBTP), gain.
   bool loudness_ran() const { return ran_ && loud_; }
   const std::vector<float>& last_loudness() const { return h_loud_; }
+  // Limiter of the last run's programs (kernels_loudness.cu): true if that run limited; then last_limiter() holds
+  // 2 P floats, per program k at 2 k: the largest reduction (dB) and the output's true peak (dBTP).
+  bool limiter_ran() const { return ran_ && lim_; }
+  const std::vector<float>& last_limiter() const { return h_lim_; }
 
   void set_noise(const float* noise, long long n);
   void set_inject(const std::string& name, int item, const void* data, long long count);
@@ -308,6 +314,10 @@ class Model {
     void* twin = nullptr;      // its 16-bit PCM (PCM16, FLAC) or G.711 (ULAW, ALAW) twin
     float* loud = nullptr;     // [3][P] lufs | dBTP | gain of loudness normalisation; the gain feeds the resampling
     float* wav24 = nullptr;    // resampling pass only: the run's 24 kHz waveform, item b at s24_off_[b]
+    float* lim = nullptr;      // [3][P] t | max reduction (dB) | output true peak (dBTP) of the limiter; t feeds the
+                               // resampling
+    float* lim_p = nullptr;    // limiter: the detector p and the limited waveform v, both indexed like wav24
+    float* lim_v = nullptr;
   };
   // Linear / Conv1d on the precision-critical path: split-TF32 tensor cores when precision==1 and
   // the weight has a TcW32, fp32 SIMT otherwise.  Returns true when the result went to the operand planes of `o`
@@ -397,7 +407,7 @@ class Model {
   // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC streams, their
   // per-item byte offsets (host) and the encoder's tables and scratch
   Encoding enc_ = Encoding::F32;
-  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_, wav24A_;
+  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_, wav24A_, limA_, limWavA_;
   std::vector<long long> flac_off_;
   // program table of the current run (P + 1 item offsets); s24_off_ [B + 1]: each item's offset in the run's 24 kHz
   // waveform, where a program is contiguous
@@ -412,6 +422,10 @@ class Model {
   // loudness normalisation of the current run; h_loud_ = the host copy of Run::loud (program-major)
   bool loud_ = false; LoudParams loud_par_{};
   std::vector<float> h_loud_;
+  // the limiter of the current run (it measures through the loudness kernels, so loud_par_ serves it too); h_lim_ =
+  // the host copy of Run::lim's report rows (program-major)
+  bool lim_ = false;
+  std::vector<float> h_lim_;
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
   std::vector<long long> sample_off_;                                      // [P + 1] at the output rate
   int* h_pred_dur_ = nullptr; size_t h_pred_dur_cap_ = 0;                  // pinned: per-row integer durations of the last run

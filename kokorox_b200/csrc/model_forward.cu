@@ -655,10 +655,12 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   const int K = k1 - k0;
   long long *d_p_in = nullptr, *d_p_len = nullptr, *d_p_out = nullptr;
   long long max_out = 0, max_len24 = 0;
-  // loudness normalisation: per-program 2400-sample segment energies (offsets seg_off) and true-peak scratch
+  // loudness normalisation and the limiter: per-program 2400-sample segment energies (offsets seg_off), true-peak and
+  // limiter scratch
   long long* d_seg_off = nullptr;
   float* energy = nullptr;
   unsigned* peak = nullptr;
+  unsigned* lim_acc = nullptr;
   if (resample_ && K > 0) {
     std::vector<long long> p_in(K), p_len(K), p_out(K), seg_off(K);
     long long nseg = 0;
@@ -677,12 +679,13 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     upload(d_p_in, p_in.data(), K * sizeof(long long));
     upload(d_p_len, p_len.data(), K * sizeof(long long));
     upload(d_p_out, p_out.data(), K * sizeof(long long));
-    if (loud_) {
+    if (loud_ || lim_) {
       d_seg_off = A.alloc<long long>(K);
       energy = A.alloc<float>((size_t)std::max(nseg, 1LL));
       peak = A.alloc<unsigned>(K);
       upload(d_seg_off, seg_off.data(), K * sizeof(long long));
     }
+    if (lim_) lim_acc = A.alloc<unsigned>((size_t)2 * K);
   }
 
   // ---- length regulation (K4/K5)
@@ -891,13 +894,20 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   if (K == 0) return;   // every program of this group goes on into the next
   const int P = n_prog();
   float* gain = nullptr;
-  if (loud_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
+  const float* wav = r.wav24;
+  if (loud_ || lim_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
     gain = r.loud + 2 * (size_t)P + k0;
     launch_loudness(r.wav24, d_p_in, d_p_len, d_seg_off, loud_par_, energy, peak, r.loud + k0, r.loud + P + k0, gain,
-                    K, max_len24, st);
+                    K, max_len24, st, lim_ ? r.lim_p : nullptr);
+  }
+  if (lim_) {   // the limited waveform v is resampled instead, with the static trim t as its gain (r.lim = t | report)
+    launch_limiter(r.wav24, r.lim_p, d_p_in, d_p_len, loud_par_, gain, r.lim_v, nullptr, lim_acc, r.lim + k0,
+                   r.lim + P + k0, r.lim + 2 * (size_t)P + k0, K, max_len24, st);
+    wav = r.lim_v;
+    gain = r.lim + k0;
   }
   // grids span the longest program (64-bit sample indices); CTAs past a shorter program's end return at once
-  launch_resample(r.wav24, d_p_in, d_p_len, d_p_out, d_taps_, rs_U_, rs_D_, rs_H_, gain, r.audio, pcm,
+  launch_resample(wav, d_p_in, d_p_len, d_p_out, d_taps_, rs_U_, rs_D_, rs_H_, gain, r.audio, pcm,
                   law ? static_cast<unsigned char*>(r.twin) : nullptr, enc_ == Encoding::ALAW ? 1 : 0, K, max_out, st);
 }
 

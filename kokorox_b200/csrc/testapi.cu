@@ -126,6 +126,39 @@ KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64
   });
 }
 
+KKX_API int kkx_test_limiter(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
+                             int32_t ceiling_centi_dbtp, float* gain, float* G, float* v, float* t,
+                             float* max_reduction_db, float* true_peak_dbtp) {
+  return run(device, [&] {
+    if (!x || !lens || B < 1) throw ArgError("kkx_test_limiter: bad argument");
+    std::vector<long long> in_off(B), in_len(B), seg_off(B);
+    long long ni = 0, nseg = 0, max_len = 0;
+    for (int b = 0; b < B; b++) {
+      if (lens[b] < 1) throw ArgError("kkx_test_limiter: every item needs >= 1 sample");
+      in_off[b] = ni; in_len[b] = lens[b]; seg_off[b] = nseg;
+      ni += lens[b]; nseg += lens[b] / kLoudSeg; max_len = std::max<long long>(max_len, lens[b]);
+    }
+    const LoudParams P = loudness_params(target_centi_lufs / 100.0, ceiling_centi_dbtp / 100.0, true);
+    DevBuf dx(x, (size_t)ni * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8), dso(seg_off.data(), B * 8);
+    DevBuf de(nullptr, (size_t)std::max(nseg, 1LL) * 4), dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4);
+    DevBuf dpm(nullptr, (size_t)ni * 4), dv(nullptr, (size_t)ni * 4), dG(nullptr, (size_t)ni * 4);
+    DevBuf dacc(nullptr, (size_t)B * 2 * 4), dl(nullptr, (size_t)B * 3 * 4);
+    float* r = dr.as<float>();
+    float* l = dl.as<float>();
+    launch_loudness(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), dso.as<long long>(), P, de.as<float>(),
+                    dp.as<unsigned>(), r, r + B, r + 2 * B, B, max_len, 0, dpm.as<float>());
+    launch_limiter(dx.as<float>(), dpm.as<float>(), dio.as<long long>(), dil.as<long long>(), P, r + 2 * B,
+                   dv.as<float>(), dG.as<float>(), dacc.as<unsigned>(), l, l + B, l + 2 * B, B, max_len, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    if (gain) KKX_CUDA(cudaMemcpy(gain, r + 2 * B, B * 4, cudaMemcpyDeviceToHost));
+    if (G) KKX_CUDA(cudaMemcpy(G, dG.p, (size_t)ni * 4, cudaMemcpyDeviceToHost));
+    if (v) KKX_CUDA(cudaMemcpy(v, dv.p, (size_t)ni * 4, cudaMemcpyDeviceToHost));
+    if (t) KKX_CUDA(cudaMemcpy(t, l, B * 4, cudaMemcpyDeviceToHost));
+    if (max_reduction_db) KKX_CUDA(cudaMemcpy(max_reduction_db, l + B, B * 4, cudaMemcpyDeviceToHost));
+    if (true_peak_dbtp) KKX_CUDA(cudaMemcpy(true_peak_dbtp, l + 2 * B, B * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
 KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
                               uint8_t* dst, int64_t capacity, int64_t* byte_offsets) {
   long long total = 0;

@@ -108,6 +108,9 @@ def load_library(path: Optional[str] = None):
         lib.kkx_test_resample_taps.restype = i64
         lib.kkx_test_resample.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(i16), P(u8)]
         lib.kkx_last_loudness.argtypes = [vp, i32, P(f32), P(f32), P(f32)]
+        lib.kkx_last_limiter.argtypes = [vp, i32, P(f32), P(f32)]
+        lib.kkx_test_limiter.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(f32), P(f32), P(f32), P(f32),
+                                         P(f32)]
         lib.kkx_test_loudness_design.argtypes = [C.c_double, P(C.c_double), P(f32), i64]
         lib.kkx_test_loudness_design.restype = i64
         lib.kkx_test_loudness.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(f32), P(f32)]
@@ -558,6 +561,18 @@ class B200Koko:
         lufs, tp, gain = (np.zeros(max(n, 1), np.float32) for _ in range(3))
         self._check(self._lib.kkx_last_loudness(self._ctx, n, _fp(lufs), _fp(tp), _fp(gain)))
         return lufs[:n], tp[:n], gain[:n]
+
+    def last_limiter(self):
+        """What the lookahead limiter (option ``limiter``) did in this session's last synchronous call:
+        ``(max_reduction_db, true_peak_dbtp)``, two float32 arrays in item order -- program order after
+        ``infer_programs``.  ``max_reduction_db`` is >= 0 (0: the item was not touched); ``true_peak_dbtp`` is the
+        output's true peak.  Raises KkxError when that call ran with the limiter off.  Coalesced and ``submit``
+        batches are not reported."""
+        self._require()
+        n = max(int(self._lib.kkx_get_stat(self._ctx, b"limiter_items")), 0)
+        red, tp = (np.zeros(max(n, 1), np.float32) for _ in range(2))
+        self._check(self._lib.kkx_last_limiter(self._ctx, n, _fp(red), _fp(tp)))
+        return red[:n], tp[:n]
 
     # -- device-resident path (bench `value`) ---------------------------------------------
     def stage(self, tokens, styles, speeds) -> None:
