@@ -216,9 +216,9 @@ KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes);
  *   encoding: KKX_ENC_F32 (4 bytes per sample), _PCM16 (2), _ULAW / _ALAW (1, G.711 as kkx_infer_batch_g711), _FLAC.
  *   Program k's output is bytes [out_byte_offsets[k], out_byte_offsets[k+1]) of *out_bytes (offsets in bytes for every
  *   encoding); out_sample_offsets (nullable, [n_programs + 1]) in output-rate samples; out_pred_dur (nullable) is
- *   indexed like tokens.  One pass (no "max_tokens" split).  Afterwards kkx_last_loudness and the "loudness_items"
- *   stat report per program (their batch is n_programs).  A FLAC program holds at most 2^36 - 1 samples (the
- *   STREAMINFO field; longer is KKX_ERR_ARG).  Release the buffer with kkx_release_programs.
+ *   indexed like tokens.  One pass (no "max_tokens" split).  Afterwards kkx_last_loudness, kkx_last_loudness_range
+ *   and the "loudness_items" stat report per program (their batch is n_programs).  A FLAC program holds at most
+ *   2^36 - 1 samples (the STREAMINFO field; longer is KKX_ERR_ARG).  Release the buffer with kkx_release_programs.
  *   KKX_ERR_ARG, with the session left as it was, for: a null out_bytes or out_byte_offsets; n_programs outside
  *   1..batch; program_offsets null, not starting at 0, not ending at batch, or not strictly increasing (no empty
  *   program); encoding outside 0..4.
@@ -342,8 +342,8 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                    do not depend on its batch, frame group or pass.  One loudness across several items (program
  *                    loudness of a request split into chunks) is kkx_infer_programs.  Rule 5 caps the gain, so an
  *                    item whose peak-to-loudness ratio exceeds ceiling - target comes back quieter than the target;
- *                    "limiter" reaches it.  Not provided: compression, measurement at the output rate, momentary /
- *                    short-term loudness and loudness range, a measure-only mode.
+ *                    "limiter" reaches it.  Measurement without normalisation, loudness range and maximum momentary /
+ *                    short-term loudness: "loudness_report".  Not provided: compression, measurement at the output rate.
  *   "limiter"     lookahead true-peak limiter: 0 (DEFAULT) = off, every bit, byte and launch as without it; 1 = on.
  *                 Any other value is KKX_ERR_ARG and the session keeps its setting.  One setting per session, followed
  *                 by the same entry points as "loudness_target" for runs that start after the call.  It works on each
@@ -379,22 +379,61 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                 "lim_trim" -- 3 launches more than loudness alone per frame group that completes a program (6 more
  *                 than plain output when "loudness_target" is 0; a resampling pass runs also at 24000).
  *                 Not provided: compression, a limiter at the output rate, user-set lookahead / release / Rmax.
+ *   "loudness_report"  the EBU R128 / Tech 3341 report of every item (program): 0 (DEFAULT) = off, every bit, byte and
+ *                 launch as without it; 1 = on.  Any other value is KKX_ERR_ARG and the session keeps its setting.  One
+ *                 setting per session, followed by the same entry points as "loudness_target" for runs that start
+ *                 after the call.  Each item (program of kkx_infer_programs) is measured on its 24 kHz model waveform x,
+ *                 the x that rules 1-4 of "loudness_target" measure.
+ *                 Measure-only: with "loudness_target" = 0 and "limiter" = 0, every returned sample, byte and FLAC file
+ *                 is bit-identical to the same run with the option off, at every "out_rate" and in every encoding; the
+ *                 applied gain is exactly 1 (rule 5's ceiling does not apply: measuring never rescales).  With
+ *                 "loudness_target" or "limiter" on, the option adds the statistics alone: gains, samples and
+ *                 kkx_last_loudness are as without it.
+ *                 After a synchronous call that ran with it, kkx_last_loudness succeeds also when "loudness_target"
+ *                 was 0 (gain = the applied g: 1 in measure-only, step 1's g under the limiter), and
+ *                 kkx_last_loudness_range reports, on the segment energies e_i of rule 2 (K-weighted sum of squares of
+ *                 segment i, 2400 samples; n_seg = floor(n / 2400)):
+ *                 1. Momentary: z_j = (e_j + e_{j+1} + e_{j+2} + e_{j+3}) / 9600 for every whole 400 ms block (rule 2's
+ *                    z_j), summed in double in ascending order; M = -0.691 + 10 log10(max_j z_j).
+ *                 2. Short-term: s_j = (sum over i = j .. j + 29 of e_i) / 72000 for every whole 3 s window on the
+ *                    100 ms hop from sample 0 (j = 0 .. n_seg - 30), summed in double in ascending i;
+ *                    l_s = -0.691 + 10 log10 s_j; S = -0.691 + 10 log10(max_j s_j).
+ *                 3. Gates (EBU Tech 3342): absolute l_s > -70; relative Gamma = -0.691 + 10 log10(mean s over the
+ *                    absolute-gated windows) - 20, l_s > Gamma (strict comparisons, as in rule 3).
+ *                 4. Range: the m windows that pass, their s sorted a_0 <= .. <= a_{m-1}; lo = floor((10 (m - 1) +
+ *                    50) / 100), hi = floor((95 (m - 1) + 50) / 100) (nearest rank, halves up, in integers);
+ *                    LRA = 10 log10(a_hi / a_lo) LU (0 for m = 1).
+ *                 5. Undefined: M is NaN without a whole 400 ms block (n < 9600); S and LRA are NaN without a whole 3 s
+ *                    window (n < 72000); LRA is NaN when no window passes the gates.  M and S are -inf for silence.
+ *                 6. The values describe x, unscaled (as kkx_last_loudness does): under a static gain g the output's M
+ *                    and S are these plus 20 log10 g and its LRA is the same; with the limiter on they are not the
+ *                    output's values.
+ *                 Every value is a function of the program's samples alone: not of its batch, position, frame group,
+ *                 "max_tokens" pass, coalescing or kkx_submit.  Device work: the three loudness launches (also when
+ *                 "loudness_target" is 0), then "loud_short" (one thread per 3 s window) and "loud_range" (one CTA per
+ *                 program: maxima, gates, and the 10 % / 95 % points by an exact radix select) -- 2 launches more than
+ *                 loudness alone per frame group that completes a program; measure-only at 24000 adds 3 + 2 + 1 (the
+ *                 resampling pass-through, without a gain) to plain output.
+ *                 Not provided: measurement at the output rate or of the limiter's output, a momentary / short-term
+ *                 time series (a loudness curve), reports of coalesced and kkx_submit batches.
  * kkx_get_stat keys: "launches", "last_frames", "gpu_us", "precision", "coalesced_batches",
  * "coalesced_requests", "coalesced_largest", "async_batches", "async_requests", "frame_groups",
  * "group_first:<g>" (first item of frame group g of the last run), "weights_sessions" (sessions sharing this
  * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate", "loudness_target",
  * "true_peak_max", "loudness_items" (items -- programs after kkx_infer_programs -- kkx_last_loudness reports now; 0
- * if it would fail with KKX_ERR_STATE), "limiter", "limiter_items" (the same for kkx_last_limiter). */
+ * if it would fail with KKX_ERR_STATE), "limiter", "limiter_items" (the same for kkx_last_limiter), "loudness_report"
+ * (the option's value). */
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value);
 KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "last_frames", "gpu_us" ... */
 
-/* What loudness normalisation measured and applied in the last SYNCHRONOUS call on the ctx (kkx_infer without
- * "coalesce", kkx_infer_batch and its _voices / _pcm16 / _g711 / _flac forms, kkx_run_staged), in item order, over
- * every pass of a "max_tokens" split; after kkx_infer_programs, in program order (one entry per program).  Per item: lufs = integrated loudness L (NaN when undefined), true_peak_dbtp =
- * 20 log10 tp of the unscaled item (-inf for silence), gain = the applied g.  Each pointer is nullable and receives
- * `batch` floats.  KKX_ERR_STATE if no synchronous call has completed or that call ran with "loudness_target" = 0;
- * KKX_ERR_ARG if `batch` is not that call's item count.  Coalesced callers and kkx_submit batches are normalised
- * but not reported here (a batch of several callers has no per-caller report). */
+/* What loudness normalisation (or "loudness_report") measured and applied in the last SYNCHRONOUS call on the ctx
+ * (kkx_infer without "coalesce", kkx_infer_batch and its _voices / _pcm16 / _g711 / _flac forms, kkx_run_staged), in
+ * item order, over every pass of a "max_tokens" split; after kkx_infer_programs, in program order (one entry per
+ * program).  Per item: lufs = integrated loudness L (NaN when undefined), true_peak_dbtp = 20 log10 tp of the unscaled
+ * item (-inf for silence), gain = the applied g.  Each pointer is nullable and receives `batch` floats.
+ * KKX_ERR_STATE if no synchronous call has completed or that call ran with "loudness_target" = 0 and
+ * "loudness_report" = 0; KKX_ERR_ARG if `batch` is not that call's item count.  Coalesced callers and kkx_submit
+ * batches are normalised but not reported here (a batch of several callers has no per-caller report). */
 KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* true_peak_dbtp, float* gain);
 
 /* What the limiter ("limiter" = 1) did in the last SYNCHRONOUS call, with kkx_last_loudness's scope, order and errors
@@ -402,6 +441,15 @@ KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* t
  * -20 log10(t min over i of G[i]) (>= 0; 0 = untouched), true_peak_dbtp = 20 log10(t tp_v), the output's true peak.
  * Each pointer is nullable and receives `batch` floats. */
 KKX_API int kkx_last_limiter(kkx_ctx* ctx, int32_t batch, float* max_reduction_db, float* true_peak_dbtp);
+
+/* The EBU R128 statistics of "loudness_report" (rules 1-6 there) for the last SYNCHRONOUS call, with kkx_last_loudness's
+ * scope, order and errors (KKX_ERR_STATE when that call ran with "loudness_report" = 0; KKX_ERR_ARG when `batch` is
+ * not its item or program count).  Per item (program): loudness_range_lu = LRA (EBU Tech 3342), max_momentary_lufs =
+ * M, max_short_term_lufs = S; NaN where undefined.  They describe the unscaled 24 kHz waveform: under the applied gain
+ * g the output's M and S are 20 log10 g higher and its LRA is the same.  Each pointer is nullable and receives `batch`
+ * floats. */
+KKX_API int kkx_last_loudness_range(kkx_ctx* ctx, int32_t batch, float* loudness_range_lu, float* max_momentary_lufs,
+                                    float* max_short_term_lufs);
 
 /* Per-kernel device timing of the last run (CUDA events on the library's stream, one after every
  * launch).  kkx_profile_json writes {"conv_flops": F, "gpu_us": T, "kernels": {name: [launches,

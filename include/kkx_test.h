@@ -148,6 +148,11 @@ KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64
 KKX_API int kkx_test_limiter(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
                              int32_t ceiling_centi_dbtp, float* gain, float* G, float* v, float* t,
                              float* max_reduction_db, float* true_peak_dbtp);
+/* EBU R128 loudness range and maxima (kernels_loudness.cu, kkx.h kkx_last_loudness_range), on B items packed as for
+ * kkx_test_loudness: the launches a "loudness_report" run makes (loud_energy, loud_peak, loud_gain, then loud_short
+ * and loud_range).  Per item: lra (LU), m_max and s_max (LUFS); NaN = undefined.  Every output pointer is nullable. */
+KKX_API int kkx_test_loudness_range(int device, const float* x, int32_t B, const int64_t* lens, float* lra,
+                                    float* m_max, float* s_max);
 KKX_API const char* kkx_test_last_error(void);
 
 #ifdef __cplusplus

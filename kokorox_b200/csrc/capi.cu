@@ -65,12 +65,17 @@ struct kkx_ctx {
   int64_t async_batches = 0, async_requests = 0;
 
   // Loudness report of the last synchronous call (kkx_last_loudness), guarded by `mu`: 3 floats per item (LUFS, dBTP,
-  // gain), appended pass by pass; valid once the call has succeeded, `normalised` if its runs had the option on.
+  // gain), appended pass by pass; valid once the call has succeeded, `measured` if its runs had "loudness_target" or
+  // "loudness_report" on.
   std::vector<float> loud;
-  bool loud_valid = false, loud_normalised = false;
+  bool loud_valid = false, loud_measured = false;
   // Limiter report of the same call (kkx_last_limiter), kept alongside: 2 floats per item (max reduction dB, dBTP).
   std::vector<float> lim;
   bool lim_ran = false;
+  // Loudness range report of the same call (kkx_last_loudness_range): 3 floats per item (LRA, max momentary, max
+  // short-term).
+  std::vector<float> rng;
+  bool rng_ran = false;
 };
 
 static thread_local std::string g_err;
@@ -236,11 +241,12 @@ static void hand_out(kkx_ctx* ctx, void* host, size_t cap) {
 
 KKX_API void kkx_release(kkx_ctx* ctx, float* audio);
 
-// kkx_last_loudness / kkx_last_limiter bookkeeping of a synchronous call (caller holds ctx->mu): begin, one note per
-// model run, done.  Coalesced and asynchronous batches leave the reports alone.
+// kkx_last_loudness / kkx_last_limiter / kkx_last_loudness_range bookkeeping of a synchronous call (caller holds
+// ctx->mu): begin, one note per model run, done.  Coalesced and asynchronous batches leave the reports alone.
 static void loud_begin(kkx_ctx* ctx) {
-  ctx->loud.clear(); ctx->loud_valid = false; ctx->loud_normalised = false;
+  ctx->loud.clear(); ctx->loud_valid = false; ctx->loud_measured = false;
   ctx->lim.clear(); ctx->lim_ran = false;
+  ctx->rng.clear(); ctx->rng_ran = false;
 }
 static void loud_note(kkx_ctx* ctx) {
   const Model& m = *ctx->model;
@@ -248,8 +254,12 @@ static void loud_note(kkx_ctx* ctx) {
     ctx->lim_ran = true;
     ctx->lim.insert(ctx->lim.end(), m.last_limiter().begin(), m.last_limiter().end());
   }
+  if (m.loudness_range_ran()) {
+    ctx->rng_ran = true;
+    ctx->rng.insert(ctx->rng.end(), m.last_loudness_range().begin(), m.last_loudness_range().end());
+  }
   if (!m.loudness_ran()) return;
-  ctx->loud_normalised = true;
+  ctx->loud_measured = true;
   ctx->loud.insert(ctx->loud.end(), m.last_loudness().begin(), m.last_loudness().end());
 }
 static void loud_done(kkx_ctx* ctx) { ctx->loud_valid = true; }
@@ -885,6 +895,10 @@ KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
       if (value != 0 && value != 1)
         throw ArgError("limiter " + std::to_string(value) + " is not supported: give 0 (off) or 1 (on)");
       o.limiter = (int)value;
+    } else if (k == "loudness_report") {
+      if (value != 0 && value != 1)
+        throw ArgError("loudness_report " + std::to_string(value) + " is not supported: give 0 (off) or 1 (on)");
+      o.loudness_report = (int)value;
     }
     else throw ArgError("unknown option: " + k);
   });
@@ -901,8 +915,9 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   if (k == "out_rate") return ctx->model->opt.out_rate;
   if (k == "loudness_target") return ctx->model->opt.loudness_target;
   if (k == "true_peak_max") return ctx->model->opt.true_peak_max;
-  if (k == "loudness_items") return ctx->loud_valid && ctx->loud_normalised ? (int64_t)(ctx->loud.size() / 3) : 0;
+  if (k == "loudness_items") return ctx->loud_valid && ctx->loud_measured ? (int64_t)(ctx->loud.size() / 3) : 0;
   if (k == "limiter") return ctx->model->opt.limiter;
+  if (k == "loudness_report") return ctx->model->opt.loudness_report;
   if (k == "limiter_items") return ctx->loud_valid && ctx->lim_ran ? (int64_t)(ctx->lim.size() / 2) : 0;
   if (k == "coalesced_batches") return ctx->coalesced_batches;
   if (k == "coalesced_requests") return ctx->coalesced_requests;
@@ -931,7 +946,8 @@ KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* t
   std::lock_guard<std::mutex> lk(ctx->mu);
   return guarded(ctx, [&] {
     if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
-    if (!ctx->loud_normalised) throw StateError("the last synchronous call ran with loudness normalisation off");
+    if (!ctx->loud_measured)
+      throw StateError("the last synchronous call ran with loudness normalisation and the loudness report off");
     const int64_t n = (int64_t)(ctx->loud.size() / 3);
     if (batch != n)
       throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
@@ -956,6 +972,25 @@ KKX_API int kkx_last_limiter(kkx_ctx* ctx, int32_t batch, float* max_reduction_d
     for (int64_t b = 0; b < n; b++) {
       if (max_reduction_db) max_reduction_db[b] = ctx->lim[b * 2];
       if (true_peak_dbtp) true_peak_dbtp[b] = ctx->lim[b * 2 + 1];
+    }
+  });
+}
+
+KKX_API int kkx_last_loudness_range(kkx_ctx* ctx, int32_t batch, float* loudness_range_lu, float* max_momentary_lufs,
+                                    float* max_short_term_lufs) {
+  int rc = check_ctx(ctx);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(ctx, [&] {
+    if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
+    if (!ctx->rng_ran) throw StateError("the last synchronous call ran with the loudness report off");
+    const int64_t n = (int64_t)(ctx->rng.size() / 3);
+    if (batch != n)
+      throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
+    for (int64_t b = 0; b < n; b++) {
+      if (loudness_range_lu) loudness_range_lu[b] = ctx->rng[b * 3];
+      if (max_momentary_lufs) max_momentary_lufs[b] = ctx->rng[b * 3 + 1];
+      if (max_short_term_lufs) max_short_term_lufs[b] = ctx->rng[b * 3 + 2];
     }
   });
 }

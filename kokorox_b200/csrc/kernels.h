@@ -305,6 +305,12 @@ void launch_resample(const float* x, const long long* in_off, const long long* i
 //                    G (nullable, indexed like x) = the smoothed gain, and per item t[b] (the static trim),
 //                    red_db[b] (max reduction, dB) and out_db[b] (the output's true peak, dBTP).  acc: [2 B] scratch.
 //                    Three launches: "lim_envelope", "loud_peak" (on v), "lim_trim".
+//   loudness_params(report = true): a "loudness_report" session; with target 0 and no limiter it is measure-only:
+//                    no normalisation and no cap, the gain is exactly 1.
+//   launch_loudness_range: after launch_loudness, on its in_len / seg_off / energy: per item lra[b] (LU), m_max[b]
+//                    and s_max[b] (LUFS), NaN = undefined (kkx.h kkx_last_loudness_range).  st: scratch of
+//                    in_len[b] / 2400 doubles per item at seg_off[b] (the short-term energies).  Two launches:
+//                    "loud_short", "loud_range".
 constexpr int kLoudSeg = 2400, kLoudWarm = 4800, kTpTaps = 81;
 // limiter constants (kkx.h "limiter"): lookahead, FIR guard, largest reduction (dB), release slope (dB per sample)
 constexpr int kLimHa = 120, kLimHb = 10, kLimW = 4800;
@@ -316,13 +322,15 @@ struct LoudParams {
   int normalise = 1, limiter = 0;   // limiter: cap at ceiling + kLimRmax, also when L is undefined
 };
 void loudness_design(double fs, double kw[10], std::vector<float>* tp_taps);
-LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter = false);
+LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter = false, bool report = false);
 void launch_loudness(const float* x, const long long* in_off, const long long* in_len, const long long* seg_off,
                      const LoudParams& P, float* energy, unsigned* peak, float* lufs, float* tp_db, float* gain, int B,
                      long long max_len, cudaStream_t st, float* pmax = nullptr);
 void launch_limiter(const float* x, const float* pmax, const long long* in_off, const long long* in_len,
                     const LoudParams& P, const float* gain, float* v, float* G, unsigned* acc, float* t, float* red_db,
                     float* out_db, int B, long long max_len, cudaStream_t st);
+void launch_loudness_range(const long long* in_len, const long long* seg_off, const float* energy, double* st,
+                           float* lra, float* m_max, float* s_max, int B, long long max_len, cudaStream_t stream);
 
 // Lossless FLAC of 16-bit mono PCM (kernels_flac.cu; the bitstream rules are in kkx.h, kkx_infer_batch_flac).
 //   Item b is pcm[soff[b] .. soff[b + 1]) (>= 1 sample) and has flac_frames(n_b) frames of 4096 samples; foff[b + 1]

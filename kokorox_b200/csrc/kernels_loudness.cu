@@ -1,7 +1,8 @@
 // kernels_loudness.cu -- loudness normalisation (K14): ITU-R BS.1770 integrated loudness of each utterance's 24 kHz
 // waveform, its true peak, and the static gain that brings it to the session's target under a true-peak ceiling
-// (kkx.h "loudness_target" / "true_peak_max"), and the lookahead true-peak limiter (kkx.h "limiter", at the end of
-// this file).  The gains themselves are applied by resample_kernel (kernels_signal.cu).
+// (kkx.h "loudness_target" / "true_peak_max"), the lookahead true-peak limiter (kkx.h "limiter") and the EBU R128
+// loudness range and maxima (kkx.h "loudness_report", at the end of this file).  The gains themselves are applied by
+// resample_kernel (kernels_signal.cu).
 //
 // Per item (n samples x at 24 kHz):
 //   loud_energy  one thread per 2400-sample segment s (the 100 ms hop): the K-weighting cascade (shelf, then
@@ -49,7 +50,7 @@ void loudness_design(double fs, double kw[10], std::vector<float>* tp_taps) {
   if (tp_taps) poly_design(4, 1, tp_taps);   // 4 * firwin(81, 1/4, ("kaiser", 5.0))
 }
 
-LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter) {
+LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter, bool report) {
   LoudParams P{};
   double kw[10];
   std::vector<float> taps;
@@ -59,7 +60,8 @@ LoudParams loudness_params(double target_lufs, double ceiling_dbtp, bool limiter
   for (int i = 0; i < kTpTaps; i++) P.tp[i] = taps[i];
   P.target_lufs = target_lufs;
   P.ceiling_dbtp = ceiling_dbtp;
-  P.normalise = limiter ? target_lufs != 0.0 : 1;   // a limiter session may run without a loudness target
+  // a limiter or report session may run without a loudness target (report alone: measure-only, g = 1, no cap)
+  P.normalise = limiter || report ? target_lufs != 0.0 : 1;
   P.limiter = limiter ? 1 : 0;
   return P;
 }
@@ -213,7 +215,8 @@ __global__ void __launch_bounds__(kLgThreads) loud_gain_kernel(const long long* 
   const float tp = __uint_as_float(peak[b]);
   double g = 1.0;
   if (P.normalise && !isnan(L)) g = pow(10.0, (P.target_lufs - L) / 20.0);
-  if (P.limiter || !isnan(L)) {   // rule 5's cap; the limiter's sits Rmax higher and always applies (kkx.h "limiter")
+  // rule 5's cap (not when measuring only); the limiter's sits Rmax higher and always applies (kkx.h "limiter")
+  if (P.limiter || (P.normalise && !isnan(L))) {
     const double cap = pow(10.0, (P.ceiling_dbtp + (P.limiter ? kLimRmax : 0.0)) / 20.0);
     if ((double)tp * g > cap) g = cap / (double)tp;
   }
@@ -406,6 +409,155 @@ void launch_limiter(const float* x, const float* pmax, const long long* in_off, 
   post_launch("loud_peak", st);
   lim_trim_kernel<<<(B + 127) / 128, 128, 0, st>>>(acc, P.ceiling_dbtp, B, t, red_db, out_db);
   post_launch("lim_trim", st);
+}
+
+// ------------------------------------------------------------------------------------------ loudness range, maxima
+// kkx.h "loudness_report" / kkx_last_loudness_range (EBU Tech 3341 / 3342), on loud_energy's segment energies e_i.
+//   loud_short  one thread per 3 s window j (segments j .. j + 29 on the 100 ms hop): s_j = the 30 energies summed in
+//               double in ascending i, / 72000; written to st at the item's seg_off, like the energies.
+//   loud_range  one CTA per item: max z_j (z as loud_gain forms it) and max s_j by fixed-shape reductions (max is
+//               exact); the absolute and relative gates with block_sum; then the order statistics a_lo and a_hi of the
+//               gated s_j by an MSD radix select on their 64-bit patterns (non-negative doubles order like their
+//               bits): 8 passes of 8-bit digits, each counting the candidates of both ranks into two 256-bin shared
+//               histograms, after which one warp per rank picks the digit.  Counts are exact, so the result does not
+//               depend on the order in which windows are visited, and the shared memory is fixed whatever the number
+//               of windows (tens of thousands for a long program).
+constexpr int kStSegs = 30;   // segments per 3 s window
+
+__global__ void __launch_bounds__(kLeThreads) loud_short_kernel(const long long* __restrict__ in_len,
+                                                                const long long* __restrict__ seg_off,
+                                                                const float* __restrict__ energy,
+                                                                double* __restrict__ st) {
+  const int b = blockIdx.y;
+  const long long nwin = in_len[b] / kLoudSeg - (kStSegs - 1);
+  const long long j = (long long)blockIdx.x * kLeThreads + threadIdx.x;
+  if (j >= nwin) return;
+  const float* e = energy + seg_off[b] + j;
+  double s = (double)__ldg(e);
+#pragma unroll
+  for (int i = 1; i < kStSegs; i++) s += (double)__ldg(e + i);
+  st[seg_off[b] + j] = s / (double)(kStSegs * kLoudSeg);
+}
+
+__device__ double block_max(double v, double* red) {   // fixed-shape tree, like block_sum
+  const int t = threadIdx.x;
+  __syncthreads();
+  red[t] = v;
+  __syncthreads();
+  for (int h = kLgThreads / 2; h > 0; h >>= 1) {
+    if (t < h) red[t] = fmax(red[t], red[t + h]);
+    __syncthreads();
+  }
+  return red[0];
+}
+
+__global__ void __launch_bounds__(kLgThreads) loud_range_kernel(const long long* __restrict__ in_len,
+                                                                const long long* __restrict__ seg_off,
+                                                                const float* __restrict__ energy,
+                                                                const double* __restrict__ st,
+                                                                float* __restrict__ lra, float* __restrict__ m_max,
+                                                                float* __restrict__ s_max) {
+  __shared__ double red_d[kLgThreads];
+  __shared__ long long red_n[kLgThreads];
+  __shared__ unsigned hist[2][256];
+  __shared__ unsigned long long pre[2];   // the decided high bits of a_lo, a_hi
+  __shared__ unsigned rank[2];            // their ranks among the candidates that share those bits
+  const int b = blockIdx.x, t = threadIdx.x;
+  const long long nseg = in_len[b] / kLoudSeg;
+  const long long nblk = nseg - 3, nwin = nseg - (kStSegs - 1);   // whole 400 ms blocks, whole 3 s windows
+  const float* e = energy + seg_off[b];
+  const double* s = st + seg_off[b];
+  // maxima: z, s >= 0, so 0 is the identity; an all-silent item gives 0 and -inf LUFS
+  double zm = 0.0, sm = 0.0;
+  for (long long j = t; j < nblk; j += kLgThreads)
+    zm = fmax(zm, ((double)e[j] + (double)e[j + 1] + (double)e[j + 2] + (double)e[j + 3]) / (4.0 * kLoudSeg));
+  for (long long j = t; j < nwin; j += kLgThreads) sm = fmax(sm, s[j]);
+  zm = block_max(zm, red_d);
+  sm = block_max(sm, red_d);
+  double range = NAN;
+  if (nwin > 0) {
+    // EBU Tech 3342 gates: absolute l_s > -70, relative l_s > -0.691 + 10 log10(mean s) - 20 (strict)
+    auto level = [](double v) { return -0.691 + 10.0 * log10(v); };   // v = 0: -inf, gated out
+    double sa = 0.0;
+    long long ca = 0;
+    for (long long j = t; j < nwin; j += kLgThreads)
+      if (level(s[j]) > -70.0) { sa += s[j]; ca++; }
+    const double s1 = block_sum(sa, red_d);
+    const long long c1 = block_sum(ca, red_n);
+    if (c1 > 0) {
+      const double rel = level(s1 / (double)c1) - 20.0;
+      auto gated = [&](double v) { const double l = level(v); return l > -70.0 && l > rel; };
+      long long cm = 0;
+      for (long long j = t; j < nwin; j += kLgThreads) cm += gated(s[j]) ? 1 : 0;
+      const long long m = block_sum(cm, red_n);
+      if (m > 0) {
+        // nearest rank of the 10 % and 95 % points, halves rounded up
+        if (t < 2) {
+          pre[t] = 0ull;
+          rank[t] = (unsigned)(((t == 0 ? 10 : 95) * (m - 1) + 50) / 100);
+        }
+        for (int pass = 0; pass < 8; pass++) {
+          const int shift = 56 - 8 * pass;
+          const unsigned long long mask = pass == 0 ? 0ull : ~0ull << (shift + 8);
+          for (int i = t; i < 2 * 256; i += kLgThreads) (&hist[0][0])[i] = 0u;
+          __syncthreads();
+          const unsigned long long p0 = pre[0], p1 = pre[1];
+          for (long long j = t; j < nwin; j += kLgThreads) {
+            const double v = s[j];
+            if (!gated(v)) continue;
+            const unsigned long long u = (unsigned long long)__double_as_longlong(v);
+            const unsigned d = (unsigned)(u >> shift) & 255u;
+            if ((u & mask) == p0) atomicAdd(&hist[0][d], 1u);
+            if ((u & mask) == p1) atomicAdd(&hist[1][d], 1u);
+          }
+          __syncthreads();
+          if (t < 64) {   // warp w: the bin in which rank[w] falls, 8 bins per lane, a warp scan of the lane totals
+            const int w = t >> 5, lane = t & 31;
+            unsigned c[8], tot = 0u;
+#pragma unroll
+            for (int k = 0; k < 8; k++) { c[k] = hist[w][lane * 8 + k]; tot += c[k]; }
+            unsigned inc = tot;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+              const unsigned u = __shfl_up_sync(0xffffffffu, inc, o);
+              if (lane >= o) inc += u;
+            }
+            const unsigned r = rank[w];
+            unsigned below = inc - tot;
+            if (r >= below && r < inc) {   // exactly one lane
+#pragma unroll
+              for (int k = 0; k < 8; k++) {
+                if (r < below + c[k]) {
+                  rank[w] = r - below;
+                  pre[w] |= (unsigned long long)(lane * 8 + k) << shift;
+                  break;
+                }
+                below += c[k];
+              }
+            }
+          }
+          __syncthreads();
+        }
+        range = 10.0 * log10(__longlong_as_double((long long)pre[1]) / __longlong_as_double((long long)pre[0]));
+      }
+    }
+  }
+  if (t != 0) return;
+  lra[b] = (float)range;
+  m_max[b] = nblk > 0 ? (float)(-0.691 + 10.0 * log10(zm)) : NAN;
+  s_max[b] = nwin > 0 ? (float)(-0.691 + 10.0 * log10(sm)) : NAN;
+}
+
+void launch_loudness_range(const long long* in_len, const long long* seg_off, const float* energy, double* st,
+                           float* lra, float* m_max, float* s_max, int B, long long max_len, cudaStream_t stream) {
+  if (g_dry_run) return;
+  if (B < 1 || B > 65535) throw ArgError("launch_loudness_range: batch out of range");
+  const long long max_seg = max_len / kLoudSeg;
+  const long long ge = std::max(1LL, (max_seg + kLeThreads - 1) / kLeThreads);
+  loud_short_kernel<<<dim3((unsigned)ge, B), kLeThreads, 0, stream>>>(in_len, seg_off, energy, st);
+  post_launch("loud_short", stream);
+  loud_range_kernel<<<B, kLgThreads, 0, stream>>>(in_len, seg_off, energy, st, lra, m_max, s_max);
+  post_launch("loud_range", stream);
 }
 
 }  // namespace kkx

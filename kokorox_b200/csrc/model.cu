@@ -795,14 +795,16 @@ void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_off
   }
 }
 
-// The resampling pass of this run: off at 24 kHz unless G.711 codes, loudness normalisation or the limiter are wanted
-// (then a pass-through, U = D = 1, which applies the gain).  The taps live on the device per Model and are rebuilt only when
-// the rate changes.
+// The resampling pass of this run: off at 24 kHz unless G.711 codes, loudness normalisation, the limiter or the
+// loudness report are wanted (then a pass-through, U = D = 1, which applies the gain, or none when only measuring).
+// The taps live on the device per Model and are rebuilt only when the rate changes.
 void Model::prepare_resample() {
   loud_ = opt.loudness_target != 0;
   lim_ = opt.limiter != 0;
-  if (loud_ || lim_) loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0, lim_);
-  resample_ = opt.out_rate != 24000 || enc_ == Encoding::ULAW || enc_ == Encoding::ALAW || loud_ || lim_;
+  rep_ = opt.loudness_report != 0;
+  if (loud_ || lim_ || rep_)
+    loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0, lim_, rep_);
+  resample_ = opt.out_rate != 24000 || enc_ == Encoding::ULAW || enc_ == Encoding::ALAW || loud_ || lim_ || rep_;
   rs_U_ = 1; rs_D_ = 1; rs_H_ = 0;
   if (opt.out_rate == 24000) return;
   std::vector<float> taps;
@@ -913,9 +915,13 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
     grow(wav24A_, (size_t)s24_off_[B_] * sizeof(float));
     r.wav24 = wav24A_.alloc<float>(s24_off_[B_]);
   }
-  if (loud_ || lim_) {
+  if (loud_ || lim_ || rep_) {
     grow(loudA_, (size_t)P * 3 * sizeof(float));
     r.loud = loudA_.alloc<float>((size_t)P * 3);
+  }
+  if (rep_) {
+    grow(rngA_, (size_t)P * 3 * sizeof(float));
+    r.rng = rngA_.alloc<float>((size_t)P * 3);
   }
   if (lim_) {
     grow(limA_, (size_t)P * 3 * sizeof(float));
@@ -951,6 +957,7 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
   }
   h_loud_.clear();
   h_lim_.clear();
+  h_rng_.clear();
   sink_filled_ = false;
   float* sink = (host_sink && !debug_) ? host_sink(total_samples_) : nullptr;
   // (both streams are idle here: the previous run synchronised them, and the outputs were sized above)
@@ -1003,12 +1010,19 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
     }
     KKX_CUDA(cudaStreamSynchronize(stream_));
     if (sink) { KKX_CUDA(cudaStreamSynchronize(copy_stream_)); sink_filled_ = true; }
-    if (loud_) {   // [3][P] on the device -> program-major on the host
+    if (loud_ || rep_) {   // [3][P] on the device -> program-major on the host
       std::vector<float> rows((size_t)P * 3);
       KKX_CUDA(cudaMemcpy(rows.data(), r.loud, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
       h_loud_.resize(rows.size());
       for (int k = 0; k < P; k++)
         for (int j = 0; j < 3; j++) h_loud_[(size_t)k * 3 + j] = rows[(size_t)j * P + k];
+    }
+    if (rep_) {    // LRA | max momentary | max short-term, [3][P] -> program-major on the host
+      std::vector<float> rows((size_t)P * 3);
+      KKX_CUDA(cudaMemcpy(rows.data(), r.rng, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
+      h_rng_.resize(rows.size());
+      for (int k = 0; k < P; k++)
+        for (int j = 0; j < 3; j++) h_rng_[(size_t)k * 3 + j] = rows[(size_t)j * P + k];
     }
     if (lim_) {    // report rows 1, 2 of [3][P] -> program-major on the host
       std::vector<float> rows((size_t)P * 2);

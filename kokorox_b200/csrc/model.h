@@ -176,6 +176,9 @@ struct Options {
   int true_peak_max = -100;
   // lookahead true-peak limiter (kkx.h "limiter"): 0 = off, 1 = on
   int limiter = 0;
+  // EBU R128 loudness report (kkx.h "loudness_report"): 0 = off, 1 = measure every program (without a target or the
+  // limiter: measure only, the output is unchanged)
+  int loudness_report = 0;
 };
 
 // Device-resident weights of one checkpoint on one GPU: every layout the kernels read (fp32 SIMT, bf16 / split-TF32
@@ -274,10 +277,15 @@ class Model {
   long long encoded_bytes() const;
   void fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
                      int32_t* pred_dur);
-  // Loudness of the last run's programs (kernels_loudness.cu): true if that run normalised; then last_loudness()
-  // holds 3 P floats, per program k at 3 k: integrated loudness (LUFS, NaN = undefined), true peak (dBTP), gain.
-  bool loudness_ran() const { return ran_ && loud_; }
+  // Loudness of the last run's programs (kernels_loudness.cu): true if that run normalised or reported; then
+  // last_loudness() holds 3 P floats, per program k at 3 k: integrated loudness (LUFS, NaN = undefined), true peak
+  // (dBTP), gain.
+  bool loudness_ran() const { return ran_ && (loud_ || rep_); }
   const std::vector<float>& last_loudness() const { return h_loud_; }
+  // Loudness range and maxima of the last run's programs: true if that run reported; then last_loudness_range()
+  // holds 3 P floats, per program k at 3 k: LRA (LU), max momentary and max short-term loudness (LUFS); NaN = undefined.
+  bool loudness_range_ran() const { return ran_ && rep_; }
+  const std::vector<float>& last_loudness_range() const { return h_rng_; }
   // Limiter of the last run's programs (kernels_loudness.cu): true if that run limited; then last_limiter() holds
   // 2 P floats, per program k at 2 k: the largest reduction (dB) and the output's true peak (dBTP).
   bool limiter_ran() const { return ran_ && lim_; }
@@ -318,6 +326,7 @@ class Model {
                                // resampling
     float* lim_p = nullptr;    // limiter: the detector p and the limited waveform v, both indexed like wav24
     float* lim_v = nullptr;
+    float* rng = nullptr;      // [3][P] LRA | max momentary | max short-term loudness of the loudness report
   };
   // Linear / Conv1d on the precision-critical path: split-TF32 tensor cores when precision==1 and
   // the weight has a TcW32, fp32 SIMT otherwise.  Returns true when the result went to the operand planes of `o`
@@ -407,7 +416,7 @@ class Model {
   // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC streams, their
   // per-item byte offsets (host) and the encoder's tables and scratch
   Encoding enc_ = Encoding::F32;
-  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_, wav24A_, limA_, limWavA_;
+  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_, wav24A_, limA_, limWavA_, rngA_;
   std::vector<long long> flac_off_;
   // program table of the current run (P + 1 item offsets); s24_off_ [B + 1]: each item's offset in the run's 24 kHz
   // waveform, where a program is contiguous
@@ -426,6 +435,10 @@ class Model {
   // the host copy of Run::lim's report rows (program-major)
   bool lim_ = false;
   std::vector<float> h_lim_;
+  // the loudness report of the current run (through the loudness kernels and loud_par_ as well); h_rng_ = the host
+  // copy of Run::rng (program-major)
+  bool rep_ = false;
+  std::vector<float> h_rng_;
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
   std::vector<long long> sample_off_;                                      // [P + 1] at the output rate
   int* h_pred_dur_ = nullptr; size_t h_pred_dur_cap_ = 0;                  // pinned: per-row integer durations of the last run

@@ -655,10 +655,11 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   const int K = k1 - k0;
   long long *d_p_in = nullptr, *d_p_len = nullptr, *d_p_out = nullptr;
   long long max_out = 0, max_len24 = 0;
-  // loudness normalisation and the limiter: per-program 2400-sample segment energies (offsets seg_off), true-peak and
-  // limiter scratch
+  // loudness normalisation, the limiter and the loudness report: per-program 2400-sample segment energies (offsets
+  // seg_off), true-peak, limiter and short-term energy scratch
   long long* d_seg_off = nullptr;
   float* energy = nullptr;
+  double* short_e = nullptr;
   unsigned* peak = nullptr;
   unsigned* lim_acc = nullptr;
   if (resample_ && K > 0) {
@@ -679,13 +680,14 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     upload(d_p_in, p_in.data(), K * sizeof(long long));
     upload(d_p_len, p_len.data(), K * sizeof(long long));
     upload(d_p_out, p_out.data(), K * sizeof(long long));
-    if (loud_ || lim_) {
+    if (loud_ || lim_ || rep_) {
       d_seg_off = A.alloc<long long>(K);
       energy = A.alloc<float>((size_t)std::max(nseg, 1LL));
       peak = A.alloc<unsigned>(K);
       upload(d_seg_off, seg_off.data(), K * sizeof(long long));
     }
     if (lim_) lim_acc = A.alloc<unsigned>((size_t)2 * K);
+    if (rep_) short_e = A.alloc<double>((size_t)std::max(nseg, 1LL));
   }
 
   // ---- length regulation (K4/K5)
@@ -895,10 +897,16 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   const int P = n_prog();
   float* gain = nullptr;
   const float* wav = r.wav24;
-  if (loud_ || lim_) {   // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
+  // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
+  if (loud_ || lim_ || rep_) {
     gain = r.loud + 2 * (size_t)P + k0;
     launch_loudness(r.wav24, d_p_in, d_p_len, d_seg_off, loud_par_, energy, peak, r.loud + k0, r.loud + P + k0, gain,
                     K, max_len24, st, lim_ ? r.lim_p : nullptr);
+  }
+  if (rep_) {   // the report on the same energies, before the limiter (r.rng = LRA | max momentary | max short-term)
+    launch_loudness_range(d_p_len, d_seg_off, energy, short_e, r.rng + k0, r.rng + P + k0, r.rng + 2 * (size_t)P + k0,
+                          K, max_len24, st);
+    if (!loud_ && !lim_) gain = nullptr;   // measure-only: the resampling pass is the plain output's arithmetic
   }
   if (lim_) {   // the limited waveform v is resampled instead, with the static trim t as its gain (r.lim = t | report)
     launch_limiter(r.wav24, r.lim_p, d_p_in, d_p_len, loud_par_, gain, r.lim_v, nullptr, lim_acc, r.lim + k0,

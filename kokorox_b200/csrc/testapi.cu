@@ -126,6 +126,34 @@ KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64
   });
 }
 
+KKX_API int kkx_test_loudness_range(int device, const float* x, int32_t B, const int64_t* lens, float* lra,
+                                    float* m_max, float* s_max) {
+  return run(device, [&] {
+    if (!x || !lens || B < 1) throw ArgError("kkx_test_loudness_range: bad argument");
+    std::vector<long long> in_off(B), in_len(B), seg_off(B);
+    long long ni = 0, nseg = 0, max_len = 0;
+    for (int b = 0; b < B; b++) {
+      if (lens[b] < 1) throw ArgError("kkx_test_loudness_range: every item needs >= 1 sample");
+      in_off[b] = ni; in_len[b] = lens[b]; seg_off[b] = nseg;
+      ni += lens[b]; nseg += lens[b] / kLoudSeg; max_len = std::max<long long>(max_len, lens[b]);
+    }
+    const LoudParams P = loudness_params(0.0, -1.0, false, true);   // measure-only
+    DevBuf dx(x, (size_t)ni * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8), dso(seg_off.data(), B * 8);
+    DevBuf de(nullptr, (size_t)std::max(nseg, 1LL) * 4), dst(nullptr, (size_t)std::max(nseg, 1LL) * 8);
+    DevBuf dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4), dq(nullptr, (size_t)B * 3 * 4);
+    float* r = dr.as<float>();
+    float* q = dq.as<float>();
+    launch_loudness(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), dso.as<long long>(), P, de.as<float>(),
+                    dp.as<unsigned>(), r, r + B, r + 2 * B, B, max_len, 0);
+    launch_loudness_range(dil.as<long long>(), dso.as<long long>(), de.as<float>(), dst.as<double>(), q, q + B,
+                          q + 2 * B, B, max_len, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    if (lra) KKX_CUDA(cudaMemcpy(lra, q, B * 4, cudaMemcpyDeviceToHost));
+    if (m_max) KKX_CUDA(cudaMemcpy(m_max, q + B, B * 4, cudaMemcpyDeviceToHost));
+    if (s_max) KKX_CUDA(cudaMemcpy(s_max, q + 2 * B, B * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
 KKX_API int kkx_test_limiter(int device, const float* x, int32_t B, const int64_t* lens, int32_t target_centi_lufs,
                              int32_t ceiling_centi_dbtp, float* gain, float* G, float* v, float* t,
                              float* max_reduction_db, float* true_peak_dbtp) {

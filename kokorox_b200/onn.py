@@ -109,6 +109,8 @@ def load_library(path: Optional[str] = None):
         lib.kkx_test_resample.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(i16), P(u8)]
         lib.kkx_last_loudness.argtypes = [vp, i32, P(f32), P(f32), P(f32)]
         lib.kkx_last_limiter.argtypes = [vp, i32, P(f32), P(f32)]
+        lib.kkx_last_loudness_range.argtypes = [vp, i32, P(f32), P(f32), P(f32)]
+        lib.kkx_test_loudness_range.argtypes = [C.c_int, P(f32), i32, P(i64), P(f32), P(f32), P(f32)]
         lib.kkx_test_limiter.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(f32), P(f32), P(f32), P(f32),
                                          P(f32)]
         lib.kkx_test_loudness_design.argtypes = [C.c_double, P(C.c_double), P(f32), i64]
@@ -551,11 +553,11 @@ class B200Koko:
         return outs
 
     def last_loudness(self):
-        """What loudness normalisation (option ``loudness_target``) measured and applied in this session's last
-        synchronous call: ``(lufs, true_peak_dbtp, gain)``, three float32 arrays in item order -- program order after
-        ``infer_programs`` -- (``lufs`` is NaN where
-        the loudness is undefined: items under 400 ms, silence).  Raises KkxError when that call ran with the option
-        off.  Coalesced and ``submit`` batches are not reported."""
+        """What loudness normalisation (option ``loudness_target``) or the loudness report (option
+        ``loudness_report``) measured and applied in this session's last synchronous call: ``(lufs, true_peak_dbtp,
+        gain)``, three float32 arrays in item order -- program order after ``infer_programs`` -- (``lufs`` is NaN where
+        the loudness is undefined: items under 400 ms, silence; ``gain`` is 1 when only measuring).  Raises KkxError
+        when that call ran with both options off.  Coalesced and ``submit`` batches are not reported."""
         self._require()
         n = max(int(self._lib.kkx_get_stat(self._ctx, b"loudness_items")), 0)
         lufs, tp, gain = (np.zeros(max(n, 1), np.float32) for _ in range(3))
@@ -573,6 +575,18 @@ class B200Koko:
         red, tp = (np.zeros(max(n, 1), np.float32) for _ in range(2))
         self._check(self._lib.kkx_last_limiter(self._ctx, n, _fp(red), _fp(tp)))
         return red[:n], tp[:n]
+
+    def last_loudness_range(self):
+        """The EBU R128 statistics the loudness report (option ``loudness_report``) measured in this session's last
+        synchronous call: ``(loudness_range_lu, max_momentary_lufs, max_short_term_lufs)``, three float32 arrays in
+        item order -- program order after ``infer_programs``.  They describe the unscaled 24 kHz waveform; NaN where
+        undefined (no whole 400 ms block, no whole 3 s window, or no window passing the gates).  Raises KkxError when
+        that call ran with the report off.  Coalesced and ``submit`` batches are not reported."""
+        self._require()
+        n = max(int(self._lib.kkx_get_stat(self._ctx, b"loudness_items")), 0)
+        lra, mm, sm = (np.zeros(max(n, 1), np.float32) for _ in range(3))
+        self._check(self._lib.kkx_last_loudness_range(self._ctx, n, _fp(lra), _fp(mm), _fp(sm)))
+        return lra[:n], mm[:n], sm[:n]
 
     # -- device-resident path (bench `value`) ---------------------------------------------
     def stage(self, tokens, styles, speeds) -> None:
