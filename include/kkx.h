@@ -224,7 +224,8 @@ KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes);
  *   program); encoding outside 0..4.
  *   Not provided: pauses, cross-fades or silence trimming at the joins (the reference joins chunks as they are);
  *   programs through kkx_infer, coalescing, kkx_submit, kkx_infer_batch_voices or kkx_run_staged; a "max_tokens" split
- *   of a program call; streaming a program before its last item is done; MP3 or Opus. */
+ *   of a program call; streaming a program before its last item is done; Opus.  MP3 programs: kkx_infer_programs_mp3
+ *   (the bitrate does not fit in the encoding code). */
 #define KKX_ENC_F32 0   /* f32 samples, 4 bytes each */
 #define KKX_ENC_PCM16 1
 #define KKX_ENC_ULAW 2
@@ -238,6 +239,66 @@ KKX_API int kkx_infer_programs(kkx_ctx* ctx, int32_t batch, const int64_t* token
                                int64_t* out_sample_offsets /* [n_programs + 1], nullable */,
                                int32_t* out_pred_dur /* nullable, indexed like tokens */);
 KKX_API void kkx_release_programs(kkx_ctx* ctx, void* bytes);
+
+/* kkx_infer_batch_mp3: like kkx_infer_batch_flac, but item b comes back as one MP3 file (MPEG audio Layer III,
+ *   constant bitrate): bytes [out_byte_offsets[b], out_byte_offsets[b+1]) of *out_bytes (out_byte_offsets required,
+ *   out_sample_offsets nullable).  kkx_infer_programs_mp3: kkx_infer_programs' arguments and rules with kbps in place
+ *   of encoding, one MP3 file per program.  Release either buffer with kkx_release_mp3.  Encoded on the device after
+ *   the forward pass; kkx_last_loudness, kkx_last_limiter and kkx_last_loudness_range report as after a PCM16 call.
+ *   Input: the int16 samples p[0..n) that kkx_infer_batch_pcm16 returns for the item (program) at the session's
+ *   "out_rate", taken as p / 32768; samples outside [0, n) are zero.
+ *   Format: mono (mode 11), no CRC (protection bit 1), private / copyright / original / emphasis 0, no bit reservoir
+ *   (main_data_begin 0), long blocks only (window_switching_flag 0, block type 0), no scalefactors
+ *   (scalefac_compress 0, so every slen is 0 in MPEG-1 and LSF coding; scfsi 0, preflag 0, scalefac_scale 0), no
+ *   ID3 tag, no Xing / Info / LAME frame.  Version by "out_rate": MPEG-1 at 32000, 44100, 48000 (two granules of
+ *   576 samples a frame); MPEG-2 LSF at 16000, 22050, 24000 and MPEG-2.5 at 8000, 11025, 12000 (one granule a
+ *   frame).  MPEG-2.5 is not part of ISO/IEC 13818-3, but common decoders play it.
+ *   kbps: MPEG-1 32, 40, 48, 56, 64, 80, 96, 112, 128, 160, 192, 224, 256, 320; MPEG-2 / 2.5 8, 16, 24, 32, 40, 48,
+ *   56, 64, 80, 96, 112, 128, 144, 160; 0 = 192 at the MPEG-1 rates and 160 at the others (at the model's 24000 the
+ *   format allows at most 160).  Any other value is KKX_ERR_ARG (the message names the version and its table) with
+ *   the session left as it was, as is a null out_bytes or out_byte_offsets and, for programs, any program-table
+ *   error of kkx_infer_programs.
+ *   Frames: with A = 144000 kbps / rate (MPEG-1) or 72000 kbps / rate, frame f of a file takes bytes
+ *   [floor(f A), floor((f + 1) A)) (64-bit integers); its padding bit is its length minus floor(A).  The decoded
+ *   signal is the input delayed by D = 1057 samples (one granule of MDCT overlap, 576, plus the analysis / synthesis
+ *   filterbank, 481).  A file has F = ceil((n + D) / samples per frame) frames, so a standard decoder emits every
+ *   input sample, and floor(F A) bytes.  Granule g of a file (frame g / 2 of MPEG-1, frame g otherwise) codes the
+ *   MDCT of subband slots 18 (g - 1) .. 18 g + 17, slot s being the filterbank output over input samples
+ *   32 s - 480 .. 32 s + 31.  A granule's bit budget is min(4095, its share of the frame's main-data bits); in an
+ *   MPEG-1 frame granule 0 takes floor(half) and granule 1 the rest (granule 1's data follows granule 0's directly).
+ *   Unused bits are zero.
+ *   Analysis: the ISO 11172-3 polyphase filterbank (window C[i] of Table C.1, matrixing cos((2k + 1)(i - 16) pi / 64)),
+ *   odd samples of odd subbands negated, the 18-point MDCT of block type 0 with the sine window (scaled by 1/9, the
+ *   inverse of the standard IMDCT), the eight alias-reduction butterflies with c_i = -0.6, -0.535, -0.33, -0.185,
+ *   -0.095, -0.041, -0.0142, -0.0037.
+ *   Quantisation: ix = nint((|xr| / 2^((gg - 210) / 4))^0.75 - 0.0946), nint(v) = floor(v + 0.5).  A gg fits when
+ *   no ix exceeds 8206 (15 + 2^13 - 1) and the granule's part2_3_length (below) is within its budget.  gg is found by
+ *   lo = 0, hi = 255; while lo < hi { mid = (lo + hi) / 2; if fits(mid) hi = mid else lo = mid + 1 } -- written
+ *   down so that every implementation takes the same steps where the bit count is not monotone.  There is no
+ *   psychoacoustic model: the quantisation noise is white across the spectrum; the tests pin the signal-to-noise
+ *   ratio of decoded speech per rate.
+ *   Regions: strip trailing zero pairs; then take quadruples whose values are all <= 1 into count1, from the top
+ *   down; big_values is what remains (in pairs).  One Huffman table for all three big_values regions: among the
+ *   tables whose range covers the largest value there (table 0 when it is 0; for tables 16..31 the linbits decide),
+ *   the one with the fewest bits, ties to the lowest number.  region0_count 7, region1_count 7.  Count1 uses the
+ *   cheaper of tables A and B, ties to A.  part2_3_length = the bits of the codes, linbits and sign bits.
+ *   Purity and identity as for FLAC programs: a file's bytes are a function of its samples alone (batch, position,
+ *   frame groups and other programs do not matter), a one-item program returns exactly the kkx_infer_batch_mp3 bytes
+ *   of that item, and no floating-point atomics or launch-shape-dependent results enter.
+ *   Not provided: VBR or ABR, the bit reservoir, a psychoacoustic model, short blocks, scalefactors, per-region
+ *   Huffman tables, the Xing / LAME tag (encoder delay for gapless playback), ID3, CRC, Opus, a "max_tokens" split. */
+KKX_API int kkx_infer_batch_mp3(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                                const float* styles, const float* speeds, int32_t kbps, uint8_t** out_bytes,
+                                int64_t* out_byte_offsets /* [batch + 1], required */,
+                                int64_t* out_sample_offsets /* [batch + 1], nullable */, int32_t* out_pred_dur);
+KKX_API int kkx_infer_programs_mp3(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
+                                   const float* styles, const float* speeds,
+                                   int32_t n_programs, const int32_t* program_offsets /* [n_programs + 1] */,
+                                   int32_t kbps, uint8_t** out_bytes,
+                                   int64_t* out_byte_offsets /* [n_programs + 1], required */,
+                                   int64_t* out_sample_offsets /* [n_programs + 1], nullable */,
+                                   int32_t* out_pred_dur /* nullable, indexed like tokens */);
+KKX_API void kkx_release_mp3(kkx_ctx* ctx, uint8_t* bytes);
 
 /* ---- output containers (host-side byte work after the pcm16 / f32 result; no GPU involved, no ctx needed).
  * kkx_wav_header_pcm16: the 44-byte RIFF/WAVE header of the WebSocket server's `encode_audio`

@@ -130,6 +130,16 @@ KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64
  * and their offsets into byte_offsets [B + 1]; returns the total byte count or < 0. */
 KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
                               uint8_t* dst, int64_t capacity, int64_t* byte_offsets);
+/* MP3 encoder (kernels_mp3.cu) on caller-supplied PCM, like kkx_test_flac: kbps as in kkx_infer_batch_mp3 (0 = the
+ * default of the rate's version).  Returns the total byte count or < 0. */
+KKX_API int64_t kkx_test_mp3(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate, int32_t kbps,
+                             uint8_t* dst, int64_t capacity, int64_t* byte_offsets);
+/* Host only: the MP3 encoder's tables.  Huffman table t (0..31): the pair (x, y) at codes / lens
+ * [t * 256 + x * xlen[t] + y] (len 0: no entry), xlen [32] (0: no such table), linbits [32], the count1 tables A and B at c1_codes / c1_lens
+ * [k * 16 + 8v + 4w + 2x + y], and the 512-tap analysis window C[i] of ISO 11172-3 Table C.1.  Any pointer may be
+ * null.  Returns 0. */
+KKX_API int kkx_test_mp3_tables(uint32_t* codes, uint8_t* lens, int32_t* xlen, int32_t* linbits, uint32_t* c1_codes,
+                                uint8_t* c1_lens, double* window);
 /* Loudness normalisation (kernels_loudness.cu, kkx.h "loudness_target").
  * kkx_test_loudness_design: host only -- the K-weighting biquads the library designs in double for sample rate fs
  *   (kweight[10], nullable: shelf b0 b1 b2 a1 a2, then high-pass b0 b1 b2 a1 a2; a0 = 1) and the fp32 taps of the

@@ -345,6 +345,37 @@ bool flac_rate_ok(int rate);
 void launch_flac(const short* pcm, const long long* soff, const int* foff, int B, int F, int rate, void* work,
                  unsigned char* out, long long* item_off, cudaStream_t st);
 
+// Constant-bitrate MPEG audio Layer III of 16-bit mono PCM (kernels_mp3.cu; the stream rules are in kkx.h,
+// kkx_infer_batch_mp3).  A stream of n samples has mp3_frames(fmt, n) frames; frame f of it takes bytes
+// [floor(f anum / rate), floor((f + 1) anum / rate)), so every offset is known before the encoder runs.
+struct Mp3Format {
+  int rate = 0, kbps = 0;
+  int version = 0;        // header version bits: 3 = MPEG-1, 2 = MPEG-2 (LSF), 0 = MPEG-2.5
+  int sr_index = 0, br_index = 0;
+  int ngr = 0, spf = 0;   // granules (of 576 samples) and samples per frame
+  int side = 0;           // side-information bytes (17 MPEG-1, 9 otherwise)
+  long long anum = 0;     // 144000 kbps (MPEG-1) or 72000 kbps: frame bytes A = anum / rate
+};
+// The decoded signal is the input delayed by this many samples: one granule (the MDCT overlap) plus the analysis /
+// synthesis filterbank pair (512 - 31).
+constexpr int kMp3Delay = 576 + 481;
+// The format of (rate, kbps); kbps 0 = 192 at the MPEG-1 rates, 160 otherwise.  Throws ArgError naming the version
+// and its bitrate table for any other value, and for a rate that is not an "out_rate" value.
+Mp3Format mp3_format(int rate, int kbps);
+long long mp3_frames(const Mp3Format& fmt, long long n);        // ceil((n + kMp3Delay) / spf)
+long long mp3_bytes(const Mp3Format& fmt, long long frames);    // floor(frames anum / rate)
+// The analysis constants (window, matrixing and MDCT cosines, butterflies) as mp3_const_bytes() bytes, built on the
+// host in double precision; launch_mp3 reads them from device memory.
+size_t mp3_const_bytes();
+void mp3_consts(void* host_dst);
+// Item b is pcm[soff[b] .. soff[b + 1]) (>= 1 sample), frames [foff[b], foff[b + 1]) of F, bytes
+// [boff[b], boff[b + 1]) of out (boff [B + 1] = prefix of mp3_bytes).  One launch, profile name "mp3_encode".
+void launch_mp3(const short* pcm, const long long* soff, const int* foff, const long long* boff, int B, int F,
+                const Mp3Format& fmt, const void* consts, unsigned char* out, cudaStream_t st);
+// Host copies of the library's Huffman tables and analysis window (kkx_test_mp3_tables)
+void mp3_tables(uint32_t* codes, uint8_t* lens, int32_t* xlen, int32_t* linbits, uint32_t* c1_codes, uint8_t* c1_lens,
+                double* window);
+
 // mix_styles (koko.rs:1255-1306) on a device-resident voice table [V][511][256]
 void launch_mix_styles(const float* table, const int* mix_off, const int* voice_ids, const float* portions,
                        const int* rows, float* styles, int B, cudaStream_t st);

@@ -10,6 +10,7 @@
 //                 the header and CRC-16 of the frame, then the frame's bytes; the CTA of an item's first frame also
 //                 writes the item's 42-byte head (STREAMINFO needs the item's smallest and largest frame).
 #include "kernels.h"
+#include "bitpack.cuh"
 
 namespace kkx {
 
@@ -29,16 +30,6 @@ struct FlacFrame {        // analysis result of one frame
   int kind, order, porder;
   unsigned char k[kParts];  // Rice parameter of each partition (FIXED)
 };
-
-// item b owns frames [foff[b], foff[b + 1]); the last b with foff[b] <= f
-__device__ __forceinline__ int frame_item(const int* foff, int B, int f) {
-  int lo = 0, hi = B - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (__ldg(foff + mid) <= f) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
 
 __host__ __device__ inline int utf8_len(unsigned v) {
   return v < 0x80 ? 1 : v < 0x800 ? 2 : v < 0x10000 ? 3 : v < 0x200000 ? 4 : v < 0x4000000 ? 5 : 6;
@@ -278,17 +269,6 @@ __global__ void __launch_bounds__(1024) flac_scan_kernel(const FlacFrame* __rest
 }
 
 // ---------------------------------------------------------------------------------------------- packing
-// MSB-first bit buffer in 32-bit words: stream bit i is bit 31 - (i & 31) of word i >> 5.  nbits <= 32.
-__device__ __forceinline__ void put_bits(unsigned* buf, int pos, unsigned v, int nbits) {
-  if (nbits <= 0) return;
-  const unsigned long long w = (unsigned long long)v << (64 - nbits - (pos & 31));
-  const unsigned hi = (unsigned)(w >> 32), lo = (unsigned)w;
-  if (hi) atomicOr(buf + (pos >> 5), hi);
-  if (lo) atomicOr(buf + (pos >> 5) + 1, lo);
-}
-__device__ __forceinline__ unsigned get_byte(const unsigned* buf, int i) {
-  return (buf[i >> 2] >> (24 - 8 * (i & 3))) & 0xFFu;
-}
 // CRC-16 (poly 0x8005, init 0, unreflected, no final xor) is linear: crc(A || B) = crc(A) * x^(8 |B|) ^ crc(B).
 __device__ __forceinline__ unsigned crc16_mulmod(unsigned a, unsigned b) {   // a * b mod (x^16 + 0x8005)
   unsigned r = 0;

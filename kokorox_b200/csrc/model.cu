@@ -776,7 +776,7 @@ long long bytes_per_sample(Encoding e) {
 
 long long Model::encoded_bytes() const {
   if (!ran_) return 0;
-  return enc_ == Encoding::FLAC ? flac_off_[n_prog()] : total_samples_ * bytes_per_sample(enc_);
+  return is_stream(enc_) ? stream_off_[n_prog()] : total_samples_ * bytes_per_sample(enc_);
 }
 
 void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
@@ -785,11 +785,11 @@ void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_off
   fetch(nullptr, 0, sample_offsets, pred_dur);
   if (byte_offsets)
     for (int k = 0; k <= n_prog(); k++)
-      byte_offsets[k] = enc_ == Encoding::FLAC ? flac_off_[k] : sample_off_[k] * bytes_per_sample(enc_);
+      byte_offsets[k] = is_stream(enc_) ? stream_off_[k] : sample_off_[k] * bytes_per_sample(enc_);
   if (dst) {
     const long long n = encoded_bytes();
     if (capacity_bytes < n) throw ArgError("output buffer too small");
-    const void* src = enc_ == Encoding::FLAC ? flacA_.base() : enc_ == Encoding::F32 ? audioA_.base() : twinA_.base();
+    const void* src = is_stream(enc_) ? streamA_.base() : enc_ == Encoding::F32 ? audioA_.base() : twinA_.base();
     KKX_CUDA(cudaMemcpyAsync(dst, src, (size_t)n, cudaMemcpyDeviceToHost, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
   }
@@ -847,9 +847,10 @@ void Model::grow(Arena& a, size_t bytes) {
 }
 
 // ============================================================================ forward
-void Model::run(Encoding enc, const std::vector<int>& programs) {
+void Model::run(Encoding enc, const std::vector<int>& programs, int kbps) {
   if (!staged_ || B_ <= 0) throw StateError("no batch staged");
   if (!programs.empty()) check_programs(B_, (int)programs.size() - 1, programs.data());
+  const Mp3Format mp3 = enc == Encoding::MP3 ? mp3_format(opt.out_rate, kbps) : Mp3Format();
   KKX_CUDA(cudaSetDevice(device_));
   ran_ = false;
   enc_ = enc;
@@ -930,30 +931,42 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
     r.lim_p = limWavA_.alloc<float>(s24_off_[B_]);
     r.lim_v = limWavA_.alloc<float>(s24_off_[B_]);
   }
-  // FLAC: the encoder's tables -- sample offsets, frames per program (4096 samples each) as a prefix, program byte
-  // offsets -- and its output, ready before the forward pass so that the encoder follows it without a host round trip
+  // FLAC / MP3: the encoder's tables -- sample offsets, frames per program (4096 samples each for FLAC, closed form
+  // for MP3) as a prefix, program byte offsets (MP3: known here; FLAC: found by the encoder) -- and its output, ready
+  // before the forward pass so that the encoder follows it without a host round trip
   struct { int F = 0; long long *soff = nullptr, *ioff = nullptr; int* foff = nullptr; void* work = nullptr;
            unsigned char* out = nullptr; } fl;
-  if (enc == Encoding::FLAC) {
+  if (is_stream(enc)) {
+    const bool flac = enc == Encoding::FLAC;
     std::vector<int> foff(P + 1, 0);
+    std::vector<long long> boff(P + 1, 0);
     for (int k = 0; k < P; k++) {
       const long long n = sample_off_[k + 1] - sample_off_[k];
-      if (n > kMaxFlacSamples) throw ArgError("program too long for one FLAC stream (2^36 - 1 samples at most)");
-      const long long nf = flac_frames(n);
-      if (foff[k] + nf > 0x7FFFFFFFLL) throw ArgError("batch too long for one FLAC encode");
+      if (flac && n > kMaxFlacSamples) throw ArgError("program too long for one FLAC stream (2^36 - 1 samples at most)");
+      const long long nf = flac ? flac_frames(n) : mp3_frames(mp3, n);
+      if (foff[k] + nf > 0x7FFFFFFFLL) throw ArgError(flac ? "batch too long for one FLAC encode" : "batch too long for one MP3 encode");
       foff[k + 1] = foff[k] + (int)nf;
+      if (!flac) boff[k + 1] = boff[k] + mp3_bytes(mp3, nf);
     }
     fl.F = foff[P];
-    const size_t bound = (size_t)flac_bound(P, fl.F, total_samples_);
-    grow(flacA_, bound);
-    fl.out = flacA_.alloc<unsigned char>(bound);
-    grow(flacTabA_, 3 * ((size_t)(P + 1) * sizeof(long long) + 256) + flac_work_bytes(fl.F));
-    fl.soff = flacTabA_.alloc<long long>(P + 1);
-    fl.foff = flacTabA_.alloc<int>(P + 1);
-    fl.ioff = flacTabA_.alloc<long long>(P + 1);
-    fl.work = flacTabA_.alloc_bytes(flac_work_bytes(fl.F));
+    const size_t bound = flac ? (size_t)flac_bound(P, fl.F, total_samples_) : (size_t)boff[P];
+    const size_t work = flac ? flac_work_bytes(fl.F) : mp3_const_bytes();
+    grow(streamA_, bound);
+    fl.out = streamA_.alloc<unsigned char>(bound);
+    grow(streamTabA_, 3 * ((size_t)(P + 1) * sizeof(long long) + 256) + work);
+    fl.soff = streamTabA_.alloc<long long>(P + 1);
+    fl.foff = streamTabA_.alloc<int>(P + 1);
+    fl.ioff = streamTabA_.alloc<long long>(P + 1);
+    fl.work = streamTabA_.alloc_bytes(work);
     upload(fl.soff, sample_off_.data(), (size_t)(P + 1) * sizeof(long long));
     upload(fl.foff, foff.data(), (size_t)(P + 1) * sizeof(int));
+    if (!flac) {
+      std::vector<unsigned char> consts(work);
+      mp3_consts(consts.data());
+      upload(fl.ioff, boff.data(), (size_t)(P + 1) * sizeof(long long));
+      upload(fl.work, consts.data(), work);
+      stream_off_ = boff;
+    }
   }
   h_loud_.clear();
   h_lim_.clear();
@@ -1004,10 +1017,12 @@ void Model::run(Encoding enc, const std::vector<int>& programs) {
     if (enc == Encoding::FLAC) {
       launch_flac(static_cast<const short*>(r.twin), fl.soff, fl.foff, P, fl.F, opt.out_rate, fl.work, fl.out, fl.ioff,
                   stream_);
-      flac_off_.assign(P + 1, 0);
-      KKX_CUDA(cudaMemcpyAsync(flac_off_.data(), fl.ioff, (size_t)(P + 1) * sizeof(long long),
+      stream_off_.assign(P + 1, 0);
+      KKX_CUDA(cudaMemcpyAsync(stream_off_.data(), fl.ioff, (size_t)(P + 1) * sizeof(long long),
                                cudaMemcpyDeviceToHost, stream_));
     }
+    if (enc == Encoding::MP3)
+      launch_mp3(static_cast<const short*>(r.twin), fl.soff, fl.foff, fl.ioff, P, fl.F, mp3, fl.work, fl.out, stream_);
     KKX_CUDA(cudaStreamSynchronize(stream_));
     if (sink) { KKX_CUDA(cudaStreamSynchronize(copy_stream_)); sink_filled_ = true; }
     if (loud_ || rep_) {   // [3][P] on the device -> program-major on the host

@@ -242,8 +242,9 @@ struct ConvOpt {
 };
 
 // What a run returns besides the f32 waveform, which every run writes: its 16-bit PCM twin, the G.711 codes of that
-// PCM (mu-law / A-law), or one FLAC stream per item encoded from it (kkx.h).
-enum class Encoding { F32, PCM16, ULAW, ALAW, FLAC };
+// PCM (mu-law / A-law), or one FLAC or MP3 stream per item encoded from it (kkx.h).
+enum class Encoding { F32, PCM16, ULAW, ALAW, FLAC, MP3 };
+inline bool is_stream(Encoding e) { return e == Encoding::FLAC || e == Encoding::MP3; }
 
 class Model {
  public:
@@ -264,16 +265,17 @@ class Model {
   // soon as the group's iSTFT is done, overlapping the device->host copy with the next group's kernels.
   std::function<float*(long long)> host_sink;
   bool sink_filled() const { return sink_filled_; }
-  // A FLAC run launches the encoder (kernels_flac.cu) after the forward pass: gpu_us does not include it.
+  // A FLAC or MP3 run launches the encoder (kernels_flac.cu, kernels_mp3.cu) after the forward pass: gpu_us does not
+  // include it.  kbps: the MP3 bitrate (mp3_format; 0 = the default), ignored by the other encodings.
   // programs: the run's program table (check_programs, P + 1 item offsets); every output -- sample offsets, the
   // encoded bytes, FLAC streams, loudness -- is per program, a program being one utterance whose 24 kHz waveform is
   // the concatenation of its items' (kkx.h, kkx_infer_programs).  Empty = one item per program.
-  void run(Encoding enc = Encoding::F32, const std::vector<int>& programs = {});
+  void run(Encoding enc = Encoding::F32, const std::vector<int>& programs = {}, int kbps = 0);
   long long total_samples() const { return total_samples_; }
   // The f32 waveform of the last run, whatever its encoding; sample_offsets [P + 1] per program.
   void fetch(float* dst, long long capacity, int64_t* sample_offsets, int32_t* pred_dur);
-  // The output of the last run in its encoding: 4 bytes per sample for F32, 2 for PCM16, 1 for G.711, the FLAC
-  // streams back to back.  byte_offsets [P + 1] locate each program's bytes.
+  // The output of the last run in its encoding: 4 bytes per sample for F32, 2 for PCM16, 1 for G.711, the FLAC or
+  // MP3 streams back to back.  byte_offsets [P + 1] locate each program's bytes.
   long long encoded_bytes() const;
   void fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
                      int32_t* pred_dur);
@@ -319,7 +321,7 @@ class Model {
     std::vector<int> T;        // frames per item (host)
     Level styL;                // one item of B rows (style FC GEMMs)
     float* audio = nullptr;    // [total_samples_] the f32 waveform at the output rate
-    void* twin = nullptr;      // its 16-bit PCM (PCM16, FLAC) or G.711 (ULAW, ALAW) twin
+    void* twin = nullptr;      // its 16-bit PCM (PCM16, FLAC, MP3) or G.711 (ULAW, ALAW) twin
     float* loud = nullptr;     // [3][P] lufs | dBTP | gain of loudness normalisation; the gain feeds the resampling
     float* wav24 = nullptr;    // resampling pass only: the run's 24 kHz waveform, item b at s24_off_[b]
     float* lim = nullptr;      // [3][P] t | max reduction (dB) | output true peak (dBTP) of the limiter; t feeds the
@@ -413,11 +415,11 @@ class Model {
   std::vector<int> tok_len_;
   int* d_ids_ = nullptr; float* d_styles_ = nullptr; float* d_speeds_ = nullptr;
   Level tokL_;
-  // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC streams, their
-  // per-item byte offsets (host) and the encoder's tables and scratch
+  // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC or MP3 streams, their
+  // per-program byte offsets (host) and the encoder's tables and scratch
   Encoding enc_ = Encoding::F32;
-  Arena audioA_, twinA_, loudA_, flacA_, flacTabA_, wav24A_, limA_, limWavA_, rngA_;
-  std::vector<long long> flac_off_;
+  Arena audioA_, twinA_, loudA_, streamA_, streamTabA_, wav24A_, limA_, limWavA_, rngA_;
+  std::vector<long long> stream_off_;
   // program table of the current run (P + 1 item offsets); s24_off_ [B + 1]: each item's offset in the run's 24 kHz
   // waveform, where a program is contiguous
   std::vector<int> prog_;

@@ -887,7 +887,7 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   }
   capture("conv_post", cp, 24, 0, 22, G120, b0);
   const bool law = enc_ == Encoding::ULAW || enc_ == Encoding::ALAW;
-  short* pcm = enc_ == Encoding::PCM16 || enc_ == Encoding::FLAC ? static_cast<short*>(r.twin) : nullptr;
+  short* pcm = enc_ == Encoding::PCM16 || is_stream(enc_) ? static_cast<short*>(r.twin) : nullptr;
   if (!resample_) {   // the output is the 24 kHz waveform: program layout == item layout
     launch_istft(cp, 24, G120.d_off, G120.d_len, r.audio, pcm, d_s24, opt.precision == 1, B, G120.max_len, st);
     return;

@@ -218,6 +218,45 @@ KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const i
   return rc == KKX_OK ? (int64_t)total : (int64_t)rc;
 }
 
+KKX_API int64_t kkx_test_mp3(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate, int32_t kbps,
+                             uint8_t* dst, int64_t capacity, int64_t* byte_offsets) {
+  long long total = 0;
+  const int rc = run(device, [&] {
+    if (!pcm || !lens || !byte_offsets || B < 1) throw ArgError("kkx_test_mp3: bad argument");
+    const Mp3Format fmt = mp3_format(rate, kbps);
+    std::vector<long long> soff(B + 1, 0), boff(B + 1, 0);
+    std::vector<int> foff(B + 1, 0);
+    for (int b = 0; b < B; b++) {
+      if (lens[b] < 1) throw ArgError("kkx_test_mp3: every item needs >= 1 sample");
+      soff[b + 1] = soff[b] + lens[b];
+      const long long nf = mp3_frames(fmt, lens[b]);
+      foff[b + 1] = foff[b] + (int)nf;
+      boff[b + 1] = boff[b] + mp3_bytes(fmt, nf);
+    }
+    std::vector<unsigned char> consts(mp3_const_bytes());
+    mp3_consts(consts.data());
+    DevBuf dp(pcm, (size_t)soff[B] * 2), ds(soff.data(), (B + 1) * 8), df(foff.data(), (B + 1) * 4);
+    DevBuf db(boff.data(), (B + 1) * 8), dc(consts.data(), consts.size()), dout(nullptr, (size_t)boff[B]);
+    launch_mp3(dp.as<short>(), ds.as<long long>(), df.as<int>(), db.as<long long>(), B, foff[B], fmt, dc.p,
+               dout.as<unsigned char>(), 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    for (int b = 0; b <= B; b++) byte_offsets[b] = boff[b];
+    total = boff[B];
+    if (dst) {
+      if (capacity < total) throw ArgError("kkx_test_mp3: dst too small");
+      KKX_CUDA(cudaMemcpy(dst, dout.p, (size_t)total, cudaMemcpyDeviceToHost));
+    }
+  });
+  if (rc != KKX_OK) return rc;
+  return (int64_t)total;
+}
+
+KKX_API int kkx_test_mp3_tables(uint32_t* codes, uint8_t* lens, int32_t* xlen, int32_t* linbits, uint32_t* c1_codes,
+                                uint8_t* c1_lens, double* window) {
+  mp3_tables(codes, lens, xlen, linbits, c1_codes, c1_lens, window);
+  return KKX_OK;
+}
+
 KKX_API int kkx_test_conv(int device, const float* in, int rows_in, int ldi, int Ci, const float* w,
                           const float* bias, int Co, int ks, int dil, int pad, int stride,
                           const float* pscale, const float* pshift, int pact, float pslope,

@@ -78,6 +78,12 @@ def load_library(path: Optional[str] = None):
                                            P(i64), P(i32)]
         lib.kkx_release_programs.argtypes = [vp, vp]
         lib.kkx_release_programs.restype = None
+        lib.kkx_infer_batch_mp3.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), i32, P(P(u8)), P(i64), P(i64),
+                                            P(i32)]
+        lib.kkx_infer_programs_mp3.argtypes = [vp, i32, P(i64), P(i32), P(f32), P(f32), i32, P(i32), i32, P(P(u8)),
+                                               P(i64), P(i64), P(i32)]
+        lib.kkx_release_mp3.argtypes = [vp, P(u8)]
+        lib.kkx_release_mp3.restype = None
         lib.kkx_wav_header_pcm16.argtypes = [P(C.c_uint8), i64, i32]
         lib.kkx_wav_header_f32_stream.argtypes = [P(C.c_uint8), i32, i32]
         lib.kkx_encode_wav16_base64.argtypes = [P(i16), i64, i32, C.c_char_p, i64]
@@ -118,6 +124,10 @@ def load_library(path: Optional[str] = None):
         lib.kkx_test_loudness.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(f32), P(f32)]
         lib.kkx_test_flac.argtypes = [C.c_int, P(i16), i32, P(i64), i32, P(u8), i64, P(i64)]
         lib.kkx_test_flac.restype = i64
+        lib.kkx_test_mp3.argtypes = [C.c_int, P(i16), i32, P(i64), i32, i32, P(u8), i64, P(i64)]
+        lib.kkx_test_mp3.restype = i64
+        lib.kkx_test_mp3_tables.argtypes = [P(C.c_uint32), P(u8), P(i32), P(i32), P(C.c_uint32), P(u8),
+                                            P(C.c_double)]
         lib.kkx_test_attention_batch.argtypes = [C.c_int, P(f32), C.c_int, P(i32), P(i32), C.c_int, C.c_int, P(f32)]
         lib.kkx_debug_stage.argtypes = [vp, C.c_char_p, i32, P(f32), i64, P(i64), P(i64)]
         lib.kkx_debug_stage.restype = i64
@@ -529,7 +539,8 @@ class B200Koko:
         per program."""
         self._require()
         if encoding not in self._ENCODINGS:
-            raise KkxError(-1, f"encoding must be one of {sorted(self._ENCODINGS)}, got {encoding!r}")
+            hint = " (MP3: infer_programs_mp3)" if encoding == "mp3" else ""
+            raise KkxError(-1, f"encoding must be one of {sorted(self._ENCODINGS)}, got {encoding!r}{hint}")
         code, ctype = self._ENCODINGS[encoding]
         B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
         prog = np.ascontiguousarray(np.asarray(program_offsets, dtype=np.int32).reshape(-1))
@@ -548,6 +559,51 @@ class B200Koko:
                 self._lib.kkx_release_programs(self._ctx, buf)
         else:
             outs = self._adopt(C.cast(buf, C.POINTER(ctype)), boff // C.sizeof(ctype))
+        if return_durations:
+            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
+        return outs
+
+    def infer_batch_mp3(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float], kbps: int = 0,
+                        return_durations: bool = False):
+        """Like infer_batch_flac, but item b comes back as one constant-bitrate MP3 file (``bytes``, Content-Type
+        audio/mpeg) of the int16 samples infer_batch_pcm16 returns, at the session's ``out_rate``, encoded on the
+        device.  ``kbps`` is a Layer III bitrate of the rate's MPEG version, 0 = 192 at 32 / 44.1 / 48 kHz and 160
+        at the other rates (kkx.h kkx_infer_batch_mp3)."""
+        self._require()
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
+        buf = C.POINTER(C.c_uint8)()
+        boff = np.zeros(B + 1, dtype=np.int64)
+        dur = np.zeros(int(offs[-1]), dtype=np.int32)
+        self._check(self._lib.kkx_infer_batch_mp3(
+            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
+            _fp(st), _fp(sp), int(kbps), C.byref(buf), boff.ctypes.data_as(C.POINTER(C.c_int64)), None,
+            dur.ctypes.data_as(C.POINTER(C.c_int32))))
+        try:
+            outs = [C.string_at(C.addressof(buf.contents) + int(boff[b]), int(boff[b + 1] - boff[b])) for b in range(B)]
+        finally:
+            self._lib.kkx_release_mp3(self._ctx, buf)
+        if return_durations:
+            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
+        return outs
+
+    def infer_programs_mp3(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
+                           program_offsets: Sequence[int], kbps: int = 0, return_durations: bool = False):
+        """infer_programs with one MP3 file (``bytes``) per program, under the rules of infer_batch_mp3."""
+        self._require()
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
+        prog = np.ascontiguousarray(np.asarray(program_offsets, dtype=np.int32).reshape(-1))
+        P = max(prog.size - 1, 0)
+        buf = C.POINTER(C.c_uint8)()
+        boff = np.zeros(P + 1, dtype=np.int64)
+        dur = np.zeros(int(offs[-1]), dtype=np.int32)
+        self._check(self._lib.kkx_infer_programs_mp3(
+            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
+            _fp(st), _fp(sp), P, prog.ctypes.data_as(C.POINTER(C.c_int32)), int(kbps), C.byref(buf),
+            boff.ctypes.data_as(C.POINTER(C.c_int64)), None, dur.ctypes.data_as(C.POINTER(C.c_int32))))
+        try:
+            outs = [C.string_at(C.addressof(buf.contents) + int(boff[k]), int(boff[k + 1] - boff[k])) for k in range(P)]
+        finally:
+            self._lib.kkx_release_mp3(self._ctx, buf)
         if return_durations:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
