@@ -9,6 +9,7 @@
 #include <condition_variable>
 #include <cstring>
 #include <deque>
+#include <initializer_list>
 #include <mutex>
 #include <map>
 #include <numeric>
@@ -64,18 +65,12 @@ struct kkx_ctx {
   std::atomic<int> async_batch{64};      // most requests the worker merges into one ragged batch
   int64_t async_batches = 0, async_requests = 0;
 
-  // Loudness report of the last synchronous call (kkx_last_loudness), guarded by `mu`: 3 floats per item (LUFS, dBTP,
-  // gain), appended pass by pass; valid once the call has succeeded, `measured` if its runs had "loudness_target" or
-  // "loudness_report" on.
-  std::vector<float> loud;
-  bool loud_valid = false, loud_measured = false;
-  // Limiter report of the same call (kkx_last_limiter), kept alongside: 2 floats per item (max reduction dB, dBTP).
-  std::vector<float> lim;
-  bool lim_ran = false;
-  // Loudness range report of the same call (kkx_last_loudness_range): 3 floats per item (LRA, max momentary, max
-  // short-term).
-  std::vector<float> rng;
-  bool rng_ran = false;
+  // Per-item report of the last synchronous call (kkx_last_loudness / _limiter / _loudness_range), guarded by `mu`:
+  // kReportRows floats per item (output.h), appended pass by pass; `groups` = the row groups its runs produced, valid
+  // once the call has succeeded.
+  std::vector<float> report;
+  unsigned report_groups = 0;
+  bool report_valid = false;
 };
 
 static thread_local std::string g_err;
@@ -244,25 +239,19 @@ KKX_API void kkx_release(kkx_ctx* ctx, float* audio);
 // kkx_last_loudness / kkx_last_limiter / kkx_last_loudness_range bookkeeping of a synchronous call (caller holds
 // ctx->mu): begin, one note per model run, done.  Coalesced and asynchronous batches leave the reports alone.
 static void loud_begin(kkx_ctx* ctx) {
-  ctx->loud.clear(); ctx->loud_valid = false; ctx->loud_measured = false;
-  ctx->lim.clear(); ctx->lim_ran = false;
-  ctx->rng.clear(); ctx->rng_ran = false;
+  ctx->report.clear(); ctx->report_groups = 0; ctx->report_valid = false;
 }
 static void loud_note(kkx_ctx* ctx) {
   const Model& m = *ctx->model;
-  if (m.limiter_ran()) {
-    ctx->lim_ran = true;
-    ctx->lim.insert(ctx->lim.end(), m.last_limiter().begin(), m.last_limiter().end());
-  }
-  if (m.loudness_range_ran()) {
-    ctx->rng_ran = true;
-    ctx->rng.insert(ctx->rng.end(), m.last_loudness_range().begin(), m.last_loudness_range().end());
-  }
-  if (!m.loudness_ran()) return;
-  ctx->loud_measured = true;
-  ctx->loud.insert(ctx->loud.end(), m.last_loudness().begin(), m.last_loudness().end());
+  if (!m.report_groups()) return;
+  ctx->report_groups |= m.report_groups();
+  ctx->report.insert(ctx->report.end(), m.last_report().begin(), m.last_report().end());
 }
-static void loud_done(kkx_ctx* ctx) { ctx->loud_valid = true; }
+static void loud_done(kkx_ctx* ctx) { ctx->report_valid = true; }
+// items of the last synchronous call's report with row group `group`, 0 without one
+static int64_t report_items(const kkx_ctx* ctx, unsigned group) {
+  return ctx->report_valid && (ctx->report_groups & group) ? (int64_t)(ctx->report.size() / kReportRows) : 0;
+}
 
 // The argument contract of one utterance (kkx.h): checked before a request is queued anywhere.
 static int validate_request(const int64_t* tokens, int32_t n_tokens, const float* style256, float speed) {
@@ -957,10 +946,10 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   if (k == "out_rate") return ctx->model->opt.out_rate;
   if (k == "loudness_target") return ctx->model->opt.loudness_target;
   if (k == "true_peak_max") return ctx->model->opt.true_peak_max;
-  if (k == "loudness_items") return ctx->loud_valid && ctx->loud_measured ? (int64_t)(ctx->loud.size() / 3) : 0;
+  if (k == "loudness_items") return report_items(ctx, kRepLoudness);
   if (k == "limiter") return ctx->model->opt.limiter;
   if (k == "loudness_report") return ctx->model->opt.loudness_report;
-  if (k == "limiter_items") return ctx->loud_valid && ctx->lim_ran ? (int64_t)(ctx->lim.size() / 2) : 0;
+  if (k == "limiter_items") return report_items(ctx, kRepLimiter);
   if (k == "coalesced_batches") return ctx->coalesced_batches;
   if (k == "coalesced_requests") return ctx->coalesced_requests;
   if (k == "coalesced_largest") return ctx->coalesced_largest;
@@ -982,59 +971,43 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   return -1;
 }
 
-KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* true_peak_dbtp, float* gain) {
+// Row group `group` of the last synchronous call's report: per item b, rows row0, row0 + 1, ... into cols[0], cols[1],
+// ... (null columns are skipped).  `off`: the error when that call did not produce the group.
+static int last_report(kkx_ctx* ctx, int32_t batch, unsigned group, const char* off, int row0,
+                       std::initializer_list<float*> cols) {
   int rc = check_ctx(ctx);
   if (rc) return rc;
   std::lock_guard<std::mutex> lk(ctx->mu);
   return guarded(ctx, [&] {
-    if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
-    if (!ctx->loud_measured)
-      throw StateError("the last synchronous call ran with loudness normalisation and the loudness report off");
-    const int64_t n = (int64_t)(ctx->loud.size() / 3);
+    if (!ctx->report_valid) throw StateError("no synchronous call has completed on this session");
+    if (!(ctx->report_groups & group)) throw StateError(off);
+    const int64_t n = (int64_t)(ctx->report.size() / kReportRows);
     if (batch != n)
       throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
-    for (int64_t b = 0; b < n; b++) {
-      if (lufs) lufs[b] = ctx->loud[b * 3];
-      if (true_peak_dbtp) true_peak_dbtp[b] = ctx->loud[b * 3 + 1];
-      if (gain) gain[b] = ctx->loud[b * 3 + 2];
+    int row = row0;
+    for (float* c : cols) {
+      if (c)
+        for (int64_t b = 0; b < n; b++) c[b] = ctx->report[b * kReportRows + row];
+      row++;
     }
   });
 }
 
+KKX_API int kkx_last_loudness(kkx_ctx* ctx, int32_t batch, float* lufs, float* true_peak_dbtp, float* gain) {
+  return last_report(ctx, batch, kRepLoudness,
+                     "the last synchronous call ran with loudness normalisation and the loudness report off", 0,
+                     {lufs, true_peak_dbtp, gain});
+}
+
 KKX_API int kkx_last_limiter(kkx_ctx* ctx, int32_t batch, float* max_reduction_db, float* true_peak_dbtp) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
-    if (!ctx->lim_ran) throw StateError("the last synchronous call ran with the limiter off");
-    const int64_t n = (int64_t)(ctx->lim.size() / 2);
-    if (batch != n)
-      throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
-    for (int64_t b = 0; b < n; b++) {
-      if (max_reduction_db) max_reduction_db[b] = ctx->lim[b * 2];
-      if (true_peak_dbtp) true_peak_dbtp[b] = ctx->lim[b * 2 + 1];
-    }
-  });
+  return last_report(ctx, batch, kRepLimiter, "the last synchronous call ran with the limiter off", 7,
+                     {max_reduction_db, true_peak_dbtp});
 }
 
 KKX_API int kkx_last_loudness_range(kkx_ctx* ctx, int32_t batch, float* loudness_range_lu, float* max_momentary_lufs,
                                     float* max_short_term_lufs) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    if (!ctx->loud_valid) throw StateError("no synchronous call has completed on this session");
-    if (!ctx->rng_ran) throw StateError("the last synchronous call ran with the loudness report off");
-    const int64_t n = (int64_t)(ctx->rng.size() / 3);
-    if (batch != n)
-      throw ArgError("batch " + std::to_string(batch) + " does not match the last call's " + std::to_string(n) + " items");
-    for (int64_t b = 0; b < n; b++) {
-      if (loudness_range_lu) loudness_range_lu[b] = ctx->rng[b * 3];
-      if (max_momentary_lufs) max_momentary_lufs[b] = ctx->rng[b * 3 + 1];
-      if (max_short_term_lufs) max_short_term_lufs[b] = ctx->rng[b * 3 + 2];
-    }
-  });
+  return last_report(ctx, batch, kRepRange, "the last synchronous call ran with the loudness report off", 3,
+                     {loudness_range_lu, max_momentary_lufs, max_short_term_lufs});
 }
 
 KKX_API int kkx_profile_enable(kkx_ctx* ctx, int enable) {

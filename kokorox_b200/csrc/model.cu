@@ -170,7 +170,6 @@ Model::~Model() {
   if (stream_) cudaStreamSynchronize(stream_);
   if (stream2_) cudaStreamSynchronize(stream2_);
   clear_graphs();
-  if (d_taps_) cudaFree(d_taps_);
   if (d_voices_) cudaFree(d_voices_);
   if (d_noise_) cudaFree(d_noise_);
   if (h_pred_dur_) cudaFreeHost(h_pred_dur_);
@@ -768,15 +767,9 @@ void check_programs(int B, int P, const int32_t* p) {
     if (p[k + 1] <= p[k]) throw ArgError("program_offsets must be strictly increasing (no empty program)");
 }
 
-namespace {
-long long bytes_per_sample(Encoding e) {
-  return e == Encoding::F32 ? sizeof(float) : e == Encoding::ULAW || e == Encoding::ALAW ? 1 : sizeof(short);
-}
-}  // namespace
-
 long long Model::encoded_bytes() const {
   if (!ran_) return 0;
-  return is_stream(enc_) ? stream_off_[n_prog()] : total_samples_ * bytes_per_sample(enc_);
+  return is_stream(plan_.enc) ? streams_.boff[n_prog()] : total_samples_ * bytes_per_sample(plan_.enc);
 }
 
 void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
@@ -785,38 +778,13 @@ void Model::fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_off
   fetch(nullptr, 0, sample_offsets, pred_dur);
   if (byte_offsets)
     for (int k = 0; k <= n_prog(); k++)
-      byte_offsets[k] = is_stream(enc_) ? stream_off_[k] : sample_off_[k] * bytes_per_sample(enc_);
+      byte_offsets[k] = is_stream(plan_.enc) ? streams_.boff[k] : sample_off_[k] * bytes_per_sample(plan_.enc);
   if (dst) {
     const long long n = encoded_bytes();
     if (capacity_bytes < n) throw ArgError("output buffer too small");
-    const void* src = is_stream(enc_) ? streamA_.base() : enc_ == Encoding::F32 ? audioA_.base() : twinA_.base();
+    const void* src = is_stream(plan_.enc) ? out_.bytes : plan_.enc == Encoding::F32 ? out_.audio : out_.twin;
     KKX_CUDA(cudaMemcpyAsync(dst, src, (size_t)n, cudaMemcpyDeviceToHost, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
-  }
-}
-
-// The resampling pass of this run: off at 24 kHz unless G.711 codes, loudness normalisation, the limiter or the
-// loudness report are wanted (then a pass-through, U = D = 1, which applies the gain, or none when only measuring).
-// The taps live on the device per Model and are rebuilt only when the rate changes.
-void Model::prepare_resample() {
-  loud_ = opt.loudness_target != 0;
-  lim_ = opt.limiter != 0;
-  rep_ = opt.loudness_report != 0;
-  if (loud_ || lim_ || rep_)
-    loud_par_ = loudness_params(opt.loudness_target / 100.0, opt.true_peak_max / 100.0, lim_, rep_);
-  resample_ = opt.out_rate != 24000 || enc_ == Encoding::ULAW || enc_ == Encoding::ALAW || loud_ || lim_ || rep_;
-  rs_U_ = 1; rs_D_ = 1; rs_H_ = 0;
-  if (opt.out_rate == 24000) return;
-  std::vector<float> taps;
-  if (resample_design(opt.out_rate, &taps, &rs_U_, &rs_D_, &rs_H_) < 0)
-    throw ArgError("out_rate " + std::to_string(opt.out_rate) + " is not supported");
-  if (taps_rate_ != opt.out_rate) {
-    KKX_CUDA(cudaStreamSynchronize(stream_));
-    if (d_taps_) cudaFree(d_taps_);
-    d_taps_ = nullptr; taps_rate_ = 0;
-    KKX_CUDA(cudaMalloc(&d_taps_, taps.size() * sizeof(float)));
-    KKX_CUDA(cudaMemcpy(d_taps_, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice));
-    taps_rate_ = opt.out_rate;
   }
 }
 
@@ -833,27 +801,18 @@ void Model::fetch(float* dst, long long capacity, int64_t* sample_offsets, int32
   }
   if (dst) {
     if (capacity < total_samples_) throw ArgError("audio buffer too small");
-    KKX_CUDA(cudaMemcpyAsync(dst, audioA_.base(), total_samples_ * sizeof(float), cudaMemcpyDeviceToHost, stream_));
+    KKX_CUDA(cudaMemcpyAsync(dst, out_.audio, total_samples_ * sizeof(float), cudaMemcpyDeviceToHost, stream_));
     KKX_CUDA(cudaStreamSynchronize(stream_));
   }
-}
-
-// A grow-only output buffer, reset for the run; when it is too small the stream must be done with the old one.
-void Model::grow(Arena& a, size_t bytes) {
-  a.reset();
-  if (bytes <= a.capacity()) return;
-  KKX_CUDA(cudaStreamSynchronize(stream_));
-  a.reserve(bytes + bytes / 4);
 }
 
 // ============================================================================ forward
 void Model::run(Encoding enc, const std::vector<int>& programs, int kbps) {
   if (!staged_ || B_ <= 0) throw StateError("no batch staged");
   if (!programs.empty()) check_programs(B_, (int)programs.size() - 1, programs.data());
-  const Mp3Format mp3 = enc == Encoding::MP3 ? mp3_format(opt.out_rate, kbps) : Mp3Format();
   KKX_CUDA(cudaSetDevice(device_));
+  plan_ = output_plan(opt, enc, kbps, out_, stream_);   // (a rejected option or bitrate changes nothing)
   ran_ = false;
-  enc_ = enc;
   if (programs.empty()) {
     prog_.resize(B_ + 1);
     for (int b = 0; b <= B_; b++) prog_[b] = b;
@@ -862,7 +821,6 @@ void Model::run(Encoding enc, const std::vector<int>& programs, int kbps) {
   }
   const int P = n_prog();
   use_lane(0);
-  prepare_resample();
   g_launch_stats = &stats;
   stats.launches = 0;
   stats.conv_flops = 0;
@@ -901,76 +859,16 @@ void Model::run(Encoding enc, const std::vector<int>& programs, int kbps) {
   sample_off_.assign(P + 1, 0);
   for (int k = 0; k < P; k++) {
     const long long n24 = s24_off_[prog_[k + 1]] - s24_off_[prog_[k]];
-    sample_off_[k + 1] = sample_off_[k] + (n24 * rs_U_ + rs_D_ - 1) / rs_D_;
+    sample_off_[k + 1] = sample_off_[k] + plan_.out_len(n24);
   }
   total_samples_ = sample_off_[P];
   last_frames = tot;
-  grow(audioA_, (size_t)total_samples_ * sizeof(float));
-  r.audio = audioA_.alloc<float>(total_samples_);
-  if (enc != Encoding::F32) {
-    const size_t bytes = (size_t)total_samples_ * bytes_per_sample(enc);
-    grow(twinA_, bytes);
-    r.twin = twinA_.alloc_bytes(bytes);
-  }
-  if (resample_) {
-    grow(wav24A_, (size_t)s24_off_[B_] * sizeof(float));
-    r.wav24 = wav24A_.alloc<float>(s24_off_[B_]);
-  }
-  if (loud_ || lim_ || rep_) {
-    grow(loudA_, (size_t)P * 3 * sizeof(float));
-    r.loud = loudA_.alloc<float>((size_t)P * 3);
-  }
-  if (rep_) {
-    grow(rngA_, (size_t)P * 3 * sizeof(float));
-    r.rng = rngA_.alloc<float>((size_t)P * 3);
-  }
-  if (lim_) {
-    grow(limA_, (size_t)P * 3 * sizeof(float));
-    r.lim = limA_.alloc<float>((size_t)P * 3);
-    grow(limWavA_, (size_t)s24_off_[B_] * 2 * sizeof(float) + 256);   // two arrays, the second 256-byte aligned
-    r.lim_p = limWavA_.alloc<float>(s24_off_[B_]);
-    r.lim_v = limWavA_.alloc<float>(s24_off_[B_]);
-  }
-  // FLAC / MP3: the encoder's tables -- sample offsets, frames per program (4096 samples each for FLAC, closed form
-  // for MP3) as a prefix, program byte offsets (MP3: known here; FLAC: found by the encoder) -- and its output, ready
-  // before the forward pass so that the encoder follows it without a host round trip
-  struct { int F = 0; long long *soff = nullptr, *ioff = nullptr; int* foff = nullptr; void* work = nullptr;
-           unsigned char* out = nullptr; } fl;
-  if (is_stream(enc)) {
-    const bool flac = enc == Encoding::FLAC;
-    std::vector<int> foff(P + 1, 0);
-    std::vector<long long> boff(P + 1, 0);
-    for (int k = 0; k < P; k++) {
-      const long long n = sample_off_[k + 1] - sample_off_[k];
-      if (flac && n > kMaxFlacSamples) throw ArgError("program too long for one FLAC stream (2^36 - 1 samples at most)");
-      const long long nf = flac ? flac_frames(n) : mp3_frames(mp3, n);
-      if (foff[k] + nf > 0x7FFFFFFFLL) throw ArgError(flac ? "batch too long for one FLAC encode" : "batch too long for one MP3 encode");
-      foff[k + 1] = foff[k] + (int)nf;
-      if (!flac) boff[k + 1] = boff[k] + mp3_bytes(mp3, nf);
-    }
-    fl.F = foff[P];
-    const size_t bound = flac ? (size_t)flac_bound(P, fl.F, total_samples_) : (size_t)boff[P];
-    const size_t work = flac ? flac_work_bytes(fl.F) : mp3_const_bytes();
-    grow(streamA_, bound);
-    fl.out = streamA_.alloc<unsigned char>(bound);
-    grow(streamTabA_, 3 * ((size_t)(P + 1) * sizeof(long long) + 256) + work);
-    fl.soff = streamTabA_.alloc<long long>(P + 1);
-    fl.foff = streamTabA_.alloc<int>(P + 1);
-    fl.ioff = streamTabA_.alloc<long long>(P + 1);
-    fl.work = streamTabA_.alloc_bytes(work);
-    upload(fl.soff, sample_off_.data(), (size_t)(P + 1) * sizeof(long long));
-    upload(fl.foff, foff.data(), (size_t)(P + 1) * sizeof(int));
-    if (!flac) {
-      std::vector<unsigned char> consts(work);
-      mp3_consts(consts.data());
-      upload(fl.ioff, boff.data(), (size_t)(P + 1) * sizeof(long long));
-      upload(fl.work, consts.data(), work);
-      stream_off_ = boff;
-    }
-  }
-  h_loud_.clear();
-  h_lim_.clear();
-  h_rng_.clear();
+  // FLAC / MP3: the encoder's tables are on the device before the forward pass, so that the encoder follows it
+  // without a host round trip
+  streams_ = is_stream(enc) ? stream_tables(plan_, sample_off_) : StreamTables();
+  out_.reserve(plan_, total_samples_, s24_off_[B_], P, streams_, stream_);
+  upload(out_.tables, streams_.host.data(), streams_.host.size());
+  report_.clear();
   sink_filled_ = false;
   float* sink = (host_sink && !debug_) ? host_sink(total_samples_) : nullptr;
   // (both streams are idle here: the previous run synchronised them, and the outputs were sized above)
@@ -1008,43 +906,22 @@ void Model::run(Encoding enc, const std::vector<int>& programs, int kbps) {
         KKX_CUDA(cudaEventRecord(ev_grp_, stream_));
         KKX_CUDA(cudaStreamWaitEvent(copy_stream_, ev_grp_, 0));
         if (s1 > s0)
-          KKX_CUDA(cudaMemcpyAsync(sink + s0, r.audio + s0, (size_t)(s1 - s0) * sizeof(float), cudaMemcpyDeviceToHost, copy_stream_));
+          KKX_CUDA(cudaMemcpyAsync(sink + s0, out_.audio + s0, (size_t)(s1 - s0) * sizeof(float), cudaMemcpyDeviceToHost, copy_stream_));
       }
       b0 = b1;
       k0 = k1;
     }
     KKX_CUDA(cudaEventRecord(ev1_, stream_));
-    if (enc == Encoding::FLAC) {
-      launch_flac(static_cast<const short*>(r.twin), fl.soff, fl.foff, P, fl.F, opt.out_rate, fl.work, fl.out, fl.ioff,
-                  stream_);
-      stream_off_.assign(P + 1, 0);
-      KKX_CUDA(cudaMemcpyAsync(stream_off_.data(), fl.ioff, (size_t)(P + 1) * sizeof(long long),
-                               cudaMemcpyDeviceToHost, stream_));
-    }
-    if (enc == Encoding::MP3)
-      launch_mp3(static_cast<const short*>(r.twin), fl.soff, fl.foff, fl.ioff, P, fl.F, mp3, fl.work, fl.out, stream_);
+    if (is_stream(enc))
+      encode_streams(plan_, streams_, static_cast<const short*>(out_.twin), out_.tables, out_.bytes, stream_);
     KKX_CUDA(cudaStreamSynchronize(stream_));
     if (sink) { KKX_CUDA(cudaStreamSynchronize(copy_stream_)); sink_filled_ = true; }
-    if (loud_ || rep_) {   // [3][P] on the device -> program-major on the host
-      std::vector<float> rows((size_t)P * 3);
-      KKX_CUDA(cudaMemcpy(rows.data(), r.loud, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
-      h_loud_.resize(rows.size());
+    if (plan_.measure) {   // [kReportRows][P] on the device -> program-major on the host
+      std::vector<float> rows((size_t)P * kReportRows);
+      KKX_CUDA(cudaMemcpy(rows.data(), out_.report, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
+      report_.resize(rows.size());
       for (int k = 0; k < P; k++)
-        for (int j = 0; j < 3; j++) h_loud_[(size_t)k * 3 + j] = rows[(size_t)j * P + k];
-    }
-    if (rep_) {    // LRA | max momentary | max short-term, [3][P] -> program-major on the host
-      std::vector<float> rows((size_t)P * 3);
-      KKX_CUDA(cudaMemcpy(rows.data(), r.rng, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
-      h_rng_.resize(rows.size());
-      for (int k = 0; k < P; k++)
-        for (int j = 0; j < 3; j++) h_rng_[(size_t)k * 3 + j] = rows[(size_t)j * P + k];
-    }
-    if (lim_) {    // report rows 1, 2 of [3][P] -> program-major on the host
-      std::vector<float> rows((size_t)P * 2);
-      KKX_CUDA(cudaMemcpy(rows.data(), r.lim + P, rows.size() * sizeof(float), cudaMemcpyDeviceToHost));
-      h_lim_.resize(rows.size());
-      for (int k = 0; k < P; k++)
-        for (int j = 0; j < 2; j++) h_lim_[(size_t)k * 2 + j] = rows[(size_t)j * P + k];
+        for (int j = 0; j < kReportRows; j++) report_[(size_t)k * kReportRows + j] = rows[(size_t)j * P + k];
     }
   } catch (...) {
     cudaStreamSynchronize(stream_);

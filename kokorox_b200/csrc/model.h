@@ -2,6 +2,7 @@
 #pragma once
 #include "common.h"
 #include "kernels.h"
+#include "output.h"
 #include <deque>
 #include <functional>
 #include <map>
@@ -241,11 +242,6 @@ struct ConvOpt {
   float* attn_scratch = nullptr;
 };
 
-// What a run returns besides the f32 waveform, which every run writes: its 16-bit PCM twin, the G.711 codes of that
-// PCM (mu-law / A-law), or one FLAC or MP3 stream per item encoded from it (kkx.h).
-enum class Encoding { F32, PCM16, ULAW, ALAW, FLAC, MP3 };
-inline bool is_stream(Encoding e) { return e == Encoding::FLAC || e == Encoding::MP3; }
-
 class Model {
  public:
   Model(const std::string& weights_path, int device);
@@ -279,19 +275,11 @@ class Model {
   long long encoded_bytes() const;
   void fetch_encoded(void* dst, long long capacity_bytes, int64_t* byte_offsets, int64_t* sample_offsets,
                      int32_t* pred_dur);
-  // Loudness of the last run's programs (kernels_loudness.cu): true if that run normalised or reported; then
-  // last_loudness() holds 3 P floats, per program k at 3 k: integrated loudness (LUFS, NaN = undefined), true peak
-  // (dBTP), gain.
-  bool loudness_ran() const { return ran_ && (loud_ || rep_); }
-  const std::vector<float>& last_loudness() const { return h_loud_; }
-  // Loudness range and maxima of the last run's programs: true if that run reported; then last_loudness_range()
-  // holds 3 P floats, per program k at 3 k: LRA (LU), max momentary and max short-term loudness (LUFS); NaN = undefined.
-  bool loudness_range_ran() const { return ran_ && rep_; }
-  const std::vector<float>& last_loudness_range() const { return h_rng_; }
-  // Limiter of the last run's programs (kernels_loudness.cu): true if that run limited; then last_limiter() holds
-  // 2 P floats, per program k at 2 k: the largest reduction (dB) and the output's true peak (dBTP).
-  bool limiter_ran() const { return ran_ && lim_; }
-  const std::vector<float>& last_limiter() const { return h_lim_; }
+  // The report of the last run's programs (output.h): the row groups it produced (kRepLoudness | kRepRange |
+  // kRepLimiter; 0 = none), and then last_report() holds kReportRows floats per program k at kReportRows k, in the
+  // device table's row order.
+  unsigned report_groups() const { return ran_ ? plan_.groups() : 0; }
+  const std::vector<float>& last_report() const { return report_; }
 
   void set_noise(const float* noise, long long n);
   void set_inject(const std::string& name, int item, const void* data, long long count);
@@ -320,15 +308,6 @@ class Model {
     int* total = nullptr;      // [B]     T_b
     std::vector<int> T;        // frames per item (host)
     Level styL;                // one item of B rows (style FC GEMMs)
-    float* audio = nullptr;    // [total_samples_] the f32 waveform at the output rate
-    void* twin = nullptr;      // its 16-bit PCM (PCM16, FLAC, MP3) or G.711 (ULAW, ALAW) twin
-    float* loud = nullptr;     // [3][P] lufs | dBTP | gain of loudness normalisation; the gain feeds the resampling
-    float* wav24 = nullptr;    // resampling pass only: the run's 24 kHz waveform, item b at s24_off_[b]
-    float* lim = nullptr;      // [3][P] t | max reduction (dB) | output true peak (dBTP) of the limiter; t feeds the
-                               // resampling
-    float* lim_p = nullptr;    // limiter: the detector p and the limited waveform v, both indexed like wav24
-    float* lim_v = nullptr;
-    float* rng = nullptr;      // [3][P] LRA | max momentary | max short-term loudness of the loudness report
   };
   // Linear / Conv1d on the precision-critical path: split-TF32 tensor cores when precision==1 and
   // the weight has a TcW32, fp32 SIMT otherwise.  Returns true when the result went to the operand planes of `o`
@@ -415,32 +394,17 @@ class Model {
   std::vector<int> tok_len_;
   int* d_ids_ = nullptr; float* d_styles_ = nullptr; float* d_speeds_ = nullptr;
   Level tokL_;
-  // outputs of the current run (Run::audio / twin / loud point into them), grow-only; the FLAC or MP3 streams, their
-  // per-program byte offsets (host) and the encoder's tables and scratch
-  Encoding enc_ = Encoding::F32;
-  Arena audioA_, twinA_, loudA_, streamA_, streamTabA_, wav24A_, limA_, limWavA_, rngA_;
-  std::vector<long long> stream_off_;
+  // the output stage of the current run: its plan, buffers, encoder tables (FLAC / MP3: the programs' byte offsets)
+  // and the host copy of its report (program-major)
+  OutputPlan plan_;
+  OutputBuffers out_;
+  StreamTables streams_;
+  std::vector<float> report_;
   // program table of the current run (P + 1 item offsets); s24_off_ [B + 1]: each item's offset in the run's 24 kHz
   // waveform, where a program is contiguous
   std::vector<int> prog_;
   std::vector<long long> s24_off_;
   int n_prog() const { return (int)prog_.size() - 1; }
-  void grow(Arena& a, size_t bytes);
-  // output resampling of the current run (opt.out_rate): U / D, half length H; d_taps_ holds the filter of taps_rate_
-  bool resample_ = false; int rs_U_ = 1, rs_D_ = 1, rs_H_ = 0;
-  float* d_taps_ = nullptr; int taps_rate_ = 0;
-  void prepare_resample();
-  // loudness normalisation of the current run; h_loud_ = the host copy of Run::loud (program-major)
-  bool loud_ = false; LoudParams loud_par_{};
-  std::vector<float> h_loud_;
-  // the limiter of the current run (it measures through the loudness kernels, so loud_par_ serves it too); h_lim_ =
-  // the host copy of Run::lim's report rows (program-major)
-  bool lim_ = false;
-  std::vector<float> h_lim_;
-  // the loudness report of the current run (through the loudness kernels and loud_par_ as well); h_rng_ = the host
-  // copy of Run::rng (program-major)
-  bool rep_ = false;
-  std::vector<float> h_rng_;
   float* d_voices_ = nullptr; int n_voices_ = 0;                           // [V][511][256] voice table
   std::vector<long long> sample_off_;                                      // [P + 1] at the output rate
   int* h_pred_dur_ = nullptr; size_t h_pred_dur_cap_ = 0;                  // pinned: per-row integer durations of the last run

@@ -649,46 +649,6 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
   upload(d_ph_off, ph_off.data(), B * sizeof(int));
   upload(d_s_loc, s_loc.data(), B * sizeof(long long));
   upload(d_s24, s24_off_.data() + b0, B * sizeof(long long));
-  // output resampling: the iSTFT writes each item into r.wav24 at its run-wide offset, so that a program is one
-  // contiguous span there; once a program's last item is done (programs [k0, k1) here) the resampling pass reads
-  // the span (p_in, p_len) and writes r.audio at the program's output-rate offset (p_out)
-  const int K = k1 - k0;
-  long long *d_p_in = nullptr, *d_p_len = nullptr, *d_p_out = nullptr;
-  long long max_out = 0, max_len24 = 0;
-  // loudness normalisation, the limiter and the loudness report: per-program 2400-sample segment energies (offsets
-  // seg_off), true-peak, limiter and short-term energy scratch
-  long long* d_seg_off = nullptr;
-  float* energy = nullptr;
-  double* short_e = nullptr;
-  unsigned* peak = nullptr;
-  unsigned* lim_acc = nullptr;
-  if (resample_ && K > 0) {
-    std::vector<long long> p_in(K), p_len(K), p_out(K), seg_off(K);
-    long long nseg = 0;
-    for (int k = 0; k < K; k++) {
-      p_in[k] = s24_off_[prog_[k0 + k]];
-      p_len[k] = s24_off_[prog_[k0 + k + 1]] - p_in[k];
-      p_out[k] = sample_off_[k0 + k];
-      max_out = std::max(max_out, sample_off_[k0 + k + 1] - p_out[k]);
-      max_len24 = std::max(max_len24, p_len[k]);
-      seg_off[k] = nseg;
-      nseg += p_len[k] / kLoudSeg;
-    }
-    d_p_in = A.alloc<long long>(K);
-    d_p_len = A.alloc<long long>(K);
-    d_p_out = A.alloc<long long>(K);
-    upload(d_p_in, p_in.data(), K * sizeof(long long));
-    upload(d_p_len, p_len.data(), K * sizeof(long long));
-    upload(d_p_out, p_out.data(), K * sizeof(long long));
-    if (loud_ || lim_ || rep_) {
-      d_seg_off = A.alloc<long long>(K);
-      energy = A.alloc<float>((size_t)std::max(nseg, 1LL));
-      peak = A.alloc<unsigned>(K);
-      upload(d_seg_off, seg_off.data(), K * sizeof(long long));
-    }
-    if (lim_) lim_acc = A.alloc<unsigned>((size_t)2 * K);
-    if (rep_) short_e = A.alloc<double>((size_t)std::max(nseg, 1LL));
-  }
 
   // ---- length regulation (K4/K5)
   int* idx = A.alloc<int>(FR.rows);
@@ -886,37 +846,23 @@ void Model::frame_phase(Run& r, int b0, int b1, int k0, int k1, bool dry) {
     launch_conv_f32(c, st);
   }
   capture("conv_post", cp, 24, 0, 22, G120, b0);
-  const bool law = enc_ == Encoding::ULAW || enc_ == Encoding::ALAW;
-  short* pcm = enc_ == Encoding::PCM16 || is_stream(enc_) ? static_cast<short*>(r.twin) : nullptr;
-  if (!resample_) {   // the output is the 24 kHz waveform: program layout == item layout
-    launch_istft(cp, 24, G120.d_off, G120.d_len, r.audio, pcm, d_s24, opt.precision == 1, B, G120.max_len, st);
+  // Without post-processing the iSTFT writes the output itself (program layout == item layout).  Otherwise it writes
+  // each item into the 24 kHz waveform at its run-wide offset, so that a program is one contiguous span there, and the
+  // programs this group completes (k0 .. k1) go through the output stage.
+  if (!plan_.post) {
+    launch_istft(cp, 24, G120.d_off, G120.d_len, out_.audio, plan_.pcm() ? static_cast<short*>(out_.twin) : nullptr,
+                 d_s24, opt.precision == 1, B, G120.max_len, st);
     return;
   }
-  launch_istft(cp, 24, G120.d_off, G120.d_len, r.wav24, nullptr, d_s24, opt.precision == 1, B, G120.max_len, st);
-  if (K == 0) return;   // every program of this group goes on into the next
-  const int P = n_prog();
-  float* gain = nullptr;
-  const float* wav = r.wav24;
-  // measured on the 24 kHz waveform; the gain rides on the resampling pass (r.loud = lufs | dBTP | gain)
-  if (loud_ || lim_ || rep_) {
-    gain = r.loud + 2 * (size_t)P + k0;
-    launch_loudness(r.wav24, d_p_in, d_p_len, d_seg_off, loud_par_, energy, peak, r.loud + k0, r.loud + P + k0, gain,
-                    K, max_len24, st, lim_ ? r.lim_p : nullptr);
-  }
-  if (rep_) {   // the report on the same energies, before the limiter (r.rng = LRA | max momentary | max short-term)
-    launch_loudness_range(d_p_len, d_seg_off, energy, short_e, r.rng + k0, r.rng + P + k0, r.rng + 2 * (size_t)P + k0,
-                          K, max_len24, st);
-    if (!loud_ && !lim_) gain = nullptr;   // measure-only: the resampling pass is the plain output's arithmetic
-  }
-  if (lim_) {   // the limited waveform v is resampled instead, with the static trim t as its gain (r.lim = t | report)
-    launch_limiter(r.wav24, r.lim_p, d_p_in, d_p_len, loud_par_, gain, r.lim_v, nullptr, lim_acc, r.lim + k0,
-                   r.lim + P + k0, r.lim + 2 * (size_t)P + k0, K, max_len24, st);
-    wav = r.lim_v;
-    gain = r.lim + k0;
-  }
-  // grids span the longest program (64-bit sample indices); CTAs past a shorter program's end return at once
-  launch_resample(wav, d_p_in, d_p_len, d_p_out, d_taps_, rs_U_, rs_D_, rs_H_, gain, r.audio, pcm,
-                  law ? static_cast<unsigned char*>(r.twin) : nullptr, enc_ == Encoding::ALAW ? 1 : 0, K, max_out, st);
+  launch_istft(cp, 24, G120.d_off, G120.d_len, out_.wav24, nullptr, d_s24, opt.precision == 1, B, G120.max_len, st);
+  if (k1 == k0) return;
+  std::vector<long long> len24(k1 - k0);
+  for (int k = k0; k < k1; k++) len24[k - k0] = s24_off_[prog_[k + 1]] - s24_off_[prog_[k]];
+  Spans sp = make_spans(len24, s24_off_[prog_[k0]], sample_off_[k0], plan_.U, plan_.D);
+  long long* d_sp = A.alloc<long long>(sp.host.size());
+  upload(d_sp, sp.host.data(), sp.bytes());
+  sp.place(d_sp);
+  post_programs(plan_, sp, out_, k0, n_prog(), A, st);
 }
 
 }  // namespace kkx

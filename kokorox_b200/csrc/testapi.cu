@@ -21,6 +21,40 @@ struct DevBuf {
   ~DevBuf() { if (p) cudaFree(p); }
   template <class T> T* as() { return static_cast<T*>(p); }
 };
+// B items of >= 1 sample back to back, as the output stage's span table (make_spans) on the device.
+struct ItemSpans {
+  Spans s;
+  DevBuf d;
+  ItemSpans(int B, const int64_t* lens, int U, int D, const char* who)
+      : s(build(B, lens, U, D, who)), d(s.host.data(), s.bytes()) { s.place(d.as<long long>()); }
+  static Spans build(int B, const int64_t* lens, int U, int D, const char* who) {
+    for (int b = 0; b < B; b++)
+      if (lens[b] < 1) throw ArgError(std::string(who) + ": every item needs >= 1 sample");
+    return make_spans(std::vector<long long>(lens, lens + B), 0, 0, U, D);
+  }
+};
+// pcm16 items of >= 1 sample through the output stage's encoder (stream_tables, encode_streams); returns the byte
+// offsets [B + 1] and, when dst is given, copies the streams there
+long long encode_items(const OutputPlan& p, const int16_t* pcm, int B, const int64_t* lens, uint8_t* dst,
+                       int64_t capacity, int64_t* byte_offsets, const char* who) {
+  std::vector<long long> soff(B + 1, 0);
+  for (int b = 0; b < B; b++) {
+    if (lens[b] < 1) throw ArgError(std::string(who) + ": every item needs >= 1 sample");
+    soff[b + 1] = soff[b] + lens[b];
+  }
+  StreamTables t = stream_tables(p, soff);
+  DevBuf dp(pcm, (size_t)soff[B] * 2), dt(nullptr, t.dev_bytes), dout(nullptr, t.bound);
+  KKX_CUDA(cudaMemcpy(dt.p, t.host.data(), t.host.size(), cudaMemcpyHostToDevice));
+  encode_streams(p, t, dp.as<short>(), dt.p, dout.as<unsigned char>(), 0);
+  KKX_CUDA(cudaDeviceSynchronize());
+  for (int b = 0; b <= B; b++) byte_offsets[b] = t.boff[b];
+  const long long total = t.boff[B];
+  if (dst) {
+    if (capacity < total) throw ArgError(std::string(who) + ": dst too small");
+    KKX_CUDA(cudaMemcpy(dst, dout.p, (size_t)total, cudaMemcpyDeviceToHost));
+  }
+  return total;
+}
 template <class F> int run(int device, F&& f) {
   try {
     int n = 0;
@@ -71,20 +105,14 @@ KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64
     std::vector<float> taps;
     int U = 1, D = 1, H = 0;
     if (out_rate != 24000 && resample_design(out_rate, &taps, &U, &D, &H) < 0) throw ArgError("rejected out_rate");
-    std::vector<long long> in_off(B), in_len(B), out_off(B);
-    long long ni = 0, no = 0, max_out = 0;
-    for (int b = 0; b < B; b++) {
-      if (lens[b] < 1) throw ArgError("kkx_test_resample: every item needs >= 1 sample");
-      const long long m = (lens[b] * U + D - 1) / D;
-      in_off[b] = ni; in_len[b] = lens[b]; out_off[b] = no;
-      ni += lens[b]; no += m; max_out = std::max(max_out, m);
-    }
-    DevBuf dx(x, (size_t)ni * 4), dt(taps.data(), taps.size() * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8);
-    DevBuf doo(out_off.data(), B * 8), dout(nullptr, (size_t)no * 4), dpcm(nullptr, pcm ? (size_t)no * 2 : 0);
+    const ItemSpans sp(B, lens, U, D, "kkx_test_resample");
+    const long long ni = sp.s.in_end, no = sp.s.out_end;
+    DevBuf dx(x, (size_t)ni * 4), dt(taps.data(), taps.size() * 4);
+    DevBuf dout(nullptr, (size_t)no * 4), dpcm(nullptr, pcm ? (size_t)no * 2 : 0);
     DevBuf dcode(nullptr, codes && law >= 0 ? (size_t)no : 0);
-    launch_resample(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), doo.as<long long>(),
-                    taps.empty() ? nullptr : dt.as<float>(), U, D, H, nullptr, dout.as<float>(), pcm ? dpcm.as<short>() : nullptr,
-                    codes && law >= 0 ? dcode.as<unsigned char>() : nullptr, law > 0 ? 1 : 0, B, max_out, 0);
+    launch_resample(dx.as<float>(), sp.s.in_off, sp.s.in_len, sp.s.out_off, taps.empty() ? nullptr : dt.as<float>(), U,
+                    D, H, nullptr, dout.as<float>(), pcm ? dpcm.as<short>() : nullptr,
+                    codes && law >= 0 ? dcode.as<unsigned char>() : nullptr, law > 0 ? 1 : 0, B, sp.s.max_out, 0);
     KKX_CUDA(cudaDeviceSynchronize());
     KKX_CUDA(cudaMemcpy(out, dout.p, (size_t)no * 4, cudaMemcpyDeviceToHost));
     if (pcm) KKX_CUDA(cudaMemcpy(pcm, dpcm.p, (size_t)no * 2, cudaMemcpyDeviceToHost));
@@ -106,19 +134,14 @@ KKX_API int kkx_test_loudness(int device, const float* x, int32_t B, const int64
                               int32_t ceiling_centi_dbtp, float* lufs, float* true_peak_dbtp, float* gain) {
   return run(device, [&] {
     if (!x || !lens || B < 1) throw ArgError("kkx_test_loudness: bad argument");
-    std::vector<long long> in_off(B), in_len(B), seg_off(B);
-    long long ni = 0, nseg = 0, max_len = 0;
-    for (int b = 0; b < B; b++) {
-      if (lens[b] < 1) throw ArgError("kkx_test_loudness: every item needs >= 1 sample");
-      in_off[b] = ni; in_len[b] = lens[b]; seg_off[b] = nseg;
-      ni += lens[b]; nseg += lens[b] / kLoudSeg; max_len = std::max<long long>(max_len, lens[b]);
-    }
+    const ItemSpans sp(B, lens, 1, 1, "kkx_test_loudness");
+    const Spans& s = sp.s;
     const LoudParams P = loudness_params(target_centi_lufs / 100.0, ceiling_centi_dbtp / 100.0);
-    DevBuf dx(x, (size_t)ni * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8), dso(seg_off.data(), B * 8);
-    DevBuf de(nullptr, (size_t)std::max(nseg, 1LL) * 4), dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4);
+    DevBuf dx(x, (size_t)s.in_end * 4);
+    DevBuf de(nullptr, (size_t)std::max(s.nseg, 1LL) * 4), dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4);
     float* r = dr.as<float>();
-    launch_loudness(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), dso.as<long long>(), P, de.as<float>(),
-                    dp.as<unsigned>(), r, r + B, r + 2 * B, B, max_len, 0);
+    launch_loudness(dx.as<float>(), s.in_off, s.in_len, s.seg_off, P, de.as<float>(), dp.as<unsigned>(), r, r + B,
+                    r + 2 * B, B, s.max_len, 0);
     KKX_CUDA(cudaDeviceSynchronize());
     if (lufs) KKX_CUDA(cudaMemcpy(lufs, r, B * 4, cudaMemcpyDeviceToHost));
     if (true_peak_dbtp) KKX_CUDA(cudaMemcpy(true_peak_dbtp, r + B, B * 4, cudaMemcpyDeviceToHost));
@@ -130,23 +153,17 @@ KKX_API int kkx_test_loudness_range(int device, const float* x, int32_t B, const
                                     float* m_max, float* s_max) {
   return run(device, [&] {
     if (!x || !lens || B < 1) throw ArgError("kkx_test_loudness_range: bad argument");
-    std::vector<long long> in_off(B), in_len(B), seg_off(B);
-    long long ni = 0, nseg = 0, max_len = 0;
-    for (int b = 0; b < B; b++) {
-      if (lens[b] < 1) throw ArgError("kkx_test_loudness_range: every item needs >= 1 sample");
-      in_off[b] = ni; in_len[b] = lens[b]; seg_off[b] = nseg;
-      ni += lens[b]; nseg += lens[b] / kLoudSeg; max_len = std::max<long long>(max_len, lens[b]);
-    }
+    const ItemSpans sp(B, lens, 1, 1, "kkx_test_loudness_range");
+    const Spans& s = sp.s;
     const LoudParams P = loudness_params(0.0, -1.0, false, true);   // measure-only
-    DevBuf dx(x, (size_t)ni * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8), dso(seg_off.data(), B * 8);
-    DevBuf de(nullptr, (size_t)std::max(nseg, 1LL) * 4), dst(nullptr, (size_t)std::max(nseg, 1LL) * 8);
+    DevBuf dx(x, (size_t)s.in_end * 4);
+    DevBuf de(nullptr, (size_t)std::max(s.nseg, 1LL) * 4), dst(nullptr, (size_t)std::max(s.nseg, 1LL) * 8);
     DevBuf dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4), dq(nullptr, (size_t)B * 3 * 4);
     float* r = dr.as<float>();
     float* q = dq.as<float>();
-    launch_loudness(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), dso.as<long long>(), P, de.as<float>(),
-                    dp.as<unsigned>(), r, r + B, r + 2 * B, B, max_len, 0);
-    launch_loudness_range(dil.as<long long>(), dso.as<long long>(), de.as<float>(), dst.as<double>(), q, q + B,
-                          q + 2 * B, B, max_len, 0);
+    launch_loudness(dx.as<float>(), s.in_off, s.in_len, s.seg_off, P, de.as<float>(), dp.as<unsigned>(), r, r + B,
+                    r + 2 * B, B, s.max_len, 0);
+    launch_loudness_range(s.in_len, s.seg_off, de.as<float>(), dst.as<double>(), q, q + B, q + 2 * B, B, s.max_len, 0);
     KKX_CUDA(cudaDeviceSynchronize());
     if (lra) KKX_CUDA(cudaMemcpy(lra, q, B * 4, cudaMemcpyDeviceToHost));
     if (m_max) KKX_CUDA(cudaMemcpy(m_max, q + B, B * 4, cudaMemcpyDeviceToHost));
@@ -159,24 +176,20 @@ KKX_API int kkx_test_limiter(int device, const float* x, int32_t B, const int64_
                              float* max_reduction_db, float* true_peak_dbtp) {
   return run(device, [&] {
     if (!x || !lens || B < 1) throw ArgError("kkx_test_limiter: bad argument");
-    std::vector<long long> in_off(B), in_len(B), seg_off(B);
-    long long ni = 0, nseg = 0, max_len = 0;
-    for (int b = 0; b < B; b++) {
-      if (lens[b] < 1) throw ArgError("kkx_test_limiter: every item needs >= 1 sample");
-      in_off[b] = ni; in_len[b] = lens[b]; seg_off[b] = nseg;
-      ni += lens[b]; nseg += lens[b] / kLoudSeg; max_len = std::max<long long>(max_len, lens[b]);
-    }
+    const ItemSpans sp(B, lens, 1, 1, "kkx_test_limiter");
+    const Spans& s = sp.s;
+    const long long ni = s.in_end;
     const LoudParams P = loudness_params(target_centi_lufs / 100.0, ceiling_centi_dbtp / 100.0, true);
-    DevBuf dx(x, (size_t)ni * 4), dio(in_off.data(), B * 8), dil(in_len.data(), B * 8), dso(seg_off.data(), B * 8);
-    DevBuf de(nullptr, (size_t)std::max(nseg, 1LL) * 4), dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4);
+    DevBuf dx(x, (size_t)ni * 4);
+    DevBuf de(nullptr, (size_t)std::max(s.nseg, 1LL) * 4), dp(nullptr, B * 4), dr(nullptr, (size_t)B * 3 * 4);
     DevBuf dpm(nullptr, (size_t)ni * 4), dv(nullptr, (size_t)ni * 4), dG(nullptr, (size_t)ni * 4);
     DevBuf dacc(nullptr, (size_t)B * 2 * 4), dl(nullptr, (size_t)B * 3 * 4);
     float* r = dr.as<float>();
     float* l = dl.as<float>();
-    launch_loudness(dx.as<float>(), dio.as<long long>(), dil.as<long long>(), dso.as<long long>(), P, de.as<float>(),
-                    dp.as<unsigned>(), r, r + B, r + 2 * B, B, max_len, 0, dpm.as<float>());
-    launch_limiter(dx.as<float>(), dpm.as<float>(), dio.as<long long>(), dil.as<long long>(), P, r + 2 * B,
-                   dv.as<float>(), dG.as<float>(), dacc.as<unsigned>(), l, l + B, l + 2 * B, B, max_len, 0);
+    launch_loudness(dx.as<float>(), s.in_off, s.in_len, s.seg_off, P, de.as<float>(), dp.as<unsigned>(), r, r + B,
+                    r + 2 * B, B, s.max_len, 0, dpm.as<float>());
+    launch_limiter(dx.as<float>(), dpm.as<float>(), s.in_off, s.in_len, P, r + 2 * B, dv.as<float>(), dG.as<float>(),
+                   dacc.as<unsigned>(), l, l + B, l + 2 * B, B, s.max_len, 0);
     KKX_CUDA(cudaDeviceSynchronize());
     if (gain) KKX_CUDA(cudaMemcpy(gain, r + 2 * B, B * 4, cudaMemcpyDeviceToHost));
     if (G) KKX_CUDA(cudaMemcpy(G, dG.p, (size_t)ni * 4, cudaMemcpyDeviceToHost));
@@ -193,27 +206,10 @@ KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const i
   const int rc = run(device, [&] {
     if (!pcm || !lens || !byte_offsets || B < 1) throw ArgError("kkx_test_flac: bad argument");
     if (!flac_rate_ok(rate)) throw ArgError("kkx_test_flac: rejected rate");
-    std::vector<long long> soff(B + 1, 0);
-    std::vector<int> foff(B + 1, 0);
-    for (int b = 0; b < B; b++) {
-      if (lens[b] < 1) throw ArgError("kkx_test_flac: every item needs >= 1 sample");
-      soff[b + 1] = soff[b] + lens[b];
-      foff[b + 1] = foff[b] + (int)flac_frames(lens[b]);
-    }
-    const int F = foff[B];
-    DevBuf dp(pcm, (size_t)soff[B] * 2), ds(soff.data(), (B + 1) * 8), df(foff.data(), (B + 1) * 4);
-    DevBuf dio(nullptr, (B + 1) * 8), dw(nullptr, flac_work_bytes(F)), dout(nullptr, (size_t)flac_bound(B, F, soff[B]));
-    launch_flac(dp.as<short>(), ds.as<long long>(), df.as<int>(), B, F, rate, dw.p, dout.as<unsigned char>(),
-                dio.as<long long>(), 0);
-    KKX_CUDA(cudaDeviceSynchronize());
-    std::vector<long long> io(B + 1);
-    KKX_CUDA(cudaMemcpy(io.data(), dio.p, (B + 1) * 8, cudaMemcpyDeviceToHost));
-    for (int b = 0; b <= B; b++) byte_offsets[b] = io[b];
-    total = io[B];
-    if (dst) {
-      if (capacity < total) throw ArgError("kkx_test_flac: dst too small");
-      KKX_CUDA(cudaMemcpy(dst, dout.p, (size_t)total, cudaMemcpyDeviceToHost));
-    }
+    OutputPlan p;
+    p.enc = Encoding::FLAC;
+    p.rate = rate;
+    total = encode_items(p, pcm, B, lens, dst, capacity, byte_offsets, "kkx_test_flac");
   });
   return rc == KKX_OK ? (int64_t)total : (int64_t)rc;
 }
@@ -223,29 +219,11 @@ KKX_API int64_t kkx_test_mp3(int device, const int16_t* pcm, int32_t B, const in
   long long total = 0;
   const int rc = run(device, [&] {
     if (!pcm || !lens || !byte_offsets || B < 1) throw ArgError("kkx_test_mp3: bad argument");
-    const Mp3Format fmt = mp3_format(rate, kbps);
-    std::vector<long long> soff(B + 1, 0), boff(B + 1, 0);
-    std::vector<int> foff(B + 1, 0);
-    for (int b = 0; b < B; b++) {
-      if (lens[b] < 1) throw ArgError("kkx_test_mp3: every item needs >= 1 sample");
-      soff[b + 1] = soff[b] + lens[b];
-      const long long nf = mp3_frames(fmt, lens[b]);
-      foff[b + 1] = foff[b] + (int)nf;
-      boff[b + 1] = boff[b] + mp3_bytes(fmt, nf);
-    }
-    std::vector<unsigned char> consts(mp3_const_bytes());
-    mp3_consts(consts.data());
-    DevBuf dp(pcm, (size_t)soff[B] * 2), ds(soff.data(), (B + 1) * 8), df(foff.data(), (B + 1) * 4);
-    DevBuf db(boff.data(), (B + 1) * 8), dc(consts.data(), consts.size()), dout(nullptr, (size_t)boff[B]);
-    launch_mp3(dp.as<short>(), ds.as<long long>(), df.as<int>(), db.as<long long>(), B, foff[B], fmt, dc.p,
-               dout.as<unsigned char>(), 0);
-    KKX_CUDA(cudaDeviceSynchronize());
-    for (int b = 0; b <= B; b++) byte_offsets[b] = boff[b];
-    total = boff[B];
-    if (dst) {
-      if (capacity < total) throw ArgError("kkx_test_mp3: dst too small");
-      KKX_CUDA(cudaMemcpy(dst, dout.p, (size_t)total, cudaMemcpyDeviceToHost));
-    }
+    OutputPlan p;
+    p.enc = Encoding::MP3;
+    p.rate = rate;
+    p.mp3 = mp3_format(rate, kbps);
+    total = encode_items(p, pcm, B, lens, dst, capacity, byte_offsets, "kkx_test_mp3");
   });
   if (rc != KKX_OK) return rc;
   return (int64_t)total;

@@ -468,17 +468,40 @@ class B200Koko:
             return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
         return outs
 
+    def _encoded(self, entry, tokens, styles, speeds, args, ctype, release=None, n_out=None, byte_offsets=False,
+                 return_durations=False):
+        """The body of the encoded entry points: pack the batch, call ``entry(ctx, batch..., *args, &buf, offsets[,
+        None], durations)`` and return one output per item (or per program: ``n_out`` of them).  ``ctype``: the
+        element type of the returned views into the library's buffer, or None for one ``bytes`` each, copied out before
+        the buffer goes back through ``release``.  ``byte_offsets``: the entry point returns byte offsets and takes a
+        sample-offset pointer after them."""
+        self._require()
+        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
+        n = B if n_out is None else n_out
+        buf = entry.argtypes[6 + len(args)]._type_()   # the result pointer, of the type the entry point declares
+        boff = np.zeros(n + 1, dtype=np.int64)
+        dur = np.zeros(int(offs[-1]), dtype=np.int32)
+        tail = (None,) if byte_offsets else ()
+        self._check(entry(
+            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
+            _fp(st), _fp(sp), *args, C.byref(buf), boff.ctypes.data_as(C.POINTER(C.c_int64)), *tail,
+            dur.ctypes.data_as(C.POINTER(C.c_int32))))
+        if ctype is None:
+            base = C.cast(buf, C.c_void_p).value
+            try:
+                outs = [C.string_at(base + int(boff[k]), int(boff[k + 1] - boff[k])) for k in range(n)]
+            finally:
+                release(self._ctx, buf)
+        else:
+            outs = self._adopt(C.cast(buf, C.POINTER(ctype)), boff // C.sizeof(ctype) if byte_offsets else boff)
+        if return_durations:
+            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
+        return outs
+
     def infer_batch_pcm16(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float]):
         """Like infer_batch, but returns int16 PCM (trunc(clamp(s,-1,1)*32767), kokorox-websocket lib.rs:699-703),
         converted inside the iSTFT kernel; the device->host copy is half the size."""
-        self._require()
-        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
-        pcm = C.POINTER(C.c_int16)()
-        soff = np.zeros(B + 1, dtype=np.int64)
-        self._check(self._lib.kkx_infer_batch_pcm16(
-            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
-            _fp(st), _fp(sp), C.byref(pcm), soff.ctypes.data_as(C.POINTER(C.c_int64)), None))
-        return self._adopt(pcm, soff)
+        return self._encoded(self._lib.kkx_infer_batch_pcm16, tokens, styles, speeds, (), C.c_int16)
 
     def infer_batch_g711(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float], law: str = "ulaw",
                          return_durations: bool = False):
@@ -489,18 +512,8 @@ class B200Koko:
         laws = {"ulaw": 0, "alaw": 1}
         if law not in laws:
             raise KkxError(-1, f"law must be 'ulaw' or 'alaw', got {law!r}")
-        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
-        codes = C.POINTER(C.c_uint8)()
-        soff = np.zeros(B + 1, dtype=np.int64)
-        dur = np.zeros(int(offs[-1]), dtype=np.int32)
-        self._check(self._lib.kkx_infer_batch_g711(
-            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
-            _fp(st), _fp(sp), laws[law], C.byref(codes), soff.ctypes.data_as(C.POINTER(C.c_int64)),
-            dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        outs = self._adopt(codes, soff)
-        if return_durations:
-            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
-        return outs
+        return self._encoded(self._lib.kkx_infer_batch_g711, tokens, styles, speeds, (laws[law],), C.c_uint8,
+                             return_durations=return_durations)
 
     def infer_batch_flac(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
                          return_durations: bool = False):
@@ -508,26 +521,18 @@ class B200Koko:
         audio/flac) at the session's ``out_rate``, encoded on the device; decoding it gives exactly the int16 samples
         infer_batch_pcm16 returns.  The files are copied out of the library's buffer, which is released before this
         returns."""
-        self._require()
-        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
-        buf = C.POINTER(C.c_uint8)()
-        boff = np.zeros(B + 1, dtype=np.int64)
-        dur = np.zeros(int(offs[-1]), dtype=np.int32)
-        self._check(self._lib.kkx_infer_batch_flac(
-            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
-            _fp(st), _fp(sp), C.byref(buf), boff.ctypes.data_as(C.POINTER(C.c_int64)), None,
-            dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        try:
-            outs = [C.string_at(C.addressof(buf.contents) + int(boff[b]), int(boff[b + 1] - boff[b])) for b in range(B)]
-        finally:
-            self._lib.kkx_release_flac(self._ctx, buf)
-        if return_durations:
-            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
-        return outs
+        return self._encoded(self._lib.kkx_infer_batch_flac, tokens, styles, speeds, (), None,
+                             self._lib.kkx_release_flac, byte_offsets=True, return_durations=return_durations)
 
     # encoding name -> (KKX_ENC_* code, element type of the returned arrays; None = one ``bytes`` per program)
     _ENCODINGS = {"f32": (0, C.c_float), "pcm16": (1, C.c_int16), "ulaw": (2, C.c_uint8), "alaw": (3, C.c_uint8),
                   "flac": (4, None)}
+
+    @staticmethod
+    def _programs(program_offsets):
+        """(P, int32 offsets [P + 1]) of a program table as the C ABI takes it."""
+        prog = np.ascontiguousarray(np.asarray(program_offsets, dtype=np.int32).reshape(-1))
+        return max(prog.size - 1, 0), prog
 
     def infer_programs(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
                        program_offsets: Sequence[int], encoding: str = "f32", return_durations: bool = False):
@@ -542,26 +547,10 @@ class B200Koko:
             hint = " (MP3: infer_programs_mp3)" if encoding == "mp3" else ""
             raise KkxError(-1, f"encoding must be one of {sorted(self._ENCODINGS)}, got {encoding!r}{hint}")
         code, ctype = self._ENCODINGS[encoding]
-        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
-        prog = np.ascontiguousarray(np.asarray(program_offsets, dtype=np.int32).reshape(-1))
-        P = max(prog.size - 1, 0)
-        buf = C.c_void_p()
-        boff = np.zeros(P + 1, dtype=np.int64)
-        dur = np.zeros(int(offs[-1]), dtype=np.int32)
-        self._check(self._lib.kkx_infer_programs(
-            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
-            _fp(st), _fp(sp), P, prog.ctypes.data_as(C.POINTER(C.c_int32)), code, C.byref(buf),
-            boff.ctypes.data_as(C.POINTER(C.c_int64)), None, dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        if ctype is None:
-            try:
-                outs = [C.string_at(buf.value + int(boff[k]), int(boff[k + 1] - boff[k])) for k in range(P)]
-            finally:
-                self._lib.kkx_release_programs(self._ctx, buf)
-        else:
-            outs = self._adopt(C.cast(buf, C.POINTER(ctype)), boff // C.sizeof(ctype))
-        if return_durations:
-            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
-        return outs
+        P, prog = self._programs(program_offsets)
+        return self._encoded(self._lib.kkx_infer_programs, tokens, styles, speeds,
+                             (P, prog.ctypes.data_as(C.POINTER(C.c_int32)), code), ctype,
+                             self._lib.kkx_release_programs, P, True, return_durations)
 
     def infer_batch_mp3(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float], kbps: int = 0,
                         return_durations: bool = False):
@@ -569,44 +558,16 @@ class B200Koko:
         audio/mpeg) of the int16 samples infer_batch_pcm16 returns, at the session's ``out_rate``, encoded on the
         device.  ``kbps`` is a Layer III bitrate of the rate's MPEG version, 0 = 192 at 32 / 44.1 / 48 kHz and 160
         at the other rates (kkx.h kkx_infer_batch_mp3)."""
-        self._require()
-        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
-        buf = C.POINTER(C.c_uint8)()
-        boff = np.zeros(B + 1, dtype=np.int64)
-        dur = np.zeros(int(offs[-1]), dtype=np.int32)
-        self._check(self._lib.kkx_infer_batch_mp3(
-            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
-            _fp(st), _fp(sp), int(kbps), C.byref(buf), boff.ctypes.data_as(C.POINTER(C.c_int64)), None,
-            dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        try:
-            outs = [C.string_at(C.addressof(buf.contents) + int(boff[b]), int(boff[b + 1] - boff[b])) for b in range(B)]
-        finally:
-            self._lib.kkx_release_mp3(self._ctx, buf)
-        if return_durations:
-            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
-        return outs
+        return self._encoded(self._lib.kkx_infer_batch_mp3, tokens, styles, speeds, (int(kbps),), None,
+                             self._lib.kkx_release_mp3, byte_offsets=True, return_durations=return_durations)
 
     def infer_programs_mp3(self, tokens: Sequence[Sequence[int]], styles, speeds: Sequence[float],
                            program_offsets: Sequence[int], kbps: int = 0, return_durations: bool = False):
         """infer_programs with one MP3 file (``bytes``) per program, under the rules of infer_batch_mp3."""
-        self._require()
-        B, flat, offs, st, sp = self._pack(tokens, styles, speeds)
-        prog = np.ascontiguousarray(np.asarray(program_offsets, dtype=np.int32).reshape(-1))
-        P = max(prog.size - 1, 0)
-        buf = C.POINTER(C.c_uint8)()
-        boff = np.zeros(P + 1, dtype=np.int64)
-        dur = np.zeros(int(offs[-1]), dtype=np.int32)
-        self._check(self._lib.kkx_infer_programs_mp3(
-            self._ctx, B, flat.ctypes.data_as(C.POINTER(C.c_int64)), offs.ctypes.data_as(C.POINTER(C.c_int32)),
-            _fp(st), _fp(sp), P, prog.ctypes.data_as(C.POINTER(C.c_int32)), int(kbps), C.byref(buf),
-            boff.ctypes.data_as(C.POINTER(C.c_int64)), None, dur.ctypes.data_as(C.POINTER(C.c_int32))))
-        try:
-            outs = [C.string_at(C.addressof(buf.contents) + int(boff[k]), int(boff[k + 1] - boff[k])) for k in range(P)]
-        finally:
-            self._lib.kkx_release_mp3(self._ctx, buf)
-        if return_durations:
-            return outs, [dur[int(offs[b]):int(offs[b + 1])].copy() for b in range(B)]
-        return outs
+        P, prog = self._programs(program_offsets)
+        return self._encoded(self._lib.kkx_infer_programs_mp3, tokens, styles, speeds,
+                             (P, prog.ctypes.data_as(C.POINTER(C.c_int32)), int(kbps)), None,
+                             self._lib.kkx_release_mp3, P, True, return_durations)
 
     def last_loudness(self):
         """What loudness normalisation (option ``loudness_target``) or the loudness report (option
