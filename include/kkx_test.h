@@ -163,6 +163,61 @@ KKX_API int kkx_test_limiter(int device, const float* x, int32_t B, const int64_
  * and loud_range).  Per item: lra (LU), m_max and s_max (LUFS); NaN = undefined.  Every output pointer is nullable. */
 KKX_API int kkx_test_loudness_range(int device, const float* x, int32_t B, const int64_t* lens, float* lra,
                                     float* m_max, float* s_max);
+/* Signal-path kernels.  These hooks take the caller's row layout: items at offsets into host buffers that already hold
+ * the gap rows between them (the model's Level layout), and every output buffer is pre-filled by the caller and copied
+ * back whole, so that anything a kernel writes outside its items shows.
+ * kkx_test_sine_source: harmonic source (kernels_signal.cu sine_phase, then sine_source).  f0 [rows_f0], item b at
+ *   f0_off[b] with L_b = f0_len[b] = 2T_b coarse steps; noise (nullable: the on-device Philox generator keyed by `seed`)
+ *   [t * 9 + h] of item-local sample t, one buffer every item reads from offset 0 like kkx_set_noise, noise_n >=
+ *   300 * max L_b * 9 floats; lin_w [9], lin_b [1] (m_source.l_linear).  phase (nullable) receives the coarse phase, items
+ *   back to back as [9][L_b]; har the source, items back to back (300 L_b samples each). */
+KKX_API int kkx_test_sine_source(int device, const float* f0, int rows_f0, int B, const int* f0_off, const int* f0_len,
+                                 const float* noise, int64_t noise_n, uint64_t seed, const float* lin_w, const float* lin_b,
+                                 float* phase, float* har);
+/* kkx_test_stft: STFT (n_fft 20, hop 5) of B items of x (n_x samples; item b has 5 (F_b - 1) samples at s_off[b]) ->
+ *   har [rows_h, 24] (magnitudes in columns 0..10, phases in 11..21), item b at h_off[b] with F_b = h_len[b] frames;
+ *   replicate_pad 0 = reflect padding. */
+KKX_API int kkx_test_stft(int device, const float* x, int64_t n_x, int B, const int64_t* s_off, const int* h_off,
+                          const int* h_len, int rows_h, int replicate_pad, float* har);
+/* kkx_test_istft: head + iSTFT of conv_post rows cp [rows, 24] (item b at h_off[b], F_b = h_len[b] frames) -> audio
+ *   [n_audio], item b's 5 (F_b - 1) samples at s_off[b] (a multiple of 4); pcm (nullable) the 16-bit twin at the same
+ *   offsets.  fast = 1 is the tensor-core configuration's SFU variant, 0 the libm variant. */
+KKX_API int kkx_test_istft(int device, const float* cp, int rows, int B, const int* h_off, const int* h_len, int fast,
+                           int64_t n_audio, const int64_t* s_off, float* audio, int16_t* pcm);
+/* kkx_test_durations: duration head and length regulator (duration, dur_scan, then expand_idx and gather_rows).
+ *   logits [rows_tok, 50] with item b at tok_off[b] (1 <= N_b = tok_len[b] <= 512), speeds [B] -> dur_float and pred_dur
+ *   [rows_tok], cum [B][512] (exclusive prefix sums), total [B] (frames T_b) and fr_off [B]: the frame level the model
+ *   builds (32 gap rows, 8-row alignment), whose row count the call returns (or < 0).  Every output pointer is
+ *   nullable; idx [rows_fr] and out [rows_fr, ldo] are written only when both are given and capacity_rows >= rows_fr
+ *   (otherwise the call is a size query): out[fr_off[b] + j, ocol + c] = feat[tok_off[b] + idx[fr_off[b] + j], c],
+ *   feat [rows_tok, C]. */
+KKX_API int64_t kkx_test_durations(int device, const float* logits, const float* speeds, const float* feat, int C, int ldo,
+                                   int ocol, int B, const int* tok_off, const int* tok_len, int rows_tok, float* dur_float,
+                                   int32_t* pred_dur, int32_t* cum, int32_t* total, int32_t* fr_off, int32_t* idx,
+                                   float* out, int64_t capacity_rows);
+/* kkx_test_pool_up: depthwise ConvTranspose1d(k3, s2, p1, op1) on lrelu(x * scale_b + shift_b, slope): x [rows_in, C]
+ *   with item b at in_off[b] (T_b = in_len[b] rows), scale / shift [B][C], w [C][3], bias [C]; item b's 2T_b output rows
+ *   at out_off[b].  Cpad == 0: the fp32 kernel, out float [rows_out, C]; Cpad >= C: the bf16 operand kernel, out bf16
+ *   bits [rows_out, Cpad], which also zeroes the gap rows and pad columns. */
+KKX_API int kkx_test_pool_up(int device, const float* x, int rows_in, int C, int B, const int* in_off, const int* in_len,
+                             const float* scale, const float* shift, float slope, const float* w, const float* bias,
+                             const int* out_off, int rows_out, int Cpad, void* out);
+/* kkx_test_post_conv: generator conv_post in the tensor-core configuration (kernels_arb.cu, post variant): x
+ *   [rows, 128] fp32 with item b at off[b] (len[b] rows, >= 32 gap rows around each), w [22][7][128] (out channel, tap,
+ *   in channel; rounded to bf16 here), bias [22] -> out [rows, 24] = Conv1d(128, 22, 7, pad 3) of bf16(lrelu(x, slope))
+ *   in columns 0..21 of the item rows. */
+KKX_API int kkx_test_post_conv(int device, const float* x, int rows, int B, const int* off, const int* len, const float* w,
+                               const float* bias, float slope, float* out);
+/* kkx_test_curve_conv: Conv1d(1, 1, k3, s2, p1) of the F0 / N curves: x [rows_x], item b at x_off[b] (x_len[b] values)
+ *   -> out[out_off[b] + t, ocol] of out [rows_out, ldo], t < out_len[b]. */
+KKX_API int kkx_test_curve_conv(int device, const float* x, int rows_x, int B, const int* x_off, const int* x_len,
+                                const float* w3, const float* bias, float* out, int rows_out, int ldo, int ocol,
+                                const int* out_off, const int* out_len);
+/* kkx_test_add_rows_stats: a += b in place on the item rows (a, b [rows, C], item b at off[b]) and the chunk statistics
+ *   part [B][ceil(max len / 128)][2][C] of the sum; with out_bf16 (bf16 bits [rows, C], nullable) the sum goes there
+ *   only and `a` is left as it was. */
+KKX_API int kkx_test_add_rows_stats(int device, float* a, const float* b, int rows, int C, int B, const int* off,
+                                    const int* len, uint16_t* out_bf16, float* part);
 KKX_API const char* kkx_test_last_error(void);
 
 #ifdef __cplusplus

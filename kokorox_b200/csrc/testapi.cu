@@ -684,4 +684,214 @@ KKX_API int kkx_test_arb_conv_stream(int device, const float* x, int B, const in
                        want_bf16, out, sums, 0);
 }
 
+// ---- signal-path kernels (kernels_signal.cu, kernels_tc.cu pool_up_bf16, kernels_arb.cu post variant).  Every hook
+// takes the caller's row layout (offsets into host buffers that already hold the gap rows) and copies the whole output
+// buffer back, so that tests see what the kernels wrote outside the items too.
+static std::vector<int> level_tiles(int B, const int* len, int MT) {
+  std::vector<int> t(B + 1, 0);
+  for (int b = 0; b < B; b++) t[b + 1] = t[b] + (len[b] + MT - 1) / MT;
+  return t;
+}
+static int max_of(int B, const int* len) {
+  int m = 0;
+  for (int b = 0; b < B; b++) m = std::max(m, len[b]);
+  return m;
+}
+
+KKX_API int kkx_test_sine_source(int device, const float* f0, int rows_f0, int B, const int* f0_off, const int* f0_len,
+                                 const float* noise, int64_t noise_n, uint64_t seed, const float* lin_w, const float* lin_b,
+                                 float* phase, float* har) {
+  return run(device, [&] {
+    if (!f0 || !f0_off || !f0_len || !lin_w || !lin_b || !har || B < 1) throw ArgError("kkx_test_sine_source: bad argument");
+    std::vector<int> ph_off(B);
+    std::vector<long long> s_off(B);
+    long long nph = 0, ns = 0, max_s = 0;
+    for (int b = 0; b < B; b++) {
+      if (f0_len[b] < 1 || f0_off[b] < 0 || f0_off[b] + f0_len[b] > rows_f0) throw ArgError("kkx_test_sine_source: bad item");
+      ph_off[b] = (int)nph; nph += 9LL * f0_len[b];
+      s_off[b] = ns; ns += 300LL * f0_len[b];
+      max_s = std::max(max_s, 300LL * f0_len[b]);
+    }
+    if (noise && noise_n < max_s * 9) throw ArgError("kkx_test_sine_source: noise buffer smaller than 300 * L * 9");
+    DevBuf df0(f0, (size_t)rows_f0 * 4), dfo(f0_off, B * 4), dfl(f0_len, B * 4), dpo(ph_off.data(), B * 4);
+    DevBuf dso(s_off.data(), B * 8), dnz(noise, noise ? (size_t)noise_n * 4 : 0), dw(lin_w, 9 * 4), dlb(lin_b, 4);
+    DevBuf dph(nullptr, (size_t)nph * 4), dout(har, (size_t)ns * 4);
+    launch_sine_phase(df0.as<float>(), dfo.as<int>(), dfl.as<int>(), dph.as<float>(), dpo.as<int>(), B, 0);
+    launch_sine_source(df0.as<float>(), dfo.as<int>(), dfl.as<int>(), dph.as<float>(), dpo.as<int>(),
+                       noise ? dnz.as<float>() : nullptr, (unsigned long long)seed, dw.as<float>(), dlb.as<float>(),
+                       dout.as<float>(), dso.as<long long>(), B, max_s, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    if (phase) KKX_CUDA(cudaMemcpy(phase, dph.p, (size_t)nph * 4, cudaMemcpyDeviceToHost));
+    KKX_CUDA(cudaMemcpy(har, dout.p, (size_t)ns * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int kkx_test_stft(int device, const float* x, int64_t n_x, int B, const int64_t* s_off, const int* h_off,
+                          const int* h_len, int rows_h, int replicate_pad, float* har) {
+  return run(device, [&] {
+    if (!x || !s_off || !h_off || !h_len || !har || B < 1) throw ArgError("kkx_test_stft: bad argument");
+    for (int b = 0; b < B; b++)
+      if (h_len[b] < 2 || s_off[b] < 0 || s_off[b] + 5LL * (h_len[b] - 1) > n_x || h_off[b] + h_len[b] > rows_h)
+        throw ArgError("kkx_test_stft: bad item");
+    DevBuf dx(x, (size_t)n_x * 4), dso(s_off, B * 8), dho(h_off, B * 4), dhl(h_len, B * 4);
+    DevBuf dh(har, (size_t)rows_h * 24 * 4);
+    launch_stft(dx.as<float>(), dso.as<long long>(), dh.as<float>(), 24, dho.as<int>(), dhl.as<int>(), replicate_pad, B,
+                max_of(B, h_len), 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(har, dh.p, (size_t)rows_h * 24 * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int kkx_test_istft(int device, const float* cp, int rows, int B, const int* h_off, const int* h_len, int fast,
+                           int64_t n_audio, const int64_t* s_off, float* audio, int16_t* pcm) {
+  return run(device, [&] {
+    if (!cp || !h_off || !h_len || !s_off || !audio || B < 1) throw ArgError("kkx_test_istft: bad argument");
+    for (int b = 0; b < B; b++)
+      if (h_len[b] < 2 || (s_off[b] & 3) || s_off[b] + 5LL * (h_len[b] - 1) > n_audio || h_off[b] + h_len[b] > rows)
+        throw ArgError("kkx_test_istft: bad item (audio offsets must be multiples of 4 samples)");
+    DevBuf dc(cp, (size_t)rows * 24 * 4), dho(h_off, B * 4), dhl(h_len, B * 4), dso(s_off, B * 8);
+    DevBuf da(audio, (size_t)n_audio * 4), dp(pcm, pcm ? (size_t)n_audio * 2 : 0);
+    launch_istft(dc.as<float>(), 24, dho.as<int>(), dhl.as<int>(), da.as<float>(), pcm ? dp.as<short>() : nullptr,
+                 dso.as<long long>(), fast, B, max_of(B, h_len), 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(audio, da.p, (size_t)n_audio * 4, cudaMemcpyDeviceToHost));
+    if (pcm) KKX_CUDA(cudaMemcpy(pcm, dp.p, (size_t)n_audio * 2, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int64_t kkx_test_durations(int device, const float* logits, const float* speeds, const float* feat, int C, int ldo,
+                                   int ocol, int B, const int* tok_off, const int* tok_len, int rows_tok, float* dur_float,
+                                   int32_t* pred_dur, int32_t* cum, int32_t* total, int32_t* fr_off, int32_t* idx,
+                                   float* out, int64_t capacity_rows) {
+  long long rows_fr = 0;
+  const int rc = run(device, [&] {
+    if (!logits || !speeds || !tok_off || !tok_len || B < 1 || C < 0 || ocol < 0 || ocol + C > ldo)
+      throw ArgError("kkx_test_durations: bad argument");
+    for (int b = 0; b < B; b++)
+      if (tok_len[b] < 1 || tok_len[b] > 512 || tok_off[b] < 0 || tok_off[b] + tok_len[b] > rows_tok)
+        throw ArgError("kkx_test_durations: bad item (1 <= N <= 512)");
+    DevBuf dl(logits, (size_t)rows_tok * 50 * 4), dsp(speeds, B * 4), dto(tok_off, B * 4), dtl(tok_len, B * 4);
+    DevBuf dpd(nullptr, (size_t)rows_tok * 4), ddf(nullptr, (size_t)rows_tok * 4);
+    DevBuf dcum(nullptr, (size_t)B * 512 * 4), dtot(nullptr, B * 4);
+    KKX_CUDA(cudaMemset(dpd.p, 0, (size_t)rows_tok * 4));
+    KKX_CUDA(cudaMemset(ddf.p, 0xFF, (size_t)rows_tok * 4));
+    KKX_CUDA(cudaMemset(dcum.p, 0xFF, (size_t)B * 512 * 4));
+    const int max_tok = max_of(B, tok_len);
+    launch_duration(dl.as<float>(), 50, dsp.as<float>(), dpd.as<int>(), ddf.as<float>(), dto.as<int>(), dtl.as<int>(), B,
+                    max_tok, 0);
+    launch_dur_scan(dpd.as<int>(), dcum.as<int>(), 512, dtot.as<int>(), dto.as<int>(), dtl.as<int>(), B, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    std::vector<int> tot(B);
+    KKX_CUDA(cudaMemcpy(tot.data(), dtot.p, B * 4, cudaMemcpyDeviceToHost));
+    if (dur_float) KKX_CUDA(cudaMemcpy(dur_float, ddf.p, (size_t)rows_tok * 4, cudaMemcpyDeviceToHost));
+    if (pred_dur) KKX_CUDA(cudaMemcpy(pred_dur, dpd.p, (size_t)rows_tok * 4, cudaMemcpyDeviceToHost));
+    if (cum) KKX_CUDA(cudaMemcpy(cum, dcum.p, (size_t)B * 512 * 4, cudaMemcpyDeviceToHost));
+    if (total) memcpy(total, tot.data(), B * 4);
+    // the frame level the model builds from the totals (Model::make_level: 32 gap rows, 8-row alignment)
+    std::vector<int> fo(B);
+    long long o = kGapRows;
+    for (int b = 0; b < B; b++) { fo[b] = (int)o; o = (o + tot[b] + kGapRows + 7) & ~7LL; }
+    rows_fr = o;
+    if (fr_off) memcpy(fr_off, fo.data(), B * 4);
+    if (!idx || !out || capacity_rows < rows_fr) return;   // size query
+    if (!feat) throw ArgError("kkx_test_durations: feat missing");
+    DevBuf dfo(fo.data(), B * 4), dfl(tot.data(), B * 4), didx(idx, (size_t)rows_fr * 4);
+    DevBuf dfeat(feat, (size_t)rows_tok * C * 4), dout(out, (size_t)rows_fr * ldo * 4);
+    const int max_fr = max_of(B, tot.data());
+    launch_expand_idx(dcum.as<int>(), 512, dtl.as<int>(), didx.as<int>(), dfo.as<int>(), dfl.as<int>(), B, max_fr, 0);
+    launch_gather_rows(dfeat.as<float>(), C, dto.as<int>(), didx.as<int>(), dfo.as<int>(), dfl.as<int>(), C,
+                       dout.as<float>(), ldo, ocol, B, max_fr, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(idx, didx.p, (size_t)rows_fr * 4, cudaMemcpyDeviceToHost));
+    KKX_CUDA(cudaMemcpy(out, dout.p, (size_t)rows_fr * ldo * 4, cudaMemcpyDeviceToHost));
+  });
+  return rc == KKX_OK ? (int64_t)rows_fr : (int64_t)rc;
+}
+
+KKX_API int kkx_test_pool_up(int device, const float* x, int rows_in, int C, int B, const int* in_off, const int* in_len,
+                             const float* scale, const float* shift, float slope, const float* w, const float* bias,
+                             const int* out_off, int rows_out, int Cpad, void* out) {
+  return run(device, [&] {
+    if (!x || !in_off || !in_len || !scale || !shift || !w || !bias || !out_off || !out || B < 1 || (Cpad && Cpad < C))
+      throw ArgError("kkx_test_pool_up: bad argument");
+    const size_t ob = Cpad ? (size_t)rows_out * Cpad * 2 : (size_t)rows_out * C * 4;
+    DevBuf dx(x, (size_t)rows_in * C * 4), dio(in_off, B * 4), dil(in_len, B * 4), doo(out_off, B * 4);
+    DevBuf dsc(scale, (size_t)B * C * 4), dsh(shift, (size_t)B * C * 4), dw(w, (size_t)C * 3 * 4), db(bias, C * 4);
+    DevBuf dout(out, ob);
+    if (Cpad)
+      launch_pool_up_bf16(dx.as<float>(), C, dsc.as<float>(), dsh.as<float>(), slope, dw.as<float>(), db.as<float>(), C,
+                          dout.p, Cpad, rows_out, dio.as<int>(), dil.as<int>(), doo.as<int>(), B, max_of(B, in_len), 0);
+    else
+      launch_pool_up(dx.as<float>(), C, dsc.as<float>(), dsh.as<float>(), slope, dw.as<float>(), db.as<float>(), C,
+                     dout.as<float>(), C, dio.as<int>(), dil.as<int>(), doo.as<int>(), B, max_of(B, in_len), 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(out, dout.p, ob, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int kkx_test_post_conv(int device, const float* x, int rows, int B, const int* off, const int* len, const float* w,
+                               const float* bias, float slope, float* out) {
+  return run(device, [&] {
+    if (!x || !off || !len || !w || !bias || !out || B < 1) throw ArgError("kkx_test_post_conv: bad argument");
+    if (!arb_conv_supported(128, 7, 1, B)) throw ArgError("kkx_test_post_conv: unsupported batch");
+    long long sum_m = 0;
+    for (int b = 0; b < B; b++) {
+      if (len[b] < 1 || off[b] < kGapRows || off[b] + len[b] + kGapRows > rows) throw ArgError("kkx_test_post_conv: bad item");
+      sum_m += len[b];
+    }
+    // conv_post zero-padded to 128 output channels, bf16 [128][7][128], as the model packs it (WeightSet::make_tc)
+    std::vector<uint16_t> hw((size_t)128 * 7 * 128, 0);
+    for (size_t i = 0; i < (size_t)22 * 7 * 128; i++) hw[i] = host_bf16(w[i]);
+    std::vector<float> b128(128, 0.f);
+    memcpy(b128.data(), bias, 22 * 4);
+    const std::vector<int> tiles = level_tiles(B, len, arb_tile_rows(128));
+    DevBuf dx(x, (size_t)rows * 128 * 4), dw(hw.data(), hw.size() * 2), db(b128.data(), 128 * 4);
+    DevBuf doff(off, B * 4), dlen(len, B * 4), dts(tiles.data(), (B + 1) * 4), dout(out, (size_t)rows * 24 * 4);
+    alignas(64) unsigned char tmB[128];
+    make_tmap_bf16(tmB, dw.p, 7LL * 128, 128, 7LL * 128, tc_box_n(128));
+    ArbConvArgs a;
+    a.C = 128; a.ks = 7; a.dil = 1; a.pad = 3; a.off = doff.as<int>(); a.len = dlen.as<int>(); a.B = B;
+    a.sum_m = sum_m; a.tile_start = dts.as<int>(); a.total_tiles = tiles[B];
+    a.x = dx.p; a.in_bf16 = 0; a.tmB = tmB; a.bias = db.as<float>();
+    a.out_f32 = dout.as<float>(); a.post = 1; a.cout = 22; a.ldo = 24; a.slope = slope;
+    launch_arb_conv(a, 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(out, dout.p, (size_t)rows * 24 * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int kkx_test_curve_conv(int device, const float* x, int rows_x, int B, const int* x_off, const int* x_len,
+                                const float* w3, const float* bias, float* out, int rows_out, int ldo, int ocol,
+                                const int* out_off, const int* out_len) {
+  return run(device, [&] {
+    if (!x || !x_off || !x_len || !w3 || !bias || !out || !out_off || !out_len || B < 1 || ocol < 0 || ocol >= ldo)
+      throw ArgError("kkx_test_curve_conv: bad argument");
+    DevBuf dx(x, (size_t)rows_x * 4), dxo(x_off, B * 4), dxl(x_len, B * 4), dw(w3, 3 * 4), db(bias, 4);
+    DevBuf doo(out_off, B * 4), dol(out_len, B * 4), dout(out, (size_t)rows_out * ldo * 4);
+    launch_curve_conv(dx.as<float>(), dxo.as<int>(), dxl.as<int>(), dw.as<float>(), db.as<float>(), dout.as<float>(), ldo,
+                      ocol, doo.as<int>(), dol.as<int>(), B, max_of(B, out_len), 0);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(out, dout.p, (size_t)rows_out * ldo * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
+KKX_API int kkx_test_add_rows_stats(int device, float* a, const float* b, int rows, int C, int B, const int* off,
+                                    const int* len, uint16_t* out_bf16, float* part) {
+  return run(device, [&] {
+    if (!a || !b || !off || !len || !part || B < 1) throw ArgError("kkx_test_add_rows_stats: bad argument");
+    const int max_len = max_of(B, len);
+    const size_t np = (size_t)B * ((max_len + kStatRows - 1) / kStatRows) * 2 * C;
+    DevBuf da(a, (size_t)rows * C * 4), db(b, (size_t)rows * C * 4), doff(off, B * 4), dlen(len, B * 4);
+    DevBuf dob(out_bf16, out_bf16 ? (size_t)rows * C * 2 : 0), dp(nullptr, np * 4);
+    KKX_CUDA(cudaMemset(dp.p, 0xFF, np * 4));
+    // in place, as the model calls it (x += x_source)
+    launch_add_rows_stats(da.as<float>(), db.as<float>(), da.as<float>(), C, dp.as<float>(), doff.as<int>(), dlen.as<int>(),
+                          B, max_len, 0, out_bf16 ? dob.p : nullptr);
+    KKX_CUDA(cudaDeviceSynchronize());
+    KKX_CUDA(cudaMemcpy(a, da.p, (size_t)rows * C * 4, cudaMemcpyDeviceToHost));
+    if (out_bf16) KKX_CUDA(cudaMemcpy(out_bf16, dob.p, (size_t)rows * C * 2, cudaMemcpyDeviceToHost));
+    KKX_CUDA(cudaMemcpy(part, dp.p, np * 4, cudaMemcpyDeviceToHost));
+  });
+}
+
 }  // extern "C"
