@@ -185,7 +185,7 @@ KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes);
  *            e folded to u = e >= 0 ? 2e : -2e - 1 and coded as (u >> k) zeros, a one, the low k bits.  Cost
  *            8 + 16 o + 6 + sum over partitions (4 + sum (u >> k) + n_part (k + 1)) bits; ties go to the smaller
  *            o, then q, then k.  VERBATIM (02, bs x 16 bits) only if strictly cheaper (8 + 16 bs bits), so no
- *            frame is larger than verbatim.  No Rice escapes, no LPC.
+ *            frame is larger than verbatim.  No Rice escapes.  LPC subframes only with "flac_lpc_order" (below).
  *   Release the buffer with kkx_release_flac.  KKX_ERR_ARG for a null out_bytes or out_byte_offsets. */
 KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                                  const float* styles, const float* speeds, uint8_t** out_bytes,
@@ -477,13 +477,47 @@ KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, i
  *                 resampling pass-through, without a gain) to plain output.
  *                 Not provided: measurement at the output rate or of the limiter's output, a momentary / short-term
  *                 time series (a loudness curve), reports of coalesced and kkx_submit batches.
+ *   "flac_lpc_order"  linear prediction in FLAC output: 0 (DEFAULT) = off, every byte and launch as without it, for
+ *                 every entry point; p in 1..12 (12: the streamable-subset limit up to 48 kHz, RFC 9639 section 7) adds
+ *                 one LPC candidate of order p per frame.  Any other value is KKX_ERR_ARG and the session keeps its
+ *                 setting.  One setting per session, followed by kkx_infer_batch_flac and by KKX_ENC_FLAC
+ *                 kkx_infer_programs runs that start after the call; no other encoding is affected.  Frame i's
+ *                 subframe (x = its bs int16 samples), in addition to the kkx_infer_batch_flac rules:
+ *                 1. Eligibility: CONSTANT frames stay CONSTANT; a frame has an LPC candidate only if p < bs.
+ *                 2. Window (integers only): M[k] = nint(2^15 0.5 (1 - cos(pi (k + 0.5) / 1024))), k = 0..1023,
+ *                    nint(v) = floor(v + 0.5), designed in double on the host.  L = bs >> 2; W[i] = 2^15 for
+ *                    L <= i < bs - L; for i < L, W[i] = W[bs - 1 - i] = M[(i 1024) / L] (integer division; L = 0:
+ *                    no taper).  xw[i] = (x[i] W[i] + 2^14) >> 15 (arithmetic shift).
+ *                 3. Autocorrelation: R[l] = sum over i = l..bs-1 of xw[i] xw[i - l], l = 0..p, exact in int64
+ *                    (|R| < 2^42), then converted to double (exact).
+ *                 4. Levinson-Durbin in IEEE binary64, one rounding per operation, no fused multiply-add, in this
+ *                    order: err = R[0]; for i = 1..p: acc = R[i]; for j = 1..i-1 ascending acc = acc - a[j] R[i - j];
+ *                    k = acc / err; a'[j] = a[j] - k a[i - j] for j = 1..i-1 (the old a), a'[i] = k;
+ *                    err = err (1 - k k).  No candidate if R[0] = 0 or err <= 0 after any step.
+ *                 5. Quantisation, precision 12: cmax = max |a_j|, no candidate if 0; e = the exponent of
+ *                    frexp(cmax) (cmax = m 2^e, 0.5 <= m < 1); shift = min(15, 11 - e), no candidate if < 0; ef = 0,
+ *                    for j = 1..p: ef = ef + a_j 2^shift, q_j = clamp(floor(ef + 0.5), -2048, 2047), ef = ef - q_j.
+ *                 6. Residual: e[s] = x[s] - ((sum over j = 1..p of q_j x[s - j]) >> shift), s = p..bs-1 (the sum
+ *                    exact in int32); no candidate if any folded u >= 2^20.
+ *                 7. Cost 8 + 16 p + 4 + 5 + 12 p + 6 + the partition / Rice cost of FIXED with o = p (partition
+ *                    order q with (bs >> q) > p, ties to the smaller q, then k).  The cheaper of the best FIXED and
+ *                    the LPC candidate is picked, ties going to FIXED; VERBATIM only if strictly cheaper than that
+ *                    pick.  So no frame is larger than with the option off, and a stream where LPC never wins is
+ *                    byte-identical to it.
+ *                 8. Bitstream: subframe header 0, type 32 + p - 1, wasted bits 0; p warm-up samples (16 bits each);
+ *                    precision - 1 = 11 (4 bits); shift (5-bit two's complement, 0..15); q_1..q_p (12 bits each, q_1
+ *                    multiplies x[s - 1]); the residual as for FIXED (method 00, 4-bit partition order, 4-bit k per
+ *                    partition, the first partition holding (bs >> q) - p residuals).
+ *                 Frame headers, CRCs, STREAMINFO and MD5 = 0 as without the option.  Purity and identity as for FLAC
+ *                 programs: a file's bytes are a function of its samples alone.  Device work: the same three
+ *                 launches; flac_analyze runs its LPC variant, which designs the predictor on the block it holds.
  * kkx_get_stat keys: "launches", "last_frames", "gpu_us", "precision", "coalesced_batches",
  * "coalesced_requests", "coalesced_largest", "async_batches", "async_requests", "frame_groups",
  * "group_first:<g>" (first item of frame group g of the last run), "weights_sessions" (sessions sharing this
  * ctx's device weight set), "weights_bytes", "weights_from_onnx", "graph_replays", "out_rate", "loudness_target",
  * "true_peak_max", "loudness_items" (items -- programs after kkx_infer_programs -- kkx_last_loudness reports now; 0
  * if it would fail with KKX_ERR_STATE), "limiter", "limiter_items" (the same for kkx_last_limiter), "loudness_report"
- * (the option's value). */
+ * (the option's value), "flac_lpc_order" (the option's value). */
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value);
 KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key); /* "launches", "last_frames", "gpu_us" ... */
 

@@ -130,6 +130,12 @@ KKX_API int kkx_test_resample(int device, const float* x, int32_t B, const int64
  * and their offsets into byte_offsets [B + 1]; returns the total byte count or < 0. */
 KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
                               uint8_t* dst, int64_t capacity, int64_t* byte_offsets);
+/* The same with "flac_lpc_order" = order (0..12; 0 gives kkx_test_flac's bytes). */
+KKX_API int64_t kkx_test_flac_lpc(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
+                                  int32_t order, uint8_t* dst, int64_t capacity, int64_t* byte_offsets);
+/* Host only: the LPC window's taper table M [1024] of "flac_lpc_order" rule 2 (kkx.h), as the encoder uploads it.
+ * Returns 0, or < 0 for a null m1024. */
+KKX_API int kkx_test_flac_lpc_window(int32_t* m1024);
 /* MP3 encoder (kernels_mp3.cu) on caller-supplied PCM, like kkx_test_flac: kbps as in kkx_infer_batch_mp3 (0 = the
  * default of the rate's version).  Returns the total byte count or < 0. */
 KKX_API int64_t kkx_test_mp3(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate, int32_t kbps,

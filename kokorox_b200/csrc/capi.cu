@@ -930,6 +930,11 @@ KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
       if (value != 0 && value != 1)
         throw ArgError("loudness_report " + std::to_string(value) + " is not supported: give 0 (off) or 1 (on)");
       o.loudness_report = (int)value;
+    } else if (k == "flac_lpc_order") {
+      if (value < 0 || value > kMaxLpcOrder)
+        throw ArgError("flac_lpc_order " + std::to_string(value) +
+                       " is not supported: give 0 (off) or an LPC order in 1..12");
+      o.flac_lpc_order = (int)value;
     }
     else throw ArgError("unknown option: " + k);
   });
@@ -949,6 +954,7 @@ KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
   if (k == "loudness_items") return report_items(ctx, kRepLoudness);
   if (k == "limiter") return ctx->model->opt.limiter;
   if (k == "loudness_report") return ctx->model->opt.loudness_report;
+  if (k == "flac_lpc_order") return ctx->model->opt.flac_lpc_order;
   if (k == "limiter_items") return report_items(ctx, kRepLimiter);
   if (k == "coalesced_batches") return ctx->coalesced_batches;
   if (k == "coalesced_requests") return ctx->coalesced_requests;

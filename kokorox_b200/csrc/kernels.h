@@ -336,14 +336,19 @@ void launch_loudness_range(const long long* in_len, const long long* seg_off, co
 //   Item b is pcm[soff[b] .. soff[b + 1]) (>= 1 sample) and has flac_frames(n_b) frames of 4096 samples; foff[b + 1]
 //   is the prefix sum of those counts (F = foff[B] frames).  launch_flac writes item b's stream to
 //   out[item_off[b] .. item_off[b + 1]) (item_off [B + 1], device); out must hold flac_bound(B, F, samples) bytes and
-//   work flac_work_bytes(F).  rate: one of the nine "out_rate" values.  Three launches, profile names
-//   "flac_analyze", "flac_scan", "flac_pack".
+//   work flac_work_bytes(F).  rate: one of the nine "out_rate" values.  lpc_order: kkx.h "flac_lpc_order", 0 (off)
+//   or 1..kMaxLpcOrder; it adds one LPC candidate per frame and never makes a frame larger.  Three launches with LPC
+//   off and on, profile names "flac_analyze", "flac_scan", "flac_pack"; with LPC on, flac_analyze is its LPC variant
+//   (the predictor is designed on the block the CTA already holds, and one more Rice-cost row is filled).
+//   flac_lpc_window: host copy of the LPC window's taper table M [1024] (kkx_test_flac_lpc_window).
+constexpr int kMaxLpcOrder = 12;
 long long flac_frames(long long n);
 long long flac_bound(long long n_items, long long n_frames, long long n_samples);
 size_t flac_work_bytes(long long n_frames);
 bool flac_rate_ok(int rate);
-void launch_flac(const short* pcm, const long long* soff, const int* foff, int B, int F, int rate, void* work,
-                 unsigned char* out, long long* item_off, cudaStream_t st);
+void flac_lpc_window(int* m1024);
+void launch_flac(const short* pcm, const long long* soff, const int* foff, int B, int F, int rate, int lpc_order,
+                 void* work, unsigned char* out, long long* item_off, cudaStream_t st);
 
 // Constant-bitrate MPEG audio Layer III of 16-bit mono PCM (kernels_mp3.cu; the stream rules are in kkx.h,
 // kkx_infer_batch_mp3).  A stream of n samples has mp3_frames(fmt, n) frames; frame f of it takes bytes

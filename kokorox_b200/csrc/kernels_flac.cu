@@ -1,16 +1,20 @@
 // kernels_flac.cu -- lossless FLAC encoding of 16-bit mono PCM on the device (kkx_infer_batch_flac, kkx.h).
 //
 // Every item becomes one FLAC stream (RFC 9639, streamable subset): a 42-byte head (fLaC + STREAMINFO), then frames
-// of 4096 samples, each with one CONSTANT, FIXED (order 0..4, Rice partitions) or VERBATIM subframe.  The choice and
-// every byte are a pure function of the item's samples (integer arithmetic only, ties broken by a fixed rule), so an
-// item encodes to the same bytes whatever batch it is in.  Three launches:
-//   flac_analyze  one CTA per frame: cost of every (order, partition order, Rice parameter) -> choice + frame size
+// of 4096 samples, each with one CONSTANT, FIXED (order 0..4, Rice partitions), LPC (order p = "flac_lpc_order", when
+// that is on) or VERBATIM subframe.  The choice and every byte are a pure function of the item's samples (integer
+// arithmetic, plus the LPC coefficient design in IEEE binary64 with one rounding per operation in a fixed order; ties
+// broken by a fixed rule), so an item encodes to the same bytes whatever batch it is in.  Three launches:
+//   flac_analyze  one CTA per frame: cost of every (order, partition order, Rice parameter) -> choice + frame size;
+//                 its LPC variant first designs the frame's order-p predictor (window, autocorrelation, Levinson-
+//                 Durbin, quantisation) on the block it already holds in shared memory
 //   flac_scan     one CTA: byte offset of every frame and every item
 //   flac_pack     one CTA per frame: bit positions by a block scan, codes OR-ed into a shared bit buffer, CRC-8 of
 //                 the header and CRC-16 of the frame, then the frame's bytes; the CTA of an item's first frame also
 //                 writes the item's 42-byte head (STREAMINFO needs the item's smallest and largest frame).
 #include "kernels.h"
 #include "bitpack.cuh"
+#include <cmath>
 
 namespace kkx {
 
@@ -22,14 +26,21 @@ constexpr int kMaxPorder = 8;         // 256 partitions at most
 constexpr int kParts = 1 << kMaxPorder;
 constexpr int kOrders = 5, kRice = 15;
 constexpr int kHead = 42;             // "fLaC" + metadata block header + 34-byte STREAMINFO
+constexpr int kLpcPrec = 12;          // quantised coefficient precision (bits)
+constexpr int kLpcWin = 1024;         // entries of the window's taper table M
 
-enum : int { SUB_CONSTANT = 0, SUB_FIXED = 1, SUB_VERBATIM = 2 };
+enum : int { SUB_CONSTANT = 0, SUB_FIXED = 1, SUB_VERBATIM = 2, SUB_LPC = 3 };
 
 struct FlacFrame {        // analysis result of one frame
   int bytes;              // whole frame, header and CRC-16 included
   int kind, order, porder;
-  unsigned char k[kParts];  // Rice parameter of each partition (FIXED)
+  unsigned char k[kParts];  // Rice parameter of each partition (FIXED, LPC)
+  int shift;                // LPC: quantisation shift and coefficients q_1..q_order
+  short q[kMaxLpcOrder];
 };
+
+// M[k] = nint(2^15 * 0.5 * (1 - cos(pi (k + 0.5) / 1024))), designed in double on the host, uploaded once per device
+__device__ int g_lpc_window[kLpcWin];
 
 __host__ __device__ inline int utf8_len(unsigned v) {
   return v < 0x80 ? 1 : v < 0x800 ? 2 : v < 0x10000 ? 3 : v < 0x200000 ? 4 : v < 0x4000000 ? 5 : 6;
@@ -81,23 +92,90 @@ __device__ __forceinline__ unsigned fold_residual(const T* x, int s, int o) {
   return e >= 0 ? 2u * (unsigned)e : 2u * (unsigned)(-e) - 1u;
 }
 
+__device__ __forceinline__ unsigned fold(int e) { return e >= 0 ? 2u * (unsigned)e : 2u * (unsigned)(-e) - 1u; }
+
+// LPC residual at sample s >= p: x[s] - ((sum_j q_j x[s - j]) >> shift), the sum exact in int32 (< 2^30)
+__device__ __forceinline__ int lpc_residual(const short* x, int s, int p, const int* q, int shift) {
+  int acc = 0;
+  for (int j = 0; j < p; j++) acc += q[j] * (int)x[s - 1 - j];
+  return (int)x[s] - (acc >> shift);
+}
+
 __device__ __forceinline__ int finest_porder(int bs) { return min(kMaxPorder, __ffs(bs) - 1); }
+
+struct LpcDesign { int valid, shift, q[kMaxLpcOrder]; };
+
+// Levinson-Durbin and quantisation of kkx.h's "flac_lpc_order" rules 4-5 on one thread: binary64 with one rounding
+// per operation (the _rn intrinsics are never contracted into a fused multiply-add), in the order the rules give.
+// Every loop has compile-time bounds (guarded by p), so the arrays live in registers.
+__device__ __forceinline__ LpcDesign lpc_design(const long long (&Rl)[kMaxLpcOrder + 1], int p) {
+  LpcDesign out{};
+  double R[kMaxLpcOrder + 1], a[kMaxLpcOrder + 1] = {};
+#pragma unroll
+  for (int l = 0; l <= kMaxLpcOrder; l++) R[l] = (double)Rl[l];   // |R| < 2^42: exact
+  if (R[0] == 0.0) return out;
+  double err = R[0];
+#pragma unroll
+  for (int i = 1; i <= kMaxLpcOrder; i++) {
+    if (i > p) break;
+    double acc = R[i];
+#pragma unroll
+    for (int j = 1; j < i; j++) acc = __dsub_rn(acc, __dmul_rn(a[j], R[i - j]));
+    const double k = __ddiv_rn(acc, err);
+    double na[kMaxLpcOrder + 1];
+#pragma unroll
+    for (int j = 1; j < i; j++) na[j] = __dsub_rn(a[j], __dmul_rn(k, a[i - j]));
+#pragma unroll
+    for (int j = 1; j < i; j++) a[j] = na[j];
+    a[i] = k;
+    err = __dmul_rn(err, __dsub_rn(1.0, __dmul_rn(k, k)));
+    if (!(err > 0.0)) return out;
+  }
+  double cmax = 0.0;
+#pragma unroll
+  for (int j = 1; j <= kMaxLpcOrder; j++)
+    if (j <= p) cmax = fmax(cmax, fabs(a[j]));
+  if (cmax == 0.0) return out;
+  int e;
+  frexp(cmax, &e);
+  const int shift = min(15, kLpcPrec - 1 - e);
+  if (shift < 0) return out;
+  const double scale = ldexp(1.0, shift);
+  double ef = 0.0;
+#pragma unroll
+  for (int j = 1; j <= kMaxLpcOrder; j++) {
+    if (j > p) break;
+    ef = __dadd_rn(ef, __dmul_rn(a[j], scale));
+    const double qd = fmin(fmax(floor(__dadd_rn(ef, 0.5)), -2048.0), 2047.0);
+    out.q[j - 1] = (int)qd;
+    ef = __dsub_rn(ef, qd);
+  }
+  out.shift = shift;
+  out.valid = 1;
+  return out;
+}
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------- analysis
-// Shared: the block, then the Rice sums S[o][k][p] = sum over residual samples of finest partition p of (u >> k).  An
-// order-o sum leaves out the o warm-up samples, so the first partition holds (bs >> q) - o residuals at every level.
-// Sums of neighbours give the coarser partition orders; all fit in 32 bits (at most 4096 samples of u < 2^20).
+// Shared: the block, then the Rice sums S[r][k][p] = sum over residual samples of finest partition p of (u >> k), one
+// row r per candidate predictor: FIXED orders 0..4, and (kLpc) the frame's LPC predictor of order p as row 5.  A row
+// with w warm-up samples (w = o, or p) leaves those out, so the first partition holds (bs >> q) - w residuals at every
+// level.  Sums of neighbours give the coarser partition orders; all fit in 32 bits (at most 4096 samples of u < 2^20).
+// kLpc = false is the encoder without "flac_lpc_order"; p is ignored there.
+template <bool kLpc>
 __global__ void __launch_bounds__(kThreads) flac_analyze_kernel(const short* __restrict__ pcm,
                                                                 const long long* __restrict__ soff,
-                                                                const int* __restrict__ foff, int B, int rate,
+                                                                const int* __restrict__ foff, int B, int rate, int p,
                                                                 FlacFrame* __restrict__ frames) {
+  constexpr int kRows = kLpc ? kOrders + 1 : kOrders;
   extern __shared__ unsigned char fa_smem[];
   short* xs = reinterpret_cast<short*>(fa_smem);
-  unsigned* S = reinterpret_cast<unsigned*>(fa_smem + kBlock * sizeof(short));          // [kOrders * kRice][kParts]
-  unsigned* cost = S + kOrders * kRice * kParts;                                        // [o][q]
-  unsigned char* kbest = reinterpret_cast<unsigned char*>(cost + kOrders * (kMaxPorder + 1));  // [o][2^q - 1 + j]
+  unsigned* S = reinterpret_cast<unsigned*>(fa_smem + kBlock * sizeof(short));          // [kRows * kRice][kParts]
+  unsigned* cost = S + kRows * kRice * kParts;                                          // [r][q]
+  unsigned char* kbest = reinterpret_cast<unsigned char*>(cost + kRows * (kMaxPorder + 1));  // [r][2^q - 1 + j]
   __shared__ int s_choice[3];
+  __shared__ __align__(16) long long s_R[kLpc ? kThreads / 32 : 1][16];   // [warp][lag], 16-byte rows
+  __shared__ LpcDesign s_lpc;
 
   const int f = blockIdx.x, t = threadIdx.x;
   const int b = frame_item(foff, B, f);
@@ -107,8 +185,9 @@ __global__ void __launch_bounds__(kThreads) flac_analyze_kernel(const short* __r
   const int bs = (int)min((long long)kBlock, n - s0);
   const short* xg = pcm + soff[b] + s0;
   for (int i = t; i < bs; i += kThreads) xs[i] = xg[i];
-  for (int i = t; i < kOrders * kRice * kParts; i += kThreads) S[i] = 0u;
-  for (int i = t; i < kOrders * (kMaxPorder + 1); i += kThreads) cost[i] = 0u;
+  if (!kLpc)   // (the LPC variant first uses S as the windowed block)
+    for (int i = t; i < kRows * kRice * kParts; i += kThreads) S[i] = 0u;
+  for (int i = t; i < kRows * (kMaxPorder + 1); i += kThreads) cost[i] = 0u;
   __syncthreads();
   const int first = xs[0];
   bool same = true;
@@ -122,27 +201,81 @@ __global__ void __launch_bounds__(kThreads) flac_analyze_kernel(const short* __r
     return;
   }
 
+  bool lpc = false;   // the frame has an LPC candidate (uniform over the CTA)
+  if constexpr (kLpc) {
+    if (t == 0) s_lpc.valid = 0;
+    if (p < bs) {
+      // window (integers only), then R[l] = sum_i xw[i] xw[i - l], exact in int64 whatever the order of the sums
+      int* xw = reinterpret_cast<int*>(S);
+      const int L = bs >> 2;
+      for (int i = t; i < bs; i += kThreads) {
+        int w = 1 << 15;
+        if (i < L) w = g_lpc_window[(i * kLpcWin) / L];
+        else if (i >= bs - L) w = g_lpc_window[((bs - 1 - i) * kLpcWin) / L];
+        xw[i] = ((int)xs[i] * w + (1 << 14)) >> 15;
+      }
+      __syncthreads();
+      long long r[kMaxLpcOrder + 1];
+#pragma unroll
+      for (int l = 0; l <= kMaxLpcOrder; l++) r[l] = 0;
+      for (int i = t; i < bs; i += kThreads) {
+        const int v = xw[i];
+#pragma unroll
+        for (int l = 0; l <= kMaxLpcOrder; l++)
+          if (l <= p && i >= l) r[l] += (long long)(v * xw[i - l]);   // |xw| <= 2^15: the product fits in int32
+      }
+#pragma unroll
+      for (int l = 0; l <= kMaxLpcOrder; l++) {
+#pragma unroll
+        for (int d = 16; d; d >>= 1) r[l] += __shfl_xor_sync(0xffffffffu, r[l], d);
+        if ((t & 31) == 0) s_R[t >> 5][l] = r[l];
+      }
+      __syncthreads();
+      if (t == 0) {
+        long long R[kMaxLpcOrder + 1];
+#pragma unroll
+        for (int l = 0; l <= kMaxLpcOrder; l++) {
+          R[l] = 0;
+#pragma unroll
+          for (int w = 0; w < kThreads / 32; w++) R[l] += s_R[w][l];
+        }
+        s_lpc = lpc_design(R, p);
+      }
+    }
+    for (int i = t; i < kRows * kRice * kParts; i += kThreads) S[i] = 0u;
+    __syncthreads();
+    lpc = s_lpc.valid != 0;
+  }
+
   const int qmax = finest_porder(bs);
   const int pf = bs >> qmax;                 // finest partition size
+  bool wide = false;                         // an LPC residual folds to u >= 2^20: no LPC candidate
   {
-    unsigned acc[kOrders][kRice];
+    int lq[kLpc ? kMaxLpcOrder : 1];
+    int lshift = 0;
+    if constexpr (kLpc) {
 #pragma unroll
-    for (int o = 0; o < kOrders; o++)
+      for (int j = 0; j < kMaxLpcOrder; j++) lq[j] = j < p ? s_lpc.q[j] : 0;
+      lshift = s_lpc.shift;
+    }
+    unsigned acc[kRows][kRice];
+#pragma unroll
+    for (int o = 0; o < kRows; o++)
 #pragma unroll
       for (int k = 0; k < kRice; k++) acc[o][k] = 0u;
     const int c0 = t * kPer, c1 = min(c0 + kPer, bs);
-    int p = c0 / pf;
+    int pt = c0 / pf;
     for (int s = c0; s < c1; s++) {
       const int ps = s / pf;
-      if (ps != p) {   // flush the previous partition's share (integer adds: the order of arrival does not matter)
+      if (ps != pt) {   // flush the previous partition's share (integer adds: the order of arrival does not matter)
 #pragma unroll
-        for (int o = 0; o < kOrders; o++)
+        for (int o = 0; o < kRows; o++)
 #pragma unroll
           for (int k = 0; k < kRice; k++) {
-            if (acc[o][k]) atomicAdd(&S[(o * kRice + k) * kParts + p], acc[o][k]);
+            if (acc[o][k]) atomicAdd(&S[(o * kRice + k) * kParts + pt], acc[o][k]);
             acc[o][k] = 0u;
           }
-        p = ps;
+        pt = ps;
       }
 #pragma unroll
       for (int o = 0; o < kOrders; o++) {
@@ -152,29 +285,46 @@ __global__ void __launch_bounds__(kThreads) flac_analyze_kernel(const short* __r
           for (int k = 0; k < kRice; k++) acc[o][k] += u >> k;
         }
       }
+      if constexpr (kLpc) {
+        if (lpc && s >= p) {
+          int a = 0;
+#pragma unroll
+          for (int j = 0; j < kMaxLpcOrder; j++)
+            if (j < p) a += lq[j] * (int)xs[s - 1 - j];
+          const unsigned u = fold((int)xs[s] - (a >> lshift));
+          wide |= u >= (1u << 20);
+#pragma unroll
+          for (int k = 0; k < kRice; k++) acc[kOrders][k] += u >> k;
+        }
+      }
     }
     if (c0 < c1) {
 #pragma unroll
-      for (int o = 0; o < kOrders; o++)
+      for (int o = 0; o < kRows; o++)
 #pragma unroll
         for (int k = 0; k < kRice; k++)
-          if (acc[o][k]) atomicAdd(&S[(o * kRice + k) * kParts + p], acc[o][k]);
+          if (acc[o][k]) atomicAdd(&S[(o * kRice + k) * kParts + pt], acc[o][k]);
     }
   }
-  __syncthreads();
+  if constexpr (kLpc) {
+    if (__syncthreads_or(wide)) lpc = false;
+  } else {
+    __syncthreads();
+  }
 
   // from the finest level up: per partition the cheapest k (ties: smaller k), then merge neighbours in place.  The
   // sum of level q's partition j sits at index j << (qmax - q).
   for (int q = qmax; q >= 0; q--) {
     const int np = 1 << q, psize = bs >> q, sh = qmax - q;
 #pragma unroll
-    for (int o = 0; o < kOrders; o++) {
+    for (int o = 0; o < kRows; o++) {
+      const int warm = o < kOrders ? o : p;
       // the cheapest k of a partition costs at most n_part (2^20 >> 14) + 15 n_part bits, so a level's total fits in
       // 32 bits; one atomic per warp (the 64-bit shared atomic is a compare-and-swap loop)
       unsigned part = 0u;
-      if (psize > o) {
+      if (psize > warm && (o < kOrders || lpc)) {
         for (int j = t; j < np; j += kThreads) {
-          const long long cnt = psize - (j == 0 ? o : 0);
+          const long long cnt = psize - (j == 0 ? warm : 0);
           unsigned long long best = ~0ull;
           int kb = 0;
           for (int k = 0; k < kRice; k++) {
@@ -191,7 +341,7 @@ __global__ void __launch_bounds__(kThreads) flac_analyze_kernel(const short* __r
     __syncthreads();
     if (q > 0) {
       const int nh = np >> 1;
-      for (int w = t; w < kOrders * kRice * nh; w += kThreads) {
+      for (int w = t; w < kRows * kRice * nh; w += kThreads) {
         const int ok = w / nh, j = w - ok * nh;
         S[ok * kParts + ((2 * j) << sh)] += S[ok * kParts + ((2 * j + 1) << sh)];
       }
@@ -208,19 +358,35 @@ __global__ void __launch_bounds__(kThreads) flac_analyze_kernel(const short* __r
         const unsigned long long c = 8ull + 16ull * o + 6ull + cost[o * (kMaxPorder + 1) + q];
         if (c < best) { best = c; bo = o; bq = q; }
       }
+    int kind = SUB_FIXED;
+    if (kLpc && lpc) {   // the cheapest partition order of the LPC predictor; it replaces FIXED only when cheaper
+      unsigned long long lbest = ~0ull;
+      int lq = 0;
+      for (int q = 0; q <= qmax; q++) {
+        if ((bs >> q) <= p) continue;
+        const unsigned long long c = 8ull + 16ull * p + 4 + 5 + 12ull * p + 6 + cost[kOrders * (kMaxPorder + 1) + q];
+        if (c < lbest) { lbest = c; lq = q; }
+      }
+      if (lbest < best) { best = lbest; kind = SUB_LPC; bo = p; bq = lq; }
+    }
     const unsigned long long verbatim = 8ull + 16ull * bs;
-    const int kind = verbatim < best ? SUB_VERBATIM : SUB_FIXED;
+    if (verbatim < best) kind = SUB_VERBATIM;
     const unsigned long long bits = kind == SUB_VERBATIM ? verbatim : best;
     FlacFrame& fr = frames[f];
     fr.kind = kind; fr.order = bo; fr.porder = bq;
     fr.bytes = header_bytes(fi, bs, rate) + (int)((bits + 7) / 8) + 2;
+    if (kLpc && kind == SUB_LPC) fr.shift = s_lpc.shift;
     s_choice[0] = kind; s_choice[1] = bo; s_choice[2] = bq;
   }
   __syncthreads();
-  if (s_choice[0] == SUB_FIXED) {
-    const int o = s_choice[1], np = 1 << s_choice[2];
-    for (int j = t; j < np; j += kThreads) frames[f].k[j] = kbest[o * (2 * kParts - 1) + (np - 1) + j];
+  if (s_choice[0] == SUB_FIXED || s_choice[0] == SUB_LPC) {
+    const int row = s_choice[0] == SUB_LPC ? kOrders : s_choice[1], np = 1 << s_choice[2];
+    for (int j = t; j < np; j += kThreads) frames[f].k[j] = kbest[row * (2 * kParts - 1) + (np - 1) + j];
   }
+  // one coefficient per thread, plain 16-bit stores.  (A thread-0 loop over j < p was compiled, CUDA 12.9 for
+  // sm_100a, into paired 32-bit stores whose upper half came from the wrong register: flac_pack then rebuilt other
+  // residuals than the ones costed here.)
+  if (kLpc && s_choice[0] == SUB_LPC && t < p) frames[f].q[t] = (short)s_lpc.q[t];
 }
 
 // ---------------------------------------------------------------------------------------------- offsets
@@ -311,6 +477,7 @@ __global__ void __launch_bounds__(kThreads) flac_pack_kernel(const short* __rest
   __shared__ unsigned bits[kWords];
   __shared__ unsigned short crc_tab[256];
   __shared__ unsigned char ks[kParts];
+  __shared__ int lq[kMaxLpcOrder];
   __shared__ int warp_sum[kThreads / 32];
   __shared__ unsigned s_crc;
   __shared__ int s_hdr;
@@ -323,10 +490,13 @@ __global__ void __launch_bounds__(kThreads) flac_pack_kernel(const short* __rest
   const int bs = (int)min((long long)kBlock, n - s0);
   const FlacFrame& fr = frames[f];
   const int nbytes = fr.bytes, kind = fr.kind, o = fr.order, q = fr.porder;
+  const bool lpc = kind == SUB_LPC;
+  const int shift = lpc ? fr.shift : 0;
   const short* xg = pcm + soff[b] + s0;
   for (int i = t; i < bs; i += kThreads) xs[i] = xg[i];
   for (int i = t; i < kWords; i += kThreads) bits[i] = 0u;
-  for (int i = t; i < kParts; i += kThreads) ks[i] = kind == SUB_FIXED && i < (1 << q) ? fr.k[i] : 0;
+  for (int i = t; i < kParts; i += kThreads) ks[i] = (kind == SUB_FIXED || lpc) && i < (1 << q) ? fr.k[i] : 0;
+  if (lpc && t < o) lq[t] = fr.q[t];
   {
     unsigned c = (unsigned)t << 8;
     for (int i = 0; i < 8; i++) c = (c << 1) ^ ((c & 0x8000u) ? 0x8005u : 0u);
@@ -372,15 +542,18 @@ __global__ void __launch_bounds__(kThreads) flac_pack_kernel(const short* __rest
     if (t == 0) put_bits(bits, sub, 0x02u, 8);
     for (int s = t; s < bs; s += kThreads) put_bits(bits, sub + 8 + 16 * s, (unsigned short)xs[s], 16);
   } else {
-    // element s: a warm-up sample (16 bits) for s < o; else [method + partition order (6 bits) if s == o]
-    // [Rice parameter (4 bits) if s starts a partition] then the code: (u >> k) zeros, a one, the low k bits
+    // element s: a warm-up sample (16 bits) for s < o; else [if s == o: (LPC: precision - 1 (4 bits), shift
+    // (5 bits), o coefficients (12 bits each)) method + partition order (6 bits)] [Rice parameter (4 bits) if s starts
+    // a partition] then the code: (u >> k) zeros, a one, the low k bits
     const int psize = bs >> q;
     const int c0 = t * kPer, c1 = min(c0 + kPer, bs);
+    const int head = lpc ? 4 + 5 + kLpcPrec * o : 0;
+    auto residual = [&](int s) { return lpc ? fold(lpc_residual(xs, s, o, lq, shift)) : fold_residual(xs, s, o); };
     int len = 0;
     for (int s = c0; s < c1; s++) {
       if (s < o) { len += 16; continue; }
       const int k = ks[s / psize];
-      len += (int)(fold_residual(xs, s, o) >> k) + 1 + k + (s == o ? 10 : (s % psize == 0 ? 4 : 0));
+      len += (int)(residual(s) >> k) + 1 + k + (s == o ? head + 10 : (s % psize == 0 ? 4 : 0));
     }
     int x = len;
 #pragma unroll
@@ -401,13 +574,19 @@ __global__ void __launch_bounds__(kThreads) flac_pack_kernel(const short* __rest
     }
     __syncthreads();
     int pos = sub + 8 + (wid ? warp_sum[wid - 1] : 0) + x - len;
-    if (t == 0) put_bits(bits, sub, 0x10u | (unsigned)(o << 1), 8);
+    if (t == 0) put_bits(bits, sub, lpc ? 0x40u | (unsigned)((o - 1) << 1) : 0x10u | (unsigned)(o << 1), 8);
     for (int s = c0; s < c1; s++) {
       if (s < o) { put_bits(bits, pos, (unsigned short)xs[s], 16); pos += 16; continue; }
       const int k = ks[s / psize];
+      if (s == o && lpc) {
+        put_bits(bits, pos, kLpcPrec - 1, 4);
+        put_bits(bits, pos + 4, (unsigned)shift, 5);
+        pos += 9;
+        for (int j = 0; j < o; j++, pos += kLpcPrec) put_bits(bits, pos, (unsigned)lq[j] & 0xFFFu, kLpcPrec);
+      }
       if (s == o) { put_bits(bits, pos, (unsigned)q, 6); pos += 6; }
       if (s == o || s % psize == 0) { put_bits(bits, pos, (unsigned)k, 4); pos += 4; }
-      const unsigned u = fold_residual(xs, s, o);
+      const unsigned u = residual(s);
       pos += (int)(u >> k);
       put_bits(bits, pos, (1u << k) | (u & ((1u << k) - 1u)), k + 1);
       pos += k + 1;
@@ -476,22 +655,41 @@ size_t flac_work_bytes(long long n_frames) {
 
 bool flac_rate_ok(int rate) { return rate_code(rate) >= 0; }
 
-static size_t analyze_smem() {
-  return kBlock * sizeof(short) + (size_t)kOrders * kRice * kParts * sizeof(unsigned) +
-         kOrders * (kMaxPorder + 1) * sizeof(unsigned) + kOrders * (2 * kParts - 1);
+void flac_lpc_window(int* m) {
+  const double pi = 3.14159265358979323846;
+  for (int k = 0; k < kLpcWin; k++)
+    m[k] = (int)std::floor(32768.0 * (0.5 * (1.0 - std::cos(pi * (k + 0.5) / kLpcWin))) + 0.5);
 }
 
-void launch_flac(const short* pcm, const long long* soff, const int* foff, int B, int F, int rate, void* work,
-                 unsigned char* out, long long* item_off, cudaStream_t st) {
+static size_t analyze_smem(int rows) {
+  return kBlock * sizeof(short) + (size_t)rows * kRice * kParts * sizeof(unsigned) +
+         rows * (kMaxPorder + 1) * sizeof(unsigned) + rows * (2 * kParts - 1);
+}
+
+void launch_flac(const short* pcm, const long long* soff, const int* foff, int B, int F, int rate, int lpc_order,
+                 void* work, unsigned char* out, long long* item_off, cudaStream_t st) {
   if (g_dry_run) return;
   if (!flac_rate_ok(rate)) throw ArgError("launch_flac: no FLAC sample-rate code for " + std::to_string(rate) + " Hz");
   if (B < 1 || F < B) throw ArgError("launch_flac: every item needs at least one sample");
+  if (lpc_order < 0 || lpc_order > kMaxLpcOrder) throw ArgError("launch_flac: LPC order outside 0..12");
   FlacFrame* frames = static_cast<FlacFrame*>(work);
   long long* frame_off = reinterpret_cast<long long*>(reinterpret_cast<char*>(work) +
                                                       (((size_t)F * sizeof(FlacFrame) + 255) & ~size_t(255)));
-  const size_t smem = analyze_smem();
-  prepare_smem_launch<flac_analyze_kernel>((int)smem);
-  flac_analyze_kernel<<<F, kThreads, smem, st>>>(pcm, soff, foff, B, rate, frames);
+  if (lpc_order == 0) {
+    const size_t smem = analyze_smem(kOrders);
+    prepare_smem_launch<flac_analyze_kernel<false>>((int)smem);
+    flac_analyze_kernel<false><<<F, kThreads, smem, st>>>(pcm, soff, foff, B, rate, 0, frames);
+  } else {
+    static DevOnce once;
+    const int dev = prepare_smem_launch<flac_analyze_kernel<true>>((int)analyze_smem(kOrders + 1));
+    once.run(dev, [] {
+      int m[kLpcWin];
+      flac_lpc_window(m);
+      KKX_CUDA(cudaMemcpyToSymbol(g_lpc_window, m, sizeof m));
+    });
+    const size_t smem = analyze_smem(kOrders + 1);
+    flac_analyze_kernel<true><<<F, kThreads, smem, st>>>(pcm, soff, foff, B, rate, lpc_order, frames);
+  }
   post_launch("flac_analyze", st);
   flac_scan_kernel<<<1, 1024, 0, st>>>(frames, foff, B, F, frame_off, item_off);
   post_launch("flac_scan", st);

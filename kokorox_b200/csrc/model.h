@@ -180,6 +180,8 @@ struct Options {
   // EBU R128 loudness report (kkx.h "loudness_report"): 0 = off, 1 = measure every program (without a target or the
   // limiter: measure only, the output is unchanged)
   int loudness_report = 0;
+  // FLAC linear prediction (kkx.h "flac_lpc_order"): 0 = off, 1..12 = one LPC candidate of that order per frame
+  int flac_lpc_order = 0;
 };
 
 // Device-resident weights of one checkpoint on one GPU: every layout the kernels read (fp32 SIMT, bf16 / split-TF32

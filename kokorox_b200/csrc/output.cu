@@ -38,6 +38,7 @@ OutputPlan output_plan(const Options& opt, Encoding enc, int kbps, OutputBuffers
   p.enc = enc;
   p.rate = opt.out_rate;
   if (enc == Encoding::MP3) p.mp3 = mp3_format(opt.out_rate, kbps);
+  if (enc == Encoding::FLAC) p.flac_lpc = opt.flac_lpc_order;
   p.loud = opt.loudness_target != 0;
   p.limit = opt.limiter != 0;
   p.report = opt.loudness_report != 0;
@@ -147,7 +148,7 @@ void encode_streams(const OutputPlan& p, StreamTables& t, const short* pcm, void
   long long* boff = reinterpret_cast<long long*>(base + L.boff);
   const int* foff = reinterpret_cast<const int*>(base + L.foff);
   if (p.enc == Encoding::FLAC) {
-    launch_flac(pcm, soff, foff, t.P, t.F, p.rate, base + L.work, out, boff, st);
+    launch_flac(pcm, soff, foff, t.P, t.F, p.rate, p.flac_lpc, base + L.work, out, boff, st);
     KKX_CUDA(cudaMemcpyAsync(t.boff.data(), boff, (size_t)(t.P + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
   } else {
     launch_mp3(pcm, soff, foff, boff, t.P, t.F, p.mp3, base + L.work, out, st);

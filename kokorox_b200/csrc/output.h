@@ -27,6 +27,7 @@ enum : unsigned { kRepLoudness = 1, kRepRange = 2, kRepLimiter = 4 };
 struct OutputPlan {
   Encoding enc = Encoding::F32;
   int rate = 24000;                     // the output rate
+  int flac_lpc = 0;                     // FLAC: the LPC order (kkx.h "flac_lpc_order"), 0 = off
   bool loud = false;                    // normalise to a loudness target
   bool limit = false;                   // the lookahead limiter
   bool report = false;                  // the loudness report

@@ -214,6 +214,28 @@ KKX_API int64_t kkx_test_flac(int device, const int16_t* pcm, int32_t B, const i
   return rc == KKX_OK ? (int64_t)total : (int64_t)rc;
 }
 
+KKX_API int64_t kkx_test_flac_lpc(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate,
+                                  int32_t order, uint8_t* dst, int64_t capacity, int64_t* byte_offsets) {
+  long long total = 0;
+  const int rc = run(device, [&] {
+    if (!pcm || !lens || !byte_offsets || B < 1) throw ArgError("kkx_test_flac_lpc: bad argument");
+    if (!flac_rate_ok(rate)) throw ArgError("kkx_test_flac_lpc: rejected rate");
+    if (order < 0 || order > kMaxLpcOrder) throw ArgError("kkx_test_flac_lpc: order outside 0..12");
+    OutputPlan p;
+    p.enc = Encoding::FLAC;
+    p.rate = rate;
+    p.flac_lpc = order;
+    total = encode_items(p, pcm, B, lens, dst, capacity, byte_offsets, "kkx_test_flac_lpc");
+  });
+  return rc == KKX_OK ? (int64_t)total : (int64_t)rc;
+}
+
+KKX_API int kkx_test_flac_lpc_window(int32_t* m1024) {
+  if (!m1024) return KKX_ERR_ARG;
+  flac_lpc_window(m1024);
+  return KKX_OK;
+}
+
 KKX_API int64_t kkx_test_mp3(int device, const int16_t* pcm, int32_t B, const int64_t* lens, int32_t rate, int32_t kbps,
                              uint8_t* dst, int64_t capacity, int64_t* byte_offsets) {
   long long total = 0;

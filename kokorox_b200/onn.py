@@ -124,6 +124,9 @@ def load_library(path: Optional[str] = None):
         lib.kkx_test_loudness.argtypes = [C.c_int, P(f32), i32, P(i64), i32, i32, P(f32), P(f32), P(f32)]
         lib.kkx_test_flac.argtypes = [C.c_int, P(i16), i32, P(i64), i32, P(u8), i64, P(i64)]
         lib.kkx_test_flac.restype = i64
+        lib.kkx_test_flac_lpc.argtypes = [C.c_int, P(i16), i32, P(i64), i32, i32, P(u8), i64, P(i64)]
+        lib.kkx_test_flac_lpc.restype = i64
+        lib.kkx_test_flac_lpc_window.argtypes = [P(i32)]
         lib.kkx_test_mp3.argtypes = [C.c_int, P(i16), i32, P(i64), i32, i32, P(u8), i64, P(i64)]
         lib.kkx_test_mp3.restype = i64
         lib.kkx_test_mp3_tables.argtypes = [P(C.c_uint32), P(u8), P(i32), P(i32), P(C.c_uint32), P(u8),
