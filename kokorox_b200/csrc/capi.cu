@@ -1,7 +1,7 @@
 // capi.cu -- the extern "C" boundary (include/kkx.h).  Every entry point catches all C++
 // exceptions and converts them to a negative return code + message: nothing unwinds or aborts
 // across the ABI (the reference `expect`s on bad outputs, ort_koko.rs:82,86, and its CLI turns a
-// panic into abort(); a library must not).
+// panic into abort(); a library must not).  The entry points take their C linkage from the declarations in the headers.
 #include "../../include/kkx.h"
 #include "../../include/kkx_test.h"
 #include "model.h"
@@ -13,7 +13,7 @@
 #include <mutex>
 #include <map>
 #include <numeric>
-#include <set>
+#include <functional>
 #include <sstream>
 #include <atomic>
 #include <thread>
@@ -25,7 +25,10 @@ struct kkx_ctx {
   std::mutex mu;  // single-flight like the reference's Mutex<Session> (ort_koko.rs:14,77-78)
   // pinned result buffers; their own lock, so that kkx_release never waits for the step `mu` is held across
   std::mutex pool_mu;
-  std::map<void*, size_t> pinned;        // result buffers handed out -> capacity (bytes)
+  // One result buffer (cap in bytes), referenced once by every pointer handed out into it: a plain result is a block
+  // with one reference, a coalesced batch one block with a reference per caller's view.
+  struct Block { void* base; size_t cap; int refs; };
+  std::map<void*, Block*> handed;        // every pointer handed to a caller -> its block
   std::vector<std::pair<void*, size_t>> pinned_free;  // returned buffers kept for reuse
   size_t pinned_free_bytes = 0;
   size_t pinned_hi = 0;                  // largest request so far: big buffers are sized alike so they recycle
@@ -37,7 +40,6 @@ struct kkx_ctx {
     const int64_t* tokens; int32_t n; const float* style; float speed; int32_t* pred_dur;
     float* audio = nullptr; int64_t samples = 0; int rc = 0; std::string err; bool done = false;
   };
-  struct SharedBuf { float* base; size_t cap; int refs; };   // cap in bytes
   std::mutex qmu;
   std::condition_variable qcv;
   std::deque<Waiter*> queue;
@@ -45,25 +47,24 @@ struct kkx_ctx {
   long long max_tokens = 40960;  // tokens per pass of one call (64 x 512-token utterances + slack)
   std::atomic<int> coalesce_max{0};      // 0/1 = off (reference behaviour); >1 = largest batch a leader gathers
   std::atomic<int> coalesce_wait_us{0};  // how long a leader waits for company before it runs
-  int64_t coalesced_batches = 0, coalesced_requests = 0, coalesced_largest = 0;
-  std::map<float*, SharedBuf*> views;   // per-caller view -> the shared buffer it pins (guarded by pool_mu)
+  int64_t coalesced_batches = 0, coalesced_requests = 0, coalesced_largest = 0;   // guarded by qmu
 
   // Asynchronous requests (kkx_submit / kkx_poll / kkx_wait): a worker thread owned by the ctx drains the queue in
   // FIFO batches, so a caller can hand in sentence k+1 and go on sending sentence k (websocket lib.rs:371-376).
   struct AsyncReq {
     std::vector<int64_t> tokens; float style[256]; std::vector<int32_t> dur;
     Waiter w{};
-    bool done = false, taken = false;
+    bool taken = false;
   };
   std::mutex amu;
   std::condition_variable acv_work, acv_done;
   std::map<int64_t, std::unique_ptr<AsyncReq>> tickets;
-  std::deque<AsyncReq*> aqueue;
+  std::deque<Waiter*> aqueue;
   std::thread worker;
   bool worker_started = false, astop = false;
   int64_t next_ticket = 1;
   std::atomic<int> async_batch{64};      // most requests the worker merges into one ragged batch
-  int64_t async_batches = 0, async_requests = 0;
+  int64_t async_batches = 0, async_requests = 0;                                 // guarded by amu
 
   // Per-item report of the last synchronous call (kkx_last_loudness / _limiter / _loudness_range), guarded by `mu`:
   // kReportRows floats per item (output.h), appended pass by pass; `groups` = the row groups its runs produced, valid
@@ -75,9 +76,12 @@ struct kkx_ctx {
 
 static thread_local std::string g_err;
 static constexpr int kMaxCoalesce = 512;
+// Most tokens in one batch the coalescing leader or the async worker gathers: the 64 x 512-token working set the
+// step is sized for.
+static constexpr long long kBatchTokens = 64 * 512;
 
 template <class F>
-static int guarded(kkx_ctx* ctx, F&& f) {
+static int guarded(F&& f) {
   std::string msg;
   int rc = KKX_OK;
   try {
@@ -91,12 +95,25 @@ static int guarded(kkx_ctx* ctx, F&& f) {
   } catch (...) { rc = KKX_ERR_CUDA; msg = "unknown error"; }
   g_launch_stats = nullptr;
   g_dry_run = false;
-  (void)ctx;
   g_err = msg;
   return rc;
 }
 
-extern "C" {
+static int check_ctx(kkx_ctx* ctx) {
+  if (!ctx) { g_err = "null ctx"; return KKX_ERR_ARG; }
+  if (!ctx->model) { g_err = "Session is not initialized."; return KKX_ERR_STATE; }
+  return KKX_OK;
+}
+
+// Every entry point that works on the session: `f` runs single-flight under ctx->mu, its exception becomes the
+// return code and kkx_last_error's message.
+template <class F>
+static int session_call(kkx_ctx* ctx, F&& f) {
+  const int rc = check_ctx(ctx);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  return guarded(f);
+}
 
 KKX_API const char* kkx_version(void) { return "kkx 0.1 sm_100a"; }
 
@@ -119,7 +136,7 @@ KKX_API int kkx_create(const char* weights_path, int device_ordinal, kkx_ctx** o
   if (rc != KKX_OK) return rc;
   kkx_ctx* ctx = new (std::nothrow) kkx_ctx();
   if (!ctx) { g_err = "out of memory"; return KKX_ERR_CUDA; }
-  rc = guarded(nullptr, [&] { ctx->model.reset(new Model(weights_path, device_ordinal)); });
+  rc = guarded([&] { ctx->model.reset(new Model(weights_path, device_ordinal)); });
   if (rc != KKX_OK) { delete ctx; return rc; }
   *out = ctx;
   return KKX_OK;
@@ -129,7 +146,7 @@ KKX_API int kkx_create(const char* weights_path, int device_ordinal, kkx_ctx** o
 // as a KKXW file.  Lets a deployment convert once and lets the CPU test-suite check the ONNX reader without a GPU.
 KKX_API int kkx_convert_model_file(const char* src_path, const char* dst_kkxw_path, int32_t* out_tensors) {
   if (!src_path || !dst_kkxw_path) { g_err = "kkx_convert_model_file: null argument"; return KKX_ERR_ARG; }
-  return guarded(nullptr, [&] {
+  return guarded([&] {
     WeightFile wf(src_path);
     std::vector<std::string> names;
     for (auto& sp : kokoro_tensor_specs()) names.push_back(sp.first);
@@ -180,11 +197,9 @@ KKX_API void kkx_destroy(kkx_ctx* ctx) {
   }
   try {
     if (ctx->model) cudaSetDevice(ctx->model->device());
-    for (auto& p : ctx->pinned) cudaFreeHost(p.first);
+    for (auto& h : ctx->handed)
+      if (--h.second->refs == 0) { cudaFreeHost(h.second->base); delete h.second; }
     for (auto& p : ctx->pinned_free) cudaFreeHost(p.first);
-    std::set<kkx_ctx::SharedBuf*> shared;
-    for (auto& v : ctx->views) shared.insert(v.second);
-    for (auto* sb : shared) { cudaFreeHost(sb->base); delete sb; }
     ctx->model.reset();
   } catch (...) {}
   delete ctx;
@@ -195,13 +210,7 @@ KKX_API void kkx_destroy(kkx_ctx* ctx) {
 // caller still reads it.
 KKX_API const char* kkx_last_error(const kkx_ctx* ctx) { (void)ctx; return g_err.c_str(); }
 
-static int check_ctx(kkx_ctx* ctx) {
-  if (!ctx) { g_err = "null ctx"; return KKX_ERR_ARG; }
-  if (!ctx->model) { g_err = "Session is not initialized."; return KKX_ERR_STATE; }
-  return KKX_OK;
-}
-
-// shared tail of the infer entry points: a pooled pinned result buffer of at least `need` bytes
+// A pooled pinned result buffer of at least `need` bytes
 static void* take_pinned(kkx_ctx* ctx, size_t need, size_t* cap_out) {
   void* host = nullptr;
   size_t cap = 0, hi = 0;
@@ -229,25 +238,30 @@ static void* take_pinned(kkx_ctx* ctx, size_t need, size_t* cap_out) {
   *cap_out = cap;
   return host;
 }
-static void hand_out(kkx_ctx* ctx, void* host, size_t cap) {
+// Result buffer `base` handed out at the addresses `at`, one reference each; kkx_release recycles it with the last.
+static void hand_out(kkx_ctx* ctx, void* base, size_t cap, const std::vector<void*>& at) {
   std::lock_guard<std::mutex> pl(ctx->pool_mu);
-  ctx->pinned[host] = cap;
+  auto* b = new kkx_ctx::Block{base, cap, (int)at.size()};
+  for (void* p : at) ctx->handed[p] = b;
 }
 
 KKX_API void kkx_release(kkx_ctx* ctx, float* audio);
 
-// kkx_last_loudness / kkx_last_limiter / kkx_last_loudness_range bookkeeping of a synchronous call (caller holds
-// ctx->mu): begin, one note per model run, done.  Coalesced and asynchronous batches leave the reports alone.
-static void loud_begin(kkx_ctx* ctx) {
-  ctx->report.clear(); ctx->report_groups = 0; ctx->report_valid = false;
-}
-static void loud_note(kkx_ctx* ctx) {
+// The report of a synchronous call (kkx_last_loudness / _limiter / _loudness_range; caller holds ctx->mu; throws):
+// `runs(note)` runs the model one or more times and calls note() after each run, which appends that run's rows; the
+// report restarts before `runs` and is valid once it has returned.  Coalesced and asynchronous batches do not come
+// through here, so they leave the report alone (kkx.h).
+template <class F>
+static void record_report(kkx_ctx* ctx, F&& runs) {
   const Model& m = *ctx->model;
-  if (!m.report_groups()) return;
-  ctx->report_groups |= m.report_groups();
-  ctx->report.insert(ctx->report.end(), m.last_report().begin(), m.last_report().end());
+  ctx->report.clear(); ctx->report_groups = 0; ctx->report_valid = false;
+  runs([&] {
+    if (!m.report_groups()) return;
+    ctx->report_groups |= m.report_groups();
+    ctx->report.insert(ctx->report.end(), m.last_report().begin(), m.last_report().end());
+  });
+  ctx->report_valid = true;
 }
-static void loud_done(kkx_ctx* ctx) { ctx->report_valid = true; }
 // items of the last synchronous call's report with row group `group`, 0 without one
 static int64_t report_items(const kkx_ctx* ctx, unsigned group) {
   return ctx->report_valid && (ctx->report_groups & group) ? (int64_t)(ctx->report.size() / kReportRows) : 0;
@@ -265,9 +279,9 @@ static int validate_request(const int64_t* tokens, int32_t n_tokens, const float
 
 // One ragged batch through the model into a pooled pinned buffer (caller holds ctx->mu; throws).  The buffer is
 // handed to the model as a sink: every frame group's audio is copied out on a second stream while the next
-// group computes.
+// group computes.  `note` follows the run (record_report).
 static void run_staged_locked(kkx_ctx* ctx, float** host_out, size_t* cap_out, int64_t* out_sample_offsets,
-                              int32_t* out_pred_dur) {
+                              int32_t* out_pred_dur, const std::function<void()>& note) {
   Model& m = *ctx->model;
   float* host = nullptr;
   size_t cap = 0;
@@ -275,6 +289,7 @@ static void run_staged_locked(kkx_ctx* ctx, float** host_out, size_t* cap_out, i
   try {
     m.run();
     m.host_sink = nullptr;
+    note();
     const long long n = m.total_samples();
     if (!host) host = static_cast<float*>(take_pinned(ctx, n * sizeof(float), &cap));
     m.fetch(m.sink_filled() ? nullptr : host, n, out_sample_offsets, out_pred_dur);
@@ -303,13 +318,12 @@ static void recycle_pinned(kkx_ctx* ctx, void* host, size_t cap) {
 // apart from one host-side concatenation.
 static void run_batch_locked(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                              const float* styles, const float* speeds, float** host_out, size_t* cap_out,
-                             int64_t* out_sample_offsets, int32_t* out_pred_dur, bool report = false) {
+                             int64_t* out_sample_offsets, int32_t* out_pred_dur, const std::function<void()>& note) {
   if (batch <= 0 || !tok_offsets) throw ArgError("batch must be >= 1");
   const long long budget = ctx->max_tokens;
   if (batch == 1 || (long long)tok_offsets[batch] - tok_offsets[0] <= budget) {
     ctx->model->stage(batch, tokens, tok_offsets, styles, speeds);
-    run_staged_locked(ctx, host_out, cap_out, out_sample_offsets, out_pred_dur);
-    if (report) loud_note(ctx);
+    run_staged_locked(ctx, host_out, cap_out, out_sample_offsets, out_pred_dur, note);
     return;
   }
   if (!styles) throw ArgError("null input pointer");
@@ -324,9 +338,8 @@ static void run_batch_locked(kkx_ctx* ctx, int32_t batch, const int64_t* tokens,
       Part p{nullptr, 0, b0, b1};
       ctx->model->stage(b1 - b0, tokens, tok_offsets + b0, styles + (size_t)b0 * 256, speeds + b0);
       run_staged_locked(ctx, &p.host, &p.cap, so.data(),
-                        out_pred_dur ? out_pred_dur + (tok_offsets[b0] - tok_offsets[0]) : nullptr);
+                        out_pred_dur ? out_pred_dur + (tok_offsets[b0] - tok_offsets[0]) : nullptr, note);
       parts.push_back(p);
-      if (report) loud_note(ctx);
       for (int i = 0; i < b1 - b0; i++) soff[b0 + i + 1] = soff[b0] + so[i + 1];
       b0 = b1;
     }
@@ -347,26 +360,23 @@ static void run_batch_locked(kkx_ctx* ctx, int32_t batch, const int64_t* tokens,
 KKX_API int kkx_infer_batch(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                     const float* styles, const float* speeds, float** out_audio,
                     int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_audio) *out_audio = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
+  return session_call(ctx, [&] {
     if (!out_audio) throw ArgError("out_audio is null");
+    *out_audio = nullptr;
     float* host = nullptr;
     size_t cap = 0;
-    loud_begin(ctx);
-    run_batch_locked(ctx, batch, tokens, tok_offsets, styles, speeds, &host, &cap, out_sample_offsets, out_pred_dur,
-                     true);
-    loud_done(ctx);
-    hand_out(ctx, host, cap);
+    record_report(ctx, [&](const std::function<void()>& note) {
+      run_batch_locked(ctx, batch, tokens, tok_offsets, styles, speeds, &host, &cap, out_sample_offsets, out_pred_dur,
+                       note);
+    });
+    hand_out(ctx, host, cap, {host});
     *out_audio = host;
   });
 }
 
-// Leader side of the coalescer: run `batch` as one ragged batch; on failure re-run the requests one by one so
-// that only the offending caller sees the error.
-static void serve_coalesced(kkx_ctx* ctx, const std::vector<kkx_ctx::Waiter*>& batch, bool count = true) {
+// Leader side of the coalescer and of the async worker: run `batch` as one ragged batch; on failure re-run the
+// requests one by one so that only the offending caller sees the error.  True when the batch ran as one.
+static bool serve_coalesced(kkx_ctx* ctx, const std::vector<kkx_ctx::Waiter*>& batch) {
   const int B = (int)batch.size();
   std::vector<int32_t> offs(B + 1, 0);
   for (int i = 0; i < B; i++) offs[i + 1] = offs[i] + std::max(batch[i]->n, 0);
@@ -382,31 +392,28 @@ static void serve_coalesced(kkx_ctx* ctx, const std::vector<kkx_ctx::Waiter*>& b
     memcpy(&styles[(size_t)i * 256], w.style, 256 * sizeof(float));
     speeds[i] = w.speed;
   }
+  const std::function<void()> no_report = [] {};
   std::lock_guard<std::mutex> lk(ctx->mu);
   float* host = nullptr;
   size_t cap = 0;
   int rc = KKX_ERR_ARG;
   if (args_ok)
-    rc = guarded(ctx, [&] {
-      run_batch_locked(ctx, B, toks.data(), offs.data(), styles.data(), speeds.data(), &host, &cap, soff.data(), dur.data());
+    rc = guarded([&] {
+      run_batch_locked(ctx, B, toks.data(), offs.data(), styles.data(), speeds.data(), &host, &cap, soff.data(),
+                       dur.data(), no_report);
     });
   if (rc == KKX_OK) {
-    auto* sb = new kkx_ctx::SharedBuf{host, cap, B};
-    std::lock_guard<std::mutex> pl(ctx->pool_mu);
+    std::vector<void*> views(B);
     for (int i = 0; i < B; i++) {
       kkx_ctx::Waiter& w = *batch[i];
       w.audio = host + soff[i];
       w.samples = soff[i + 1] - soff[i];   // >= 200: every token lasts at least one frame, so view addresses are distinct
       if (w.pred_dur) memcpy(w.pred_dur, &dur[offs[i]], (size_t)w.n * sizeof(int32_t));
       w.rc = KKX_OK;
-      ctx->views[w.audio] = sb;
+      views[i] = w.audio;
     }
-    if (count) {     // (the asynchronous worker keeps its own counters)
-      ctx->coalesced_batches++;
-      ctx->coalesced_requests += B;
-      ctx->coalesced_largest = std::max<int64_t>(ctx->coalesced_largest, B);
-    }
-    return;
+    hand_out(ctx, host, cap, views);
+    return true;
   }
   for (int i = 0; i < B; i++) {   // isolate the failure
     kkx_ctx::Waiter& w = *batch[i];
@@ -414,19 +421,46 @@ static void serve_coalesced(kkx_ctx* ctx, const std::vector<kkx_ctx::Waiter*>& b
     int64_t s1[2] = {0, 0};
     float* h1 = nullptr;
     size_t c1 = 0;
-    w.rc = guarded(ctx, [&] {
+    w.rc = guarded([&] {
       if (!w.tokens || !w.style) throw ArgError("null argument");
-      run_batch_locked(ctx, 1, w.tokens, o1, w.style, &w.speed, &h1, &c1, s1, w.pred_dur);
+      run_batch_locked(ctx, 1, w.tokens, o1, w.style, &w.speed, &h1, &c1, s1, w.pred_dur, no_report);
     });
     if (w.rc == KKX_OK) {
-      hand_out(ctx, h1, c1);
+      hand_out(ctx, h1, c1, {h1});
       w.audio = h1;
       w.samples = s1[1];
-      if (count) { ctx->coalesced_batches++; ctx->coalesced_requests++; }
     } else {
       w.err = g_err;      // guarded() left the message in this (the leader's) thread
     }
   }
+  return false;
+}
+
+// The request batcher of the coalescing leader and of the async worker (caller holds `lk` on `queue`'s mutex, which
+// is released while the batch runs): takes a FIFO batch of at most `want` requests and kBatchTokens tokens off
+// `queue` and serves it.  `together` says whether it ran as one batch.
+static std::vector<kkx_ctx::Waiter*> serve_queue(kkx_ctx* ctx, std::deque<kkx_ctx::Waiter*>& queue,
+                                                 std::unique_lock<std::mutex>& lk, size_t want, const char* what,
+                                                 bool* together) {
+  std::vector<kkx_ctx::Waiter*> batch;
+  long long tok = 0;
+  while (!queue.empty() && batch.size() < want) {
+    kkx_ctx::Waiter* q = queue.front();
+    if (!batch.empty() && tok + q->n > kBatchTokens) break;
+    tok += std::max(q->n, 0);
+    batch.push_back(q);
+    queue.pop_front();
+  }
+  lk.unlock();
+  *together = false;
+  try {
+    *together = serve_coalesced(ctx, batch);
+  } catch (...) {   // (allocation failure outside guarded()): fail the batch, never leave the queue without a server
+    for (auto* w : batch) { w->rc = KKX_ERR_CUDA; w->err = std::string("internal error while serving ") + what; w->audio = nullptr; }
+  }
+  lk.lock();
+  for (auto* w : batch) w->done = true;
+  return batch;
 }
 
 static int infer_coalesced(kkx_ctx* ctx, kkx_ctx::Waiter& w) {
@@ -440,24 +474,16 @@ static int infer_coalesced(kkx_ctx* ctx, kkx_ctx::Waiter& w) {
     const int wait_us = ctx->coalesce_wait_us.load();
     if (wait_us > 0 && ctx->queue.size() < want)
       ctx->qcv.wait_for(ql, std::chrono::microseconds(wait_us), [&] { return ctx->queue.size() >= want; });
-    // FIFO, bounded by the batch size and by the 64 x 512-token working set the step is sized for
-    std::vector<kkx_ctx::Waiter*> batch;
-    long long tok = 0;
-    while (!ctx->queue.empty() && batch.size() < want) {
-      kkx_ctx::Waiter* q = ctx->queue.front();
-      if (!batch.empty() && tok + q->n > 64 * 512) break;
-      tok += std::max(q->n, 0);
-      batch.push_back(q);
-      ctx->queue.pop_front();
+    bool together = false;
+    const auto batch = serve_queue(ctx, ctx->queue, ql, want, "a coalesced batch", &together);
+    if (together) {
+      ctx->coalesced_batches++;
+      ctx->coalesced_requests += (int64_t)batch.size();
+      ctx->coalesced_largest = std::max<int64_t>(ctx->coalesced_largest, (int64_t)batch.size());
+    } else {
+      for (auto* b : batch)
+        if (b->rc == KKX_OK) { ctx->coalesced_batches++; ctx->coalesced_requests++; }
     }
-    ql.unlock();
-    try {
-      serve_coalesced(ctx, batch);
-    } catch (...) {   // (allocation failure outside guarded()): fail the batch, never leave the queue without a leader
-      for (auto* b : batch) { b->rc = KKX_ERR_CUDA; b->err = "internal error while serving a coalesced batch"; b->audio = nullptr; }
-    }
-    ql.lock();
-    for (auto* b : batch) b->done = true;
     ctx->leader = false;
     ctx->qcv.notify_all();
   }
@@ -466,70 +492,74 @@ static int infer_coalesced(kkx_ctx* ctx, kkx_ctx::Waiter& w) {
 }
 
 KKX_API int kkx_load_voices(kkx_ctx* ctx, const float* table, int32_t n_voices) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] { ctx->model->load_voices(table, n_voices); });
+  return session_call(ctx, [&] { ctx->model->load_voices(table, n_voices); });
 }
 
 KKX_API int kkx_infer_batch_voices(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                            const int32_t* mix_offsets, const int32_t* voice_ids, const float* voice_portions,
                            const int32_t* style_rows, const float* speeds, float** out_audio,
                            int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_audio) *out_audio = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
+  return session_call(ctx, [&] {
     if (!out_audio) throw ArgError("out_audio is null");
-    Model& m = *ctx->model;
-    m.stage_voices(batch, tokens, tok_offsets, mix_offsets, voice_ids, voice_portions, style_rows, speeds);
+    *out_audio = nullptr;
+    ctx->model->stage_voices(batch, tokens, tok_offsets, mix_offsets, voice_ids, voice_portions, style_rows, speeds);
     float* host = nullptr;
     size_t cap = 0;
-    loud_begin(ctx);
-    run_staged_locked(ctx, &host, &cap, out_sample_offsets, out_pred_dur);
-    loud_note(ctx);
-    loud_done(ctx);
-    hand_out(ctx, host, cap);
+    record_report(ctx, [&](const std::function<void()>& note) {
+      run_staged_locked(ctx, &host, &cap, out_sample_offsets, out_pred_dur, note);
+    });
+    hand_out(ctx, host, cap, {host});
     *out_audio = host;
   });
 }
 
 // The encoded entry points (kkx_infer_batch_pcm16 / _g711 / _flac / _mp3, kkx_infer_programs / _mp3): one pass of
-// the staged batch with `enc` (and the MP3 bitrate) and the program table (empty: one item per program), its bytes in
-// a pooled pinned buffer (caller holds ctx->mu; throws).
-static void* infer_encoded_locked(kkx_ctx* ctx, Encoding enc, int32_t batch, const int64_t* tokens,
-                                  const int32_t* tok_offsets, const float* styles, const float* speeds,
-                                  int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur,
-                                  const std::vector<int>& programs = {}, int kbps = 0) {
-  Model& m = *ctx->model;
-  m.stage(batch, tokens, tok_offsets, styles, speeds);
-  loud_begin(ctx);
-  m.run(enc, programs, kbps);
-  loud_note(ctx);
-  const long long n = m.encoded_bytes();
-  size_t cap = 0;
-  void* host = take_pinned(ctx, (size_t)n, &cap);
-  try {
-    m.fetch_encoded(host, n, out_byte_offsets, out_sample_offsets, out_pred_dur);
-  } catch (...) { cudaFreeHost(host); throw; }
-  hand_out(ctx, host, cap);
-  loud_done(ctx);
-  return host;
+// the batch with `enc` (kbps: the MP3 bitrate), its bytes in a pooled pinned buffer.  `out_name`: the out-pointer's
+// name in the messages; `byte_offsets`: whether the entry point takes out_byte_offsets (then it must not be null);
+// `bad_enc`: why the requested encoding is refused ("" = it is not); `programs`: whether the call takes a program
+// table (n_programs, program_offsets), one item per program otherwise.  Every check runs before the batch is staged,
+// so a rejected call leaves the session as it was.
+template <class T>
+static int infer_encoded(kkx_ctx* ctx, const char* out_name, T** out, bool byte_offsets, int64_t* out_byte_offsets,
+                         Encoding enc, const std::string& bad_enc, int32_t kbps, bool programs, int32_t n_programs,
+                         const int32_t* program_offsets, int32_t batch, const int64_t* tokens,
+                         const int32_t* tok_offsets, const float* styles, const float* speeds,
+                         int64_t* out_sample_offsets, int32_t* out_pred_dur) {
+  return session_call(ctx, [&] {
+    if (!out) throw ArgError(std::string(out_name) + " is null");
+    *out = nullptr;
+    if (byte_offsets && !out_byte_offsets) throw ArgError("out_byte_offsets is null");
+    if (!bad_enc.empty()) throw ArgError(bad_enc);
+    if (enc == Encoding::MP3) mp3_format(ctx->model->opt.out_rate, kbps);
+    std::vector<int> table;
+    if (programs) {
+      if (batch < 1) throw ArgError("batch must be >= 1");
+      check_programs(batch, n_programs, program_offsets);
+      table.assign(program_offsets, program_offsets + n_programs + 1);
+    }
+    Model& m = *ctx->model;
+    m.stage(batch, tokens, tok_offsets, styles, speeds);
+    void* host = nullptr;
+    size_t cap = 0;
+    record_report(ctx, [&](const std::function<void()>& note) {
+      m.run(enc, table, kbps);
+      note();
+      const long long n = m.encoded_bytes();
+      host = take_pinned(ctx, (size_t)n, &cap);
+      try {
+        m.fetch_encoded(host, n, out_byte_offsets, out_sample_offsets, out_pred_dur);
+      } catch (...) { cudaFreeHost(host); throw; }
+    });
+    hand_out(ctx, host, cap, {host});
+    *out = static_cast<T*>(host);
+  });
 }
 
 KKX_API int kkx_infer_batch_pcm16(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                           const float* styles, const float* speeds, int16_t** out_pcm,
                           int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_pcm) *out_pcm = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    if (!out_pcm) throw ArgError("out_pcm is null");
-    *out_pcm = static_cast<int16_t*>(infer_encoded_locked(ctx, Encoding::PCM16, batch, tokens, tok_offsets, styles,
-                                                          speeds, nullptr, out_sample_offsets, out_pred_dur));
-  });
+  return infer_encoded(ctx, "out_pcm", out_pcm, false, nullptr, Encoding::PCM16, "", 0, false, 0, nullptr, batch,
+                       tokens, tok_offsets, styles, speeds, out_sample_offsets, out_pred_dur);
 }
 
 KKX_API void kkx_release_pcm16(kkx_ctx* ctx, int16_t* pcm) { kkx_release(ctx, reinterpret_cast<float*>(pcm)); }
@@ -537,17 +567,9 @@ KKX_API void kkx_release_pcm16(kkx_ctx* ctx, int16_t* pcm) { kkx_release(ctx, re
 KKX_API int kkx_infer_batch_g711(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                                  const float* styles, const float* speeds, int32_t law, uint8_t** out_codes,
                                  int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_codes) *out_codes = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    if (!out_codes) throw ArgError("out_codes is null");
-    if (law != 0 && law != 1) throw ArgError("law must be 0 (mu-law) or 1 (A-law), got " + std::to_string(law));
-    *out_codes = static_cast<uint8_t*>(infer_encoded_locked(ctx, law ? Encoding::ALAW : Encoding::ULAW, batch, tokens,
-                                                            tok_offsets, styles, speeds, nullptr, out_sample_offsets,
-                                                            out_pred_dur));
-  });
+  const std::string bad = law == 0 || law == 1 ? "" : "law must be 0 (mu-law) or 1 (A-law), got " + std::to_string(law);
+  return infer_encoded(ctx, "out_codes", out_codes, false, nullptr, law ? Encoding::ALAW : Encoding::ULAW, bad, 0,
+                       false, 0, nullptr, batch, tokens, tok_offsets, styles, speeds, out_sample_offsets, out_pred_dur);
 }
 
 KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes) { kkx_release(ctx, reinterpret_cast<float*>(codes)); }
@@ -555,16 +577,8 @@ KKX_API void kkx_release_g711(kkx_ctx* ctx, uint8_t* codes) { kkx_release(ctx, r
 KKX_API int kkx_infer_batch_flac(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                                  const float* styles, const float* speeds, uint8_t** out_bytes,
                                  int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_bytes) *out_bytes = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    if (!out_bytes) throw ArgError("out_bytes is null");
-    if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
-    *out_bytes = static_cast<uint8_t*>(infer_encoded_locked(ctx, Encoding::FLAC, batch, tokens, tok_offsets, styles,
-                                                            speeds, out_byte_offsets, out_sample_offsets, out_pred_dur));
-  });
+  return infer_encoded(ctx, "out_bytes", out_bytes, true, out_byte_offsets, Encoding::FLAC, "", 0, false, 0, nullptr,
+                       batch, tokens, tok_offsets, styles, speeds, out_sample_offsets, out_pred_dur);
 }
 
 KKX_API void kkx_release_flac(kkx_ctx* ctx, uint8_t* bytes) { kkx_release(ctx, reinterpret_cast<float*>(bytes)); }
@@ -573,24 +587,13 @@ KKX_API int kkx_infer_programs(kkx_ctx* ctx, int32_t batch, const int64_t* token
                                const float* styles, const float* speeds, int32_t n_programs,
                                const int32_t* program_offsets, int32_t encoding, void** out_bytes,
                                int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_bytes) *out_bytes = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    // every check before the batch is staged: a rejected call leaves the session as it was
-    if (!out_bytes) throw ArgError("out_bytes is null");
-    if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
-    if (encoding < KKX_ENC_F32 || encoding > KKX_ENC_FLAC)
-      throw ArgError("encoding must be in 0..4 (KKX_ENC_F32 .. KKX_ENC_FLAC), got " + std::to_string(encoding) +
-                     " (MP3: kkx_infer_programs_mp3)");
-    if (batch < 1) throw ArgError("batch must be >= 1");
-    check_programs(batch, n_programs, program_offsets);
-    static const Encoding enc[] = {Encoding::F32, Encoding::PCM16, Encoding::ULAW, Encoding::ALAW, Encoding::FLAC};
-    *out_bytes = infer_encoded_locked(ctx, enc[encoding], batch, tokens, tok_offsets, styles, speeds, out_byte_offsets,
-                                      out_sample_offsets, out_pred_dur,
-                                      std::vector<int>(program_offsets, program_offsets + n_programs + 1));
-  });
+  static const Encoding enc[] = {Encoding::F32, Encoding::PCM16, Encoding::ULAW, Encoding::ALAW, Encoding::FLAC};
+  const bool ok = encoding >= KKX_ENC_F32 && encoding <= KKX_ENC_FLAC;
+  const std::string bad = ok ? "" : "encoding must be in 0..4 (KKX_ENC_F32 .. KKX_ENC_FLAC), got " +
+                                    std::to_string(encoding) + " (MP3: kkx_infer_programs_mp3)";
+  return infer_encoded(ctx, "out_bytes", out_bytes, true, out_byte_offsets, ok ? enc[encoding] : Encoding::F32, bad, 0,
+                       true, n_programs, program_offsets, batch, tokens, tok_offsets, styles, speeds,
+                       out_sample_offsets, out_pred_dur);
 }
 
 KKX_API void kkx_release_programs(kkx_ctx* ctx, void* bytes) { kkx_release(ctx, static_cast<float*>(bytes)); }
@@ -598,40 +601,16 @@ KKX_API void kkx_release_programs(kkx_ctx* ctx, void* bytes) { kkx_release(ctx, 
 KKX_API int kkx_infer_batch_mp3(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                                 const float* styles, const float* speeds, int32_t kbps, uint8_t** out_bytes,
                                 int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_bytes) *out_bytes = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    // every check before the batch is staged: a rejected call leaves the session as it was
-    if (!out_bytes) throw ArgError("out_bytes is null");
-    if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
-    mp3_format(ctx->model->opt.out_rate, kbps);
-    *out_bytes = static_cast<uint8_t*>(infer_encoded_locked(ctx, Encoding::MP3, batch, tokens, tok_offsets, styles,
-                                                            speeds, out_byte_offsets, out_sample_offsets, out_pred_dur,
-                                                            {}, kbps));
-  });
+  return infer_encoded(ctx, "out_bytes", out_bytes, true, out_byte_offsets, Encoding::MP3, "", kbps, false, 0, nullptr,
+                       batch, tokens, tok_offsets, styles, speeds, out_sample_offsets, out_pred_dur);
 }
 
 KKX_API int kkx_infer_programs_mp3(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                                    const float* styles, const float* speeds, int32_t n_programs,
                                    const int32_t* program_offsets, int32_t kbps, uint8_t** out_bytes,
                                    int64_t* out_byte_offsets, int64_t* out_sample_offsets, int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  if (out_bytes) *out_bytes = nullptr;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    if (!out_bytes) throw ArgError("out_bytes is null");
-    if (!out_byte_offsets) throw ArgError("out_byte_offsets is null");
-    mp3_format(ctx->model->opt.out_rate, kbps);
-    if (batch < 1) throw ArgError("batch must be >= 1");
-    check_programs(batch, n_programs, program_offsets);
-    *out_bytes = static_cast<uint8_t*>(infer_encoded_locked(ctx, Encoding::MP3, batch, tokens, tok_offsets, styles,
-                                                            speeds, out_byte_offsets, out_sample_offsets, out_pred_dur,
-                                                            std::vector<int>(program_offsets, program_offsets + n_programs + 1),
-                                                            kbps));
-  });
+  return infer_encoded(ctx, "out_bytes", out_bytes, true, out_byte_offsets, Encoding::MP3, "", kbps, true, n_programs,
+                       program_offsets, batch, tokens, tok_offsets, styles, speeds, out_sample_offsets, out_pred_dur);
 }
 
 KKX_API void kkx_release_mp3(kkx_ctx* ctx, uint8_t* bytes) { kkx_release(ctx, reinterpret_cast<float*>(bytes)); }
@@ -722,33 +701,16 @@ static void async_worker(kkx_ctx* ctx) {
   for (;;) {
     ctx->acv_work.wait(al, [&] { return ctx->astop || !ctx->aqueue.empty(); });
     if (ctx->astop) {
-      for (auto* r : ctx->aqueue) { r->w.rc = KKX_ERR_STATE; r->w.err = "session destroyed before the request ran"; r->done = true; }
+      for (auto* w : ctx->aqueue) { w->rc = KKX_ERR_STATE; w->err = "session destroyed before the request ran"; w->done = true; }
       ctx->aqueue.clear();
       ctx->acv_done.notify_all();
       return;
     }
-    std::vector<kkx_ctx::AsyncReq*> reqs;
-    std::vector<kkx_ctx::Waiter*> batch;
-    long long tok = 0;
-    const size_t want = (size_t)std::max(ctx->async_batch.load(), 1);
-    while (!ctx->aqueue.empty() && reqs.size() < want) {
-      kkx_ctx::AsyncReq* r = ctx->aqueue.front();
-      if (!reqs.empty() && tok + r->w.n > 64 * 512) break;
-      tok += r->w.n;
-      reqs.push_back(r);
-      batch.push_back(&r->w);
-      ctx->aqueue.pop_front();
-    }
-    al.unlock();
-    try {
-      serve_coalesced(ctx, batch, false);
-    } catch (...) {
-      for (auto* w : batch) { w->rc = KKX_ERR_CUDA; w->err = "internal error while serving an asynchronous batch"; w->audio = nullptr; }
-    }
-    al.lock();
+    bool together = false;
+    const auto batch = serve_queue(ctx, ctx->aqueue, al, (size_t)std::max(ctx->async_batch.load(), 1),
+                                   "an asynchronous batch", &together);
     ctx->async_batches++;
-    ctx->async_requests += (int64_t)reqs.size();
-    for (auto* r : reqs) r->done = true;
+    ctx->async_requests += (int64_t)batch.size();
     ctx->acv_done.notify_all();
   }
 }
@@ -775,7 +737,7 @@ KKX_API int kkx_submit(kkx_ctx* ctx, const int64_t* tokens, int32_t n_tokens, co
       ctx->worker_started = true;
     }
     const int64_t t = ctx->next_ticket++;
-    ctx->aqueue.push_back(r.get());
+    ctx->aqueue.push_back(&r->w);
     ctx->tickets[t] = std::move(r);
     *out_ticket = t;
   } catch (const std::exception& e) { g_err = e.what(); return KKX_ERR_CUDA; }
@@ -789,7 +751,7 @@ KKX_API int kkx_poll(kkx_ctx* ctx, kkx_ticket ticket) {
   std::lock_guard<std::mutex> al(ctx->amu);
   auto it = ctx->tickets.find(ticket);
   if (it == ctx->tickets.end() || it->second->taken) { g_err = "unknown ticket"; return KKX_ERR_ARG; }
-  return it->second->done ? 1 : 0;
+  return it->second->w.done ? 1 : 0;
 }
 
 KKX_API int kkx_wait(kkx_ctx* ctx, kkx_ticket ticket, float** out_audio, int64_t* out_samples, int32_t* out_pred_dur) {
@@ -804,7 +766,7 @@ KKX_API int kkx_wait(kkx_ctx* ctx, kkx_ticket ticket, float** out_audio, int64_t
     if (it == ctx->tickets.end() || it->second->taken) { g_err = "unknown ticket"; return KKX_ERR_ARG; }
     it->second->taken = true;                         // a ticket is redeemed once
     kkx_ctx::AsyncReq* p = it->second.get();
-    ctx->acv_done.wait(al, [&] { return p->done; });
+    ctx->acv_done.wait(al, [&] { return p->w.done; });
     r = std::move(it->second);
     ctx->tickets.erase(it);
   }
@@ -817,45 +779,30 @@ KKX_API int kkx_wait(kkx_ctx* ctx, kkx_ticket ticket, float** out_audio, int64_t
 
 KKX_API void kkx_release(kkx_ctx* ctx, float* audio) {
   if (!ctx || !audio) return;
-  void* host = audio;
-  size_t cap = 0;
+  kkx_ctx::Block* b = nullptr;
   {
     std::lock_guard<std::mutex> pl(ctx->pool_mu);
-    auto vit = ctx->views.find(audio);
-    if (vit != ctx->views.end()) {     // a coalesced caller's view: the shared buffer goes back with its last view
-      kkx_ctx::SharedBuf* sb = vit->second;
-      ctx->views.erase(vit);
-      if (--sb->refs > 0) return;
-      host = sb->base;
-      cap = sb->cap;
-      delete sb;
-    } else {
-      auto it = ctx->pinned.find(audio);
-      if (it == ctx->pinned.end()) return;
-      cap = it->second;
-      ctx->pinned.erase(it);
-    }
+    auto it = ctx->handed.find(audio);
+    if (it == ctx->handed.end()) return;
+    b = it->second;
+    ctx->handed.erase(it);
+    if (--b->refs > 0) return;
   }
-  recycle_pinned(ctx, host, cap);
+  recycle_pinned(ctx, b->base, b->cap);
+  delete b;
 }
 
 KKX_API int kkx_stage_batch(kkx_ctx* ctx, int32_t batch, const int64_t* tokens, const int32_t* tok_offsets,
                     const float* styles, const float* speeds) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] { ctx->model->stage(batch, tokens, tok_offsets, styles, speeds); });
+  return session_call(ctx, [&] { ctx->model->stage(batch, tokens, tok_offsets, styles, speeds); });
 }
 
 KKX_API int kkx_run_staged(kkx_ctx* ctx, int64_t* out_total_samples, int64_t* out_launches) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
-    loud_begin(ctx);
-    ctx->model->run();
-    loud_note(ctx);
-    loud_done(ctx);
+  return session_call(ctx, [&] {
+    record_report(ctx, [&](const std::function<void()>& note) {
+      ctx->model->run();
+      note();
+    });
     if (out_total_samples) *out_total_samples = ctx->model->total_samples();
     if (out_launches) *out_launches = ctx->model->stats.launches;
   });
@@ -863,17 +810,55 @@ KKX_API int kkx_run_staged(kkx_ctx* ctx, int64_t* out_total_samples, int64_t* ou
 
 KKX_API int kkx_fetch_staged(kkx_ctx* ctx, float* dst_audio, int64_t capacity, int64_t* out_sample_offsets,
                      int32_t* out_pred_dur) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] { ctx->model->fetch(dst_audio, capacity, out_sample_offsets, out_pred_dur); });
+  return session_call(ctx, [&] { ctx->model->fetch(dst_audio, capacity, out_sample_offsets, out_pred_dur); });
+}
+
+// kkx_get_stat's value of `k` (caller holds ctx->mu), -1 for an unknown key
+static int64_t session_stat(kkx_ctx* ctx, const std::string& k) {
+  if (k == "launches") return ctx->model->stats.launches;
+  if (k == "last_frames") return ctx->model->last_frames;
+  if (k == "gpu_us") return (int64_t)ctx->model->last_gpu_us;
+  if (k == "precision") return ctx->model->opt.precision;
+  if (k == "out_rate") return ctx->model->opt.out_rate;
+  if (k == "loudness_target") return ctx->model->opt.loudness_target;
+  if (k == "true_peak_max") return ctx->model->opt.true_peak_max;
+  if (k == "loudness_items") return report_items(ctx, kRepLoudness);
+  if (k == "limiter") return ctx->model->opt.limiter;
+  if (k == "loudness_report") return ctx->model->opt.loudness_report;
+  if (k == "flac_lpc_order") return ctx->model->opt.flac_lpc_order;
+  if (k == "limiter_items") return report_items(ctx, kRepLimiter);
+  if (k == "graph_replays") return ctx->model->graph_replays;
+  if (k == "frame_groups") return (int64_t)ctx->model->group_first().size();
+  if (k.rfind("group_first:", 0) == 0) {     // first item of frame group g of the last run
+    const long g = atol(k.c_str() + 12);
+    const auto& gf = ctx->model->group_first();
+    return g >= 0 && g < (long)gf.size() ? gf[g] : -1;
+  }
+  if (k == "weights_sessions") return (int64_t)ctx->model->weight_sessions();
+  if (k == "weights_bytes") return (int64_t)ctx->model->weight_set().device_bytes;
+  if (k == "weights_from_onnx") return ctx->model->weight_set().format == "onnx" ? 1 : 0;
+  {
+    std::lock_guard<std::mutex> ql(ctx->qmu);
+    if (k == "coalesced_batches") return ctx->coalesced_batches;
+    if (k == "coalesced_requests") return ctx->coalesced_requests;
+    if (k == "coalesced_largest") return ctx->coalesced_largest;
+  }
+  {
+    std::lock_guard<std::mutex> al(ctx->amu);
+    if (k == "async_batches") return ctx->async_batches;
+    if (k == "async_requests") return ctx->async_requests;
+  }
+  return -1;
+}
+
+KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
+  int64_t v = -1;
+  session_call(ctx, [&] { if (key) v = session_stat(ctx, key); });
+  return v;
 }
 
 KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
+  return session_call(ctx, [&] {
     if (!key) throw ArgError("null key");
     Options& o = ctx->model->opt;
     const std::string k(key);
@@ -940,51 +925,11 @@ KKX_API int kkx_set_option(kkx_ctx* ctx, const char* key, int64_t value) {
   });
 }
 
-KKX_API int64_t kkx_get_stat(kkx_ctx* ctx, const char* key) {
-  if (check_ctx(ctx) || !key) return -1;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  const std::string k(key);
-  if (k == "launches") return ctx->model->stats.launches;
-  if (k == "last_frames") return ctx->model->last_frames;
-  if (k == "gpu_us") return (int64_t)ctx->model->last_gpu_us;
-  if (k == "precision") return ctx->model->opt.precision;
-  if (k == "out_rate") return ctx->model->opt.out_rate;
-  if (k == "loudness_target") return ctx->model->opt.loudness_target;
-  if (k == "true_peak_max") return ctx->model->opt.true_peak_max;
-  if (k == "loudness_items") return report_items(ctx, kRepLoudness);
-  if (k == "limiter") return ctx->model->opt.limiter;
-  if (k == "loudness_report") return ctx->model->opt.loudness_report;
-  if (k == "flac_lpc_order") return ctx->model->opt.flac_lpc_order;
-  if (k == "limiter_items") return report_items(ctx, kRepLimiter);
-  if (k == "coalesced_batches") return ctx->coalesced_batches;
-  if (k == "coalesced_requests") return ctx->coalesced_requests;
-  if (k == "coalesced_largest") return ctx->coalesced_largest;
-  if (k == "graph_replays") return ctx->model->graph_replays;
-  if (k == "frame_groups") return (int64_t)ctx->model->group_first().size();
-  if (k.rfind("group_first:", 0) == 0) {     // first item of frame group g of the last run
-    const long g = atol(k.c_str() + 12);
-    const auto& gf = ctx->model->group_first();
-    return g >= 0 && g < (long)gf.size() ? gf[g] : -1;
-  }
-  if (k == "weights_sessions") return (int64_t)ctx->model->weight_sessions();
-  if (k == "weights_bytes") return (int64_t)ctx->model->weight_set().device_bytes;
-  if (k == "weights_from_onnx") return ctx->model->weight_set().format == "onnx" ? 1 : 0;
-  {
-    std::lock_guard<std::mutex> al(ctx->amu);
-    if (k == "async_batches") return ctx->async_batches;
-    if (k == "async_requests") return ctx->async_requests;
-  }
-  return -1;
-}
-
 // Row group `group` of the last synchronous call's report: per item b, rows row0, row0 + 1, ... into cols[0], cols[1],
 // ... (null columns are skipped).  `off`: the error when that call did not produce the group.
 static int last_report(kkx_ctx* ctx, int32_t batch, unsigned group, const char* off, int row0,
                        std::initializer_list<float*> cols) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
+  return session_call(ctx, [&] {
     if (!ctx->report_valid) throw StateError("no synchronous call has completed on this session");
     if (!(ctx->report_groups & group)) throw StateError(off);
     const int64_t n = (int64_t)(ctx->report.size() / kReportRows);
@@ -1017,48 +962,40 @@ KKX_API int kkx_last_loudness_range(kkx_ctx* ctx, int32_t batch, float* loudness
 }
 
 KKX_API int kkx_profile_enable(kkx_ctx* ctx, int enable) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  ctx->model->stats.profile = enable != 0;
-  return KKX_OK;
+  return session_call(ctx, [&] { ctx->model->stats.profile = enable != 0; });
 }
 
 KKX_API int64_t kkx_profile_json(kkx_ctx* ctx, char* buf, int64_t capacity) {
-  if (check_ctx(ctx)) return -1;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  std::ostringstream os;
-  os << "{\"conv_flops\": " << ctx->model->stats.conv_flops << ", \"arb_flops\": " << ctx->model->stats.arb_flops
-     << ", \"arb_bytes\": " << ctx->model->stats.arb_bytes << ", \"gpu_us\": " << ctx->model->last_gpu_us
-     << ", \"kernels\": {";
-  bool first = true;
-  for (auto& kv : ctx->model->prof_) {
-    if (!first) os << ", ";
-    first = false;
-    os << "\"" << kv.first << "\": [" << kv.second.first << ", " << kv.second.second << "]";
-  }
-  os << "}}";
-  const std::string s = os.str();
-  if (buf && capacity > 0) {
-    const size_t n = std::min<size_t>(s.size(), (size_t)capacity - 1);
-    memcpy(buf, s.data(), n);
-    buf[n] = 0;
-  }
-  return (int64_t)s.size();
+  int64_t len = -1;
+  session_call(ctx, [&] {
+    std::ostringstream os;
+    os << "{\"conv_flops\": " << ctx->model->stats.conv_flops << ", \"arb_flops\": " << ctx->model->stats.arb_flops
+       << ", \"arb_bytes\": " << ctx->model->stats.arb_bytes << ", \"gpu_us\": " << ctx->model->last_gpu_us
+       << ", \"kernels\": {";
+    bool first = true;
+    for (auto& kv : ctx->model->prof_) {
+      if (!first) os << ", ";
+      first = false;
+      os << "\"" << kv.first << "\": [" << kv.second.first << ", " << kv.second.second << "]";
+    }
+    os << "}}";
+    const std::string s = os.str();
+    if (buf && capacity > 0) {
+      const size_t n = std::min<size_t>(s.size(), (size_t)capacity - 1);
+      memcpy(buf, s.data(), n);
+      buf[n] = 0;
+    }
+    len = (int64_t)s.size();
+  });
+  return len;
 }
 
 KKX_API int kkx_set_noise(kkx_ctx* ctx, const float* noise, int64_t n) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] { ctx->model->set_noise(noise, n); });
+  return session_call(ctx, [&] { ctx->model->set_noise(noise, n); });
 }
 
 KKX_API int kkx_set_inject_item(kkx_ctx* ctx, int32_t item, const char* name, const void* data, int64_t count) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  return guarded(ctx, [&] {
+  return session_call(ctx, [&] {
     if (!name) throw ArgError("null name");
     ctx->model->set_inject(name, item, count > 0 ? data : nullptr, count);
   });
@@ -1069,32 +1006,24 @@ KKX_API int kkx_set_inject(kkx_ctx* ctx, const char* name, const void* data, int
 }
 
 KKX_API int kkx_debug_enable(kkx_ctx* ctx, int enable) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  ctx->model->set_debug(enable != 0, -1);
-  return KKX_OK;
+  return session_call(ctx, [&] { ctx->model->set_debug(enable != 0, -1); });
 }
 
 KKX_API int kkx_debug_select(kkx_ctx* ctx, int enable, int32_t item) {
-  int rc = check_ctx(ctx);
-  if (rc) return rc;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  ctx->model->set_debug(enable != 0, item);
-  return KKX_OK;
+  return session_call(ctx, [&] { ctx->model->set_debug(enable != 0, item); });
 }
 
 KKX_API int64_t kkx_debug_stage(kkx_ctx* ctx, const char* name, int32_t item, float* dst, int64_t capacity,
                         int64_t* rows, int64_t* cols) {
-  if (check_ctx(ctx) || !name) return -1;
-  std::lock_guard<std::mutex> lk(ctx->mu);
-  const DebugStage* s = ctx->model->debug_stage(name, item);
-  if (!s) { g_err = std::string("no such debug stage: ") + name; return -1; }
-  if (rows) *rows = s->rows;
-  if (cols) *cols = s->cols;
-  const int64_t n = (int64_t)s->data.size();
-  if (dst && capacity > 0) memcpy(dst, s->data.data(), (size_t)std::min(n, capacity) * sizeof(float));
+  int64_t n = -1;
+  session_call(ctx, [&] {
+    if (!name) return;
+    const DebugStage* s = ctx->model->debug_stage(name, item);
+    if (!s) { g_err = std::string("no such debug stage: ") + name; return; }
+    if (rows) *rows = s->rows;
+    if (cols) *cols = s->cols;
+    n = (int64_t)s->data.size();
+    if (dst && capacity > 0) memcpy(dst, s->data.data(), (size_t)std::min(n, capacity) * sizeof(float));
+  });
   return n;
 }
-
-}  // extern "C"
